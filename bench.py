@@ -3,7 +3,7 @@
 % of FP32 FMA peak; vs host CPU").
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload large|medium|small|large4k|synth4096]
-                  [--variant mega|wavefront|scalar] [--impl reference]
+                  [--variant mega|wavefront|scalar] [--impl reference] [--dump-outputs DIR]
   N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A step = one full render of the workload (every pixel x sample through generate -> scan -> shade -> resolve, and for
@@ -27,6 +27,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark writes nothing into the tree it runs from (which may be read-only): no bytecode caches for the modules it
+# imports beyond what build() imported (rays1bench_b200/dist.py, tests/cpu_checkers.py)
+sys.dont_write_bytecode = True
 
 WORKLOADS = {
     # name: (scene, width, height, spp, max_bounces)  -- BASELINE.json configs
@@ -63,6 +66,29 @@ def metric_name(workload):
 def workload_label(name):
     scene, w, h, spp, mb = WORKLOADS[name]
     return "%s scene %dx%d %d spp depth %d" % (scene, w, h, spp, mb)
+
+
+DUMP_BUDGET = 64_000_000   # bytes --dump-outputs may write in all
+NPY_HEADER = 128           # bytes numpy writes in front of each of the (at most three) arrays below
+
+
+def dump_outputs(out_dir, image, num_rays):
+    """--dump-outputs: what the timed path handed its caller in its last step, so that two builds can be compared output for
+    output.  image.npy = the RGB8 framebuffer [H, W, 3] (row 0 = bottom) as float32, num_rays.npy = the ray count as float64.
+    An image that does not fit the budget (the 3840x2160 workload) is replaced by a fixed, seeded sample of its pixels [n, 3]
+    that fills it; their flat indices y * W + x go to image_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    rays = np.array([num_rays], np.float64)
+    img = image.astype(np.float32)
+    room = DUMP_BUDGET - 3 * NPY_HEADER - rays.nbytes       # for image.npy and, when sampled, image_index.npy
+    if img.nbytes > room:
+        h, w = img.shape[:2]
+        n = room // (3 * 4 + 8)                              # per kept pixel: three float32 values + one float64 index
+        idx = np.sort(np.random.default_rng(0).choice(h * w, n, replace=False))
+        np.save(os.path.join(out_dir, "image_index.npy"), idx.astype(np.float64))
+        img = img.reshape(-1, 3)[idx]
+    np.save(os.path.join(out_dir, "image.npy"), img)
+    np.save(os.path.join(out_dir, "num_rays.npy"), rays)
 
 
 # ------------------------------------------------------------------------------------------------ clocks sampler
@@ -232,7 +258,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-reference-exe", action="store_true", help="skip the `rays1_latest -n 3` run of the unmodified reference executable")
     ap.add_argument("--threads", type=int, default=0, help="threads per persistent CTA (512/768/1024; 0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's image and ray count to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 path computed (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -357,6 +388,8 @@ def main():
             total_rays += int(d_rays.item()) if rank == 0 else 0  # for N > 1 the reduced total lives on rank 0
             launches += n_l
     clocks = sampler.end() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, img[:H].cpu().numpy(), int(d_rays.item()))
     ms_value = allmax(total_ms)        # max over ranks of the summed per-step device times
     ms_trace = allmax(trace_ms)
 

@@ -23,22 +23,6 @@ def oracle():
 
 
 @pytest.fixture(scope="session")
-def reflib():
-    from cpu_checkers import RefLib
-    if not RefLib.available():
-        pytest.skip("oracle/_ref/libref_rays1.so not built (needs /root/reference)")
-    return RefLib()
-
-
-@pytest.fixture(scope="session")
-def reflib4096():
-    from cpu_checkers import RefLib
-    if not RefLib.available(4096):
-        pytest.skip("oracle/_ref/libref_rays1_4096.so not built (needs /root/reference)")
-    return RefLib(4096)
-
-
-@pytest.fixture(scope="session")
 def r1():
     import rays1bench_b200
     return rays1bench_b200

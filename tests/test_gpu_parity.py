@@ -608,28 +608,6 @@ def test_bench_steps_tool_runs_the_executable(r1, tmp_path):
         assert os.path.getsize(tmp_path / ("out_%s.tga" % name)) == 18 + 80 * 60 * 3
 
 
-def test_reference_main_runs_on_the_product_library(r1, tmp_path):
-    """INTEGRATION.md section 2: the reference's own, unchanged main() (rayweek1.cpp:930-988) compiled against rays1_host.h and
-    linked with librays1_b200.so (oracle/Makefile -> oracle/_ref/rays1_refmain_b200): `-n 1 -w` renders the three scenes at the
-    reference's compiled-in workload and leaves the report blocks, out_<scene>.txt and out_<scene>.tga the reference leaves."""
-    from conftest import ROOT
-    exe = os.path.join(ROOT, "oracle", "_ref", "rays1_refmain_b200")
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/rays1_refmain_b200 not built (needs /root/reference at build time)")
-    out = subprocess.run([exe, "-n", "1", "-w"], cwd=tmp_path, capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stderr
-    lines = out.stdout.splitlines()
-    assert [l for l in lines if l in ("small", "medium", "large")] == ["small", "medium", "large"]
-    assert sum(l == "total samples:  %d" % (1280 * 720 * 250) for l in lines) == 3
-    rays = [int(l.split()[-1]) for l in lines if l.startswith("total rays:")]
-    for got, want in zip(rays, (414.19e6, 577.13e6, 631.16e6)):                    # the reference's own totals (tests/golden/ref_stats.json)
-        assert abs(got / want - 1) < 0.005
-    for name in ("small", "medium", "large"):
-        tok = open(tmp_path / ("out_%s.txt" % name)).read().split("|")
-        assert tok[0] == "latest" and tok[1].endswith("s") and tok[3].endswith(" mrays/s")
-        assert os.path.getsize(tmp_path / ("out_%s.tga" % name)) == 18 + 1280 * 720 * 3
-
-
 def test_in_process_multi_gpu_matches_single_gpu(r1, tmp_path):
     """--gpus 2 in ONE process (NCCL gather + reduce, rays1_host.cpp:render_multi) renders the same bytes and ray count."""
     if r1.device_count() < 2:

@@ -1,6 +1,5 @@
-"""The oracle (oracle/rays1_oracle.c) pinned against the reference: known answers, golden vectors recorded from the
-reference's compiled code (tests/golden, oracle/make_golden.py) and -- where oracle/_ref was built -- the reference
-library itself.  CPU only."""
+"""The oracle (oracle/rays1_oracle.c) pinned against the reference: known answers and golden vectors recorded from the
+reference's compiled code (tests/golden, oracle/make_golden.py).  CPU only."""
 import numpy as np
 import pytest
 
@@ -217,29 +216,6 @@ def test_render_edge_sizes(oracle):
     rgb, rays, _ = oracle.render(s, 16, 9, 3, max_bounces=0, threads=0)
     assert rays == 16 * 9 * 3, "with a cap of 0 every sample is exactly one ray"
     oracle.scene_destroy(s)
-
-
-# ---- against the reference library itself (only where oracle/_ref was built) ------------------------------------------
-
-@pytest.mark.parametrize("name", SCENES)
-def test_against_reference_library(oracle, reflib, name):
-    so, sr = oracle.scene_create(name), reflib.scene_create(name)
-    rec = reflib.record_paths(sr, 2048, seed=11)
-    idx, t, p, n = oracle.hit(so, rec["org"], rec["dir"])
-    assert np.array_equal(idx, rec["index"])
-    m = idx >= 0
-    assert np.array_equal(bits(t[m]), bits(rec["t"][m]))
-    assert np.array_equal(bits(n[m]), bits(rec["normal"][m]))
-    for fn in ("xorshift32", "myrand01", "myrand02"):
-        assert getattr(oracle, fn)(777) == getattr(reflib, fn)(777)
-    a, sa = oracle.random_in_unit_disk(4242)
-    b, sb = reflib.random_in_unit_disk(4242)
-    assert sa == sb and np.array_equal(a, b)
-    a, sa = oracle.myrand01_x4([5, 6, 7, 8])
-    b, sb = reflib.myrand01_x4([5, 6, 7, 8])
-    assert np.array_equal(a, b) and np.array_equal(sa, sb)
-    oracle.scene_destroy(so)
-    reflib.scene_destroy(sr)
 
 
 def replay_agreement(col, rays, g):
