@@ -140,7 +140,10 @@ int r1_deinterleave_rows(int device, const void *d_gathered, uint64_t stride, vo
                          int world, void *cuda_stream);
 
 /* Parity entry points (host buffers, n rays each, xyz interleaved) -- the device functions the kernels use. */
-/* Hitable::hit (rayweek1.cpp:152-339); index = -1 on a miss.  dir must be unit length (Ray ctor, :104-108). */
+/* Hitable::hit (rayweek1.cpp:152-339); index = -1 on a miss.  dir must be unit length (Ray ctor, :104-108).  `variant` picks
+ * the filter: R1_VARIANT_MEGAKERNEL resolves as in r1_render; SCALAR, COOP, DEFERRED and PACKED run that kernel's scan;
+ * TENSOR runs the filter of megakernel_tc3 (128-sphere accumulator chunks, the short last chunk included) and returns
+ * R1_ERR_LIMIT above 768 spheres; WAVEFRONT and DUAL have no per-ray kernel and return R1_ERR_ARG. */
 int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, float t_min, float t_max, int variant,
                   int32_t *index, float *t, float *p, float *normal);
 /* Name of the trace kernel `variant` resolves to for this scene with default tuning ("megakernel_tc3", "megakernel_pool", ...);

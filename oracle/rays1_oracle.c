@@ -325,6 +325,22 @@ ORC_API orc_scene *orc_scene_create(const char *name, int image_w, int image_h)
     return s;
 }
 
+/* A scene from its SoA as given (e.g. r1_scene_get_soa of a scene file), placeholders included, no padding added; the camera
+ * stays zero until orc_scene_set_camera.  For hit() on scenes the named builders do not make. */
+ORC_API orc_scene *orc_scene_create_from_soa(int n, const float *cx, const float *cy, const float *cz, const float *radius_sq,
+                                             const float *inv_radius, const int32_t *kind, const float *albedo, const float *param)
+{
+    if (n < 0) return NULL;
+    orc_scene *s = calloc(1, sizeof(*s));
+    scene_reserve(s, (uint32_t)n + 1);
+    size_t b = (size_t)n * 4;
+    memcpy(s->cx, cx, b); memcpy(s->cy, cy, b); memcpy(s->cz, cz, b);
+    memcpy(s->radius_sq, radius_sq, b); memcpy(s->inv_radius, inv_radius, b);
+    memcpy(s->kind, kind, b); memcpy(s->albedo, albedo, 3 * b); memcpy(s->param, param, b);
+    s->count = (uint32_t)n;
+    return s;
+}
+
 ORC_API void orc_scene_destroy(orc_scene *s)
 {
     if (!s) return;

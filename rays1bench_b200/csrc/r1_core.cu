@@ -861,12 +861,22 @@ int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, fl
     DeviceCtx *cp = nullptr;
     R1_TRY(get_ctx(scene, &cp));
     if (n < 0 || (n > 0 && (!org || !dir || !index || !t || !p || !normal))) return fail(R1_ERR_ARG, "bad argument");
+    // R1_VARIANT_MEGAKERNEL resolves as in r1_render; the variants without a per-ray kernel of their own are refused
+    r1_render_params prm;
+    memset(&prm, 0, sizeof(prm));
+    prm.variant = variant;
+    if (variant < 0 || variant > 7) return fail(R1_ERR_ARG, "unknown variant %d", variant);
+    const int v = resolve_variant(cp->dev, prm);
+    if (v == R1_VARIANT_WAVEFRONT || v == R1_VARIANT_MEGAKERNEL_DUAL) return fail(R1_ERR_ARG, "r1_trace_rays has no kernel for variant %d (wavefront, dual)", v);
+    if (v == R1_VARIANT_MEGAKERNEL_TENSOR && !cp->dev.tcb)
+        return fail(R1_ERR_LIMIT, "the tensor-core filter takes scenes of 1 .. %d spheres (this scene pads to %d)", r1::tc::kMaxSpheres, cp->dev.n32);
     if (n == 0) return R1_OK;
     if (cp->dev.n_pad > r1::kMaxStagedSpheres) return fail(R1_ERR_LIMIT, "r1_trace_rays stages at most %d spheres", r1::kMaxStagedSpheres);
     DevBuf d_org, d_dir, d_idx, d_t, d_p, d_n;
     R1_TRY(d_org.upload(org, (size_t)n * 12)); R1_TRY(d_dir.upload(dir, (size_t)n * 12));
     R1_TRY(d_idx.alloc((size_t)n * 4)); R1_TRY(d_t.alloc((size_t)n * 4)); R1_TRY(d_p.alloc((size_t)n * 12)); R1_TRY(d_n.alloc((size_t)n * 12));
-    const size_t smem = 16 + (size_t)cp->dev.n_pad * 32 + sizeof(r1::WarpScratch) * 4;
+    const size_t smem = v == R1_VARIANT_MEGAKERNEL_TENSOR ? r1::trace_rays_tc_smem_bytes(cp->dev.n32)
+                                                          : 16 + (size_t)cp->dev.n_pad * 32 + sizeof(r1::WarpScratch) * 4;
     const int grid = (n + 127) / 128;
     auto launch = [&](auto kern) -> int {
         R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -874,9 +884,10 @@ int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, fl
                                   d_n.as<float>());
         return R1_OK;
     };
-    if (variant == R1_VARIANT_MEGAKERNEL_SCALAR) R1_TRY(launch(r1::trace_rays_kernel<r1::kScanLaneScalar>));
-    else if (variant == R1_VARIANT_MEGAKERNEL_COOP) R1_TRY(launch(r1::trace_rays_kernel<r1::kScanCoop>));
-    else if (variant == R1_VARIANT_MEGAKERNEL_DEFERRED) R1_TRY(launch(r1::trace_rays_kernel<r1::kScanLaneDeferred>));
+    if (v == R1_VARIANT_MEGAKERNEL_SCALAR) R1_TRY(launch(r1::trace_rays_kernel<r1::kScanLaneScalar>));
+    else if (v == R1_VARIANT_MEGAKERNEL_COOP) R1_TRY(launch(r1::trace_rays_kernel<r1::kScanCoop>));
+    else if (v == R1_VARIANT_MEGAKERNEL_DEFERRED) R1_TRY(launch(r1::trace_rays_kernel<r1::kScanLaneDeferred>));
+    else if (v == R1_VARIANT_MEGAKERNEL_TENSOR) R1_TRY(launch(r1::trace_rays_tc_kernel));
     else R1_TRY(launch(r1::trace_rays_kernel<r1::kScanLanePacked>));
     R1_CUDA(cudaGetLastError());
     R1_CUDA(cudaDeviceSynchronize());

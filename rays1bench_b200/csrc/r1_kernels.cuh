@@ -1410,6 +1410,92 @@ __global__ void __launch_bounds__(128) trace_rays_kernel(const __grid_constant__
     n_out[3 * k] = nrm.x; n_out[3 * k + 1] = nrm.y; n_out[3 * k + 2] = nrm.z;
 }
 
+// Hitable::hit through the filter of megakernel_tc3: the same device functions (write_ray_row, mma_chunk in chunks of 128
+// spheres with the per-chunk N, the last chunk read in (n32 - 128 c) / 32 pieces of 32 columns, two TMEM loads in flight,
+// exact_candidates, hit_finalise) with the caller's t_min / t_max.  One CTA = 128 rays, one 128-column accumulator buffer, the
+// MMA issued by thread 0; no buffer pool, so only the arithmetic and the chunking of tc3 are under test here.
+constexpr int kTraceTcChunk = 128;                               // = megakernel_tc3's kChunk
+constexpr size_t trace_rays_tc_smem_bytes(int n32)
+{
+    return 128 + (size_t)n32 * tc::kRowBytes + 128 * tc::kRowBytes + (size_t)n32 * 16;
+}
+__global__ void __launch_bounds__(128, 1) trace_rays_tc_kernel(const __grid_constant__ DevScene sc, int n, const float *org, const float *dir,
+                                                               float t_min, float t_max, int32_t *index, float *t_out, float *p_out, float *n_out)
+{
+    constexpr int kChunk = kTraceTcChunk, kPieces = kChunk / 32;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw);      // [mbarrier | TMEM address | pad to 128 | B | A | exact]
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(smem_raw + 8);
+    const int n32 = sc.n32;
+    unsigned char *s_b = smem_raw + 128;
+    unsigned char *a_tile = s_b + (size_t)n32 * tc::kRowBytes;
+    float4 *s_exact = reinterpret_cast<float4 *>(a_tile + 128 * tc::kRowBytes);
+    for (int i = threadIdx.x; i < n32 * (tc::kRowBytes / 16); i += blockDim.x)
+        reinterpret_cast<uint4 *>(s_b)[i] = reinterpret_cast<const uint4 *>(sc.tcb)[i];
+    for (int i = threadIdx.x; i < n32; i += blockDim.x)
+        s_exact[i] = i < sc.n_pad ? sc.exact[i] : make_float4(0, 0, 0, 0);
+    if (threadIdx.x == 0) {
+        tc::mbar_init(full, 1);
+        tc::fence_mbar_init();
+    }
+    const int k = blockIdx.x * 128 + threadIdx.x;
+    const bool live = k < n;                                     // rays past n write a row that flags nothing
+    f3 o = mk3(0, 0, 0), d = mk3(0, 0, 0);
+    if (live) { o = mk3(org[3 * k], org[3 * k + 1], org[3 * k + 2]); d = mk3(dir[3 * k], dir[3 * k + 1], dir[3 * k + 2]); }
+    tc::write_ray_row(a_tile, threadIdx.x, o, d, live);
+    tc::fence_proxy_async();                                     // the tiles are read by the tensor core (async proxy)
+    if (threadIdx.x < 32) tc::tmem_alloc(tmem_slot, kChunk);
+    tc::tc_fence_before();
+    __syncthreads();
+    tc::tc_fence_after();
+    const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t *>(tmem_slot);
+    const uint32_t t_lane = tmem_base + ((uint32_t)((threadIdx.x >> 5) * 32) << 16);
+    const uint32_t a_smem = tc::smem_u32(a_tile), b_smem = tc::smem_u32(s_b);
+    const int nchunks = (n32 + kChunk - 1) / kChunk;
+    float t = t_max;
+    int hit = -1;
+    for (int c = 0; c < nchunks; ++c) {
+        if (threadIdx.x == 0) {
+            tc::tc_fence_after();
+            tc::mma_chunk(tmem_base, a_smem, b_smem + (uint32_t)c * (kChunk / 8) * tc::kSBO, min(kChunk, n32 - c * kChunk), tc::kLBO, tc::kSBO);
+            tc::mma_commit(full);
+        }
+        tc::mbar_wait(full, (uint32_t)c & 1u);
+        tc::tc_fence_after();
+        const int pieces = min(kPieces, (n32 - c * kChunk) >> 5);   // the last chunk may be short
+        uint32_t cand[kPieces];
+#pragma unroll
+        for (int h = 0; h < kPieces; h += 2) {
+            cand[h] = 0; cand[h + 1] = 0;
+            if (h + 1 < pieces) {
+                uint32_t v0[32], v1[32];
+                tc::tmem_ld32_issue(t_lane + 32 * h, v0);
+                tc::tmem_ld32_issue(t_lane + 32 * h + 32, v1);
+                tc::tmem_wait(v0, v1);
+                cand[h] = tc::flagged(v0);
+                cand[h + 1] = tc::flagged(v1);
+            } else if (h < pieces) {
+                uint32_t v[32];
+                tc::tmem_ld32(t_lane + 32 * h, v);
+                cand[h] = tc::flagged(v);
+            }
+        }
+        tc::tc_fence_before();
+        __syncthreads();                                         // every warp has read the buffer: the next chunk may overwrite it
+#pragma unroll
+        for (int h = 0; h < kPieces; ++h)
+            if (cand[h]) exact_candidates(cand[h], s_exact, c * kChunk + 32 * h, o, d, t_min, t, hit);
+    }
+    if (threadIdx.x < 32) tc::tmem_dealloc(tmem_base, kChunk);
+    if (!live) return;
+    f3 p = mk3(0, 0, 0), nrm = mk3(0, 0, 0);
+    if (hit >= 0) hit_finalise(s_exact[hit], load_shade(sc, hit).inv_radius, o, d, t, p, nrm);
+    index[k] = hit;
+    t_out[k] = hit >= 0 ? t : 0.0f;
+    p_out[3 * k] = p.x; p_out[3 * k + 1] = p.y; p_out[3 * k + 2] = p.z;
+    n_out[3 * k] = nrm.x; n_out[3 * k + 1] = nrm.y; n_out[3 * k + 2] = nrm.z;
+}
+
 __global__ void scatter_kernel(const __grid_constant__ DevScene sc, int n, const float *dir_in, const float *p, const float *nrm,
                                const int32_t *index, const float *rs, const float *ru, int32_t *ok, float *atten, float *dir_out)
 {

@@ -150,6 +150,18 @@ class Oracle(_Checker):
         L.orc_hw_rsqrtss.argtypes = [C.c_float]
         L.orc_render.restype = C.c_uint64
         L.orc_render.argtypes = [C.c_void_p, _bp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double)]
+        L.orc_scene_create_from_soa.restype = C.c_void_p
+        L.orc_scene_create_from_soa.argtypes = [C.c_int, _fp, _fp, _fp, _fp, _fp, _ip, _fp, _fp]
+
+    def scene_create_from_soa(self, soa):
+        """a scene holding the spheres of ``soa`` (the dict of Scene.soa() / scene_soa()) as given, for hit() on any scene;
+        destroy it with scene_destroy"""
+        c = lambda k, dt=_f: np.ascontiguousarray(soa[k], dt)  # noqa: E731
+        s = self.lib.orc_scene_create_from_soa(len(soa["cx"]), c("cx"), c("cy"), c("cz"), c("radius_sq"), c("inv_radius"), c("kind", np.int32),
+                                               c("albedo"), c("param"))
+        if not s:
+            raise ValueError("orc_scene_create_from_soa failed")
+        return s
 
     def scene_set_camera(self, s, cam22):
         self.lib.orc_scene_set_camera(s, np.ascontiguousarray(cam22, _f))

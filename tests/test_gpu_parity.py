@@ -47,7 +47,14 @@ def scenes(r1):
 
 # ---- hit() ----------------------------------------------------------------------------------------------------------
 
-@pytest.mark.parametrize("variant", ["mega", "coop", "scalar", "deferred"])
+def refuses_tensor(r1, scene, org, d):
+    """above 768 spheres the tensor-core filter has no operand: R1_ERR_LIMIT, never a silent fall-back to another scan"""
+    with pytest.raises(r1.Rays1Error, match=r"\(-4\).*768"):
+        scene.trace_rays(org, d, variant=r1.VARIANT_MEGAKERNEL_TENSOR)
+
+
+# "mega" resolves as in r1_render: the tensor-core filter on the large scene, the packed scan elsewhere
+@pytest.mark.parametrize("variant", ["mega", "coop", "scalar", "deferred", "tensor", "packed"])
 @pytest.mark.parametrize("name", ALL)
 def test_hit_matches_reference_golden(r1, scenes, golden_rays, name, variant):
     g = golden_rays[name]
@@ -57,6 +64,8 @@ def test_hit_matches_reference_golden(r1, scenes, golden_rays, name, variant):
     want_t = np.concatenate([g["seg_t"], g["edge_t"]])
     want_p = np.concatenate([g["seg_p"], g["edge_p"]])
     want_n = np.concatenate([g["seg_normal"], g["edge_normal"]])
+    if variant == "tensor" and name == "synth4096":
+        return refuses_tensor(r1, scenes[name], org, d)
     idx, t, p, n = scenes[name].trace_rays(org, d, variant=r1.VARIANTS[variant])
     assert np.array_equal(idx, want_idx), "hit sphere index differs for %d rays" % int((idx != want_idx).sum())
     m = idx >= 0
@@ -93,7 +102,7 @@ def test_hit_matches_oracle_on_fresh_rays(r1, scenes, oracle, name):
     oracle.scene_destroy(so)
 
 
-@pytest.mark.parametrize("variant", ["mega", "coop", "scalar", "deferred"])
+@pytest.mark.parametrize("variant", ["mega", "coop", "scalar", "deferred", "tensor", "packed"])
 @pytest.mark.parametrize("name", ("large", "synth4096"))
 def test_filter_is_conservative_for_far_and_grazing_rays(r1, scenes, oracle, name, variant):
     """The 8-instruction filter works in the expanded form (cancellation at |o|^2 + |c|^2): rays from far away that graze
@@ -113,6 +122,8 @@ def test_filter_is_conservative_for_far_and_grazing_rays(r1, scenes, oracle, nam
     target = ctr + side * (rad * rng.uniform(0.98, 1.02, n))[:, None]
     d = target - org; d /= np.linalg.norm(d, axis=1, keepdims=True)
     org, d = org.astype(np.float32), d.astype(np.float32)
+    if variant == "tensor" and name == "synth4096":
+        return refuses_tensor(r1, scenes[name], org, d)
     so = oracle.scene_create(name)
     want = oracle.hit(so, org, d)
     oracle.scene_destroy(so)
@@ -139,6 +150,24 @@ def tensor_filter_rays(soa, n=4096, seed=99):
     d2 = ctr + side * (rad * rng.uniform(0.98, 1.02, n))[:, None] - o2
     d2 /= np.linalg.norm(d2, axis=1, keepdims=True)
     return np.concatenate([org, o2]).astype(np.float32), np.concatenate([d, d2]).astype(np.float32)
+
+
+def tensor_filter_far_rays(soa, n=2048, seed=77):
+    """tensor_filter_rays plus rays grazing spheres from 2 000 and 20 000 units away (where the FFMA2 filter is tested too):
+    the filter's cancellation grows with |o|^2"""
+    rng = np.random.default_rng(seed)
+    org, d = tensor_filter_rays(soa, n, seed)
+    real = np.where(soa["inv_radius"] > 0)[0]
+    idx = rng.choice(real, n)
+    ctr = np.stack([soa["cx"][idx], soa["cy"][idx], soa["cz"][idx]], 1).astype(np.float64)
+    rad = 1.0 / soa["inv_radius"][idx].astype(np.float64)
+    u = rng.normal(size=(n, 3)); u /= np.linalg.norm(u, axis=1, keepdims=True)
+    u[:, 1] = np.abs(u[:, 1])                                   # stay above the ground plane
+    o3 = ctr + u * rng.choice([2000.0, 20000.0], n)[:, None]
+    side = np.cross(u, rng.normal(size=(n, 3))); side /= np.linalg.norm(side, axis=1, keepdims=True)
+    d3 = ctr + side * (rad * rng.uniform(0.98, 1.02, n))[:, None] - o3
+    d3 /= np.linalg.norm(d3, axis=1, keepdims=True)
+    return np.concatenate([org, o3.astype(np.float32)]), np.concatenate([d, d3.astype(np.float32)])
 
 
 def tensor_filter_truth(soa, org, d, margin=2.0 ** -16):
@@ -231,6 +260,15 @@ def test_default_variant_picks_the_kernel_by_scene(r1, scenes, monkeypatch):
     monkeypatch.delenv("R1_AUTO_TENSOR")
     b, rb = scenes["large"].render(96, 54, 8)
     assert np.array_equal(a, b) and ra.num_rays == rb.num_rays
+
+
+def test_trace_rays_refuses_variants_without_a_ray_kernel(r1, scenes):
+    """wavefront and dual have no per-ray kernel: refused, not answered by another scan; so is an unknown variant"""
+    for v in (r1.VARIANT_WAVEFRONT, r1.VARIANT_MEGAKERNEL_DUAL, 8, -1):
+        with pytest.raises(r1.Rays1Error, match=r"\(-1\)"):
+            scenes["large"].trace_rays([[0, 5, 20]], [[0, 0, -1]], variant=v)
+    idx, _, _, _ = scenes["large"].trace_rays([[0, 3, 20]], [[0, 0, -1]], variant=r1.VARIANT_MEGAKERNEL_TENSOR)
+    assert idx[0] >= 0
 
 
 def test_hit_empty_and_single(r1, scenes):

@@ -265,3 +265,30 @@ def test_rsqrt12_table_matches_this_cpu(oracle):
         pytest.skip("RSQRTSS table check needs an Intel CPU (this is %r)" % vendor)
     hw = np.array([oracle.lib.orc_hw_rsqrtss(float(x)) for x in xs], np.float32)
     assert np.array_equal(bits(got), bits(hw))
+
+
+@pytest.mark.parametrize("name", ALL)
+def test_scene_from_soa_hits_like_the_named_builder(r1, oracle, name):
+    """orc_scene_create_from_soa, fed with the library's SoA of a scene, answers hit() bit for bit like the oracle's own builder
+    of that scene -- so the oracle can check any scene the library loads (scene files, sweeps)"""
+    s = r1.create_scene(name, commit=False)
+    soa = s.soa()
+    s.close()
+    named = oracle.scene_create(name)
+    from_soa = oracle.scene_create_from_soa(soa)
+    try:
+        assert oracle.scene_count(from_soa) == oracle.scene_count(named) == len(soa["cx"])
+        rng = np.random.default_rng(5)
+        n = 3000
+        org = (rng.normal(size=(n, 3)) * [8, 2, 8] + [0, 2, 0]).astype(np.float32)
+        d = rng.normal(size=(n, 3))
+        d = (d / np.linalg.norm(d, axis=1, keepdims=True)).astype(np.float32)
+        for t_min, t_max in ((0.001, float(np.finfo(np.float32).max)), (0.5, 6.0)):
+            want = oracle.hit(named, org, d, t_min, t_max)
+            got = oracle.hit(from_soa, org, d, t_min, t_max)
+            assert np.array_equal(got[0], want[0]) and (want[0] >= 0).sum() > 300
+            for a, b in zip(got[1:], want[1:]):
+                assert np.array_equal(bits(a), bits(b))
+    finally:
+        oracle.scene_destroy(named)
+        oracle.scene_destroy(from_soa)

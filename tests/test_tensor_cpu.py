@@ -5,7 +5,8 @@ on the GPU by tests/test_gpu_parity.py::test_tensor_filter_is_conservative."""
 import numpy as np
 import pytest
 
-from test_gpu_parity import tensor_filter_rays, tensor_filter_truth   # ray generator and float64 truth shared with the GPU test
+from test_gpu_parity import tensor_filter_far_rays, tensor_filter_rays, tensor_filter_truth   # ray generators and float64 truth shared with the GPU tests
+from test_tensor_gpu import GRIDS, TENSOR, grid_scene                # the sphere-count sweep of the tensor path
 
 MARGIN = 2.0 ** -16
 
@@ -39,9 +40,17 @@ def ray_rows(org, d):
     return np.concatenate([hi, lo, hi[:, :10]], 1)
 
 
-@pytest.mark.parametrize("name", ("small", "medium", "large"))
-def test_tensor_operand_layout_split_and_padding(r1, name):
-    s = r1.create_scene(name, commit=False)
+def cpu_scene(r1, name, tmp_path):
+    """a built-in scene, or a sweep scene "WxH" of tests/test_tensor_gpu.py, host side only"""
+    if "x" in name:
+        return grid_scene(r1, tmp_path, *map(int, name.split("x")), commit=False)
+    return r1.create_scene(name, commit=False)
+
+
+@pytest.mark.parametrize("name", ("small", "medium", "large", "21x16", "28x27"))
+def test_tensor_operand_layout_split_and_padding(r1, name, tmp_path):
+    """incl. a 96-row last chunk (n32 = 352) and the largest operand the filter takes (760 spheres, n32 = 768: 96 KB)"""
+    s = cpu_scene(r1, name, tmp_path)
     soa = s.soa()
     op = s.tensor_operand()
     n, n32 = len(soa["cx"]), op.shape[0]
@@ -65,26 +74,37 @@ def test_tensor_operand_layout_split_and_padding(r1, name):
     s.close()
 
 
-def test_tensor_operand_limits(r1):
+def test_tensor_operand_limits(r1, tmp_path):
     import ctypes as C
     s = r1.create_scene("synth4096", commit=False)
     n32 = C.c_uint32(0)
     assert r1.lib.r1_tensor_operand(s.handle, np.zeros(16, np.uint8), 16, C.byref(n32)) == -4 and n32.value == 4096   # R1_ERR_LIMIT
     assert b"768" in r1.lib.r1_last_error()
     s.close()
+    for grid, (count, want_n32) in GRIDS.items():             # the sweep: 768 is the last accepted, 800 the first refused
+        s = grid_scene(r1, tmp_path, *grid, commit=False)
+        rc = r1.lib.r1_tensor_operand(s.handle, np.zeros(16, np.uint8), 16, C.byref(n32))
+        assert s.count() == count and n32.value == want_n32
+        if want_n32 <= 768:
+            assert rc == -1, "accepted: only the 16-byte buffer is too small"
+            assert r1.lib.r1_tensor_operand(s.handle, np.zeros(want_n32 * 128, np.uint8), want_n32 * 128, C.byref(n32)) == 0
+        else:
+            assert rc == -4 and b"768" in r1.lib.r1_last_error() and b"800" in r1.lib.r1_last_error()
+        s.close()
     s = r1.create_scene("small", commit=False)
     assert r1.lib.r1_tensor_operand(s.handle, np.zeros(16, np.uint8), 16, C.byref(n32)) == -1 and n32.value == 32       # buffer too small
     s.close()
 
 
-@pytest.mark.parametrize("name", ("medium", "large"))
-def test_tensor_filter_formulation_is_conservative(r1, oracle, name):
+@pytest.mark.parametrize("name", ("medium", "large") + tuple("%dx%d" % g for g in TENSOR))
+def test_tensor_filter_formulation_is_conservative(r1, oracle, name, tmp_path):
     """A[ray] . B[sphere] with the split operands exactly as the device and the host build them (products and sum in float64):
-    within 2^-20 S of the float64 polynomial, and every sphere the oracle's Hitable::hit returns is flagged."""
-    s = r1.create_scene(name, commit=False)
+    within 2^-20 S of the float64 polynomial, and every sphere the oracle's Hitable::hit returns is flagged.  On the sweep scenes
+    the rays include ones grazing spheres from 2 000 and 20 000 units."""
+    s = cpu_scene(r1, name, tmp_path)
     soa = s.soa()
     n = len(soa["cx"])
-    org, d = tensor_filter_rays(soa, n=1024)
+    org, d = tensor_filter_rays(soa, n=1024) if "x" not in name else tensor_filter_far_rays(soa, n=512)
     a = ray_rows(org, d).astype(np.float64)
     op = s.tensor_operand().astype(np.float64)
     b = np.concatenate([op[:, 0:11], op[:, 11:22], op[:, 22:32]], 1)      # sphere words in K order: hi | hi | lo
@@ -96,7 +116,7 @@ def test_tensor_filter_formulation_is_conservative(r1, oracle, name):
     must = (discr >= -4.0e-6 * big_s) & real[None, :]
     assert must.sum() > 500 and (e[:, :n][must] >= 0).all()
     assert (e[:, n:] < 0).all() and (e[:, :n][:, ~real] < 0).all()
-    so = oracle.scene_create(name)
+    so = oracle.scene_create_from_soa(soa)
     idx = oracle.hit(so, org, d)[0]
     oracle.scene_destroy(so)
     hit = idx >= 0
