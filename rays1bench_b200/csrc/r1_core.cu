@@ -219,14 +219,19 @@ int launch_megakernel_lanefetch(int sm_count, const r1::RenderArgs &args, const 
 }
 
 // warp sample-pool scheduling (r1::megakernel_pool): the default; R1_POOL=0 selects the per-lane unit fetch of r1::megakernel
+size_t megakernel_pool_smem(int scan, bool staged, int n_pad, int threads)
+{
+    return r1::kSmemSpheres + (staged ? (size_t)n_pad * 32 : 0) +
+           (scan == r1::kScanCoop || scan == r1::kScanLaneDeferred ? sizeof(r1::WarpScratch) * (threads / 32) : 0) + sizeof(r1::WarpPool) * (threads / 32);
+}
+
 template <int kScan, bool kStaged, int kThreads>
 int launch_megakernel_pool(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
 {
     constexpr int kBlocks = 1;
     auto kern = r1::megakernel_pool<kScan, kStaged, kThreads, kBlocks>;
-    const size_t smem = r1::kSmemSpheres + (kStaged ? (size_t)args.scene.n_pad * 32 : 0) +
-                        (kScan == r1::kScanCoop || kScan == r1::kScanLaneDeferred ? sizeof(r1::WarpScratch) * (kThreads / 32) : 0) +
-                        sizeof(r1::WarpPool) * (kThreads / 32);
+    const size_t smem = megakernel_pool_smem(kScan, kStaged, args.scene.n_pad, kThreads);
+    if (smem > 227 * 1024) return fail(R1_ERR_LIMIT, "%d threads need %zu bytes of shared memory for this scene (227 KB available)", kThreads, smem);
     R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int grid = sm_count * kBlocks;
     if (prm.blocks_per_sm > 0) grid = sm_count * prm.blocks_per_sm;
@@ -354,7 +359,11 @@ int launch_megakernel_t(int sm_count, const r1::RenderArgs &args, const r1_rende
 template <int kScan, bool kStaged>
 int launch_megakernel(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
 {
-    const int threads = prm.threads > 0 ? prm.threads : (kScan == r1::kScanCoop ? kDefaultThreadsCoop : kDefaultThreads);
+    int threads = prm.threads > 0 ? prm.threads : (kScan == r1::kScanCoop ? kDefaultThreadsCoop : kDefaultThreads);
+    // The deferred scan's 2 KB of queue per warp: with the sample pool, 1024 threads and more than 3 936 staged spheres exceed
+    // 227 KB of shared memory.  The default then runs 768 threads (the image does not depend on the thread count).
+    const bool pool = !(getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0);
+    if (prm.threads <= 0 && pool && megakernel_pool_smem(kScan, kStaged, args.scene.n_pad, threads) > 227 * 1024) threads = 768;
     if (threads == 512) return launch_megakernel_t<kScan, kStaged, 512>(sm_count, args, prm, stream);
     if (threads == 768) return launch_megakernel_t<kScan, kStaged, 768>(sm_count, args, prm, stream);
     if (threads == 1024) return launch_megakernel_t<kScan, kStaged, 1024>(sm_count, args, prm, stream);
@@ -858,6 +867,9 @@ extern "C" {
 int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, float t_min, float t_max, int variant, int32_t *index, float *t,
                   float *p, float *normal)
 {
+    // The exact test lifts discr to 2^-100 before its square root, and the cooperative and deferred scans merge roots as unsigned
+    // keys: both agree with Hitable::hit only for t_min >= 2^-24 (r1_device.cuh, exact_test).  Renders use 0.001.  !(>=) rejects NaN.
+    if (!(t_min >= 0x1p-24f)) return fail(R1_ERR_ARG, "t_min must be >= 2^-24 (5.96e-8), got %g", (double)t_min);
     DeviceCtx *cp = nullptr;
     R1_TRY(get_ctx(scene, &cp));
     if (n < 0 || (n > 0 && (!org || !dir || !index || !t || !p || !normal))) return fail(R1_ERR_ARG, "bad argument");

@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 from test_gpu_parity import tensor_filter_far_rays, tensor_filter_rays, tensor_filter_truth   # ray generators and float64 truth shared with the GPU tests
+from test_scan_edges_gpu import make_scene                           # unpadded scenes through the raw ABI
 from test_tensor_gpu import GRIDS, TENSOR, grid_scene                # the sphere-count sweep of the tensor path
 
 MARGIN = 2.0 ** -16
@@ -41,15 +42,19 @@ def ray_rows(org, d):
 
 
 def cpu_scene(r1, name, tmp_path):
-    """a built-in scene, or a sweep scene "WxH" of tests/test_tensor_gpu.py, host side only"""
+    """a built-in scene, a sweep scene "WxH" of tests/test_tensor_gpu.py or an unpadded cluster "n<count>" of
+    tests/test_scan_edges_gpu.py, host side only"""
+    if name.startswith("n") and name[1:].isdigit():
+        return make_scene(r1, name, tmp_path, commit=False)
     if "x" in name:
         return grid_scene(r1, tmp_path, *map(int, name.split("x")), commit=False)
     return r1.create_scene(name, commit=False)
 
 
-@pytest.mark.parametrize("name", ("small", "medium", "large", "21x16", "28x27"))
+@pytest.mark.parametrize("name", ("small", "medium", "large", "21x16", "28x27", "n1", "n13", "n33"))
 def test_tensor_operand_layout_split_and_padding(r1, name, tmp_path):
-    """incl. a 96-row last chunk (n32 = 352) and the largest operand the filter takes (760 spheres, n32 = 768: 96 KB)"""
+    """incl. a 96-row last chunk (n32 = 352), the largest operand the filter takes (760 spheres, n32 = 768: 96 KB) and scenes
+    not padded to 8 (1, 13 and 33 spheres: 31, 19 and 31 padding rows)"""
     s = cpu_scene(r1, name, tmp_path)
     soa = s.soa()
     op = s.tensor_operand()
