@@ -49,7 +49,12 @@ enum {
     R1_VARIANT_MEGAKERNEL_TENSOR = 6,  /* persistent threads, per-lane path state machine, the filter as a split-TF32 GEMM on the tensor
                                          cores (tcgen05.mma, accumulators in TMEM), 128 rays x 64 spheres per instruction; scenes of up
                                          to 768 spheres */
-    R1_VARIANT_MEGAKERNEL_PACKED = 7   /* persistent threads, per-lane path state machine, per-lane packed f32x2 (FFMA2) filter */
+    R1_VARIANT_MEGAKERNEL_PACKED = 7,  /* persistent threads, per-lane path state machine, per-lane packed f32x2 (FFMA2) filter */
+    /* 8 stays unassigned: callers built against earlier versions of this header may rely on it being refused as an unknown
+       variant (R1_ERR_ARG), and the ABI tests use it as their example of one. */
+    R1_VARIANT_MEGAKERNEL_TENSOR_STREAM = 9 /* the filter of R1_VARIANT_MEGAKERNEL_TENSOR with the sphere operand streamed through a
+                                               ring of 128-sphere chunks in shared memory, shared by the CTA's ray groups: scenes of
+                                               any size; threads / 128 = ray groups (1 .. 4, default 4) */
 };
 
 typedef struct r1_scene r1_scene; /* opaque: host SoA + per-device buffers */
@@ -143,12 +148,14 @@ int r1_deinterleave_rows(int device, const void *d_gathered, uint64_t stride, vo
 /* Hitable::hit (rayweek1.cpp:152-339); index = -1 on a miss.  dir must be unit length (Ray ctor, :104-108).  `variant` picks
  * the filter: R1_VARIANT_MEGAKERNEL resolves as in r1_render; SCALAR, COOP, DEFERRED and PACKED run that kernel's scan;
  * TENSOR runs the filter of megakernel_tc3 (128-sphere accumulator chunks, the short last chunk included) and returns
- * R1_ERR_LIMIT above 768 spheres; WAVEFRONT and DUAL have no per-ray kernel and return R1_ERR_ARG.  t_min must be >= 2^-24
+ * R1_ERR_LIMIT above 768 spheres; TENSOR_STREAM runs the streamed filter of megakernel_tcs at any sphere count, while every
+ * other variant returns R1_ERR_LIMIT above 4096 (they stage the scene in shared memory); WAVEFRONT and DUAL have no per-ray
+ * kernel and return R1_ERR_ARG.  t_min must be >= 2^-24
  * (renders use 0.001): below it the exact test's floored square root and the unsigned root keys of COOP and DEFERRED can differ
  * from Hitable::hit, so a smaller t_min or a NaN returns R1_ERR_ARG before any device is touched. */
 int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, float t_min, float t_max, int variant,
                   int32_t *index, float *t, float *p, float *normal);
-/* Name of the trace kernel `variant` resolves to for this scene with default tuning ("megakernel_tc3", "megakernel_pool", ...);
+/* Name of the trace kernel `variant` resolves to for this scene with default tuning ("megakernel_tc3", "megakernel_tcs", "megakernel_pool", ...);
  * static storage. */
 const char *r1_kernel_name(r1_scene *scene, int variant);
 /* Host only (no device needed): the sphere operand of the tensor-core filter for this scene -- n32 rows (sphere count padded to

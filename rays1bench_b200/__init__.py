@@ -16,8 +16,10 @@ LIB_PATH = os.environ.get("R1_LIBRARY") or os.path.join(_HERE, "librays1_b200.so
 EXE_PATH = os.path.join(_HERE, "rays1_b200")
 
 VARIANT_MEGAKERNEL, VARIANT_WAVEFRONT, VARIANT_MEGAKERNEL_SCALAR, VARIANT_MEGAKERNEL_COOP, VARIANT_MEGAKERNEL_DEFERRED, VARIANT_MEGAKERNEL_DUAL, VARIANT_MEGAKERNEL_TENSOR, VARIANT_MEGAKERNEL_PACKED = 0, 1, 2, 3, 4, 5, 6, 7
+VARIANT_MEGAKERNEL_TENSOR_STREAM = 9   # 8 stays unassigned (include/rays1_b200.h)
 VARIANTS = {"mega": VARIANT_MEGAKERNEL, "wavefront": VARIANT_WAVEFRONT, "scalar": VARIANT_MEGAKERNEL_SCALAR, "coop": VARIANT_MEGAKERNEL_COOP,
-            "deferred": VARIANT_MEGAKERNEL_DEFERRED, "dual": VARIANT_MEGAKERNEL_DUAL, "tensor": VARIANT_MEGAKERNEL_TENSOR, "packed": VARIANT_MEGAKERNEL_PACKED}
+            "deferred": VARIANT_MEGAKERNEL_DEFERRED, "dual": VARIANT_MEGAKERNEL_DUAL, "tensor": VARIANT_MEGAKERNEL_TENSOR, "packed": VARIANT_MEGAKERNEL_PACKED,
+            "tensor_stream": VARIANT_MEGAKERNEL_TENSOR_STREAM}
 MAT_NONE, MAT_LAMBERT, MAT_METAL, MAT_DIELECTRIC = -1, 0, 1, 2
 
 # the reference's compile-time workload (src/common/common.h:18-25)

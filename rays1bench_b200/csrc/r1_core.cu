@@ -312,6 +312,42 @@ int launch_megakernel_tc3_t(int sm_count, const r1::RenderArgs &args, cudaStream
     return R1_OK;
 }
 
+// streamed tensor-core filter (r1::megakernel_tcs, R1_VARIANT_MEGAKERNEL_TENSOR_STREAM): `threads` / 128 = ray groups per CTA (one
+// 128-column TMEM accumulator each), R1_TCS_STAGES = depth of the operand ring.  Shared memory does not depend on the scene.
+// Measured on synth4096 at 1280x720x250 (B200, 1000 W; DESIGN.md section 4.7, profiles/r03_bench_tensor_stream.json): 4 groups with
+// 2 / 3 / 4 / 6 stages 1279 / 1324 / 1350 / 1358 Mrays/s; 3 / 2 / 1 groups with 6 stages 1120 / 806 / 415 (PACKED: 827).
+constexpr int kDefaultTcsGroups = 4, kDefaultTcsStages = 6;
+
+template <int kGroups, int kStages>
+int launch_megakernel_tcs_t(int sm_count, const r1::RenderArgs &args, cudaStream_t stream)
+{
+    auto kern = r1::megakernel_tcs<kGroups, kStages>;
+    const size_t smem = r1::tcs_smem_bytes(kGroups, kStages);
+    if (smem > 227 * 1024) return fail(R1_ERR_LIMIT, "tensor-stream variant: %d ray groups and %d stages need %zu bytes of shared memory", kGroups, kStages, smem);
+    R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int grid = sm_count;                                         // one CTA per SM
+    const unsigned long long max_ctas = (args.n_samples + kGroups * 128 - 1) / (kGroups * 128);
+    if ((unsigned long long)grid > max_ctas) grid = (int)std::max<unsigned long long>(1, max_ctas);
+    kern<<<grid, kGroups * 128, smem, stream>>>(args);
+    R1_CUDA(cudaGetLastError());
+    return R1_OK;
+}
+
+int launch_megakernel_tcs(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
+{
+    const int groups = prm.threads > 0 ? prm.threads / 128 : kDefaultTcsGroups;
+    const int stages = getenv("R1_TCS_STAGES") ? atoi(getenv("R1_TCS_STAGES")) : kDefaultTcsStages;
+    if (groups == 4 && stages == 2) return launch_megakernel_tcs_t<4, 2>(sm_count, args, stream);
+    if (groups == 4 && stages == 3) return launch_megakernel_tcs_t<4, 3>(sm_count, args, stream);
+    if (groups == 4 && stages == 4) return launch_megakernel_tcs_t<4, 4>(sm_count, args, stream);
+    if (groups == 4 && stages == 6) return launch_megakernel_tcs_t<4, 6>(sm_count, args, stream);
+    if (groups == 3 && stages == 6) return launch_megakernel_tcs_t<3, 6>(sm_count, args, stream);
+    if (groups == 2 && stages == 6) return launch_megakernel_tcs_t<2, 6>(sm_count, args, stream);
+    if (groups == 1 && stages == 6) return launch_megakernel_tcs_t<1, 6>(sm_count, args, stream);
+    return fail(R1_ERR_ARG, "the tensor-stream variant runs 1 .. 4 groups of 128 ray threads per CTA (threads = 128 .. 512) with a 6-stage ring, "
+                            "or 4 groups with 2, 3, 4 or 6 stages (got %d groups, %d stages)", groups, stages);
+}
+
 int launch_megakernel_tc(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
 {
     if (!args.scene.tcb) return fail(R1_ERR_LIMIT, "the tensor-core filter takes scenes of 1 .. %d spheres (its operand lives in shared memory)", r1::tc::kMaxSpheres);
@@ -391,7 +427,7 @@ int validate(const r1_render_params *p)
     // the pixel accumulators hold sums of radiance * 2^24 in 64 bits, one sample saturating at 2^32 - 1 (r1_kernels.cuh): 2^20
     // samples per pixel cannot wrap them
     if (p->spp > (1 << 20)) return fail(R1_ERR_LIMIT, "spp %d exceeds the accumulator limit of 2^20 samples per pixel", p->spp);
-    if (p->variant < 0 || p->variant > 7) return fail(R1_ERR_ARG, "unknown variant %d", p->variant);
+    if (p->variant < 0 || p->variant > R1_VARIANT_MEGAKERNEL_TENSOR_STREAM || p->variant == 8) return fail(R1_ERR_ARG, "unknown variant %d", p->variant);
     return R1_OK;
 }
 
@@ -569,11 +605,13 @@ int r1_scene_commit(r1_scene *scene, int device)
     const int n = (int)scene->cx.size();
     const int n_pad = (n + 15) / 16 * 16;  // one scan supergroup = 16 spheres (the reference pads to SIMD_WIDTH = 8, rayweek1.cpp:575)
     const float inf = std::numeric_limits<float>::infinity();
-    // host image of the device block: [scan n_pad f4 | exact n_pad f4 | shade n_pad x 2 f4 | tensor-filter operand n32 x 128 B]
+    // host image of the device block: [scan n_pad f4 | exact n_pad f4 | shade n_pad x 2 f4 | tensor-filter operand n32 x 128 B].
+    // The operand is built for every scene: the streamed filter (r1::tcs_operand) finds it after `shade` at any size, while `tcb`,
+    // the resident filter's pointer, stays null above tc::kMaxSpheres.
     const int n32 = (n + 31) / 32 * 32;
     const bool tensor_ok = n32 > 0 && n32 <= r1::tc::kMaxSpheres;
     const size_t tcb_off = (size_t)n_pad * (16 + 16 + 32);
-    const size_t bytes = tcb_off + (tensor_ok ? (size_t)n32 * r1::tc::kRowBytes : 0);
+    const size_t bytes = tcb_off + (size_t)n32 * r1::tc::kRowBytes;
     std::vector<unsigned char> host(bytes, 0);
     float *scan = reinterpret_cast<float *>(host.data());
     float4 *exact = reinterpret_cast<float4 *>(host.data()) + n_pad;
@@ -612,7 +650,7 @@ int r1_scene_commit(r1_scene *scene, int device)
         }
         shade[2 * i + 1] = make_float4(inv_r, kind_bits, inv_ior, r0s);
     }
-    if (tensor_ok) build_tensor_operand(scene, host.data() + tcb_off, n32);
+    build_tensor_operand(scene, host.data() + tcb_off, n32);
     rc = take_scene_block(*scr, bytes, &c.block, &c.block_bytes);
     if (rc) return rc;
     {
@@ -753,6 +791,7 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
             else if (variant == R1_VARIANT_MEGAKERNEL_DEFERRED) rc = staged ? launch_megakernel<r1::kScanLaneDeferred, true>(x.sm_count, a, prm, stream)
                                                                                 : launch_megakernel<r1::kScanLaneDeferred, false>(x.sm_count, a, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR) rc = launch_megakernel_tc(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) rc = launch_megakernel_tcs(x.sm_count, a, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_DUAL) rc = staged ? launch_megakernel_dual<true>(x.sm_count, a, prm, stream)
                                                                             : launch_megakernel_dual<false>(x.sm_count, a, prm, stream);
             else rc = staged ? launch_megakernel<r1::kScanLaneScalar, true>(x.sm_count, a, prm, stream)
@@ -877,18 +916,20 @@ int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, fl
     r1_render_params prm;
     memset(&prm, 0, sizeof(prm));
     prm.variant = variant;
-    if (variant < 0 || variant > 7) return fail(R1_ERR_ARG, "unknown variant %d", variant);
+    if (variant < 0 || variant > R1_VARIANT_MEGAKERNEL_TENSOR_STREAM || variant == 8) return fail(R1_ERR_ARG, "unknown variant %d", variant);
     const int v = resolve_variant(cp->dev, prm);
     if (v == R1_VARIANT_WAVEFRONT || v == R1_VARIANT_MEGAKERNEL_DUAL) return fail(R1_ERR_ARG, "r1_trace_rays has no kernel for variant %d (wavefront, dual)", v);
     if (v == R1_VARIANT_MEGAKERNEL_TENSOR && !cp->dev.tcb)
         return fail(R1_ERR_LIMIT, "the tensor-core filter takes scenes of 1 .. %d spheres (this scene pads to %d)", r1::tc::kMaxSpheres, cp->dev.n32);
     if (n == 0) return R1_OK;
-    if (cp->dev.n_pad > r1::kMaxStagedSpheres) return fail(R1_ERR_LIMIT, "r1_trace_rays stages at most %d spheres", r1::kMaxStagedSpheres);
+    // the streamed filter takes any size; the other kernels stage the whole scene in shared memory
+    if (v != R1_VARIANT_MEGAKERNEL_TENSOR_STREAM && cp->dev.n_pad > r1::kMaxStagedSpheres) return fail(R1_ERR_LIMIT, "r1_trace_rays stages at most %d spheres", r1::kMaxStagedSpheres);
     DevBuf d_org, d_dir, d_idx, d_t, d_p, d_n;
     R1_TRY(d_org.upload(org, (size_t)n * 12)); R1_TRY(d_dir.upload(dir, (size_t)n * 12));
     R1_TRY(d_idx.alloc((size_t)n * 4)); R1_TRY(d_t.alloc((size_t)n * 4)); R1_TRY(d_p.alloc((size_t)n * 12)); R1_TRY(d_n.alloc((size_t)n * 12));
-    const size_t smem = v == R1_VARIANT_MEGAKERNEL_TENSOR ? r1::trace_rays_tc_smem_bytes(cp->dev.n32)
-                                                          : 16 + (size_t)cp->dev.n_pad * 32 + sizeof(r1::WarpScratch) * 4;
+    const size_t smem = v == R1_VARIANT_MEGAKERNEL_TENSOR          ? r1::trace_rays_tc_smem_bytes(cp->dev.n32)
+                        : v == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM ? r1::trace_rays_tcs_smem_bytes()
+                                                                   : 16 + (size_t)cp->dev.n_pad * 32 + sizeof(r1::WarpScratch) * 4;
     const int grid = (n + 127) / 128;
     auto launch = [&](auto kern) -> int {
         R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -900,6 +941,7 @@ int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, fl
     else if (v == R1_VARIANT_MEGAKERNEL_COOP) R1_TRY(launch(r1::trace_rays_kernel<r1::kScanCoop>));
     else if (v == R1_VARIANT_MEGAKERNEL_DEFERRED) R1_TRY(launch(r1::trace_rays_kernel<r1::kScanLaneDeferred>));
     else if (v == R1_VARIANT_MEGAKERNEL_TENSOR) R1_TRY(launch(r1::trace_rays_tc_kernel));
+    else if (v == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) R1_TRY(launch(r1::trace_rays_tcs_kernel));
     else R1_TRY(launch(r1::trace_rays_kernel<r1::kScanLanePacked>));
     R1_CUDA(cudaGetLastError());
     R1_CUDA(cudaDeviceSynchronize());
@@ -919,6 +961,7 @@ const char *r1_kernel_name(r1_scene *scene, int variant)
     case R1_VARIANT_WAVEFRONT: return "wf_intersect + wf_shade (graph loop)";
     case R1_VARIANT_MEGAKERNEL_TENSOR: return getenv("R1_TC1") ? "megakernel_tc" : (getenv("R1_TC2") ? "megakernel_tc2" : "megakernel_tc3");
     case R1_VARIANT_MEGAKERNEL_DUAL: return "megakernel_pool2";
+    case R1_VARIANT_MEGAKERNEL_TENSOR_STREAM: return "megakernel_tcs";
     default: return (getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0) ? "megakernel" : "megakernel_pool";
     }
 }

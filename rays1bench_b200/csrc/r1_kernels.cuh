@@ -1255,6 +1255,285 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tc3(const __grid_
     if (threadIdx.x < 32) tc::tmem_dealloc(tmem_base, 512);
 }
 
+// ------------------------------------------------------------------------------------------------ megakernel, streamed tensor-core filter
+// R1_VARIANT_MEGAKERNEL_TENSOR_STREAM (DESIGN.md section 4.7): megakernel_tc3's scan with the sphere operand STREAMED through a
+// ring of kStages shared-memory stages instead of resident, so that shared memory no longer depends on the scene.  A stage holds
+// one 128-sphere chunk: its 16 KB of operand rows (one contiguous range of the K-major layout) and its 2 KB of exact records,
+// brought in by two cp.async.bulk on the stage's `landed` mbarrier.
+//
+// Fills are numbered f = 0, 1, 2, ...: fill f is chunk f mod nchunks in stage f mod kStages.  Every live ray group consumes every
+// fill in order; a scan is the nchunks fills from a multiple of nchunks, so the exact tests still run in ascending sphere order.
+// Each warp releases a fill once its group's MMA on it is complete (the warp has waited for it) and its own exact tests are done:
+// byte g of the stage's ring word counts the warps of group g.  The thread whose release completes the fill -- every group still
+// consuming has all four warps in -- refills the stage with fill f + kStages (tc3's last-arriver idiom, no producer warp), so the
+// groups drift apart by at most the ring depth.  A group out of work sets its bit in `exited`: from then on it counts as done for
+// every fill, and it completes the fills only it was holding up.  The ring word {fill number | release bytes} changes atomically,
+// and a refill is claimed with a compare-and-swap on it, so a releaser and a leaving group that both see a fill complete refill
+// it once.  Fill numbers are kept modulo 2 kStages nchunks, which preserves the stage, the chunk and the mbarrier parity.
+constexpr int kTcsChunk = 128;
+constexpr int kTcsMaxStages = 8;
+constexpr uint32_t kTcsOpBytes = kTcsChunk * tc::kRowBytes;   // 16 KB of operand rows
+constexpr uint32_t kTcsStageBytes = kTcsOpBytes + kTcsChunk * 16;   // + 2 KB of exact records
+
+struct TcsControl {
+    uint64_t mma[4];                      // per group: accumulator chunk complete (tcgen05.commit; the exit arrival), count 1
+    uint64_t landed[kTcsMaxStages];       // per stage: fill landed (complete_tx)
+    uint64_t ring[kTcsMaxStages];         // per stage: fill number << 32 | byte g = warps of group g done with it
+    uint32_t arrived_a[4];                // per group: ray warps with their row written (low byte) / out of work (next byte)
+    uint32_t arrived_e[4];                // per group: ray warps that have read the current chunk
+    uint32_t exit_flag[4];
+    uint32_t exited;                      // bit g: group g is out of work and consumes no more fills
+    uint32_t tmem_base;
+    uint32_t pad_[2];
+};
+static_assert(sizeof(TcsControl) % 16 == 0, "TcsControl is followed by 16-byte aligned stages");
+
+// The sphere operand at every scene size: the end of the scene block, after the shading records (r1_scene_commit)
+__device__ __forceinline__ const unsigned char *tcs_operand(const DevScene &sc) { return reinterpret_cast<const unsigned char *>(sc.shade + 2 * (size_t)sc.n_pad); }
+
+// Fill a stage with chunk c (one thread): the rows that exist (the last chunk may be short) and the n_pad exact records that
+// exist -- n32 is padded to 32, n_pad only to 16, and the columns without a record are padding rows no ray flags.
+__device__ __forceinline__ void tcs_fill(const DevScene &sc, unsigned char *stage, uint64_t *landed, int c)
+{
+    const uint32_t op_bytes = (uint32_t)min(kTcsChunk, sc.n32 - c * kTcsChunk) * tc::kRowBytes;
+    const uint32_t ex_bytes = (uint32_t)min(kTcsChunk, sc.n_pad - c * kTcsChunk) * 16u;
+    const uint32_t bar = tc::smem_u32(landed);
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(op_bytes + ex_bytes) : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(tc::smem_u32(stage)),
+                 "l"(tcs_operand(sc) + (size_t)c * kTcsOpBytes), "r"(op_bytes), "r"(bar)
+                 : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(tc::smem_u32(stage + kTcsOpBytes)),
+                 "l"(sc.exact + (size_t)c * kTcsChunk), "r"(ex_bytes), "r"(bar)
+                 : "memory");
+}
+
+// A fill is complete when every group still consuming has all four warps in.  With every group gone nothing is refilled.
+template <int kGroups>
+__device__ __forceinline__ bool tcs_fill_complete(uint32_t released, uint32_t exited)
+{
+    bool done = exited != (1u << kGroups) - 1u;
+#pragma unroll
+    for (int g = 0; g < kGroups; ++g)
+        if (!((exited >> g) & 1u) && ((released >> (8 * g)) & 0xffu) != 4u) done = false;
+    return done;
+}
+// Refill a completed stage with fill f + kStages -- once: the compare-and-swap on the whole ring word fails for everyone else
+template <int kStages>
+__device__ __forceinline__ void tcs_refill(const DevScene &sc, TcsControl &ctl, unsigned char *stages, int s, uint64_t word, uint32_t wrap, int nchunks)
+{
+    uint32_t next = (uint32_t)(word >> 32) + kStages;
+    if (next >= wrap) next -= wrap;
+    if (atomicCAS(reinterpret_cast<unsigned long long *>(&ctl.ring[s]), word, (unsigned long long)next << 32) != word) return;
+    tcs_fill(sc, stages + (size_t)s * kTcsStageBytes, &ctl.landed[s], (int)(next % (uint32_t)nchunks));
+}
+// One warp (lane 0) of group g is done with the fill in stage s
+template <int kGroups, int kStages>
+__device__ __forceinline__ void tcs_release(const DevScene &sc, TcsControl &ctl, unsigned char *stages, int s, int g, uint32_t wrap, int nchunks)
+{
+    __threadfence_block();
+    const unsigned long long inc = 1ull << (8 * g);
+    const uint64_t word = atomicAdd(reinterpret_cast<unsigned long long *>(&ctl.ring[s]), inc) + inc;
+    __threadfence_block();                                       // the release before the read of `exited` (see tcs_leave)
+    if (tcs_fill_complete<kGroups>((uint32_t)word, *reinterpret_cast<volatile uint32_t *>(&ctl.exited))) tcs_refill<kStages>(sc, ctl, stages, s, word, wrap, nchunks);
+}
+// Group g is out of work (its warps hold no fill): it stops counting as a consumer and completes the fills that waited only for it.
+// Its bit is published before it reads the ring words, and a releaser adds its byte before it reads `exited`: of a racing pair at
+// least one sees the other, and the compare-and-swap lets only one of them refill.
+template <int kGroups, int kStages>
+__device__ __forceinline__ void tcs_leave(const DevScene &sc, TcsControl &ctl, unsigned char *stages, int g, uint32_t wrap, int nchunks)
+{
+    const uint32_t exited = atomicOr(&ctl.exited, 1u << g) | (1u << g);
+    __threadfence_block();
+#pragma unroll
+    for (int s = 0; s < kStages; ++s) {
+        const uint64_t word = *reinterpret_cast<volatile uint64_t *>(&ctl.ring[s]);
+        if (tcs_fill_complete<kGroups>((uint32_t)word, exited)) tcs_refill<kStages>(sc, ctl, stages, s, word, wrap, nchunks);
+    }
+}
+
+constexpr size_t tcs_smem_bytes(int groups, int stages)
+{
+    return (size_t)((kSmemSpheres + 127) & ~127) + ((sizeof(TcsControl) + 127) & ~(size_t)127) + (size_t)stages * kTcsStageBytes +
+           (size_t)groups * 128 * tc::kRowBytes + (size_t)groups * 4 * sizeof(WarpPool);
+}
+
+template <int kGroups, int kStages>
+__global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tcs(const __grid_constant__ RenderArgs a)
+{
+    constexpr int kChunk = kTcsChunk, kPieces = kChunk / 32;
+    static_assert(kGroups >= 1 && kGroups <= 4 && kStages >= 2 && kStages <= kTcsMaxStages, "bad configuration");
+    constexpr uint32_t kTmemCols = kGroups == 1 ? 128 : (kGroups == 2 ? 256 : 512);   // one 128-column accumulator per group
+    const bool hint = a.tc_flags & 1u;
+    // shared memory: [16 B | rsqrtss table 4 KB | control | stages kStages x 18 KB | A tiles kGroups x 16 KB | pools]
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    uint16_t *s_tab = reinterpret_cast<uint16_t *>(smem_raw + 16);
+    unsigned char *p = smem_raw + ((kSmemSpheres + 127) & ~127);
+    TcsControl &ctl = *reinterpret_cast<TcsControl *>(p);
+    p += (sizeof(TcsControl) + 127) & ~127;
+    unsigned char *s_stages = p;
+    p += (size_t)kStages * kTcsStageBytes;
+    unsigned char *s_a = p;
+    p += (size_t)kGroups * 128 * tc::kRowBytes;
+    WarpPool *pools = reinterpret_cast<WarpPool *>(p);
+
+    const int n32 = a.scene.n32;
+    const int nchunks = (n32 + kChunk - 1) / kChunk;
+    const uint32_t wrap = 2u * kStages * (uint32_t)nchunks;
+    for (int i = threadIdx.x; i < R1_RSQRT12_ENTRIES / 2; i += blockDim.x)
+        reinterpret_cast<uint32_t *>(s_tab)[i] = reinterpret_cast<const uint32_t *>(g_rsqrt12)[i];
+    if (threadIdx.x == 0) {
+        for (int g = 0; g < 4; ++g) {
+            tc::mbar_init(&ctl.mma[g], 1);
+            ctl.arrived_a[g] = 0; ctl.arrived_e[g] = 0; ctl.exit_flag[g] = 0;
+        }
+        for (int s = 0; s < kStages; ++s) {
+            tc::mbar_init(&ctl.landed[s], 1);
+            ctl.ring[s] = (uint64_t)s << 32;
+        }
+        ctl.exited = 0;
+        tc::fence_mbar_init();
+        tc::fence_proxy_async();
+        for (int s = 0; s < kStages; ++s) tcs_fill(a.scene, s_stages + (size_t)s * kTcsStageBytes, &ctl.landed[s], s % nchunks);
+    }
+    if (threadIdx.x < 32) tc::tmem_alloc(&ctl.tmem_base, kTmemCols);
+    tc::tc_fence_before();
+    __syncthreads();
+    tc::tc_fence_after();
+    const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t *>(&ctl.tmem_base);
+    const unsigned lane = threadIdx.x & 31u;
+    const int g = threadIdx.x >> 7, w = (threadIdx.x >> 5) & 3, r = threadIdx.x & 127;
+    const uint16_t *tab = s_tab;
+    const unsigned lt_mask = (1u << lane) - 1u;
+    WarpPool &pool = pools[threadIdx.x >> 5];
+    unsigned char *a_tile = s_a + (size_t)g * 128 * tc::kRowBytes;
+    const uint32_t a_smem = tc::smem_u32(a_tile), stages_smem = tc::smem_u32(s_stages);
+    const uint32_t t_acc = tmem_base + (uint32_t)(g * kChunk);
+    const uint32_t t_lane = t_acc + ((uint32_t)(w * 32) << 16);
+    bool active = false, exhausted = false;
+    PoolState ps;
+    ps.dry = false; ps.ready = 0; ps.w_next = 0; ps.w_end = 0;
+    const uint32_t lanes_x = gridDim.x * blockDim.x * a.sched_div;
+    uint32_t lp = 0, it = 0, nrays = 0, fpos = 0;               // fpos: the fill that starts this group's next scan
+    int depth = 0;
+    f3 thr = mk3(1, 1, 1), o = mk3(0, 0, 0), d = mk3(0, 0, 0);
+    Rng rng;
+    rng.k0 = 0; rng.k1 = 0;
+
+    for (;;) {
+        const bool want = !active && !exhausted;
+        const unsigned need = __ballot_sync(kFull, want);
+        if (need) pool_take(a, pool, ps, tab, lane, lt_mask, lanes_x, need, want, active, exhausted, o, d, lp, rng, thr, depth);
+        const bool warp_done = __all_sync(kFull, exhausted);
+
+        tc::write_ray_row(a_tile, r, o, d, active);
+        tc::fence_proxy_async();
+        tc::tc_fence_before();                                   // this warp's reads of the previous scan's last chunk are complete
+        __syncwarp();
+        if (lane == 0) {
+            const uint32_t mine = 1u + (warp_done ? 0x100u : 0u);
+            __threadfence_block();
+            const uint32_t tot = atomicAdd(&ctl.arrived_a[g], mine) + mine;
+            if ((tot & 0xffu) == 4u) {                           // last of the group: start the scan (or end the group)
+                *reinterpret_cast<volatile uint32_t *>(&ctl.arrived_a[g]) = 0u;
+                __threadfence_block();
+                if ((tot >> 8) == 4u) {
+                    *reinterpret_cast<volatile uint32_t *>(&ctl.exit_flag[g]) = 1u;
+                    __threadfence_block();
+                    tcs_leave<kGroups, kStages>(a.scene, ctl, s_stages, g, wrap, nchunks);
+                    tc::mbar_arrive(&ctl.mma[g]);
+                } else {
+                    const int s = (int)(fpos % kStages);
+                    tc::mbar_wait(&ctl.landed[s], (fpos / kStages) & 1u, hint);
+                    tc::tc_fence_after();
+                    tc::mma_chunk(t_acc, a_smem, stages_smem + (uint32_t)s * kTcsStageBytes, min(kChunk, n32), tc::kLBO, tc::kSBO);
+                    tc::mma_commit(&ctl.mma[g]);
+                }
+            }
+        }
+        __syncwarp();
+
+        float t = kTMax;
+        int hit = -1;
+        bool leave = false;
+        for (int c = 0; c < nchunks; ++c, ++it) {
+            tc::mbar_wait(&ctl.mma[g], it & 1u, hint);
+            if (c == 0 && *reinterpret_cast<volatile uint32_t *>(&ctl.exit_flag[g])) { leave = true; break; }
+            const uint32_t f = fpos + (uint32_t)c;
+            const int s = (int)(f % kStages);
+            tc::tc_fence_after();
+            const int pieces = min(kPieces, (n32 - c * kChunk) >> 5);   // warp-uniform: the last chunk may be short
+            uint32_t cand[kPieces];
+#pragma unroll
+            for (int h = 0; h < kPieces; h += 2) {               // two loads in flight, eight independent sign-gather chains
+                cand[h] = 0; cand[h + 1] = 0;
+                if (h + 1 < pieces) {
+                    uint32_t v0[32], v1[32];
+                    tc::tmem_ld32_issue(t_lane + 32 * h, v0);
+                    tc::tmem_ld32_issue(t_lane + 32 * h + 32, v1);
+                    tc::tmem_wait(v0, v1);
+                    cand[h] = tc::flagged(v0);
+                    cand[h + 1] = tc::flagged(v1);
+                } else if (h < pieces) {
+                    uint32_t v[32];
+                    tc::tmem_ld32(t_lane + 32 * h, v);
+                    cand[h] = tc::flagged(v);
+                }
+            }
+            tc::tc_fence_before();
+            __syncwarp();
+            if (lane == 0) {
+                __threadfence_block();
+                if (atomicAdd(&ctl.arrived_e[g], 1u) == 3u) {        // last reader: the accumulator is free for the next chunk
+                    *reinterpret_cast<volatile uint32_t *>(&ctl.arrived_e[g]) = 0u;
+                    __threadfence_block();
+                    if (c + 1 < nchunks) {
+                        const uint32_t f1 = f + 1u;
+                        const int s1 = (int)(f1 % kStages);
+                        tc::mbar_wait(&ctl.landed[s1], (f1 / kStages) & 1u, hint);
+                        tc::tc_fence_after();
+                        tc::mma_chunk(t_acc, a_smem, stages_smem + (uint32_t)s1 * kTcsStageBytes, min(kChunk, n32 - (c + 1) * kChunk), tc::kLBO, tc::kSBO);
+                        tc::mma_commit(&ctl.mma[g]);
+                    }
+                }
+            }
+            __syncwarp();
+            tc::mbar_wait(&ctl.landed[s], (f / kStages) & 1u);   // complete (the MMA read it): makes the exact records visible here
+            const float4 *s_exact = reinterpret_cast<const float4 *>(s_stages + (size_t)s * kTcsStageBytes + kTcsOpBytes) - c * kChunk;
+#pragma unroll
+            for (int h = 0; h < kPieces; ++h)
+                if (cand[h]) exact_candidates(cand[h], s_exact, c * kChunk + 32 * h, o, d, kTMin, t, hit);
+            __syncwarp();
+            if (lane == 0) tcs_release<kGroups, kStages>(a.scene, ctl, s_stages, s, g, wrap, nchunks);
+        }
+        if (leave) break;
+        fpos += (uint32_t)nchunks;
+        if (fpos >= wrap) fpos -= wrap;
+
+        if (active) {
+            ++nrays;
+            f3 contrib;
+            const float4 e = hit >= 0 ? a.scene.exact[hit] : make_float4(0, 0, 0, 0);   // the stage may hold another chunk by now
+            if (shade_step(a, hit, t, e, tab, o, d, thr, depth, rng, contrib)) {
+                accumulate_sample(a, lp, contrib);
+                active = false;
+            }
+        }
+    }
+    unsigned long long total = nrays;
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
+    if (lane == 0 && total) atomicAdd(a.num_rays, total);
+    tc::tc_fence_before();
+    __syncthreads();
+    if (threadIdx.x == 0) {                                      // no bulk copy may still be writing when the CTA ends
+        for (int s = 0; s < kStages; ++s) {
+            const uint32_t f = (uint32_t)(*reinterpret_cast<volatile uint64_t *>(&ctl.ring[s]) >> 32);
+            tc::mbar_wait(&ctl.landed[s], (f / kStages) & 1u);
+        }
+    }
+    if (threadIdx.x < 32) tc::tmem_dealloc(tmem_base, kTmemCols);
+}
+
 // TMEM read throughput: every warp reads 32 lanes x 32 columns (4 KB) per tcgen05.ld, `iters` times over its lane quarter's 512
 // columns.  Bounds the tensor-core filter: one 4-byte filter value per (ray, sphere) has to come out of TMEM.
 __global__ void __launch_bounds__(1024, 1) tmem_read_kernel(int iters, uint32_t *sink)
@@ -1490,6 +1769,93 @@ __global__ void __launch_bounds__(128, 1) trace_rays_tc_kernel(const __grid_cons
     if (!live) return;
     f3 p = mk3(0, 0, 0), nrm = mk3(0, 0, 0);
     if (hit >= 0) hit_finalise(s_exact[hit], load_shade(sc, hit).inv_radius, o, d, t, p, nrm);
+    index[k] = hit;
+    t_out[k] = hit >= 0 ? t : 0.0f;
+    p_out[3 * k] = p.x; p_out[3 * k + 1] = p.y; p_out[3 * k + 2] = p.z;
+    n_out[3 * k] = nrm.x; n_out[3 * k + 1] = nrm.y; n_out[3 * k + 2] = nrm.z;
+}
+
+// Hitable::hit through the filter of megakernel_tcs at any scene size: the chunks stream through a ring of two stages filled by
+// tcs_fill (its addressing, the short last chunk, the exact records that exist), the rest as in trace_rays_tc_kernel.  One CTA =
+// one ray group, so chunk c is simply fill c; the multi-group release protocol is exercised by the renders.
+constexpr int kTraceTcsStages = 2;
+constexpr size_t trace_rays_tcs_smem_bytes() { return 128 + (size_t)kTraceTcsStages * kTcsStageBytes + 128 * tc::kRowBytes; }
+__global__ void __launch_bounds__(128, 1) trace_rays_tcs_kernel(const __grid_constant__ DevScene sc, int n, const float *org, const float *dir,
+                                                                float t_min, float t_max, int32_t *index, float *t_out, float *p_out, float *n_out)
+{
+    constexpr int kChunk = kTcsChunk, kPieces = kChunk / 32, kStages = kTraceTcsStages;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw);      // [MMA mbarrier | stage mbarriers | TMEM address | pad to 128 | stages | A]
+    uint64_t *landed = full + 1;
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(landed + kStages);
+    unsigned char *s_stages = smem_raw + 128;
+    unsigned char *a_tile = s_stages + (size_t)kStages * kTcsStageBytes;
+    const int n32 = sc.n32;
+    const int nchunks = (n32 + kChunk - 1) / kChunk;
+    if (threadIdx.x == 0) {
+        tc::mbar_init(full, 1);
+        for (int s = 0; s < kStages; ++s) tc::mbar_init(&landed[s], 1);
+        tc::fence_mbar_init();
+        tc::fence_proxy_async();
+        for (int s = 0; s < kStages && s < nchunks; ++s) tcs_fill(sc, s_stages + (size_t)s * kTcsStageBytes, &landed[s], s);
+    }
+    const int k = blockIdx.x * 128 + threadIdx.x;
+    const bool live = k < n;                                     // rays past n write a row that flags nothing
+    f3 o = mk3(0, 0, 0), d = mk3(0, 0, 0);
+    if (live) { o = mk3(org[3 * k], org[3 * k + 1], org[3 * k + 2]); d = mk3(dir[3 * k], dir[3 * k + 1], dir[3 * k + 2]); }
+    tc::write_ray_row(a_tile, threadIdx.x, o, d, live);
+    tc::fence_proxy_async();                                     // the A tile is read by the tensor core (async proxy)
+    if (threadIdx.x < 32) tc::tmem_alloc(tmem_slot, kChunk);
+    tc::tc_fence_before();
+    __syncthreads();
+    tc::tc_fence_after();
+    const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t *>(tmem_slot);
+    const uint32_t t_lane = tmem_base + ((uint32_t)((threadIdx.x >> 5) * 32) << 16);
+    const uint32_t a_smem = tc::smem_u32(a_tile), stages_smem = tc::smem_u32(s_stages);
+    float t = t_max;
+    int hit = -1;
+    for (int c = 0; c < nchunks; ++c) {
+        const int s = c % kStages;
+        const uint32_t parity = (uint32_t)(c / kStages) & 1u;
+        if (threadIdx.x == 0) {
+            tc::mbar_wait(&landed[s], parity);
+            tc::tc_fence_after();
+            tc::mma_chunk(tmem_base, a_smem, stages_smem + (uint32_t)s * kTcsStageBytes, min(kChunk, n32 - c * kChunk), tc::kLBO, tc::kSBO);
+            tc::mma_commit(full);
+        }
+        tc::mbar_wait(full, (uint32_t)c & 1u);
+        tc::tc_fence_after();
+        const int pieces = min(kPieces, (n32 - c * kChunk) >> 5);   // the last chunk may be short
+        uint32_t cand[kPieces];
+#pragma unroll
+        for (int h = 0; h < kPieces; h += 2) {
+            cand[h] = 0; cand[h + 1] = 0;
+            if (h + 1 < pieces) {
+                uint32_t v0[32], v1[32];
+                tc::tmem_ld32_issue(t_lane + 32 * h, v0);
+                tc::tmem_ld32_issue(t_lane + 32 * h + 32, v1);
+                tc::tmem_wait(v0, v1);
+                cand[h] = tc::flagged(v0);
+                cand[h + 1] = tc::flagged(v1);
+            } else if (h < pieces) {
+                uint32_t v[32];
+                tc::tmem_ld32(t_lane + 32 * h, v);
+                cand[h] = tc::flagged(v);
+            }
+        }
+        tc::tc_fence_before();
+        tc::mbar_wait(&landed[s], parity);                       // complete: makes the bulk copy's exact records visible here
+        const float4 *s_exact = reinterpret_cast<const float4 *>(s_stages + (size_t)s * kTcsStageBytes + kTcsOpBytes) - c * kChunk;
+#pragma unroll
+        for (int h = 0; h < kPieces; ++h)
+            if (cand[h]) exact_candidates(cand[h], s_exact, c * kChunk + 32 * h, o, d, t_min, t, hit);
+        __syncthreads();                                         // every warp is done with the accumulator and with the stage
+        if (threadIdx.x == 0 && c + kStages < nchunks) tcs_fill(sc, s_stages + (size_t)s * kTcsStageBytes, &landed[s], c + kStages);
+    }
+    if (threadIdx.x < 32) tc::tmem_dealloc(tmem_base, kChunk);
+    if (!live) return;
+    f3 p = mk3(0, 0, 0), nrm = mk3(0, 0, 0);
+    if (hit >= 0) hit_finalise(sc.exact[hit], load_shade(sc, hit).inv_radius, o, d, t, p, nrm);
     index[k] = hit;
     t_out[k] = hit >= 0 ? t : 0.0f;
     p_out[3 * k] = p.x; p_out[3 * k + 1] = p.y; p_out[3 * k + 2] = p.z;
