@@ -181,6 +181,15 @@ int r1_replay_pixels(r1_scene *scene, int n, const int32_t *xy, int width, int h
                      const uint32_t *state, const uint32_t *state4, float *color_sum, uint32_t *num_rays);
 /* First `n` draws of the counter-based generator for (pixel, sample, seed): raw u32 -- for distribution tests. */
 int r1_rng_draws(uint32_t pixel, uint32_t sample, uint32_t seed, int n, uint32_t *out);
+/* The random points a render draws for n (global pixel y * width + x, sample) keys under the global `seed`, through the
+ * renderer's own generator and samplers (SFU approximations included).  out: n x (2 + 4 * bounces) floats, per key the
+ * lens-disk point (x, y), then for every depth d < bounces (ru, rs.x, rs.y, rs.z): ru = the [0,1) uniform of draw 4 + 3 d,
+ * rs = the unit-ball sample of that bounce.  With these, a CPU restatement of the integrator reproduces a render bit for bit.
+ * 0 <= bounces <= 1024. */
+int r1_sample_points(int n, const uint32_t *pixel, const uint32_t *sample, uint32_t seed, int bounces, float *out);
+/* r1_render, plus the rank's fixed-point pixel sums the bytes were resolved from: sums = r1_local_pixels() x 3 uint64
+ * (r, g, b) in local pixel order, each the sum over the pixel's samples of round(radiance * 2^24), saturated to 32 bits. */
+int r1_render_sums(r1_scene *scene, const r1_render_params *params, uint64_t *sums, uint8_t *rgb_host, r1_result *result);
 /* FP32 FMA throughput microbenchmark on `device`: independent FFMA chains (packed = 0) or FFMA2 (packed = 1).
  * Returns TFLOP/s (FMA = 2) in *tflops.  *sm_mhz_est (optional) = clock64 ticks of one thread / elapsed time: a rough
  * cross-check only -- on the B200 boxes of this project clock64 did not tick at the SM clock (it read ~300 MHz while

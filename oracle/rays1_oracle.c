@@ -819,6 +819,151 @@ ORC_API int orc_trace_sample(const orc_scene *s, int x, int y, int image_w, int 
     return n;
 }
 
+/* ------------------------------------------------------------------ the device integrator (DESIGN.md section 3)
+ * The GPU renderer does not run the reference's loop above: it keys a counter-based generator by (pixel, sample), multiplies the
+ * throughput forward, and sums every sample into 64-bit fixed point.  Restated here from that formulation -- not from the
+ * renderer's code -- so that a whole render can be compared bit for bit: sums, bytes and ray count.  The integer sums make the
+ * result independent of the order samples finish in.  What a CPU cannot reproduce are the SFU approximations the renderer
+ * samples the lens disk and the unit ball with; those come in as `points` (r1_sample_points), or, with points == NULL, are
+ * evaluated in double precision with libm (statistically the same render, not the same bits). */
+
+/* Stafford variant 13 */
+static inline uint64_t keyed_mix64(uint64_t z)
+{
+    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+    z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+    return z ^ (z >> 31);
+}
+typedef struct { uint32_t k0, k1; } keyed_rng;
+static inline uint64_t keyed_seed_mix(uint32_t seed) { return keyed_mix64(0x9E3779B97F4A7C15ull * ((uint64_t)seed + 1u)); }
+static inline keyed_rng keyed_stream(uint32_t pixel, uint32_t sample, uint64_t seed_mix)
+{
+    const uint64_t z = keyed_mix64((((uint64_t)pixel << 32) | sample) ^ seed_mix);
+    keyed_rng r = { (uint32_t)z, (uint32_t)(z >> 32) };
+    return r;
+}
+static inline uint32_t keyed_draw(keyed_rng r, uint32_t i)
+{
+    uint32_t x = r.k0 + 0x9E3779B9u * i;
+    x ^= x >> 16; x *= 0x21f0aaadu;
+    x ^= r.k1;
+    x ^= x >> 15; x *= 0x735a2d97u;
+    x ^= x >> 15;
+    return x;
+}
+static inline float keyed_rand01(keyed_rng r, uint32_t i) { return (float)(keyed_draw(r, i) >> 8) * 0x1p-24f; }
+static inline float keyed_rand02(keyed_rng r, uint32_t i) { return (float)(keyed_draw(r, i) >> 8) * 0x1p-23f; }
+
+ORC_API uint32_t orc_keyed_draw(uint32_t pixel, uint32_t sample, uint32_t seed, uint32_t i)
+{
+    return keyed_draw(keyed_stream(pixel, sample, keyed_seed_mix(seed)), i);
+}
+
+/* one sample's radiance -> 2^-24 fixed point as cvt.rni.sat.u32.f32 does it: round half to even, NaN and negatives 0,
+ * values above 2^32 - 1 saturated */
+static inline uint32_t quantise_radiance(float c)
+{
+    const float x = c * 16777216.0f;
+    if (!(x > 0.0f)) return 0u;
+    if (x >= 4294967295.0f) return 0xFFFFFFFFu;   /* the float nearest 2^32 - 1 is 2^32 */
+    return (uint32_t)rintf(x);
+}
+/* a pixel's sum -> one byte: mean, gamma 2, (int)(c * 255.99f) (rayweek1.cpp:765-775 on the fixed-point sum) */
+static inline uint8_t resolve_sum(uint64_t sum, float inv_spp)
+{
+    const float mean = ((float)sum * 0x1p-24f) * inv_spp;
+    return (uint8_t)(int)(sqrtf(mean) * 255.99f);
+}
+ORC_API uint32_t orc_quantise_radiance(float c) { return quantise_radiance(c); }
+ORC_API uint8_t orc_resolve(uint64_t sum, int spp) { return resolve_sum(sum, (float)(1.0f / spp)); }
+
+/* the interleaved row-tile partition: tile k of row_tile rows belongs to rank k % world */
+static inline int keyed_global_row(int lr, int row_tile, int rank, int world) { return ((lr / row_tile) * world + rank) * row_tile + lr % row_tile; }
+ORC_API int orc_local_rows(int height, int row_tile, int rank, int world)
+{
+    if (row_tile <= 0) row_tile = 1;
+    int rows = 0;
+    while (keyed_global_row(rows, row_tile, rank, world) < height) ++rows;
+    return rows;
+}
+
+/* the lens-disk point and the unit-ball samples in double precision: radius sqrt(u) / cbrt(u), azimuth a * pi */
+static void disk_libm(keyed_rng r, float *px, float *py)
+{
+    const double rad = sqrt((double)keyed_rand01(r, 2)), a = (double)keyed_rand02(r, 3) * M_PI;
+    *px = (float)(rad * cos(a));
+    *py = (float)(rad * sin(a));
+}
+static v3 ball_libm(keyed_rng r, uint32_t i, float u)
+{
+    const float z = 1.0f - keyed_rand02(r, i + 1);
+    const double a = (double)keyed_rand02(r, i + 2) * M_PI, rad = cbrt((double)u);
+    const double rho = rad * sqrt(fmax(0.0, 1.0 - (double)z * z));
+    return v3_make((float)(rho * cos(a)), (float)(rho * sin(a)), (float)(rad * z));
+}
+
+/* The rank's rows of a render (ascending global row, like r1_render): sums[local pixel][3], rgb[local pixel][3], *num_rays.
+ * points: per local pixel, per sample 2 + 4 max_bounces floats as r1_sample_points writes them (disk x, y; then ru, ball x, y, z
+ * per depth -- ru is drawn here, only the ball is taken from the table), or NULL.  Returns the number of local pixels. */
+ORC_API int64_t orc_render_keyed(const orc_scene *s, int width, int height, int spp, int max_bounces, uint32_t seed, int rank, int world,
+                                 int row_tile, const float *points, uint64_t *sums, uint8_t *rgb, uint64_t *num_rays)
+{
+    const int built = g_as_built;
+    g_as_built = 1;                        /* the renderer's association throughout */
+    if (row_tile <= 0) row_tile = 1;
+    const int rows = orc_local_rows(height, row_tile, rank, world);
+    const size_t per_sample = 2 + 4 * (size_t)max_bounces;
+    const uint64_t seed_mix = keyed_seed_mix(seed);
+    const float inv_w = 1.0f / width, inv_h = 1.0f / height, inv_spp = (float)(1.0f / spp);
+    uint64_t rays = 0;
+    for (int lr = 0; lr < rows; ++lr) {
+        const int y = keyed_global_row(lr, row_tile, rank, world);
+        for (int x = 0; x < width; ++x) {
+            const size_t lp = (size_t)lr * width + x;
+            uint64_t acc[3] = { 0, 0, 0 };
+            for (int smp = 0; smp < spp; ++smp) {
+                const keyed_rng key = keyed_stream((uint32_t)y * (uint32_t)width + (uint32_t)x, (uint32_t)smp, seed_mix);
+                const float *pt = points ? points + (lp * (size_t)spp + (size_t)smp) * per_sample : NULL;
+                /* primary ray: jitter from draws 0 and 1, lens disk from draws 2 and 3 */
+                const float u = (keyed_rand01(key, 0) + (float)x) * inv_w, v = (keyed_rand01(key, 1) + (float)y) * inv_h;
+                float px, py;
+                if (pt) { px = pt[0]; py = pt[1]; }
+                else disk_libm(key, &px, &py);
+                v3 o, d;
+                camera_ray(s, u, v, px, py, &o, &d);
+                v3 thr = v3_make(1, 1, 1), contrib = v3_make(0, 0, 0);
+                for (int depth = 0;; ) {
+                    ++rays;
+                    hit_rec rec;
+                    if (!scene_hit(s, o, d, 0.001f, FLT_MAX, &rec)) {
+                        const float t = 0.5f * (d.y + 1.0f), it = 1.0f - t;
+                        contrib = v3_mul(thr, v3_make(fmaf(t, 0.5f, it), fmaf(t, 0.7f, it), fmaf(t, 1.0f, it)));
+                        break;
+                    }
+                    if (depth >= max_bounces) break;                       /* black, no draw past the cap */
+                    const uint32_t draw0 = 4u + 3u * (uint32_t)depth;
+                    const float ru = keyed_rand01(key, draw0);
+                    const v3 rs = pt ? v3_make(pt[2 + 4 * depth + 1], pt[2 + 4 * depth + 2], pt[2 + 4 * depth + 3]) : ball_libm(key, draw0, ru);
+                    v3 atten, nd;
+                    if (!scatter_explicit(s, rec.index, d, rec.p, rec.normal, rs, ru, &atten, &nd)) break;   /* black */
+                    thr = v3_mul(thr, atten);
+                    o = rec.p; d = nd; ++depth;
+                }
+                acc[0] += quantise_radiance(contrib.x);
+                acc[1] += quantise_radiance(contrib.y);
+                acc[2] += quantise_radiance(contrib.z);
+            }
+            for (int c = 0; c < 3; ++c) {
+                if (sums) sums[3 * lp + c] = acc[c];
+                if (rgb) rgb[3 * lp + c] = resolve_sum(acc[c], inv_spp);
+            }
+        }
+    }
+    g_as_built = built;
+    if (num_rays) *num_rays = rays;
+    return (int64_t)rows * width;
+}
+
 /* ------------------------------------------------------------------ RNG known-answer entry points */
 
 ORC_API uint32_t orc_xorshift32(uint32_t *state) { return xorshift32(state); }

@@ -55,6 +55,7 @@ def _load():
     i32p = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
     u32p = np.ctypeslib.ndpointer(dtype=np.uint32, flags="C_CONTIGUOUS")
     u8p = np.ctypeslib.ndpointer(dtype=np.uint8, flags="C_CONTIGUOUS")
+    u64p = np.ctypeslib.ndpointer(dtype=np.uint64, flags="C_CONTIGUOUS")
     vp, ci, cf = C.c_void_p, C.c_int, C.c_float
     sig = {
         "r1_abi_version": (ci, []),
@@ -85,6 +86,8 @@ def _load():
         "r1_get_ray": (ci, [vp, ci, f32p, f32p, f32p, f32p, f32p]),
         "r1_replay_pixels": (ci, [vp, ci, i32p, ci, ci, ci, ci, u32p, u32p, f32p, u32p]),
         "r1_rng_draws": (ci, [C.c_uint32, C.c_uint32, C.c_uint32, ci, u32p]),
+        "r1_sample_points": (ci, [ci, u32p, u32p, C.c_uint32, ci, f32p]),
+        "r1_render_sums": (ci, [vp, C.POINTER(RenderParams), u64p, u8p, C.POINTER(Result)]),
         "r1_fma_peak": (ci, [ci, ci, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
         "r1_tmem_read_peak": (ci, [ci, ci, C.POINTER(C.c_double)]),
         "r1_kernel_name": (C.c_char_p, [vp, ci]),
@@ -181,6 +184,19 @@ class Scene:
         buf = rgb if rgb.size else np.zeros(16, np.uint8)
         _check(lib.r1_render(self.handle, C.byref(p), buf, C.byref(res)), "r1_render")
         return rgb, res
+
+    def render_sums(self, width=SCREEN_W, height=SCREEN_H, spp=NUM_SAMPLES_PER_PIXEL, max_bounces=MAX_BOUNCES, variant=VARIANT_MEGAKERNEL,
+                    seed=0, rank=0, world=1, row_tile=DEFAULT_ROW_TILE, device=-1, blocks_per_sm=0, threads=0):
+        """r1_render_sums: render() plus the fixed-point pixel sums the bytes were resolved from.
+        Returns (rgb[local_rows, width, 3] uint8, sums[local_rows, width, 3] uint64 in units of 2^-24, Result)."""
+        p = RenderParams(width, height, spp, max_bounces, variant, seed, rank, world, row_tile, blocks_per_sm, threads, device)
+        rows = int(lib.r1_local_rows(height, row_tile, rank, world))
+        rgb = np.zeros((rows, width, 3), np.uint8)
+        sums = np.zeros((rows, width, 3), np.uint64)
+        res = Result()
+        _check(lib.r1_render_sums(self.handle, C.byref(p), sums.reshape(-1) if sums.size else np.zeros(1, np.uint64),
+                                  rgb if rgb.size else np.zeros(16, np.uint8), C.byref(res)), "r1_render_sums")
+        return rgb, sums, res
 
     def render_device(self, d_rgb_ptr, d_num_rays_ptr, stream_ptr=None, **kw):
         """r1_render_device: asynchronous, device pointers (e.g. torch tensors' data_ptr())."""
@@ -357,6 +373,19 @@ def log_results(version, scene, results):
 def rng_draws(pixel, sample, seed, n):
     out = np.zeros(n, np.uint32)
     _check(lib.r1_rng_draws(pixel, sample, seed, n, out), "r1_rng_draws")
+    return out
+
+
+def sample_points(pixel, sample, seed, bounces):
+    """r1_sample_points: the random points a render draws for the (global pixel, sample) keys -> float32 [n, 2 + 4 bounces]:
+    lens-disk (x, y), then (ru, ball x, y, z) per depth."""
+    pixel = np.ascontiguousarray(pixel, np.uint32).reshape(-1)
+    sample = np.ascontiguousarray(sample, np.uint32).reshape(-1)
+    if pixel.shape != sample.shape:
+        raise ValueError("pixel and sample keys differ in length")
+    out = np.zeros((len(pixel), 2 + 4 * max(bounces, 0)), np.float32)   # bounces < 0: the library refuses it
+    _check(lib.r1_sample_points(len(pixel), pixel, sample, seed, bounces, out.reshape(-1) if out.size else np.zeros(1, np.float32)),
+           "r1_sample_points")
     return out
 
 

@@ -1058,6 +1058,41 @@ int r1_rng_draws(uint32_t pixel, uint32_t sample, uint32_t seed, int n, uint32_t
     return R1_OK;
 }
 
+int r1_sample_points(int n, const uint32_t *pixel, const uint32_t *sample, uint32_t seed, int bounces, float *out)
+{
+    if (n < 0 || bounces < 0 || bounces > 1024 || (n > 0 && (!pixel || !sample || !out))) return fail(R1_ERR_ARG, "bad argument");
+    if (n == 0) return R1_OK;
+    const size_t per_key = 2 + 4 * (size_t)bounces;
+    DevBuf d_pixel, d_sample, d_out;
+    R1_TRY(d_pixel.upload(pixel, (size_t)n * 4)); R1_TRY(d_sample.upload(sample, (size_t)n * 4));
+    R1_TRY(d_out.alloc((size_t)n * per_key * 4));
+    r1::sample_points_kernel<<<(n + 127) / 128, 128>>>(n, d_pixel.as<uint32_t>(), d_sample.as<uint32_t>(), r1::Rng::seed_hash(seed), bounces, d_out.as<float>());
+    R1_CUDA(cudaGetLastError());
+    R1_CUDA(cudaDeviceSynchronize());
+    R1_TRY(d_out.download(out, (size_t)n * per_key * 4));
+    return R1_OK;
+}
+
+int r1_render_sums(r1_scene *scene, const r1_render_params *params, uint64_t *sums, uint8_t *rgb_host, r1_result *result)
+{
+    R1_TRY(validate(params));
+    if (!scene || !sums || !rgb_host) return fail(R1_ERR_ARG, "null argument");
+    int ndev = 0;
+    R1_CUDA(cudaGetDeviceCount(&ndev));
+    R1_TRY(r1_render(scene, params, rgb_host, result));   // returns after the render and its copies have completed
+    const Partition part = partition(params->width, params->height, params->row_tile, params->rank, params->world);
+    if (part.npix_local == 0) return R1_OK;
+    DeviceCtx *cp = nullptr;
+    R1_TRY(get_ctx(scene, &cp, params->device));
+    Scratch *xp = nullptr;
+    R1_TRY(get_scratch(cp->device, &xp));
+    std::vector<unsigned long long> accum((size_t)part.npix_local * 4);   // (r, g, b, unused) per local pixel
+    R1_CUDA(cudaMemcpy(accum.data(), xp->accum, accum.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    for (size_t lp = 0; lp < part.npix_local; ++lp)
+        for (int c = 0; c < 3; ++c) sums[3 * lp + c] = accum[4 * lp + c];
+    return R1_OK;
+}
+
 int r1_tmem_read_peak(int device, int warps, double *bytes_per_second_per_sm)
 {
     if (!bytes_per_second_per_sm || warps < 1 || warps > 32) return fail(R1_ERR_ARG, "bad argument");

@@ -1898,6 +1898,27 @@ __global__ void rng_kernel(uint32_t pixel, uint32_t sample, uint32_t seed, int n
     }
 }
 
+// The random points of the integrator for given (pixel, sample) keys: primary_ray's lens-disk sample and shade_step's (ru, unit-ball
+// sample) of every depth, from the same device functions and draw indices -- the values a CPU cannot reproduce (SFU approximations).
+__global__ void sample_points_kernel(int n, const uint32_t *pixel, const uint32_t *sample, uint64_t seed_mix, int bounces, float *out)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    Rng rng;
+    rng.seed(pixel[k], sample[k], seed_mix);
+    float *o = out + (size_t)k * (2 + 4 * (size_t)bounces);
+    float px, py;
+    random_in_unit_disk(rng, 2, px, py);
+    o[0] = px; o[1] = py;
+    for (int depth = 0; depth < bounces; ++depth) {
+        const uint32_t draw0 = kDrawsPrimary + kDrawsPerBounce * (uint32_t)depth;
+        const float ru = rng.rand01(draw0);
+        const f3 rs = random_in_unit_sphere(rng, draw0, ru);
+        float *q = o + 2 + 4 * depth;
+        q[0] = ru; q[1] = rs.x; q[2] = rs.y; q[3] = rs.z;
+    }
+}
+
 // ------------------------------------------------------------------------------------------------ replay (parity)
 // SURVEY.md 8f rank 4: the pixel loop of render_tile (rayweek1.cpp:752-765) for one pixel per thread, driven by the
 // REFERENCE's generators from recorded states instead of the counter-based RNG: xorshift32 13/17/15 (mymath.h:17-25), the

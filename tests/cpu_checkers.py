@@ -24,6 +24,7 @@ _fp = np.ctypeslib.ndpointer(dtype=np.float32, flags="C_CONTIGUOUS")
 _ip = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
 _up = np.ctypeslib.ndpointer(dtype=np.uint32, flags="C_CONTIGUOUS")
 _bp = np.ctypeslib.ndpointer(dtype=np.uint8, flags="C_CONTIGUOUS")
+_u64p = np.ctypeslib.ndpointer(dtype=np.uint64, flags="C_CONTIGUOUS")
 
 
 def build_oracle():
@@ -152,6 +153,46 @@ class Oracle(_Checker):
         L.orc_render.argtypes = [C.c_void_p, _bp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double)]
         L.orc_scene_create_from_soa.restype = C.c_void_p
         L.orc_scene_create_from_soa.argtypes = [C.c_int, _fp, _fp, _fp, _fp, _fp, _ip, _fp, _fp]
+        L.orc_keyed_draw.restype = C.c_uint32
+        L.orc_keyed_draw.argtypes = [C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]
+        L.orc_quantise_radiance.restype = C.c_uint32
+        L.orc_quantise_radiance.argtypes = [C.c_float]
+        L.orc_resolve.restype = C.c_uint8
+        L.orc_resolve.argtypes = [C.c_uint64, C.c_int]
+        L.orc_local_rows.restype = C.c_int
+        L.orc_local_rows.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int]
+        L.orc_render_keyed.restype = C.c_int64
+        L.orc_render_keyed.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                       _u64p, _bp, C.POINTER(C.c_uint64)]
+
+    # -- the device integrator (counter-based generator, forward throughput, fixed-point sums)
+    def keyed_draw(self, pixel, sample, seed, i):
+        return int(self.lib.orc_keyed_draw(pixel, sample, seed, i))
+
+    def quantise_radiance(self, c):
+        return int(self.lib.orc_quantise_radiance(c))
+
+    def resolve(self, total, spp):
+        return int(self.lib.orc_resolve(total, spp))
+
+    def local_rows(self, height, row_tile, rank, world):
+        return int(self.lib.orc_local_rows(height, row_tile, rank, world))
+
+    def render_keyed(self, s, w, h, spp, max_bounces, seed=0, rank=0, world=1, row_tile=1, points=None):
+        """The rank's rows as the GPU renderer computes them -> (sums[rows, w, 3] uint64, rgb[rows, w, 3] uint8, num_rays).
+        points: r1.sample_points() of the rank's (pixel, sample) keys in local pixel order (bit-exact), or None (libm)."""
+        rows = self.local_rows(h, row_tile, rank, world)
+        sums = np.zeros((rows, w, 3), np.uint64)
+        rgb = np.zeros((rows, w, 3), np.uint8)
+        rays = C.c_uint64(0)
+        if points is not None:
+            points = np.ascontiguousarray(points, _f)
+            assert points.size == rows * w * spp * (2 + 4 * max_bounces), "points table does not match the rank's samples"
+        n = self.lib.orc_render_keyed(s, w, h, spp, max_bounces, seed, rank, world, row_tile,
+                                      None if points is None else points.ctypes.data, sums.reshape(-1) if sums.size else np.zeros(1, np.uint64),
+                                      rgb.reshape(-1) if rgb.size else np.zeros(1, np.uint8), C.byref(rays))
+        assert n == rows * w
+        return sums, rgb, int(rays.value)
 
     def scene_create_from_soa(self, soa):
         """a scene holding the spheres of ``soa`` (the dict of Scene.soa() / scene_soa()) as given, for hit() on any scene;

@@ -163,6 +163,15 @@ def test_no_cpu_fallback_without_a_gpu(r1):
         s.render(16, 9, 1)
     with pytest.raises(r1.Rays1Error):
         s.trace_rays(np.zeros((1, 3)), np.array([[0, 0, 1.0]]))
+    with pytest.raises(r1.Rays1Error, match=r"\(-3\)"):
+        s.render_sums(16, 9, 1)
+    with pytest.raises(r1.Rays1Error, match=r"\(-3\)"):
+        r1.sample_points([0], [0], 0, 2)
+    # arguments are checked before any device is looked up
+    with pytest.raises(r1.Rays1Error, match=r"\(-1\)"):
+        s.render_sums(16, 9, 0)
+    with pytest.raises(r1.Rays1Error, match=r"\(-1\)"):
+        r1.sample_points([0], [0], 0, -1)
     s.close()
 
 
