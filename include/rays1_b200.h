@@ -165,7 +165,8 @@ const char *r1_kernel_name(r1_scene *scene, int variant);
 int r1_tensor_operand(const r1_scene *scene, void *out, uint64_t out_bytes, uint32_t *n32_out);
 /* Values of the tensor-core FILTER (R1_VARIANT_MEGAKERNEL_TENSOR) for n rays against every sphere: e[ray * n32 + sphere], n32 =
  * sphere count padded to 32; the filter flags a sphere iff the sign bit of e is clear, and must flag every sphere Hitable::hit's
- * discriminant test (rayweek1.cpp:192-204) accepts.  layout = 0. */
+ * discriminant test (rayweek1.cpp:192-204) accepts.  layout must be 0 (the renderer's operand layout); any other value returns
+ * R1_ERR_ARG before any device is touched. */
 int r1_filter_probe(r1_scene *scene, int n, const float *org, const float *dir, int layout, float *e);
 /* Material::scatter (rayweek1.cpp:403-409, 427-433, 470-511) with the random inputs injected: rand_sphere is the
  * unit-ball sample, rand_u the [0,1) uniform. */

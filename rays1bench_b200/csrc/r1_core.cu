@@ -266,42 +266,12 @@ int launch_megakernel_dual(int sm_count, const r1::RenderArgs &args, const r1_re
     return fail(R1_ERR_ARG, "the dual variant runs 512 or 768 threads (got %d)", threads);
 }
 
-// tensor-core filter (r1::megakernel_tc, R1_VARIANT_MEGAKERNEL_TENSOR): `threads` selects the number of 128-ray groups per CTA,
-// R1_TC_CFG="chunk,buffers" the TMEM pipeline (columns per accumulator buffer, buffers per group; groups x buffers x chunk <= 512)
-template <int kGroups, int kChunk, int kBufs, bool kATmem>
-int launch_megakernel_tc_t(int sm_count, const r1::RenderArgs &args, cudaStream_t stream)
-{
-    auto kern = r1::megakernel_tc<kGroups, kChunk, kBufs, kATmem>;
-    const size_t smem = r1::tc_smem_bytes(kGroups, args.scene.n32);
-    R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = sm_count;                                         // one CTA per SM: it owns all 512 TMEM columns
-    const unsigned long long max_ctas = (args.n_samples + kGroups * 128 - 1) / (kGroups * 128);
-    if ((unsigned long long)grid > max_ctas) grid = (int)std::max<unsigned long long>(1, max_ctas);
-    kern<<<grid, kGroups * 160, smem, stream>>>(args);
-    R1_CUDA(cudaGetLastError());
-    return R1_OK;
-}
-
-template <int kGroups, int kChunk, int kBufs>
-int launch_megakernel_tc2_t(int sm_count, const r1::RenderArgs &args, cudaStream_t stream)
-{
-    auto kern = r1::megakernel_tc2<kGroups, kChunk, kBufs>;
-    const size_t smem = r1::tc2_smem_bytes(kGroups, args.scene.n32);
-    if (smem > 227 * 1024) return fail(R1_ERR_LIMIT, "tensor variant: %d ray groups need %zu bytes of shared memory for this scene", kGroups, smem);
-    R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = sm_count;
-    const unsigned long long max_ctas = (args.n_samples + kGroups * 128 - 1) / (kGroups * 128);
-    if ((unsigned long long)grid > max_ctas) grid = (int)std::max<unsigned long long>(1, max_ctas);
-    kern<<<grid, kGroups * 128, smem, stream>>>(args);
-    R1_CUDA(cudaGetLastError());
-    return R1_OK;
-}
-
+// tensor-core filter (r1::megakernel_tc3, R1_VARIANT_MEGAKERNEL_TENSOR): `threads` / 128 = ray groups per CTA
 template <int kGroups>
 int launch_megakernel_tc3_t(int sm_count, const r1::RenderArgs &args, cudaStream_t stream)
 {
     auto kern = r1::megakernel_tc3<kGroups>;
-    const size_t smem = r1::tc2_smem_bytes(kGroups, args.scene.n32);
+    const size_t smem = r1::tc3_smem_bytes(kGroups, args.scene.n32);
     if (smem > 227 * 1024) return fail(R1_ERR_LIMIT, "tensor variant: %d ray groups need %zu bytes of shared memory for this scene", kGroups, smem);
     R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int grid = sm_count;
@@ -351,37 +321,13 @@ int launch_megakernel_tcs(int sm_count, const r1::RenderArgs &args, const r1_ren
 int launch_megakernel_tc(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
 {
     if (!args.scene.tcb) return fail(R1_ERR_LIMIT, "the tensor-core filter takes scenes of 1 .. %d spheres (its operand lives in shared memory)", r1::tc::kMaxSpheres);
-    if (!getenv("R1_TC1") && !getenv("R1_TC2")) {
-        // r1::megakernel_tc3 (default): the last ray warp to arrive issues the MMA, accumulator buffers pooled among the groups;
-        // R1_TC3 (or threads / 128) = ray groups per CTA.  Measured on the large scene: 4 groups 9.70, 5: 10.34, 6: 9.92, 7: 9.69 G rays/s
-        const int groups = getenv("R1_TC3") ? atoi(getenv("R1_TC3")) : (prm.threads > 0 ? prm.threads / 128 : 5);
-        if (groups == 4) return launch_megakernel_tc3_t<4>(sm_count, args, stream);
-        if (groups == 5) return launch_megakernel_tc3_t<5>(sm_count, args, stream);
-        if (groups == 6) return launch_megakernel_tc3_t<6>(sm_count, args, stream);
-        if (groups == 7) return launch_megakernel_tc3_t<7>(sm_count, args, stream);
-        return fail(R1_ERR_ARG, "the tensor variant runs 4 .. 7 groups of 128 ray threads per CTA (threads = 512 .. 896)");
-    }
-    if (!getenv("R1_TC1")) {   // R1_TC2 = groups (A/B): r1::megakernel_tc2, one accumulator buffer (or two: R1_TC2_BUFS=2) owned by each group
-        const int groups = atoi(getenv("R1_TC2"));
-        const int bufs = getenv("R1_TC2_BUFS") ? atoi(getenv("R1_TC2_BUFS")) : 1;
-        if (groups == 4 && bufs == 2) return launch_megakernel_tc2_t<4, 64, 2>(sm_count, args, stream);
-        if (groups == 3 && bufs == 2) return launch_megakernel_tc2_t<3, 64, 2>(sm_count, args, stream);
-        if (groups == 4) return launch_megakernel_tc2_t<4, 128, 1>(sm_count, args, stream);
-        if (groups == 5) return launch_megakernel_tc2_t<5, 96, 1>(sm_count, args, stream);
-        if (groups == 6) return launch_megakernel_tc2_t<6, 64, 1>(sm_count, args, stream);
-        if (groups == 7) return launch_megakernel_tc2_t<7, 64, 1>(sm_count, args, stream);
-        return fail(R1_ERR_ARG, "R1_TC2 must be 3 .. 7");
-    }
-    // R1_TC1=1: r1::megakernel_tc, one MMA-issuing warp per group (A/B)
-    const int threads = prm.threads > 0 ? prm.threads : (getenv("R1_TC_THREADS") ? atoi(getenv("R1_TC_THREADS")) : 512);
-    int chunk = 128, bufs = 1, atmem = 0;
-    if (const char *e = getenv("R1_TC_CFG")) sscanf(e, "%d,%d,%d", &chunk, &bufs, &atmem);
-#define R1_TC_CASE(G, C, B, A) if (threads == G * 128 && chunk == C && bufs == B && atmem == A) return launch_megakernel_tc_t<G, C, B, A != 0>(sm_count, args, stream)
-    R1_TC_CASE(4, 128, 1, 0); R1_TC_CASE(4, 64, 2, 0); R1_TC_CASE(4, 96, 1, 1); R1_TC_CASE(4, 32, 3, 1);
-    R1_TC_CASE(3, 128, 1, 0); R1_TC_CASE(3, 64, 2, 0); R1_TC_CASE(3, 128, 1, 1); R1_TC_CASE(3, 64, 2, 1);
-    R1_TC_CASE(2, 128, 2, 0); R1_TC_CASE(2, 256, 1, 0); R1_TC_CASE(2, 96, 2, 1); R1_TC_CASE(2, 224, 1, 1);
-#undef R1_TC_CASE
-    return fail(R1_ERR_ARG, "tensor variant: no kernel for %d ray threads, chunk %d, %d buffers, A in %s", threads, chunk, bufs, atmem ? "TMEM" : "shared memory");
+    // ray groups per CTA; measured on the large scene: 4 groups 9.70, 5: 10.34, 6: 9.92, 7: 9.69 G rays/s
+    const int groups = prm.threads > 0 ? prm.threads / 128 : 5;
+    if (groups == 4) return launch_megakernel_tc3_t<4>(sm_count, args, stream);
+    if (groups == 5) return launch_megakernel_tc3_t<5>(sm_count, args, stream);
+    if (groups == 6) return launch_megakernel_tc3_t<6>(sm_count, args, stream);
+    if (groups == 7) return launch_megakernel_tc3_t<7>(sm_count, args, stream);
+    return fail(R1_ERR_ARG, "the tensor variant runs 4 .. 7 groups of 128 ray threads per CTA (threads = 512 .. 896)");
 }
 
 template <int kScan, bool kStaged, int kThreads>
@@ -746,7 +692,6 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
     const bool pool_sched = !(getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0);
     if (c.dev.n8 >= 256) { a.sched_kmax = pool_sched ? 8 : 1; a.sched_div = pool_sched ? 16 : 1; }
     else { a.sched_kmax = 64; a.sched_div = 16; }
-    a.tc_flags = getenv("R1_TC_FLAGS") ? (uint32_t)atoi(getenv("R1_TC_FLAGS")) : 1u;
     if (const char *e = getenv("R1_SCHED")) {  // tuning knob: "kmax,div"
         unsigned k = 0, d = 0;
         if (sscanf(e, "%u,%u", &k, &d) == 2 && k >= 1 && k <= 4096 && d >= 1 && d <= 1024) { a.sched_kmax = k; a.sched_div = d; }
@@ -959,7 +904,7 @@ const char *r1_kernel_name(r1_scene *scene, int variant)
     prm.variant = variant;
     switch (resolve_variant(cp->dev, prm)) {
     case R1_VARIANT_WAVEFRONT: return "wf_intersect + wf_shade (graph loop)";
-    case R1_VARIANT_MEGAKERNEL_TENSOR: return getenv("R1_TC1") ? "megakernel_tc" : (getenv("R1_TC2") ? "megakernel_tc2" : "megakernel_tc3");
+    case R1_VARIANT_MEGAKERNEL_TENSOR: return "megakernel_tc3";
     case R1_VARIANT_MEGAKERNEL_DUAL: return "megakernel_pool2";
     case R1_VARIANT_MEGAKERNEL_TENSOR_STREAM: return "megakernel_tcs";
     default: return (getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0) ? "megakernel" : "megakernel_pool";
@@ -968,6 +913,7 @@ const char *r1_kernel_name(r1_scene *scene, int variant)
 
 int r1_filter_probe(r1_scene *scene, int n, const float *org, const float *dir, int layout, float *e)
 {
+    if (layout != 0) return fail(R1_ERR_ARG, "r1_filter_probe: layout must be 0, got %d", layout);
     DeviceCtx *cp = nullptr;
     R1_TRY(get_ctx(scene, &cp));
     if (n < 0 || (n > 0 && (!org || !dir || !e))) return fail(R1_ERR_ARG, "bad argument");
@@ -977,11 +923,9 @@ int r1_filter_probe(r1_scene *scene, int n, const float *org, const float *dir, 
     DevBuf d_org, d_dir, d_e;
     R1_TRY(d_org.upload(org, (size_t)n * 12)); R1_TRY(d_dir.upload(dir, (size_t)n * 12));
     R1_TRY(d_e.alloc((size_t)n * n32 * 4));
-    const size_t smem = ((sizeof(r1::TcControl) + 127) & ~(size_t)127) + (size_t)n32 * r1::tc::kRowBytes + 128 * r1::tc::kRowBytes;
+    const size_t smem = r1::filter_probe_smem_bytes(n32);
     R1_CUDA(cudaFuncSetAttribute(r1::tc_filter_probe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    // layout 1 swaps the two stride fields of the shared-memory descriptors (bring-up aid; 0 is the layout the renderer uses)
-    const uint32_t lbo = layout == 1 ? r1::tc::kSBO : r1::tc::kLBO, sbo = layout == 1 ? r1::tc::kLBO : r1::tc::kSBO;
-    r1::tc_filter_probe_kernel<<<(n + 127) / 128, 160, smem>>>(cp->dev, n, d_org.as<float>(), d_dir.as<float>(), d_e.as<float>(), lbo, sbo);
+    r1::tc_filter_probe_kernel<<<(n + 127) / 128, 128, smem>>>(cp->dev, n, d_org.as<float>(), d_dir.as<float>(), d_e.as<float>());
     R1_CUDA(cudaGetLastError());
     R1_CUDA(cudaDeviceSynchronize());
     R1_TRY(d_e.download(e, (size_t)n * n32 * 4));

@@ -30,7 +30,6 @@ struct RenderArgs {
     float inv_w, inv_h, inv_spp;
     uint64_t seed;                   // Rng::seed_hash(global seed)
     uint64_t magic_chunks, magic_width, magic_row_tile;  // floor(2^64 / d) + 1: exact n / d for 32-bit n via one 64-bit mul-high (0 when d == 1)
-    uint32_t tc_flags;                   // megakernel_tc experiments (R1_TC_FLAGS): 1 = mbarrier waits suspend, 2 = one funnel-shift chain
     uint32_t sched_kmax, sched_div;      // guided self-scheduling: min(kmax, max(1, left / (lanes * div))) units per lane (megakernel) or
                                          // x 32 samples per warp (megakernel_pool) per atomic
     // sample-pool scheduling (megakernel_pool): work items are single samples g = lp * spp + s, handed out 32 at a time
@@ -597,26 +596,29 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool2(const
 }
 
 // ------------------------------------------------------------------------------------------------ megakernel, tensor-core filter
-// R1_VARIANT_MEGAKERNEL_TENSOR: the path state machine of megakernel_pool with the filter on the tensor cores (r1_tensor.cuh).
-// Three generations, all kept for A/B (DESIGN.md section 4.0): megakernel_tc below (R1_TC1=1: one MMA-issuing warp per group),
-// megakernel_tc2 (R1_TC2=groups: the last ray warp to arrive issues, every group owns its accumulator buffer) and megakernel_tc3
-// (default: the four accumulator buffers are pooled among five groups).
+// R1_VARIANT_MEGAKERNEL_TENSOR (DESIGN.md section 4.0): the path state machine of megakernel_pool with the filter on the tensor
+// cores (r1_tensor.cuh).  CTA = kGroups ray groups of 128 threads (4 warps, warp w of a group owns TMEM lanes 32 w .. 32 w + 31,
+// one ray per lane).  Per scan every thread writes its ray's lifted TF32 row into the group's A tile, and the scene's B tile
+// (resident in shared memory) is walked in chunks of 128 spheres: four tcgen05.mma (M = 128, N = 128, K = 8) per chunk into a
+// 128-column accumulator buffer, tcgen05.commit onto the group's `full` mbarrier.  No warp issues on behalf of the others: the
+// LAST ray warp of a group to arrive -- with its row written (first chunk of a scan) or with its 32 lanes of the buffer read
+// (next chunk) -- issues the tcgen05.mma itself, with arrivals counted in shared memory (atomicAdd).  The ray warps read their
+// filter values with tcgen05.ld and resolve the flagged spheres with the same exact test as every other variant -- same hits,
+// same bytes out.
 //
-// CTA = kGroups ray groups of 128 threads (4 warps, warp w of a group owns TMEM lanes 32 w .. 32 w + 31, one ray per lane) +
-// one MMA-issuing warp per group.  Per scan every thread writes its ray's lifted TF32 row into the group's A tile; the issuing
-// warp then walks the scene's B tile (resident in shared memory) in chunks of 64 spheres: four tcgen05.mma (M = 128, N = 64,
-// K = 8) per chunk into one of the group's two 64-column accumulator buffers, tcgen05.commit onto the buffer's `full` mbarrier.
-// The ray warps wait for `full`, read their 64 filter values with two tcgen05.ld, release the buffer (`empty`, one arrival per
-// warp) and resolve the flagged spheres with the same exact test as every other variant -- same hits, same bytes out.
-// TMEM columns of a group: kBufs accumulator buffers of kChunk columns (+ 32 for the ray operand if kATmem).
+// The four 128-column TMEM buffers are POOLED: a group holds one only while it scans (first MMA issued ... last chunk read) and
+// hands it back for the exact tests of the last chunk, shading, the pop and the row build, so a CTA carries more ray groups
+// (4 .. 7) than TMEM has buffers.  free_mask: bit b = buffer b is free; the last warp to write its row takes a buffer
+// (atomicAnd), the last reader of the last chunk returns it (atomicOr).
 struct TcControl {
-    uint64_t a_full[4];               // per group: the four ray warps have written their rows (count 4)
-    uint64_t full[4][4];              // per group and buffer: accumulator chunk complete (tcgen05.commit, count 1)
-    uint64_t empty[4][4];             // per group and buffer: the four ray warps have read it (count 4)
+    uint64_t full[8];                 // per group: accumulator chunk complete (tcgen05.commit; the exit arrival), count 1
+    uint32_t arrived_a[8];            // per group: ray warps with their row written (low byte) / out of work (next byte)
+    uint32_t arrived_e[8];            // per group: ray warps that have read the current chunk
+    uint32_t exit_flag[8];
+    uint32_t buf_of[8];               // per group: the buffer its current scan holds
+    uint32_t free_mask;
     uint32_t tmem_base;
-    uint32_t exit_flag[4];            // per group: set by the issuing warp once all four ray warps are out of work
-    uint32_t done[4][4];              // per group and ray warp: out of work (dry, pool empty, no live path)
-    uint32_t pad_[3];
+    uint32_t pad_[2];
 };
 static_assert(sizeof(TcControl) % 16 == 0, "TcControl is followed by 16-byte aligned tiles");
 
@@ -699,378 +701,11 @@ __device__ __forceinline__ void pool_take(const RenderArgs &a, WarpPool &pool, P
     }
 }
 
-constexpr size_t tc_smem_bytes(int groups, int n32)
-{
-    return (size_t)kSmemSpheres + sizeof(TcControl) + (size_t)n32 * tc::kRowBytes + (size_t)n32 * 16 + (size_t)groups * 128 * tc::kRowBytes +
-           (size_t)groups * 4 * sizeof(WarpPool) + 128;          // + alignment slack
-}
-
-template <int kGroups, int kChunk, int kBufs, bool kATmem>
-__global__ void __launch_bounds__(kGroups * 160, 1) megakernel_tc(const __grid_constant__ RenderArgs a)
-{
-    static_assert(kGroups >= 1 && kGroups <= 4 && kBufs >= 1 && kBufs <= 4 && kChunk % 32 == 0 && kChunk <= 256, "bad configuration");
-    // TMEM columns of group g: [g * kGroupCols, +32) = the ray operand if kATmem, then kBufs accumulator buffers of kChunk columns
-    constexpr int kGroupCols = (512 / kGroups) & ~31, kDCol = kATmem ? 32 : 0;
-    static_assert(kDCol + kBufs * kChunk <= kGroupCols, "TMEM has 512 columns");
-    constexpr int kPieces = kChunk / 32;
-    const bool hint = a.tc_flags & 1u, one_chain = a.tc_flags & 2u;
-    constexpr int kRayThreads = kGroups * 128;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    // shared memory: [16 B | rsqrtss table 4 KB | control | B tile n32 x 128 B | exact n32 x 16 B | A tiles kGroups x 16 KB | pools]
-    uint16_t *s_tab = reinterpret_cast<uint16_t *>(smem_raw + 16);
-    unsigned char *p = smem_raw + ((kSmemSpheres + 127) & ~127);
-    TcControl &ctl = *reinterpret_cast<TcControl *>(p);
-    p += (sizeof(TcControl) + 127) & ~127;
-    unsigned char *s_b = p;
-    const int n32 = a.scene.n32;
-    p += (size_t)n32 * tc::kRowBytes;
-    float4 *s_exact = reinterpret_cast<float4 *>(p);
-    p += (size_t)n32 * 16;
-    unsigned char *s_a = p;
-    p += (size_t)kGroups * 128 * tc::kRowBytes;
-    WarpPool *pools = reinterpret_cast<WarpPool *>(p);
-
-    for (int i = threadIdx.x; i < R1_RSQRT12_ENTRIES / 2; i += blockDim.x)
-        reinterpret_cast<uint32_t *>(s_tab)[i] = reinterpret_cast<const uint32_t *>(g_rsqrt12)[i];
-    for (int i = threadIdx.x; i < n32 * (tc::kRowBytes / 16); i += blockDim.x)
-        reinterpret_cast<uint4 *>(s_b)[i] = reinterpret_cast<const uint4 *>(a.scene.tcb)[i];
-    for (int i = threadIdx.x; i < n32; i += blockDim.x)
-        s_exact[i] = i < a.scene.n_pad ? a.scene.exact[i] : make_float4(0, 0, 0, 0);
-    if (threadIdx.x == 0) {
-        for (int g = 0; g < 4; ++g) {
-            tc::mbar_init(&ctl.a_full[g], 4);
-            for (int b = 0; b < 4; ++b) { tc::mbar_init(&ctl.full[g][b], 1); tc::mbar_init(&ctl.empty[g][b], 4); }
-            ctl.exit_flag[g] = 0;
-        }
-        tc::fence_mbar_init();
-    }
-    tc::fence_proxy_async();                                     // the B tile is read by the tensor core (async proxy)
-    if (threadIdx.x < 32) tc::tmem_alloc(&ctl.tmem_base, 512);
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
-    const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t *>(&ctl.tmem_base);
-    const int nchunks = (n32 + kChunk - 1) / kChunk;
-    const unsigned lane = threadIdx.x & 31u;
-    uint32_t nrays = 0;
-
-    if (threadIdx.x >= kRayThreads) {
-        // ===== MMA issuer of group g (one lane) =====
-        const int g = (threadIdx.x - kRayThreads) >> 5;
-        if (lane == 0) {
-            const uint32_t a_smem = tc::smem_u32(s_a + (size_t)g * 128 * tc::kRowBytes), b_smem = tc::smem_u32(s_b);
-            uint32_t it = 0;
-            for (uint32_t scan_no = 0;; ++scan_no) {
-                tc::mbar_wait(&ctl.a_full[g], scan_no & 1u, hint);
-                const volatile uint32_t *dn = ctl.done[g];
-                if (dn[0] && dn[1] && dn[2] && dn[3]) {          // nobody has a path left: wake the group up and leave
-                    *reinterpret_cast<volatile uint32_t *>(&ctl.exit_flag[g]) = 1u;
-                    tc::mbar_arrive(&ctl.full[g][it % kBufs]);
-                    break;
-                }
-                tc::tc_fence_after();
-                for (int c = 0; c < nchunks; ++c, ++it) {
-                    const uint32_t b = it % kBufs;
-                    tc::mbar_wait(&ctl.empty[g][b], ((it / kBufs) & 1u) ^ 1u, hint);
-                    tc::tc_fence_after();
-                    const int n = min(kChunk, n32 - c * kChunk);
-                    const uint32_t d_tmem = tmem_base + (uint32_t)(g * kGroupCols + kDCol + (int)b * kChunk);
-                    if (kATmem) tc::mma_chunk_ts(d_tmem, tmem_base + (uint32_t)(g * kGroupCols), b_smem + (uint32_t)c * (kChunk / 8) * tc::kSBO, n);
-                    else tc::mma_chunk(d_tmem, a_smem, b_smem + (uint32_t)c * (kChunk / 8) * tc::kSBO, n, tc::kLBO, tc::kSBO);
-                    tc::mma_commit(&ctl.full[g][b]);
-                }
-            }
-        }
-    } else {
-        // ===== ray warps =====
-        const int g = threadIdx.x >> 7, w = (threadIdx.x >> 5) & 3, r = threadIdx.x & 127;
-        const uint16_t *tab = s_tab;
-        const unsigned lt_mask = (1u << lane) - 1u;
-        WarpPool &pool = pools[threadIdx.x >> 5];
-        unsigned char *a_tile = s_a + (size_t)g * 128 * tc::kRowBytes;
-        const uint32_t t_row = tmem_base + ((uint32_t)(w * 32) << 16) + (uint32_t)(g * kGroupCols), t_lane = t_row + kDCol;
-        bool active = false, exhausted = false;
-        PoolState ps;
-        ps.dry = false; ps.ready = 0; ps.w_next = 0; ps.w_end = 0;
-        const uint32_t lanes_x = gridDim.x * kRayThreads * a.sched_div;
-        uint32_t lp = 0, it = 0;
-        int depth = 0;
-        f3 thr = mk3(1, 1, 1), o = mk3(0, 0, 0), d = mk3(0, 0, 0);
-        Rng rng;
-        rng.k0 = 0; rng.k1 = 0;
-
-        for (;;) {
-            const bool want = !active && !exhausted;
-            const unsigned need = __ballot_sync(kFull, want);
-            if (need) pool_take(a, pool, ps, tab, lane, lt_mask, lanes_x, need, want, active, exhausted, o, d, lp, rng, thr, depth);
-            const bool warp_done = __all_sync(kFull, exhausted);
-
-            if (kATmem) {
-                uint32_t row[tc::kK];
-                tc::ray_row(o, d, active, row);
-                tc::tmem_st32(t_row, row);
-                tc::tc_fence_before();
-            } else {
-                tc::write_ray_row(a_tile, r, o, d, active);
-                tc::fence_proxy_async();
-            }
-            __syncwarp();
-            if (lane == 0) {
-                *reinterpret_cast<volatile uint32_t *>(&ctl.done[g][w]) = warp_done ? 1u : 0u;
-                tc::mbar_arrive(&ctl.a_full[g]);
-            }
-
-            float t = kTMax;
-            int hit = -1;
-            bool leave = false;
-            for (int c = 0; c < nchunks; ++c, ++it) {
-                const uint32_t b = it % kBufs;
-                tc::mbar_wait(&ctl.full[g][b], (it / kBufs) & 1u, hint);
-                if (c == 0 && *reinterpret_cast<volatile uint32_t *>(&ctl.exit_flag[g])) { leave = true; break; }
-                tc::tc_fence_after();
-                const int pieces = min(kPieces, (n32 - c * kChunk) >> 5);   // warp-uniform: the last chunk may be short
-                uint32_t cand[kPieces];
-#pragma unroll
-                for (int h = 0; h < kPieces; ++h) {
-                    cand[h] = 0;
-                    if (h < pieces) {
-                        uint32_t v[32];
-                        tc::tmem_ld32(t_lane + b * kChunk + 32 * h, v);
-                        cand[h] = one_chain ? tc::flagged_chain(v) : tc::flagged(v);
-                    }
-                }
-                tc::tc_fence_before();
-                __syncwarp();
-                if (lane == 0) tc::mbar_arrive(&ctl.empty[g][b]);
-#pragma unroll
-                for (int h = 0; h < kPieces; ++h)
-                    if (cand[h]) exact_candidates(cand[h], s_exact, c * kChunk + 32 * h, o, d, kTMin, t, hit);
-            }
-            if (leave) break;
-
-            if (active) {
-                ++nrays;
-                f3 contrib;
-                const float4 e = hit >= 0 ? s_exact[hit] : make_float4(0, 0, 0, 0);
-                if (shade_step(a, hit, t, e, tab, o, d, thr, depth, rng, contrib)) {
-                    accumulate_sample(a, lp, contrib);
-                    active = false;
-                }
-            }
-        }
-        unsigned long long total = nrays;
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
-        if (lane == 0 && total) atomicAdd(a.num_rays, total);
-    }
-    tc::tc_fence_before();
-    __syncthreads();
-    if (threadIdx.x < 32) tc::tmem_dealloc(tmem_base, 512);
-}
-
-// megakernel_tc without issuing warps: the LAST ray warp of a group to arrive -- with its row written (first chunk of a scan) or
-// with its 32 lanes of the accumulator buffer read (next chunk) -- issues the tcgen05.mma itself.  Arrivals are counted in shared
-// memory (atomicAdd); nobody has to be woken up to issue, no warp spins on behalf of others, and a CTA holds up to 7 groups
-// (896 threads), each with ONE accumulator buffer of kChunk columns.
-struct TcControl2 {
-    uint64_t full[8][2];              // per group and buffer: accumulator chunk complete (tcgen05.commit; the exit arrival), count 1
-    uint32_t arrived_a[8];            // per group: ray warps with their row written (low byte) / out of work (next byte)
-    uint32_t arrived_e[8][2];         // per group and buffer: ray warps that have read the chunk in it
-    uint32_t exit_flag[8];
-    uint32_t tmem_base;
-    uint32_t pad_[3];
-};
-static_assert(sizeof(TcControl2) % 16 == 0, "TcControl2 is followed by 16-byte aligned tiles");
-
-constexpr size_t tc2_smem_bytes(int groups, int n32)
+constexpr size_t tc3_smem_bytes(int groups, int n32)
 {
     return (size_t)kSmemSpheres + 256 + (size_t)n32 * tc::kRowBytes + (size_t)n32 * 16 + (size_t)groups * 128 * tc::kRowBytes +
            (size_t)groups * 4 * sizeof(WarpPool) + 256;          // + alignment slack
 }
-
-template <int kGroups, int kChunk, int kBufs>
-__global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tc2(const __grid_constant__ RenderArgs a)
-{
-    static_assert(kGroups >= 1 && kGroups <= 8 && kChunk % 32 == 0 && kChunk <= 256 && (kBufs == 1 || kBufs == 2) && kGroups * kChunk * kBufs <= 512,
-                  "bad configuration");
-    constexpr int kPieces = kChunk / 32;
-    const bool hint = a.tc_flags & 1u;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    uint16_t *s_tab = reinterpret_cast<uint16_t *>(smem_raw + 16);
-    unsigned char *p = smem_raw + ((kSmemSpheres + 127) & ~127);
-    TcControl2 &ctl = *reinterpret_cast<TcControl2 *>(p);
-    p += (sizeof(TcControl2) + 127) & ~127;
-    unsigned char *s_b = p;
-    const int n32 = a.scene.n32;
-    p += (size_t)n32 * tc::kRowBytes;
-    float4 *s_exact = reinterpret_cast<float4 *>(p);
-    p += (size_t)n32 * 16;
-    unsigned char *s_a = p;
-    p += (size_t)kGroups * 128 * tc::kRowBytes;
-    WarpPool *pools = reinterpret_cast<WarpPool *>(p);
-
-    for (int i = threadIdx.x; i < R1_RSQRT12_ENTRIES / 2; i += blockDim.x)
-        reinterpret_cast<uint32_t *>(s_tab)[i] = reinterpret_cast<const uint32_t *>(g_rsqrt12)[i];
-    for (int i = threadIdx.x; i < n32 * (tc::kRowBytes / 16); i += blockDim.x)
-        reinterpret_cast<uint4 *>(s_b)[i] = reinterpret_cast<const uint4 *>(a.scene.tcb)[i];
-    for (int i = threadIdx.x; i < n32; i += blockDim.x)
-        s_exact[i] = i < a.scene.n_pad ? a.scene.exact[i] : make_float4(0, 0, 0, 0);
-    if (threadIdx.x == 0) {
-        for (int g = 0; g < 8; ++g) {
-            tc::mbar_init(&ctl.full[g][0], 1); tc::mbar_init(&ctl.full[g][1], 1);
-            ctl.arrived_a[g] = 0; ctl.arrived_e[g][0] = 0; ctl.arrived_e[g][1] = 0; ctl.exit_flag[g] = 0;
-        }
-        tc::fence_mbar_init();
-    }
-    tc::fence_proxy_async();                                     // the B tile is read by the tensor core (async proxy)
-    if (threadIdx.x < 32) tc::tmem_alloc(&ctl.tmem_base, 512);
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
-    const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t *>(&ctl.tmem_base);
-    const int nchunks = (n32 + kChunk - 1) / kChunk;
-    const unsigned lane = threadIdx.x & 31u;
-    const int g = threadIdx.x >> 7, w = (threadIdx.x >> 5) & 3, r = threadIdx.x & 127;
-    const uint16_t *tab = s_tab;
-    const unsigned lt_mask = (1u << lane) - 1u;
-    WarpPool &pool = pools[threadIdx.x >> 5];
-    unsigned char *a_tile = s_a + (size_t)g * 128 * tc::kRowBytes;
-    const uint32_t a_smem = tc::smem_u32(a_tile), b_smem = tc::smem_u32(s_b);
-    const uint32_t d_tmem = tmem_base + (uint32_t)(g * kChunk * kBufs), t_lane = d_tmem + ((uint32_t)(w * 32) << 16);
-    bool active = false, exhausted = false;
-    PoolState ps;
-    ps.dry = false; ps.ready = 0; ps.w_next = 0; ps.w_end = 0;
-    const uint32_t lanes_x = gridDim.x * blockDim.x * a.sched_div;
-    uint32_t lp = 0, it = 0, nrays = 0;
-    int depth = 0;
-    f3 thr = mk3(1, 1, 1), o = mk3(0, 0, 0), d = mk3(0, 0, 0);
-    Rng rng;
-    rng.k0 = 0; rng.k1 = 0;
-
-    for (;;) {
-        const bool want = !active && !exhausted;
-        const unsigned need = __ballot_sync(kFull, want);
-        if (need) pool_take(a, pool, ps, tab, lane, lt_mask, lanes_x, need, want, active, exhausted, o, d, lp, rng, thr, depth);
-        const bool warp_done = __all_sync(kFull, exhausted);
-
-        tc::write_ray_row(a_tile, r, o, d, active);
-        tc::fence_proxy_async();
-        tc::tc_fence_before();                                   // this warp's reads of the previous scan's last chunk are complete
-        __syncwarp();
-        if (lane == 0) {
-            const uint32_t mine = 1u + (warp_done ? 0x100u : 0u);
-            __threadfence_block();
-            const uint32_t tot = atomicAdd(&ctl.arrived_a[g], mine) + mine;
-            if ((tot & 0xffu) == 4u) {                           // last of the group: start the scan (or end the group)
-                *reinterpret_cast<volatile uint32_t *>(&ctl.arrived_a[g]) = 0u;
-                __threadfence_block();
-                if ((tot >> 8) == 4u) {
-                    *reinterpret_cast<volatile uint32_t *>(&ctl.exit_flag[g]) = 1u;
-                    __threadfence_block();
-                    tc::mbar_arrive(&ctl.full[g][it % kBufs]);
-                } else {
-                    tc::tc_fence_after();
-#pragma unroll
-                    for (int j = 0; j < kBufs; ++j)
-                        if (j < nchunks) {                       // the first kBufs chunks: every buffer is free at the start of a scan
-                            const uint32_t b = (it + j) % kBufs;
-                            tc::mma_chunk(d_tmem + b * kChunk, a_smem, b_smem + (uint32_t)j * (kChunk / 8) * tc::kSBO, min(kChunk, n32 - j * kChunk), tc::kLBO, tc::kSBO);
-                            tc::mma_commit(&ctl.full[g][b]);
-                        }
-                }
-            }
-        }
-        __syncwarp();
-
-        float t = kTMax;
-        int hit = -1;
-        bool leave = false;
-        for (int c = 0; c < nchunks; ++c, ++it) {
-            const uint32_t b = it % kBufs, t_buf = t_lane + b * kChunk;
-            tc::mbar_wait(&ctl.full[g][b], (it / kBufs) & 1u, hint);
-            if (c == 0 && *reinterpret_cast<volatile uint32_t *>(&ctl.exit_flag[g])) { leave = true; break; }
-            tc::tc_fence_after();
-            const int pieces = min(kPieces, (n32 - c * kChunk) >> 5);   // warp-uniform: the last chunk may be short
-            uint32_t cand[kPieces + 1];
-#pragma unroll
-            for (int h = 0; h < kPieces; h += 2) {               // two loads in flight, eight independent sign-gather chains
-                cand[h] = 0; cand[h + 1] = 0;
-                if (kGroups <= 5 && h + 1 < pieces) {           // (6 and 7 groups have 72 .. 80 registers: one load at a time)
-                    uint32_t v0[32], v1[32];
-                    tc::tmem_ld32_issue(t_buf + 32 * h, v0);
-                    tc::tmem_ld32_issue(t_buf + 32 * h + 32, v1);
-                    tc::tmem_wait(v0, v1);
-                    cand[h] = tc::flagged(v0);
-                    cand[h + 1] = tc::flagged(v1);
-                } else {
-                    if (h < pieces) {
-                        uint32_t v[32];
-                        tc::tmem_ld32(t_buf + 32 * h, v);
-                        cand[h] = tc::flagged(v);
-                    }
-                    if (h + 1 < pieces) {
-                        uint32_t v[32];
-                        tc::tmem_ld32(t_buf + 32 * h + 32, v);
-                        cand[h + 1] = tc::flagged(v);
-                    }
-                }
-            }
-            if (c + kBufs < nchunks) {                           // warp-uniform: this buffer is needed again in this scan
-                tc::tc_fence_before();
-                __syncwarp();
-                if (lane == 0) {
-                    __threadfence_block();
-                    if (atomicAdd(&ctl.arrived_e[g][b], 1u) == 3u) {  // last reader: the buffer is free, issue the chunk that reuses it
-                        *reinterpret_cast<volatile uint32_t *>(&ctl.arrived_e[g][b]) = 0u;
-                        __threadfence_block();
-                        tc::tc_fence_after();
-                        tc::mma_chunk(d_tmem + b * kChunk, a_smem, b_smem + (uint32_t)(c + kBufs) * (kChunk / 8) * tc::kSBO, min(kChunk, n32 - (c + kBufs) * kChunk),
-                                      tc::kLBO, tc::kSBO);
-                        tc::mma_commit(&ctl.full[g][b]);
-                    }
-                }
-                __syncwarp();
-            }
-#pragma unroll
-            for (int h = 0; h < kPieces; ++h)
-                if (cand[h]) exact_candidates(cand[h], s_exact, c * kChunk + 32 * h, o, d, kTMin, t, hit);
-        }
-        if (leave) break;
-
-        if (active) {
-            ++nrays;
-            f3 contrib;
-            const float4 e = hit >= 0 ? s_exact[hit] : make_float4(0, 0, 0, 0);
-            if (shade_step(a, hit, t, e, tab, o, d, thr, depth, rng, contrib)) {
-                accumulate_sample(a, lp, contrib);
-                active = false;
-            }
-        }
-    }
-    unsigned long long total = nrays;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
-    if (lane == 0 && total) atomicAdd(a.num_rays, total);
-    tc::tc_fence_before();
-    __syncthreads();
-    if (threadIdx.x < 32) tc::tmem_dealloc(tmem_base, 512);
-}
-
-// megakernel_tc2 with the accumulator buffers POOLED: a group holds one of the four 128-column TMEM buffers only while it scans
-// (first MMA issued ... last chunk read) and hands it back for the exact tests of the last chunk, shading, the pop and the row
-// build, so a CTA carries more ray groups (5 .. 7) than TMEM has buffers.  free_mask: bit b = buffer b is free; the last warp to
-// write its row takes a buffer (atomicAnd), the last reader of the last chunk returns it (atomicOr).
-struct TcControl3 {
-    uint64_t full[8];                 // per group: accumulator chunk complete (tcgen05.commit; the exit arrival), count 1
-    uint32_t arrived_a[8];            // per group: ray warps with their row written (low byte) / out of work (next byte)
-    uint32_t arrived_e[8];            // per group: ray warps that have read the current chunk
-    uint32_t exit_flag[8];
-    uint32_t buf_of[8];               // per group: the buffer its current scan holds
-    uint32_t free_mask;
-    uint32_t tmem_base;
-    uint32_t pad_[2];
-};
-static_assert(sizeof(TcControl3) % 16 == 0, "TcControl3 is followed by 16-byte aligned tiles");
 
 template <int kGroups>
 __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tc3(const __grid_constant__ RenderArgs a)
@@ -1078,12 +713,12 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tc3(const __grid_
     constexpr int kChunk = 128, kPool = 4;
     static_assert(kGroups >= 4 && kGroups <= 7, "bad configuration");
     constexpr int kPieces = kChunk / 32;
-    const bool hint = a.tc_flags & 1u;
+    // shared memory: [16 B | rsqrtss table 4 KB | control | B tile n32 x 128 B | exact n32 x 16 B | A tiles kGroups x 16 KB | pools]
     extern __shared__ __align__(128) unsigned char smem_raw[];
     uint16_t *s_tab = reinterpret_cast<uint16_t *>(smem_raw + 16);
     unsigned char *p = smem_raw + ((kSmemSpheres + 127) & ~127);
-    TcControl3 &ctl = *reinterpret_cast<TcControl3 *>(p);
-    p += (sizeof(TcControl3) + 127) & ~127;
+    TcControl &ctl = *reinterpret_cast<TcControl *>(p);
+    p += (sizeof(TcControl) + 127) & ~127;
     unsigned char *s_b = p;
     const int n32 = a.scene.n32;
     p += (size_t)n32 * tc::kRowBytes;
@@ -1180,7 +815,7 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tc3(const __grid_
         bool leave = false;
         uint32_t b = 0;
         for (int c = 0; c < nchunks; ++c, ++it) {
-            tc::mbar_wait(&ctl.full[g], it & 1u, hint);
+            tc::mbar_wait(&ctl.full[g], it & 1u, true);
             if (c == 0) {
                 if (*reinterpret_cast<volatile uint32_t *>(&ctl.exit_flag[g])) { leave = true; break; }
                 b = *reinterpret_cast<volatile uint32_t *>(&ctl.buf_of[g]);
@@ -1363,7 +998,6 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tcs(const __grid_
     constexpr int kChunk = kTcsChunk, kPieces = kChunk / 32;
     static_assert(kGroups >= 1 && kGroups <= 4 && kStages >= 2 && kStages <= kTcsMaxStages, "bad configuration");
     constexpr uint32_t kTmemCols = kGroups == 1 ? 128 : (kGroups == 2 ? 256 : 512);   // one 128-column accumulator per group
-    const bool hint = a.tc_flags & 1u;
     // shared memory: [16 B | rsqrtss table 4 KB | control | stages kStages x 18 KB | A tiles kGroups x 16 KB | pools]
     extern __shared__ __align__(128) unsigned char smem_raw[];
     uint16_t *s_tab = reinterpret_cast<uint16_t *>(smem_raw + 16);
@@ -1443,7 +1077,7 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tcs(const __grid_
                     tc::mbar_arrive(&ctl.mma[g]);
                 } else {
                     const int s = (int)(fpos % kStages);
-                    tc::mbar_wait(&ctl.landed[s], (fpos / kStages) & 1u, hint);
+                    tc::mbar_wait(&ctl.landed[s], (fpos / kStages) & 1u, true);
                     tc::tc_fence_after();
                     tc::mma_chunk(t_acc, a_smem, stages_smem + (uint32_t)s * kTcsStageBytes, min(kChunk, n32), tc::kLBO, tc::kSBO);
                     tc::mma_commit(&ctl.mma[g]);
@@ -1456,7 +1090,7 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tcs(const __grid_
         int hit = -1;
         bool leave = false;
         for (int c = 0; c < nchunks; ++c, ++it) {
-            tc::mbar_wait(&ctl.mma[g], it & 1u, hint);
+            tc::mbar_wait(&ctl.mma[g], it & 1u, true);
             if (c == 0 && *reinterpret_cast<volatile uint32_t *>(&ctl.exit_flag[g])) { leave = true; break; }
             const uint32_t f = fpos + (uint32_t)c;
             const int s = (int)(f % kStages);
@@ -1489,7 +1123,7 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tcs(const __grid_
                     if (c + 1 < nchunks) {
                         const uint32_t f1 = f + 1u;
                         const int s1 = (int)(f1 % kStages);
-                        tc::mbar_wait(&ctl.landed[s1], (f1 / kStages) & 1u, hint);
+                        tc::mbar_wait(&ctl.landed[s1], (f1 / kStages) & 1u, true);
                         tc::tc_fence_after();
                         tc::mma_chunk(t_acc, a_smem, stages_smem + (uint32_t)s1 * kTcsStageBytes, min(kChunk, n32 - (c + 1) * kChunk), tc::kLBO, tc::kSBO);
                         tc::mma_commit(&ctl.mma[g]);
@@ -1555,80 +1189,6 @@ __global__ void __launch_bounds__(1024, 1) tmem_read_kernel(int iters, uint32_t 
     tc::tc_fence_before();
     __syncthreads();
     if (threadIdx.x < 32) tc::tmem_dealloc(*reinterpret_cast<volatile uint32_t *>(&slot), 512);
-}
-
-// Filter values of n rays against every sphere (parity / error measurement of the tensor filter): e[ray * n32 + sphere].
-// One CTA per 128 rays: 4 ray warps + the issuing warp, the scan of megakernel_tc with kGroups = 1 and the values written out.
-constexpr int kProbeChunk = 64;
-__global__ void __launch_bounds__(160, 1) tc_filter_probe_kernel(DevScene sc, int n, const float *__restrict__ org, const float *__restrict__ dir, float *__restrict__ e_out,
-                                                               uint32_t lbo, uint32_t sbo)
-{
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    TcControl &ctl = *reinterpret_cast<TcControl *>(smem_raw);
-    unsigned char *s_b = smem_raw + ((sizeof(TcControl) + 127) & ~127);
-    const int n32 = sc.n32;
-    unsigned char *a_tile = s_b + (size_t)n32 * tc::kRowBytes;
-    for (int i = threadIdx.x; i < n32 * (tc::kRowBytes / 16); i += blockDim.x)
-        reinterpret_cast<uint4 *>(s_b)[i] = reinterpret_cast<const uint4 *>(sc.tcb)[i];
-    if (threadIdx.x == 0) {
-        tc::mbar_init(&ctl.a_full[0], 4);
-        for (int b = 0; b < 2; ++b) { tc::mbar_init(&ctl.full[0][b], 1); tc::mbar_init(&ctl.empty[0][b], 4); }
-        tc::fence_mbar_init();
-    }
-    tc::fence_proxy_async();
-    if (threadIdx.x < 32) tc::tmem_alloc(&ctl.tmem_base, 128);
-    tc::tc_fence_before();
-    __syncthreads();
-    tc::tc_fence_after();
-    const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t *>(&ctl.tmem_base);
-    const int nchunks = (n32 + kProbeChunk - 1) / kProbeChunk;
-    const unsigned lane = threadIdx.x & 31u;
-    if (threadIdx.x >= 128) {
-        if (lane == 0) {
-            tc::mbar_wait(&ctl.a_full[0], 0);
-            tc::tc_fence_after();
-            uint32_t it = 0;
-            for (int c = 0; c < nchunks; ++c, ++it) {
-                const uint32_t b = it & 1u;
-                tc::mbar_wait(&ctl.empty[0][b], ((it >> 1) & 1u) ^ 1u);
-                tc::tc_fence_after();
-                const int nn = min(kProbeChunk, n32 - c * kProbeChunk);
-                tc::mma_chunk(tmem_base + b * kProbeChunk, tc::smem_u32(a_tile), tc::smem_u32(s_b) + (uint32_t)c * (kProbeChunk / 8) * tc::kSBO, nn, lbo, sbo);
-                tc::mma_commit(&ctl.full[0][b]);
-            }
-        }
-    } else {
-        const int r = threadIdx.x, w = threadIdx.x >> 5;
-        const int ray = blockIdx.x * 128 + r;
-        const bool live = ray < n;
-        f3 o = mk3(0, 0, 0), d = mk3(0, 0, 0);
-        if (live) { o = mk3(org[3 * ray], org[3 * ray + 1], org[3 * ray + 2]); d = mk3(dir[3 * ray], dir[3 * ray + 1], dir[3 * ray + 2]); }
-        tc::write_ray_row(a_tile, r, o, d, live);
-        tc::fence_proxy_async();
-        __syncwarp();
-        if (lane == 0) tc::mbar_arrive(&ctl.a_full[0]);
-        const uint32_t t_lane = tmem_base + ((uint32_t)(w * 32) << 16);
-        uint32_t it = 0;
-        for (int c = 0; c < nchunks; ++c, ++it) {
-            const uint32_t b = it & 1u;
-            tc::mbar_wait(&ctl.full[0][b], (it >> 1) & 1u);
-            tc::tc_fence_after();
-            const int halves = n32 - c * kProbeChunk > 32 ? 2 : 1;
-            for (int h = 0; h < halves; ++h) {
-                uint32_t v[32];
-                tc::tmem_ld32(t_lane + b * kProbeChunk + 32 * h, v);
-                if (live)
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) e_out[(size_t)ray * n32 + c * kProbeChunk + 32 * h + j] = __uint_as_float(v[j]);
-            }
-            tc::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) tc::mbar_arrive(&ctl.empty[0][b]);
-        }
-    }
-    tc::tc_fence_before();
-    __syncthreads();
-    if (threadIdx.x < 32) tc::tmem_dealloc(tmem_base, 128);
 }
 
 // ------------------------------------------------------------------------------------------------ resolve
@@ -1773,6 +1333,62 @@ __global__ void __launch_bounds__(128, 1) trace_rays_tc_kernel(const __grid_cons
     t_out[k] = hit >= 0 ? t : 0.0f;
     p_out[3 * k] = p.x; p_out[3 * k + 1] = p.y; p_out[3 * k + 2] = p.z;
     n_out[3 * k] = nrm.x; n_out[3 * k + 1] = nrm.y; n_out[3 * k + 2] = nrm.z;
+}
+
+// Filter values of n rays against every sphere (parity / error measurement of the tensor filter): e[ray * n32 + sphere].
+// The MMA chunks of trace_rays_tc_kernel -- 128 spheres with the per-chunk N into one 128-column accumulator, issued by
+// thread 0 -- with the raw values written out instead of tested.
+constexpr size_t filter_probe_smem_bytes(int n32) { return 128 + (size_t)n32 * tc::kRowBytes + 128 * tc::kRowBytes; }
+__global__ void __launch_bounds__(128, 1) tc_filter_probe_kernel(const __grid_constant__ DevScene sc, int n, const float *__restrict__ org,
+                                                               const float *__restrict__ dir, float *__restrict__ e_out)
+{
+    constexpr int kChunk = kTraceTcChunk;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw);      // [mbarrier | TMEM address | pad to 128 | B | A]
+    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(smem_raw + 8);
+    const int n32 = sc.n32;
+    unsigned char *s_b = smem_raw + 128;
+    unsigned char *a_tile = s_b + (size_t)n32 * tc::kRowBytes;
+    for (int i = threadIdx.x; i < n32 * (tc::kRowBytes / 16); i += blockDim.x)
+        reinterpret_cast<uint4 *>(s_b)[i] = reinterpret_cast<const uint4 *>(sc.tcb)[i];
+    if (threadIdx.x == 0) {
+        tc::mbar_init(full, 1);
+        tc::fence_mbar_init();
+    }
+    const int ray = blockIdx.x * 128 + threadIdx.x;
+    const bool live = ray < n;                                   // rays past n write a row that flags nothing
+    f3 o = mk3(0, 0, 0), d = mk3(0, 0, 0);
+    if (live) { o = mk3(org[3 * ray], org[3 * ray + 1], org[3 * ray + 2]); d = mk3(dir[3 * ray], dir[3 * ray + 1], dir[3 * ray + 2]); }
+    tc::write_ray_row(a_tile, threadIdx.x, o, d, live);
+    tc::fence_proxy_async();                                     // the tiles are read by the tensor core (async proxy)
+    if (threadIdx.x < 32) tc::tmem_alloc(tmem_slot, kChunk);
+    tc::tc_fence_before();
+    __syncthreads();
+    tc::tc_fence_after();
+    const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t *>(tmem_slot);
+    const uint32_t t_lane = tmem_base + ((uint32_t)((threadIdx.x >> 5) * 32) << 16);
+    const uint32_t a_smem = tc::smem_u32(a_tile), b_smem = tc::smem_u32(s_b);
+    const int nchunks = (n32 + kChunk - 1) / kChunk;
+    for (int c = 0; c < nchunks; ++c) {
+        if (threadIdx.x == 0) {
+            tc::tc_fence_after();
+            tc::mma_chunk(tmem_base, a_smem, b_smem + (uint32_t)c * (kChunk / 8) * tc::kSBO, min(kChunk, n32 - c * kChunk), tc::kLBO, tc::kSBO);
+            tc::mma_commit(full);
+        }
+        tc::mbar_wait(full, (uint32_t)c & 1u);
+        tc::tc_fence_after();
+        const int pieces = min(kChunk / 32, (n32 - c * kChunk) >> 5);   // the last chunk may be short
+        for (int h = 0; h < pieces; ++h) {
+            uint32_t v[32];
+            tc::tmem_ld32(t_lane + 32 * h, v);
+            if (live)
+#pragma unroll
+                for (int j = 0; j < 32; ++j) e_out[(size_t)ray * n32 + c * kChunk + 32 * h + j] = __uint_as_float(v[j]);
+        }
+        tc::tc_fence_before();
+        __syncthreads();                                         // every warp has read the buffer: the next chunk may overwrite it
+    }
+    if (threadIdx.x < 32) tc::tmem_dealloc(tmem_base, kChunk);
 }
 
 // Hitable::hit through the filter of megakernel_tcs at any scene size: the chunks stream through a ring of two stages filled by

@@ -6,7 +6,7 @@
 // sphere vector, n = -c:
 //     sphere:  nx^2  ny^2  nz^2  nx ny  nx nz  ny nz   nx  ny  nz   kk   1          kk = |c|^2 - r^2 - margin_s
 //     ray:     dx^2  dy^2  dz^2  2dxdy  2dxdz  2dydz   2 (o.d d - o)    -1   (o.d)^2 - |o|^2 (1 - margin_r)
-// i.e. a GEMM  E[rays x spheres] = R[rays x 11] S^T  -- 128 rays x 64 spheres per tcgen05.mma.  TF32 operands carry 11
+// i.e. a GEMM  E[rays x spheres] = R[rays x 11] S^T  -- 128 rays x 128 spheres per tcgen05.mma.  TF32 operands carry 11
 // significant bits, so every feature is split  x = hi + lo  (both TF32) and the three products hi hi + lo hi + hi lo go into
 // the K dimension:  K = 11 + 11 + 10 = 32 (the constant sphere feature has no low part) = four K = 8 instructions.
 // Per test the CUDA cores are left with ONE instruction (the sign bit of e into the candidate mask) instead of eight packed FMA.
@@ -126,13 +126,6 @@ __device__ __forceinline__ void mma_tf32(uint32_t d_tmem, uint64_t adesc, uint64
                  "r"(idesc), "r"(accumulate)
                  : "memory");
 }
-// the same with the A operand in tensor memory (128 lanes x 8 columns per K step)
-__device__ __forceinline__ void mma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
-{
-    asm volatile("{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n}" ::"r"(d_tmem), "r"(a_tmem), "l"(bdesc),
-                 "r"(idesc), "r"(accumulate)
-                 : "memory");
-}
 __device__ __forceinline__ void mma_commit(uint64_t *bar) { asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory"); }
 
 // 32 consecutive columns of this thread's TMEM lane (warp w reads lanes 32 (w % 4) .. +31), complete on return
@@ -169,25 +162,7 @@ __device__ __forceinline__ void tmem_wait(uint32_t (&a)[32], uint32_t (&b)[32])
                  :
                  : "memory");
 }
-// 32 consecutive columns of this thread's TMEM lane, written (complete on return)
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t (&v)[32])
-{
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, %17, %18, %19, %20, %21, %22, %23, "
-                 "%24, %25, %26, %27, %28, %29, %30, %31, %32};" ::"r"(taddr),
-                 "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]),
-                 "r"(v[13]), "r"(v[14]), "r"(v[15]), "r"(v[16]), "r"(v[17]), "r"(v[18]), "r"(v[19]), "r"(v[20]), "r"(v[21]), "r"(v[22]), "r"(v[23]), "r"(v[24]),
-                 "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31])
-                 : "memory");
-    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-}
 // sign bits of 32 filter values into a candidate mask: first sphere -> bit 31, set = flagged (e >= 0)
-__device__ __forceinline__ uint32_t flagged_chain(const uint32_t (&v)[32])      // one chain of 32 funnel shifts
-{
-    uint32_t neg = 0;
-#pragma unroll
-    for (int j = 0; j < 32; ++j) neg = __funnelshift_l(v[j], neg, 1);
-    return ~neg;
-}
 __device__ __forceinline__ uint32_t flagged(const uint32_t (&v)[32])
 {
     // four independent funnel-shift chains of 8 (one chain of 32 is a 32-deep dependency)
@@ -250,13 +225,6 @@ __device__ __forceinline__ void mma_chunk(uint32_t d_tmem, uint32_t a_smem, uint
 #pragma unroll
     for (int k = 0; k < kK / 8; ++k)
         mma_tf32(d_tmem, smem_desc(a_smem + 2 * k * kLBO, lbo, sbo), smem_desc(b_smem + 2 * k * kLBO, lbo, sbo), idesc, k > 0);
-}
-// the same with A in tensor memory: row r = lane r, k = column a_tmem + k
-__device__ __forceinline__ void mma_chunk_ts(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_smem, int n)
-{
-    const uint32_t idesc = instr_desc(n);
-#pragma unroll
-    for (int k = 0; k < kK / 8; ++k) mma_tf32_ts(d_tmem, a_tmem + 8 * k, smem_desc(b_smem + 2 * k * kLBO, kLBO, kSBO), idesc, k > 0);
 }
 #endif  // __CUDACC__
 

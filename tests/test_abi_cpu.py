@@ -175,6 +175,18 @@ def test_no_cpu_fallback_without_a_gpu(r1):
     s.close()
 
 
+@pytest.mark.parametrize("layout", (1, -1, 2))
+def test_filter_probe_refuses_layouts_other_than_0(r1, layout):
+    """r1_filter_probe reads the operand in the renderer's layout only: any other `layout` is R1_ERR_ARG before the device is
+    looked at (this scene is not even committed)"""
+    s = r1.create_scene("small", commit=False)
+    try:
+        with pytest.raises(r1.Rays1Error, match=r"\(-1\).*layout"):
+            s.filter_probe(np.zeros((1, 3)), np.array([[0, 0, 1.0]]), 1, layout=layout)
+    finally:
+        s.close()
+
+
 @pytest.mark.parametrize("height,row_tile,world", [(720, 8, 1), (720, 8, 2), (720, 8, 8), (2160, 8, 8), (37, 8, 4), (5, 8, 8), (100, 3, 7)])
 def test_row_tile_partition_is_a_partition(r1, height, row_tile, world):
     seen = []

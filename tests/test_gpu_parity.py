@@ -204,41 +204,14 @@ def test_tensor_filter_is_conservative(r1, scenes, name):
     record("tensor_filter_flag_ratio_%s" % name, float(flagged.sum() / max(1, ((discr >= 0) & real[None, :]).sum())))
 
 
-def test_tensor_variant_renders_the_same_bytes(r1, scenes, monkeypatch):
-    """same hits, same bytes: the tensor-core filter only decides which spheres get the exact test.  Every TMEM pipeline
-    configuration (ray threads; R1_TC_CFG = columns per accumulator buffer, buffers per group, ray operand in TMEM)."""
-    cfgs = ((512, None), (512, "64,2,0"), (512, "96,1,1"), (512, "32,3,1"), (384, "128,1,0"), (384, "64,2,0"), (384, "128,1,1"), (384, "64,2,1"),
-            (256, "128,2,0"), (256, "256,1,0"), (256, "96,2,1"), (256, "224,1,1"))
+def test_tensor_renders_the_same_bytes_at_every_group_count(r1, scenes):
+    """same hits, same bytes: the tensor-core filter only decides which spheres get the exact test.  r1::megakernel_tc3 at the
+    default and at every group count it builds (threads = 128 x groups), on four frames; rank shares; the shared-memory limit."""
     for name, (w, h, spp) in (("large", (200, 117, 40)), ("medium", (160, 90, 16)), ("small", (64, 36, 8)), ("large", (7, 3, 5))):
         base, r0 = scenes[name].render(w, h, spp, variant=r1.VARIANT_MEGAKERNEL_PACKED)
-        monkeypatch.setenv("R1_TC1", "1")                        # r1::megakernel_tc: one MMA-issuing warp per group
-        for threads, cfg in cfgs:
-            if cfg:
-                monkeypatch.setenv("R1_TC_CFG", cfg)
-            else:
-                monkeypatch.delenv("R1_TC_CFG", raising=False)
-            alt, ra = scenes[name].render(w, h, spp, variant=r1.VARIANT_MEGAKERNEL_TENSOR, threads=threads)
-            assert np.array_equal(base, alt) and ra.num_rays == r0.num_rays, (name, threads, cfg)
-    monkeypatch.delenv("R1_TC_CFG", raising=False)
-    monkeypatch.delenv("R1_TC1", raising=False)
-    for groups, bufs in (("4", "1"), ("5", "1"), ("6", "1"), ("7", "1"), ("4", "2"), ("3", "2")):
-        # r1::megakernel_tc2: the last ray warp to arrive issues the MMA; ray groups per CTA, accumulator buffers owned by each group
-        monkeypatch.setenv("R1_TC2_BUFS", bufs)
-        monkeypatch.setenv("R1_TC2", groups)
-        for name, (w, h, spp) in (("large", (200, 117, 40)), ("medium", (160, 90, 16)), ("small", (64, 36, 8)), ("large", (7, 3, 5))):
-            base, r0 = scenes[name].render(w, h, spp, variant=r1.VARIANT_MEGAKERNEL_PACKED)
-            alt, ra = scenes[name].render(w, h, spp, variant=r1.VARIANT_MEGAKERNEL_TENSOR)
-            assert np.array_equal(base, alt) and ra.num_rays == r0.num_rays, (name, "tc2", groups, bufs)
-    monkeypatch.delenv("R1_TC2", raising=False)
-    monkeypatch.delenv("R1_TC2_BUFS", raising=False)
-    for groups in (None, "4", "5", "6", "7"):                    # r1::megakernel_tc3 (default): accumulator buffers pooled among the groups
-        if groups:
-            monkeypatch.setenv("R1_TC3", groups)
-        for name, (w, h, spp) in (("large", (200, 117, 40)), ("medium", (160, 90, 16)), ("small", (64, 36, 8)), ("large", (7, 3, 5))):
-            base, r0 = scenes[name].render(w, h, spp, variant=r1.VARIANT_MEGAKERNEL_PACKED)
-            alt, ra = scenes[name].render(w, h, spp, variant=r1.VARIANT_MEGAKERNEL_TENSOR)
+        for groups in (None, 4, 5, 6, 7):                        # accumulator buffers pooled among the groups
+            alt, ra = scenes[name].render(w, h, spp, variant=r1.VARIANT_MEGAKERNEL_TENSOR, threads=128 * groups if groups else 0)
             assert np.array_equal(base, alt) and ra.num_rays == r0.num_rays, (name, "tc3", groups)
-    monkeypatch.delenv("R1_TC3", raising=False)
     for world in (2, 3):
         parts = [scenes["large"].render(200, 117, 40, rank=r, world=world, variant=r1.VARIANT_MEGAKERNEL_TENSOR)[0] for r in range(world)]
         whole, _ = scenes["large"].render(200, 117, 40, variant=r1.VARIANT_MEGAKERNEL_PACKED)

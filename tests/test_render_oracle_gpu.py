@@ -220,7 +220,7 @@ def variant_runs(r1):
     for st in (2, 3, 4):
         runs["stream_stages%d" % st] = (V.VARIANT_MEGAKERNEL_TENSOR_STREAM, 512, 0, {"R1_TCS_STAGES": str(st)})
     for g in (4, 5, 6, 7):
-        runs["tc3_%dg" % g] = (V.VARIANT_MEGAKERNEL_TENSOR, 0, 0, {"R1_TC3": str(g)})
+        runs["tc3_%dg" % g] = (V.VARIANT_MEGAKERNEL_TENSOR, 128 * g, 0, {})
     return runs
 
 

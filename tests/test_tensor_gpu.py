@@ -42,7 +42,7 @@ SMEM_LIMIT = 227 * 1024
 
 
 def tc3_smem_bytes(groups, n32):
-    """r1::tc2_smem_bytes, which launch_megakernel_tc3_t checks: the rsqrt table, control, B tile and exact spheres (144 bytes
+    """r1::tc3_smem_bytes, which launch_megakernel_tc3_t checks: the rsqrt table, control, B tile and exact spheres (144 bytes
     per sphere), and per ray group the A tile (16 KB) and four warp pools (4 x 1152 bytes)"""
     return (16 + 2048 * 2) + 256 + n32 * (128 + 16) + groups * (128 * 128 + 4 * 1152) + 256
 
@@ -157,29 +157,25 @@ def fits(groups, n32):
 
 
 @pytest.mark.parametrize("grid", TENSOR, ids=["%dx%d" % g for g in TENSOR])
-def test_tensor_renders_like_packed_for_every_group_count(r1, sweep, monkeypatch, grid):
-    """variant TENSOR (tc3) against PACKED, byte for byte and ray for ray, with 4 .. 7 ray groups per CTA, on a frame, on a
-    7x3 image (fewer samples than one group has lanes) and as rank 1 of 3.  A group count whose shared memory does not fit
-    the scene is refused with R1_ERR_LIMIT -- exactly those -- and leaves nothing behind: the next render works."""
+def test_tensor_group_counts_render_like_packed(r1, sweep, grid):
+    """variant TENSOR (tc3) against PACKED, byte for byte and ray for ray, with 4 .. 7 ray groups per CTA (threads = 128 x groups),
+    on a frame, on a 7x3 image (fewer samples than one group has lanes) and as rank 1 of 3.  A group count whose shared memory
+    does not fit the scene is refused with R1_ERR_LIMIT -- exactly those -- and leaves nothing behind: the next render works."""
     s = sweep[grid]
     n32 = GRIDS[grid][1]
     cases = ((96, 54, 8, 0, 1), (7, 3, 5, 0, 1), (96, 54, 8, 1, 3))
     base = {c: s.render(c[0], c[1], c[2], rank=c[3], world=c[4], variant=r1.VARIANT_MEGAKERNEL_PACKED) for c in cases}
     assert base[cases[0]][0].any()
-    for groups in (None, "4", "6", "7"):
-        if groups:
-            monkeypatch.setenv("R1_TC3", groups)
-        else:
-            monkeypatch.delenv("R1_TC3", raising=False)
-        g = int(groups or 5)
+    for groups in (None, 4, 6, 7):
+        threads = 128 * groups if groups else 0
+        g = groups or 5
         for c in cases:
             if not fits(g, n32):
                 with pytest.raises(r1.Rays1Error, match=r"\(-4\).*shared memory"):
-                    s.render(c[0], c[1], c[2], rank=c[3], world=c[4], variant=r1.VARIANT_MEGAKERNEL_TENSOR)
+                    s.render(c[0], c[1], c[2], rank=c[3], world=c[4], variant=r1.VARIANT_MEGAKERNEL_TENSOR, threads=threads)
                 continue
-            rgb, res = s.render(c[0], c[1], c[2], rank=c[3], world=c[4], variant=r1.VARIANT_MEGAKERNEL_TENSOR)
+            rgb, res = s.render(c[0], c[1], c[2], rank=c[3], world=c[4], variant=r1.VARIANT_MEGAKERNEL_TENSOR, threads=threads)
             assert np.array_equal(rgb, base[c][0]) and res.num_rays == base[c][1].num_rays, (grid, groups, c)
-    monkeypatch.delenv("R1_TC3", raising=False)
     rgb, res = s.render(96, 54, 8, variant=r1.VARIANT_MEGAKERNEL_TENSOR)   # after any refusal: no sticky error
     assert np.array_equal(rgb, base[cases[0]][0]) and res.num_rays == base[cases[0]][1].num_rays
     whole = base[cases[0]][0]
@@ -196,3 +192,18 @@ def test_above_768_spheres_tensor_is_refused_and_default_is_packed(r1, sweep):
     base, r0 = s.render(96, 54, 8, variant=r1.VARIANT_MEGAKERNEL_PACKED)
     rgb, res = s.render(96, 54, 8)
     assert np.array_equal(rgb, base) and res.num_rays == r0.num_rays and base.any()
+
+
+def test_tensor_has_one_render_kernel_whatever_the_environment(r1, monkeypatch):
+    """R1_TC1, R1_TC2, R1_TC_FLAGS and R1_TC3 are not tuning knobs of this library: with them set, TENSOR still names
+    megakernel_tc3, and a render of the large scene is the same bytes and rays as without them."""
+    s = r1.create_large_scene()
+    try:
+        base, r0 = s.render(7, 3, 5, variant=r1.VARIANT_MEGAKERNEL_TENSOR)
+        for key, value in (("R1_TC1", "1"), ("R1_TC2", "4"), ("R1_TC_FLAGS", "2"), ("R1_TC3", "4")):
+            monkeypatch.setenv(key, value)
+        assert r1.lib.r1_kernel_name(s.handle, r1.VARIANT_MEGAKERNEL_TENSOR).decode() == "megakernel_tc3"
+        rgb, res = s.render(7, 3, 5, variant=r1.VARIANT_MEGAKERNEL_TENSOR)
+        assert np.array_equal(rgb, base) and res.num_rays == r0.num_rays
+    finally:
+        s.close()
