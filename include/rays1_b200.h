@@ -52,9 +52,15 @@ enum {
     R1_VARIANT_MEGAKERNEL_PACKED = 7,  /* persistent threads, per-lane path state machine, per-lane packed f32x2 (FFMA2) filter */
     /* 8 stays unassigned: callers built against earlier versions of this header may rely on it being refused as an unknown
        variant (R1_ERR_ARG), and the ABI tests use it as their example of one. */
-    R1_VARIANT_MEGAKERNEL_TENSOR_STREAM = 9 /* the filter of R1_VARIANT_MEGAKERNEL_TENSOR with the sphere operand streamed through a
+    R1_VARIANT_MEGAKERNEL_TENSOR_STREAM = 9, /* the filter of R1_VARIANT_MEGAKERNEL_TENSOR with the sphere operand streamed through a
                                                ring of 128-sphere chunks in shared memory, shared by the CTA's ray groups: scenes of
                                                any size; threads / 128 = ray groups (1 .. 4, default 4) */
+    /* 10 stays unassigned as well (tests use it as an unknown variant). */
+    R1_VARIANT_MEGAKERNEL_BVH = 11 /* persistent threads, per-lane path state machine, nearest hit by a per-lane stack traversal of a
+                                      binned-SAH BVH2 (leaves of <= 4 spheres, boxes widened per ray so that no sphere the exact test
+                                      accepts is skipped): scenes of any size, same bytes as every other variant.  The tree is built
+                                      on the host and uploaded on the first BVH render or trace on a device: that call's
+                                      elapsed_seconds includes it, its kernel_ms does not.  threads: 512, 768 or 1024 (default) */
 };
 
 typedef struct r1_scene r1_scene; /* opaque: host SoA + per-device buffers */
@@ -148,14 +154,15 @@ int r1_deinterleave_rows(int device, const void *d_gathered, uint64_t stride, vo
 /* Hitable::hit (rayweek1.cpp:152-339); index = -1 on a miss.  dir must be unit length (Ray ctor, :104-108).  `variant` picks
  * the filter: R1_VARIANT_MEGAKERNEL resolves as in r1_render; SCALAR, COOP, DEFERRED and PACKED run that kernel's scan;
  * TENSOR runs the filter of megakernel_tc3 (128-sphere accumulator chunks, the short last chunk included) and returns
- * R1_ERR_LIMIT above 768 spheres; TENSOR_STREAM runs the streamed filter of megakernel_tcs at any sphere count, while every
- * other variant returns R1_ERR_LIMIT above 4096 (they stage the scene in shared memory); WAVEFRONT and DUAL have no per-ray
+ * R1_ERR_LIMIT above 768 spheres; TENSOR_STREAM runs the streamed filter of megakernel_tcs and BVH the BVH traversal of
+ * megakernel_bvh at any sphere count, while every other variant returns R1_ERR_LIMIT above 4096 (they stage the scene in shared memory); WAVEFRONT and DUAL have no per-ray
  * kernel and return R1_ERR_ARG.  t_min must be >= 2^-24
  * (renders use 0.001): below it the exact test's floored square root and the unsigned root keys of COOP and DEFERRED can differ
  * from Hitable::hit, so a smaller t_min or a NaN returns R1_ERR_ARG before any device is touched. */
 int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, float t_min, float t_max, int variant,
                   int32_t *index, float *t, float *p, float *normal);
-/* Name of the trace kernel `variant` resolves to for this scene with default tuning ("megakernel_tc3", "megakernel_tcs", "megakernel_pool", ...);
+/* Name of the trace kernel `variant` resolves to for this scene with default tuning ("megakernel_tc3", "megakernel_tcs", "megakernel_bvh",
+ * "megakernel_pool", ...);
  * static storage. */
 const char *r1_kernel_name(r1_scene *scene, int variant);
 /* Host only (no device needed): the sphere operand of the tensor-core filter for this scene -- n32 rows (sphere count padded to
@@ -163,6 +170,14 @@ const char *r1_kernel_name(r1_scene *scene, int variant);
  * layout, byte offset of (row r, word k) = (r / 8) * 1024 + (k / 4) * 128 + (r % 8) * 16 + (k % 4) * 4.  out = NULL: only
  * *n32_out is set.  R1_ERR_LIMIT for empty scenes and above 768 spheres. */
 int r1_tensor_operand(const r1_scene *scene, void *out, uint64_t out_bytes, uint32_t *n32_out);
+/* Host only (no device needed): the BVH of R1_VARIANT_MEGAKERNEL_BVH for this scene, built now if it is not cached yet (adding
+ * spheres drops the cached tree).  nodes: n_nodes x 64 bytes {float lo0[3], hi0[3], lo1[3], hi1[3]; int32 child[2]; float diag[2]},
+ * node 0 = root; child >= 0: inner node, child < 0: leaf with ~child = first record << 3 | count (1 .. 4), child = -1: none;
+ * diag = bound on the box's diagonal.  leaves: n_leaf_records x 32 bytes {float cx, cy, cz, radius_sq (the scene's values); int32
+ * sphere index; 3 x 0}, ascending index within a leaf.  Spheres with inv_radius == 0 are not in the tree.  depth = deepest inner
+ * node (root = 1), at most 64.  A NULL buffer skips that copy (the counts are still returned). */
+int r1_bvh_export(const r1_scene *scene, void *nodes, uint64_t nodes_bytes, void *leaves, uint64_t leaves_bytes, uint32_t *n_nodes,
+                  uint32_t *n_leaf_records, uint32_t *depth);
 /* Values of the tensor-core FILTER (R1_VARIANT_MEGAKERNEL_TENSOR) for n rays against every sphere: e[ray * n32 + sphere], n32 =
  * sphere count padded to 32; the filter flags a sphere iff the sign bit of e is clear, and must flag every sphere Hitable::hit's
  * discriminant test (rayweek1.cpp:192-204) accepts.  layout must be 0 (the renderer's operand layout); any other value returns

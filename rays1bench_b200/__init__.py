@@ -17,9 +17,10 @@ EXE_PATH = os.path.join(_HERE, "rays1_b200")
 
 VARIANT_MEGAKERNEL, VARIANT_WAVEFRONT, VARIANT_MEGAKERNEL_SCALAR, VARIANT_MEGAKERNEL_COOP, VARIANT_MEGAKERNEL_DEFERRED, VARIANT_MEGAKERNEL_DUAL, VARIANT_MEGAKERNEL_TENSOR, VARIANT_MEGAKERNEL_PACKED = 0, 1, 2, 3, 4, 5, 6, 7
 VARIANT_MEGAKERNEL_TENSOR_STREAM = 9   # 8 stays unassigned (include/rays1_b200.h)
+VARIANT_MEGAKERNEL_BVH = 11            # 10 stays unassigned
 VARIANTS = {"mega": VARIANT_MEGAKERNEL, "wavefront": VARIANT_WAVEFRONT, "scalar": VARIANT_MEGAKERNEL_SCALAR, "coop": VARIANT_MEGAKERNEL_COOP,
             "deferred": VARIANT_MEGAKERNEL_DEFERRED, "dual": VARIANT_MEGAKERNEL_DUAL, "tensor": VARIANT_MEGAKERNEL_TENSOR, "packed": VARIANT_MEGAKERNEL_PACKED,
-            "tensor_stream": VARIANT_MEGAKERNEL_TENSOR_STREAM}
+            "tensor_stream": VARIANT_MEGAKERNEL_TENSOR_STREAM, "bvh": VARIANT_MEGAKERNEL_BVH}
 MAT_NONE, MAT_LAMBERT, MAT_METAL, MAT_DIELECTRIC = -1, 0, 1, 2
 
 # the reference's compile-time workload (src/common/common.h:18-25)
@@ -29,6 +30,12 @@ DEFAULT_ROW_TILE = 1  # rows per interleaved tile of the multi-GPU partition (li
 
 class Rays1Error(RuntimeError):
     pass
+
+
+# r1_bvh_export's records (include/rays1_b200.h)
+BVH_NODE = np.dtype([("lo0", "<f4", 3), ("hi0", "<f4", 3), ("lo1", "<f4", 3), ("hi1", "<f4", 3), ("child", "<i4", 2), ("diag", "<f4", 2)])
+BVH_LEAF = np.dtype([("exact", "<f4", 4), ("index", "<i4"), ("pad", "<i4", 3)])
+BVH_MAX_DEPTH = 64
 
 
 class Result(C.Structure):
@@ -82,6 +89,7 @@ def _load():
         "r1_trace_rays": (ci, [vp, ci, f32p, f32p, cf, cf, ci, i32p, f32p, f32p, f32p]),
         "r1_filter_probe": (ci, [vp, ci, f32p, f32p, ci, f32p]),
         "r1_tensor_operand": (ci, [vp, u8p, C.c_uint64, C.POINTER(C.c_uint32)]),
+        "r1_bvh_export": (ci, [vp, vp, C.c_uint64, vp, C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
         "r1_scatter": (ci, [vp, ci, f32p, f32p, f32p, i32p, f32p, f32p, i32p, f32p, f32p]),
         "r1_get_ray": (ci, [vp, ci, f32p, f32p, f32p, f32p, f32p]),
         "r1_replay_pixels": (ci, [vp, ci, i32p, ci, ci, ci, ci, u32p, u32p, f32p, u32p]),
@@ -234,6 +242,18 @@ class Scene:
         r, k = np.meshgrid(np.arange(n32.value), np.arange(32), indexing="ij")
         off = (r // 8) * 1024 + (k // 4) * 128 + (r % 8) * 16 + (k % 4) * 4
         return raw.view(np.float32)[off // 4]
+
+    def bvh(self):
+        """r1_bvh_export (host only): the BVH of the bvh variant as numpy arrays.  Returns (nodes, leaves, depth): nodes a structured
+        array of lo0, hi0, lo1, hi1 (float32 x 3), child (int32 x 2; < 0: leaf ~child = first << 3 | count, -1: none) and diag
+        (float32 x 2); leaves a structured array of exact (float32 x 4, the scene's cx, cy, cz, radius_sq) and index (int32)."""
+        nn, nl, depth = C.c_uint32(0), C.c_uint32(0), C.c_uint32(0)
+        _check(lib.r1_bvh_export(self.handle, None, 0, None, 0, C.byref(nn), C.byref(nl), C.byref(depth)), "r1_bvh_export")
+        nodes = np.zeros(nn.value, BVH_NODE)
+        leaves = np.zeros(nl.value, BVH_LEAF)
+        _check(lib.r1_bvh_export(self.handle, nodes.ctypes.data, nodes.nbytes, leaves.ctypes.data if nl.value else None, leaves.nbytes,
+                                 C.byref(nn), C.byref(nl), C.byref(depth)), "r1_bvh_export")
+        return nodes, leaves, int(depth.value)
 
     def filter_probe(self, org, dir_, n_spheres, layout=0):
         """r1_filter_probe: values of the tensor-core filter, shape (rays, n32); sign bit clear = sphere flagged."""

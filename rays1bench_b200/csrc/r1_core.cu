@@ -3,6 +3,7 @@
 // returns R1_ERR_CUDA if the CUDA runtime reports an error (including "no device").
 // file:line citations are relative to /root/reference/.
 #include "../../include/rays1_b200.h"
+#include "r1_bvh.h"
 #include "r1_internal.h"
 #include "r1_kernels.cuh"
 #include "r1_wavefront.cuh"
@@ -15,6 +16,7 @@
 #include <cstring>
 #include <limits>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -37,6 +39,9 @@ struct DeviceCtx {
     void *block = nullptr;
     size_t block_bytes = 0;
     r1::DevScene dev;
+    uint64_t generation = 0;            // r1_scene::generation at the commit
+    void *bvh_block = nullptr;          // R1_VARIANT_MEGAKERNEL_BVH: [nodes | leaf records], uploaded on first use
+    const float4 *bvh_nodes = nullptr, *bvh_leaves = nullptr;
 };
 
 // Per-device scratch shared by every scene of the process (pixel accumulators, counters, staging, events).
@@ -87,6 +92,8 @@ struct r1_scene {
     bool have_camera = false;
     std::map<int, DeviceCtx> ctx;
     int current = -1;  // device of the last commit
+    std::unique_ptr<r1::bvh::Bvh> bvh;  // R1_VARIANT_MEGAKERNEL_BVH: built on first need, dropped when the spheres change
+    uint64_t generation = 0;            // counts changes to the spheres
 };
 
 namespace {
@@ -96,6 +103,10 @@ constexpr size_t kSceneBlockCache = 4;   // blocks kept per device (<= 4 x 260 K
 void free_ctx(DeviceCtx &c)
 {
     if (c.device < 0) return;
+    if (c.bvh_block) {
+        cudaSetDevice(c.device);
+        cudaFree(c.bvh_block);
+    }
     bool kept = false;
     {
         std::lock_guard<std::mutex> lock(g_scratch_mutex);
@@ -352,6 +363,63 @@ int launch_megakernel(int sm_count, const r1::RenderArgs &args, const r1_render_
     return fail(R1_ERR_ARG, "threads must be 512, 768 or 1024 (got %d)", threads);
 }
 
+// BVH traversal (megakernel_pool<kScanBvh>, R1_VARIANT_MEGAKERNEL_BVH): nothing is staged, every CTA shape runs the sample pool
+// (R1_POOL=0 does not apply).  Measured at 640x360x32 (B200, DESIGN.md section 4.8), Mrays/s for 512 / 768 / 1024 threads: large
+// 7143 / 8264 / 8531, 10^5-sphere cloud 527 / 705 / 789, 10^5-sphere grid 2603 / 3331 / 3565.  Samples per atomic (sched_kmax x 32,
+// shrinking by sched_div) at 512 threads, kmax,div = 64,16 / 8,16 / 1,1: large 7143 / 7114 / 6716, cloud 527 / 529 / 525.
+constexpr int kDefaultThreadsBvh = 1024;
+constexpr uint32_t kBvhSchedKmax = 64, kBvhSchedDiv = 16;
+
+int launch_megakernel_bvh(int sm_count, const r1::RenderArgs &args, const float4 *nodes, const float4 *leaves, const r1_render_params &prm,
+                          cudaStream_t stream)
+{
+    const int threads = prm.threads > 0 ? prm.threads : kDefaultThreadsBvh;
+    const r1::BvhArgs b = { nodes, leaves };
+    R1_CUDA(cudaMemcpyToSymbolAsync(r1::c_bvh, &b, sizeof(b), 0, cudaMemcpyHostToDevice, stream));
+    if (threads == 512) return launch_megakernel_pool<r1::kScanBvh, false, 512>(sm_count, args, prm, stream);
+    if (threads == 768) return launch_megakernel_pool<r1::kScanBvh, false, 768>(sm_count, args, prm, stream);
+    if (threads == 1024) return launch_megakernel_pool<r1::kScanBvh, false, 1024>(sm_count, args, prm, stream);
+    return fail(R1_ERR_ARG, "the bvh variant runs 512, 768 or 1024 threads (got %d)", threads);
+}
+
+// The host BVH of the scene, built on first need (r1_bvh.h).
+int scene_bvh(r1_scene *scene, const r1::bvh::Bvh **out)
+{
+    if (!scene->bvh) {
+        std::unique_ptr<r1::bvh::Bvh> b(new r1::bvh::Bvh());
+        if (!r1::bvh::build(scene->cx.data(), scene->cy.data(), scene->cz.data(), scene->radius_sq.data(), scene->inv_radius.data(),
+                            (uint32_t)scene->cx.size(), *b))
+            return fail(R1_ERR_LIMIT, "the bvh takes fewer than 2^28 spheres that can be hit");
+        if (b->depth > (uint32_t)r1::bvh::kMaxDepth) return fail(R1_ERR_LIMIT, "bvh depth %u exceeds %d", b->depth, r1::bvh::kMaxDepth);
+        scene->bvh = std::move(b);
+    }
+    *out = scene->bvh.get();
+    return R1_OK;
+}
+
+// The scene's BVH on the context's device: built and uploaded on the first BVH render or trace there (a synchronous copy into an
+// allocation of its own, freed with the context).  Refused when the spheres changed after the commit: the device's shading and
+// exact records would no longer match the tree.
+int ctx_bvh(r1_scene *scene, DeviceCtx &c)
+{
+    if (c.bvh_block) return R1_OK;
+    if (c.generation != scene->generation) return fail(R1_ERR_STATE, "the scene's spheres changed after it was committed to device %d (commit it again)", c.device);
+    const r1::bvh::Bvh *b = nullptr;
+    int rc = scene_bvh(scene, &b);
+    if (rc) return rc;
+    const size_t nb = b->nodes.size() * sizeof(r1::bvh::Node), lb = b->leaves.size() * sizeof(r1::bvh::LeafRec);
+    R1_CUDA(cudaSetDevice(c.device));
+    void *blk = nullptr;
+    R1_CUDA(cudaMalloc(&blk, nb + lb + 16));
+    cudaError_t e = cudaMemcpy(blk, b->nodes.data(), nb, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && lb) e = cudaMemcpy(static_cast<unsigned char *>(blk) + nb, b->leaves.data(), lb, cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) { cudaFree(blk); return fail(R1_ERR_CUDA, "bvh upload: %s", cudaGetErrorString(e)); }
+    c.bvh_block = blk;
+    c.bvh_nodes = static_cast<const float4 *>(blk);
+    c.bvh_leaves = reinterpret_cast<const float4 *>(static_cast<unsigned char *>(blk) + nb);
+    return R1_OK;
+}
+
 // R1_VARIANT_MEGAKERNEL = the fastest megakernel for the scene.  Measured on B200: the tensor-core filter wins on the large scene
 // (485 spheres: 10.3 against 6.2 G rays/s) and loses where a scan is short (medium, 58 spheres: 25 against 34 G).  Explicit
 // tuning knobs (blocks_per_sm, threads, R1_POOL=0) address the packed kernel; R1_AUTO_TENSOR=0 keeps it everywhere.
@@ -364,6 +432,9 @@ int resolve_variant(const r1::DevScene &dev, const r1_render_params &prm)
     return R1_VARIANT_MEGAKERNEL_PACKED;
 }
 
+// 8 and 10 stay unassigned (include/rays1_b200.h)
+bool known_variant(int v) { return v >= 0 && v <= R1_VARIANT_MEGAKERNEL_BVH && v != 8 && v != 10; }
+
 int validate(const r1_render_params *p)
 {
     if (!p) return fail(R1_ERR_ARG, "null params");
@@ -373,7 +444,7 @@ int validate(const r1_render_params *p)
     // the pixel accumulators hold sums of radiance * 2^24 in 64 bits, one sample saturating at 2^32 - 1 (r1_kernels.cuh): 2^20
     // samples per pixel cannot wrap them
     if (p->spp > (1 << 20)) return fail(R1_ERR_LIMIT, "spp %d exceeds the accumulator limit of 2^20 samples per pixel", p->spp);
-    if (p->variant < 0 || p->variant > R1_VARIANT_MEGAKERNEL_TENSOR_STREAM || p->variant == 8) return fail(R1_ERR_ARG, "unknown variant %d", p->variant);
+    if (!known_variant(p->variant)) return fail(R1_ERR_ARG, "unknown variant %d", p->variant);
     return R1_OK;
 }
 
@@ -458,6 +529,8 @@ int r1_scene_add_sphere(r1_scene *scene, float cx, float cy, float cz, float rad
     if (mat_kind < R1_MAT_NONE || mat_kind > R1_MAT_DIELECTRIC) return fail(R1_ERR_ARG, "unknown material kind %d", mat_kind);
     if (mat_kind == R1_MAT_NONE && radius > 0) return fail(R1_ERR_ARG, "a sphere with radius > 0 needs a material");
     if (mat_kind == R1_MAT_METAL) param = param < 1 ? param : 1;  // Metal ctor, rayweek1.cpp:424
+    scene->bvh.reset();
+    ++scene->generation;
     scene->cx.push_back(cx); scene->cy.push_back(cy); scene->cz.push_back(cz);
     scene->radius_sq.push_back(radius * radius);
     scene->inv_radius.push_back(radius > 0 ? (1.0f / radius) : 0);
@@ -523,6 +596,27 @@ int r1_tensor_operand(const r1_scene *scene, void *out, uint64_t out_bytes, uint
     if (out_bytes < (uint64_t)n32 * r1::tc::kRowBytes) return fail(R1_ERR_ARG, "operand buffer too small: %llu < %llu bytes", (unsigned long long)out_bytes,
                                                                    (unsigned long long)n32 * r1::tc::kRowBytes);
     build_tensor_operand(scene, static_cast<unsigned char *>(out), n32);
+    return R1_OK;
+}
+
+int r1_bvh_export(const r1_scene *scene, void *nodes, uint64_t nodes_bytes, void *leaves, uint64_t leaves_bytes, uint32_t *n_nodes,
+                  uint32_t *n_leaf_records, uint32_t *depth)
+{
+    if (!scene) return fail(R1_ERR_ARG, "null scene");
+    const r1::bvh::Bvh *b = nullptr;
+    { const int rc = scene_bvh(const_cast<r1_scene *>(scene), &b); if (rc) return rc; }   // the cached tree is derived state, not a change to the scene
+    if (n_nodes) *n_nodes = (uint32_t)b->nodes.size();
+    if (n_leaf_records) *n_leaf_records = (uint32_t)b->leaves.size();
+    if (depth) *depth = b->depth;
+    const uint64_t nb = b->nodes.size() * sizeof(r1::bvh::Node), lb = b->leaves.size() * sizeof(r1::bvh::LeafRec);
+    if (nodes) {
+        if (nodes_bytes < nb) return fail(R1_ERR_ARG, "node buffer too small: %llu < %llu bytes", (unsigned long long)nodes_bytes, (unsigned long long)nb);
+        memcpy(nodes, b->nodes.data(), nb);
+    }
+    if (leaves) {
+        if (leaves_bytes < lb) return fail(R1_ERR_ARG, "leaf buffer too small: %llu < %llu bytes", (unsigned long long)leaves_bytes, (unsigned long long)lb);
+        memcpy(leaves, b->leaves.data(), lb);
+    }
     return R1_OK;
 }
 
@@ -613,6 +707,7 @@ int r1_scene_commit(r1_scene *scene, int device)
     c.dev.cam = scene->cam;
     c.dev.tcb = tensor_ok ? reinterpret_cast<const unsigned char *>(c.block) + tcb_off : nullptr;
     c.dev.n32 = n32;
+    c.generation = scene->generation;
     scene->ctx[device] = c;
     scene->current = device;
     return R1_OK;
@@ -664,6 +759,10 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
     r1_render_params prm = *params;
     if (prm.row_tile <= 0) prm.row_tile = kDefaultRowTile;
     cudaStream_t stream = (cudaStream_t)cuda_stream;
+    if (prm.variant == R1_VARIANT_MEGAKERNEL_BVH) {   // first use on this device: build / upload before the first event
+        rc = ctx_bvh(scene, c);
+        if (rc) return rc;
+    }
 
     const Partition part = partition(prm.width, prm.height, prm.row_tile, prm.rank, prm.world);
     r1::RenderArgs a;
@@ -692,6 +791,9 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
     const bool pool_sched = !(getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0);
     if (c.dev.n8 >= 256) { a.sched_kmax = pool_sched ? 8 : 1; a.sched_div = pool_sched ? 16 : 1; }
     else { a.sched_kmax = 64; a.sched_div = 16; }
+    if (prm.variant == R1_VARIANT_MEGAKERNEL_BVH) {   // traversals are short at every scene size (DESIGN.md section 4.8)
+        a.sched_kmax = kBvhSchedKmax; a.sched_div = kBvhSchedDiv;
+    }
     if (const char *e = getenv("R1_SCHED")) {  // tuning knob: "kmax,div"
         unsigned k = 0, d = 0;
         if (sscanf(e, "%u,%u", &k, &d) == 2 && k >= 1 && k <= 4096 && d >= 1 && d <= 1024) { a.sched_kmax = k; a.sched_div = d; }
@@ -737,6 +839,7 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
                                                                                 : launch_megakernel<r1::kScanLaneDeferred, false>(x.sm_count, a, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR) rc = launch_megakernel_tc(x.sm_count, a, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) rc = launch_megakernel_tcs(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_BVH) rc = launch_megakernel_bvh(x.sm_count, a, c.bvh_nodes, c.bvh_leaves, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_DUAL) rc = staged ? launch_megakernel_dual<true>(x.sm_count, a, prm, stream)
                                                                             : launch_megakernel_dual<false>(x.sm_count, a, prm, stream);
             else rc = staged ? launch_megakernel<r1::kScanLaneScalar, true>(x.sm_count, a, prm, stream)
@@ -844,6 +947,24 @@ struct DevBuf {
     template <typename T> T *as() { return reinterpret_cast<T *>(p); }
 };
 #define R1_TRY(expr) do { int rc_ = (expr); if (rc_) return rc_; } while (0)
+
+// r1_trace_rays through the BVH: any sphere count
+int trace_rays_bvh(r1_scene *scene, DeviceCtx &c, int n, const float *org, const float *dir, float t_min, float t_max, int32_t *index, float *t,
+                   float *p, float *normal)
+{
+    R1_TRY(ctx_bvh(scene, c));
+    DevBuf d_org, d_dir, d_idx, d_t, d_p, d_n;
+    R1_TRY(d_org.upload(org, (size_t)n * 12)); R1_TRY(d_dir.upload(dir, (size_t)n * 12));
+    R1_TRY(d_idx.alloc((size_t)n * 4)); R1_TRY(d_t.alloc((size_t)n * 4)); R1_TRY(d_p.alloc((size_t)n * 12)); R1_TRY(d_n.alloc((size_t)n * 12));
+    r1::trace_rays_bvh_kernel<<<(n + 127) / 128, 128>>>(c.dev, n, d_org.as<float>(), d_dir.as<float>(), t_min, t_max, d_idx.as<int32_t>(), d_t.as<float>(),
+                                                        d_p.as<float>(), d_n.as<float>(), c.bvh_nodes, c.bvh_leaves);
+    R1_CUDA(cudaGetLastError());
+    R1_CUDA(cudaDeviceSynchronize());
+    R1_TRY(d_idx.download(index, (size_t)n * 4)); R1_TRY(d_t.download(t, (size_t)n * 4));
+    R1_TRY(d_p.download(p, (size_t)n * 12)); R1_TRY(d_n.download(normal, (size_t)n * 12));
+    return R1_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -861,12 +982,13 @@ int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, fl
     r1_render_params prm;
     memset(&prm, 0, sizeof(prm));
     prm.variant = variant;
-    if (variant < 0 || variant > R1_VARIANT_MEGAKERNEL_TENSOR_STREAM || variant == 8) return fail(R1_ERR_ARG, "unknown variant %d", variant);
+    if (!known_variant(variant)) return fail(R1_ERR_ARG, "unknown variant %d", variant);
     const int v = resolve_variant(cp->dev, prm);
     if (v == R1_VARIANT_WAVEFRONT || v == R1_VARIANT_MEGAKERNEL_DUAL) return fail(R1_ERR_ARG, "r1_trace_rays has no kernel for variant %d (wavefront, dual)", v);
     if (v == R1_VARIANT_MEGAKERNEL_TENSOR && !cp->dev.tcb)
         return fail(R1_ERR_LIMIT, "the tensor-core filter takes scenes of 1 .. %d spheres (this scene pads to %d)", r1::tc::kMaxSpheres, cp->dev.n32);
     if (n == 0) return R1_OK;
+    if (v == R1_VARIANT_MEGAKERNEL_BVH) return trace_rays_bvh(scene, *cp, n, org, dir, t_min, t_max, index, t, p, normal);
     // the streamed filter takes any size; the other kernels stage the whole scene in shared memory
     if (v != R1_VARIANT_MEGAKERNEL_TENSOR_STREAM && cp->dev.n_pad > r1::kMaxStagedSpheres) return fail(R1_ERR_LIMIT, "r1_trace_rays stages at most %d spheres", r1::kMaxStagedSpheres);
     DevBuf d_org, d_dir, d_idx, d_t, d_p, d_n;
@@ -907,6 +1029,7 @@ const char *r1_kernel_name(r1_scene *scene, int variant)
     case R1_VARIANT_MEGAKERNEL_TENSOR: return "megakernel_tc3";
     case R1_VARIANT_MEGAKERNEL_DUAL: return "megakernel_pool2";
     case R1_VARIANT_MEGAKERNEL_TENSOR_STREAM: return "megakernel_tcs";
+    case R1_VARIANT_MEGAKERNEL_BVH: return "megakernel_bvh";
     default: return (getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0) ? "megakernel" : "megakernel_pool";
     }
 }

@@ -37,6 +37,12 @@ struct RenderArgs {
     uint64_t n_samples, magic_spp;       // npix_local * spp; floor(2^64 / spp) + 1 (exact g / spp for g < 2^64 / spp; 0 when spp == 1)
 };
 
+// The BVH megakernel_pool<kScanBvh> traverses (r1_bvh.h): written on the launching stream before every launch of that kernel
+// (r1_core.cu).  It is not a RenderArgs field because the wavefront kernels take a second parameter behind RenderArgs, whose
+// offset -- and so their code -- would change with its size.
+struct BvhArgs { const float4 *nodes, *leaves; };
+__constant__ BvhArgs c_bvh;
+
 constexpr int kSmemSpheres = 16 + R1_RSQRT12_ENTRIES * 2;   // megakernel: byte offset of the staged spheres (mbarrier, rsqrtss table first)
 constexpr float kFixedScale = 16777216.0f;                 // 2^24: one sample saturates at 2^32 - 1 (radiance 256; scenes stay <= 1)
 constexpr float kFixedInvScale = 5.9604644775390625e-8f;   // 2^-24
@@ -162,7 +168,7 @@ __device__ __forceinline__ bool shade_step(const RenderArgs &a, int hit, float t
 // every scan with a live ray and divergence is confined to the short fetch / generate / shade steps.
 // Replaces render_tile + color + TileRenderScheduler (rayweek1.cpp:722-842, 515-536).
 // kScan: which Hitable::hit implementation the lanes run
-enum ScanKind { kScanCoop = 0, kScanLanePacked = 1, kScanLaneScalar = 2, kScanLaneDeferred = 3 };
+enum ScanKind { kScanCoop = 0, kScanLanePacked = 1, kScanLaneScalar = 2, kScanLaneDeferred = 3, kScanBvh = 4 };   // kScanBvh: megakernel_pool only
 __host__ __device__ constexpr int scan_filter(int kScan) { return kScan == kScanLaneScalar ? 0 : 1; }
 
 // (Round-1 scheduling, kept as the A/B alternative of megakernel_pool below: R1_POOL=0.)
@@ -431,6 +437,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool(const 
         int hit = -1;
         if (kScan == kScanCoop) scan_coop<(kThreads <= 512 ? 2 : 1)>(*ws, s_scan, s_exact, n_pad, o, d, kTMin, kTMax, t, hit);
         else if (kScan == kScanLaneDeferred) scan_deferred(*reinterpret_cast<DeferScratch *>(ws), s_scan, s_exact, a.scene.n8, o, d, kTMin, kTMax, t, hit);
+        else if (kScan == kScanBvh) { if (active) bvh_trace(c_bvh.nodes, c_bvh.leaves, o, d, kTMin, t, hit); }   // idle lanes do not traverse
         else scan<scan_filter(kScan)>(s_scan, s_exact, a.scene.n8, o, d, kTMin, t, hit);
 
         // -- color() body (rayweek1.cpp:515-536)
@@ -1243,6 +1250,26 @@ __global__ void __launch_bounds__(128) trace_rays_kernel(const __grid_constant__
     if (!live) return;
     f3 p = mk3(0, 0, 0), nrm = mk3(0, 0, 0);
     if (hit >= 0) hit_finalise(s_spheres[sc.n_pad + hit], load_shade(sc, hit).inv_radius, o, d, t, p, nrm);
+    index[k] = hit;
+    t_out[k] = hit >= 0 ? t : 0.0f;
+    p_out[3 * k] = p.x; p_out[3 * k + 1] = p.y; p_out[3 * k + 2] = p.z;
+    n_out[3 * k] = nrm.x; n_out[3 * k + 1] = nrm.y; n_out[3 * k + 2] = nrm.z;
+}
+
+// Hitable::hit through the BVH (R1_VARIANT_MEGAKERNEL_BVH): bvh_trace, then hit_finalise from the scene's exact and shading
+// records by original index.  Any sphere count; nothing staged.
+__global__ void __launch_bounds__(128) trace_rays_bvh_kernel(const __grid_constant__ DevScene sc, int n, const float *org, const float *dir,
+                                                             float t_min, float t_max, int32_t *index, float *t_out, float *p_out, float *n_out,
+                                                             const float4 *nodes, const float4 *leaves)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const f3 o = mk3(org[3 * k], org[3 * k + 1], org[3 * k + 2]), d = mk3(dir[3 * k], dir[3 * k + 1], dir[3 * k + 2]);
+    float t = t_max;
+    int hit = -1;
+    bvh_trace(nodes, leaves, o, d, t_min, t, hit);
+    f3 p = mk3(0, 0, 0), nrm = mk3(0, 0, 0);
+    if (hit >= 0) hit_finalise(__ldg(sc.exact + hit), load_shade(sc, hit).inv_radius, o, d, t, p, nrm);
     index[k] = hit;
     t_out[k] = hit >= 0 ? t : 0.0f;
     p_out[3 * k] = p.x; p_out[3 * k + 1] = p.y; p_out[3 * k + 2] = p.z;

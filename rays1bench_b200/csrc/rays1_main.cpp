@@ -1,7 +1,7 @@
 // rays1_main.cpp -- the reference's executable surface: `./rays1_b200 [-w] [-n N]` renders small, medium and large,
 // prints the reference's report blocks and writes out_<scene>.txt (and out_<scene>.tga with -w), exactly as
 // src/latest/rayweek1.cpp:930-988 does.  Extra flags (not in the reference) select what it fixes at compile time:
-//   --gpus N  --variant mega|wavefront|packed|tensor|tensor-stream|scalar|coop|deferred|dual  --width W --height H --spp S --bounces B  --scene NAME (repeatable)
+//   --gpus N  --variant mega|wavefront|packed|tensor|tensor-stream|bvh|scalar|coop|deferred|dual  --width W --height H --spp S --bounces B  --scene NAME (repeatable)
 //   --scene-file PATH (text scene description, see rays1_host.cpp)
 #include <cstdio>
 #include <cstdlib>
@@ -46,6 +46,7 @@ int main(int argc, const char *argv[])
             else if (!strcmp(v, "tensor")) cfg.variant = R1_VARIANT_MEGAKERNEL_TENSOR;
             else if (!strcmp(v, "tensor-stream")) cfg.variant = R1_VARIANT_MEGAKERNEL_TENSOR_STREAM;
             else if (!strcmp(v, "packed")) cfg.variant = R1_VARIANT_MEGAKERNEL_PACKED;
+            else if (!strcmp(v, "bvh")) cfg.variant = R1_VARIANT_MEGAKERNEL_BVH;
             else { printf("Invalid variant: %s\n", v); exit(2); }
         }
     }

@@ -2,6 +2,8 @@
 """Writes scene description files for rays1_b200 --scene-file (SURVEY.md 8f rank 3: sphere-count sweeps without a
 recompile).  `--preset large` reproduces create_large_scene() (src/latest/rayweek1.cpp:654-719 of the reference) through
 the file format; `--grid W H` builds the same recipe on a W x H grid (66 x 62 = the synthetic 4096-sphere scene).
+`--cloud N [--seed S]` scatters N overlapping spheres of radii 0.02 .. 2 through a cube above a ground sphere: unlike the flat
+grids, a hard case for a bounding volume hierarchy.
 
   python tools/make_scene.py --grid 30 16 --out large.r1scene
   ./rays1bench_b200/rays1_b200 --scene-file large.r1scene --spp 64
@@ -48,14 +50,45 @@ def grid_scene(gw, gh, ior_mod, lookfrom, focus):
     return camera, spheres
 
 
+def cloud_scene(n, seed=1):
+    """n spheres, centres uniform in a cube of side 2 n^(1/3) (at least 4) above the ground, radii log-uniform in [0.02, 2]
+    (about 30 % of the cube's volume summed over the spheres: heavy overlap), 70 % Lambertian, 20 % metal, 10 % glass; then the
+    ground sphere (radius 10 000) and a camera outside the cube looking at its centre."""
+    rng = np.random.default_rng(seed)
+    f = np.float32
+    half = max(2.0, float(n) ** (1.0 / 3.0))
+    c = rng.uniform(-half, half, (n, 3))
+    c[:, 1] += half + 0.5
+    r = np.exp(rng.uniform(np.log(0.02), np.log(2.0), n))
+    kind = rng.choice([0, 1, 2], n, p=[0.7, 0.2, 0.1])
+    col = rng.uniform(0.1, 0.9, (n, 3))
+    fuzz = rng.uniform(0.0, 0.5, n)
+    spheres = []
+    for i in range(n):
+        x, y, z = (f(v) for v in c[i])
+        if kind[i] == 0:
+            spheres.append((x, y, z, f(r[i]), 0, *(f(v) for v in col[i]), 0))
+        elif kind[i] == 1:
+            spheres.append((x, y, z, f(r[i]), 1, *(f(v) for v in col[i]), f(fuzz[i])))
+        else:
+            spheres.append((x, y, z, f(r[i]), 2, 1, 1, 1, f(1.5)))
+    spheres.append((0, f(-10000), 0, 10000, 0, 0.5, 0.5, 0.5, 0))
+    camera = (0, 1.6 * half + 1, 3.2 * half + 3, 0, half, 0, 50, 0.02, float(np.hypot(0.6 * half + 1, 3.2 * half + 3)))
+    return camera, spheres
+
+
 def main():
     import rays1bench_b200 as r1
     ap = argparse.ArgumentParser()
     ap.add_argument("--preset", choices=["large", "synth4096"])
     ap.add_argument("--grid", type=int, nargs=2, metavar=("W", "H"))
+    ap.add_argument("--cloud", type=int, metavar="N")
+    ap.add_argument("--seed", type=int, default=1)
     ap.add_argument("--out", required=True)
     args = ap.parse_args()
-    if args.preset == "large" or (not args.preset and not args.grid):
+    if args.cloud:
+        cam, sph = cloud_scene(args.cloud, args.seed)
+    elif args.preset == "large" or (not args.preset and not args.grid):
         cam, sph = grid_scene(30, 16, 0, (3, 8, 15), 10.0)
     elif args.preset == "synth4096":
         cam, sph = grid_scene(66, 62, 480, (6, 16, 30), 20.0)
