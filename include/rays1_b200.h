@@ -178,6 +178,22 @@ int r1_tensor_operand(const r1_scene *scene, void *out, uint64_t out_bytes, uint
  * node (root = 1), at most 64.  A NULL buffer skips that copy (the counts are still returned). */
 int r1_bvh_export(const r1_scene *scene, void *nodes, uint64_t nodes_bytes, void *leaves, uint64_t leaves_bytes, uint32_t *n_nodes,
                   uint32_t *n_leaf_records, uint32_t *depth);
+/* Builders of r1_scene_build_bvh.  HOST: the tree r1_bvh_export returns (binned SAH, built on the host and cached in the scene).
+ * DEVICE: a linear BVH (Morton codes, radix sort, Karras' radix tree, leaves of <= 4 spheres) built on the device from the
+ * committed scene; a pure function of the scene, in r1_bvh_export's layout, depth at most 62 (DESIGN.md section 4.9). */
+enum { R1_BVH_BUILD_HOST = 0, R1_BVH_BUILD_DEVICE = 1 };
+/* Builds the BVH of R1_VARIANT_MEGAKERNEL_BVH for `device` now (< 0: device of the last commit) and makes it the tree that BVH
+ * renders and traces there use, replacing any tree the device holds.  HOST: the host tree (cached in the scene) uploaded;
+ * DEVICE: the linear BVH, built on the device from the committed scene.  Synchronous.  device_ms (optional): CUDA events around
+ * the device work (the upload for HOST; every kernel and the sort for DEVICE).  R1_ERR_ARG for a null scene, an unknown builder
+ * or (DEVICE) a sphere that can be hit with a non-finite centre or radius_sq; R1_ERR_STATE if the scene is not committed there or
+ * its spheres changed since; R1_ERR_LIMIT from 2^28 spheres that can be hit.  A re-commit drops the device's tree: the next BVH
+ * render or trace builds and uploads the host tree again. */
+int r1_scene_build_bvh(r1_scene *scene, int device, int builder, double *device_ms);
+/* The tree `device` (< 0: device of the last commit) holds, in r1_bvh_export's layout; R1_ERR_STATE if it holds none, R1_ERR_ARG
+ * for a null scene or a buffer smaller than the tree.  A NULL buffer skips that copy (the counts are still returned). */
+int r1_bvh_export_device(r1_scene *scene, int device, void *nodes, uint64_t nodes_bytes, void *leaves, uint64_t leaves_bytes,
+                         uint32_t *n_nodes, uint32_t *n_leaf_records, uint32_t *depth);
 /* Values of the tensor-core FILTER (R1_VARIANT_MEGAKERNEL_TENSOR) for n rays against every sphere: e[ray * n32 + sphere], n32 =
  * sphere count padded to 32; the filter flags a sphere iff the sign bit of e is clear, and must flag every sphere Hitable::hit's
  * discriminant test (rayweek1.cpp:192-204) accepts.  layout must be 0 (the renderer's operand layout); any other value returns

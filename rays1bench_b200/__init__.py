@@ -36,6 +36,7 @@ class Rays1Error(RuntimeError):
 BVH_NODE = np.dtype([("lo0", "<f4", 3), ("hi0", "<f4", 3), ("lo1", "<f4", 3), ("hi1", "<f4", 3), ("child", "<i4", 2), ("diag", "<f4", 2)])
 BVH_LEAF = np.dtype([("exact", "<f4", 4), ("index", "<i4"), ("pad", "<i4", 3)])
 BVH_MAX_DEPTH = 64
+BVH_BUILD_HOST, BVH_BUILD_DEVICE = 0, 1   # builders of r1_scene_build_bvh
 
 
 class Result(C.Structure):
@@ -90,6 +91,8 @@ def _load():
         "r1_filter_probe": (ci, [vp, ci, f32p, f32p, ci, f32p]),
         "r1_tensor_operand": (ci, [vp, u8p, C.c_uint64, C.POINTER(C.c_uint32)]),
         "r1_bvh_export": (ci, [vp, vp, C.c_uint64, vp, C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+        "r1_scene_build_bvh": (ci, [vp, ci, ci, C.POINTER(C.c_double)]),
+        "r1_bvh_export_device": (ci, [vp, ci, vp, C.c_uint64, vp, C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
         "r1_scatter": (ci, [vp, ci, f32p, f32p, f32p, i32p, f32p, f32p, i32p, f32p, f32p]),
         "r1_get_ray": (ci, [vp, ci, f32p, f32p, f32p, f32p, f32p]),
         "r1_replay_pixels": (ci, [vp, ci, i32p, ci, ci, ci, ci, u32p, u32p, f32p, u32p]),
@@ -253,6 +256,24 @@ class Scene:
         leaves = np.zeros(nl.value, BVH_LEAF)
         _check(lib.r1_bvh_export(self.handle, nodes.ctypes.data, nodes.nbytes, leaves.ctypes.data if nl.value else None, leaves.nbytes,
                                  C.byref(nn), C.byref(nl), C.byref(depth)), "r1_bvh_export")
+        return nodes, leaves, int(depth.value)
+
+    def build_bvh(self, builder=BVH_BUILD_DEVICE, device=-1):
+        """r1_scene_build_bvh: builds the bvh variant's tree for `device` (-1: the device of the last commit) with `builder` and makes
+        it the tree BVH renders and traces there use.  Returns the device time of the build (or of the upload, for BVH_BUILD_HOST)
+        in ms."""
+        ms = C.c_double(0)
+        _check(lib.r1_scene_build_bvh(self.handle, device, builder, C.byref(ms)), "r1_scene_build_bvh")
+        return ms.value
+
+    def bvh_on_device(self, device=-1):
+        """r1_bvh_export_device: the tree `device` holds, as (nodes, leaves, depth) in the arrays of bvh()."""
+        nn, nl, depth = C.c_uint32(0), C.c_uint32(0), C.c_uint32(0)
+        _check(lib.r1_bvh_export_device(self.handle, device, None, 0, None, 0, C.byref(nn), C.byref(nl), C.byref(depth)), "r1_bvh_export_device")
+        nodes = np.zeros(nn.value, BVH_NODE)
+        leaves = np.zeros(nl.value, BVH_LEAF)
+        _check(lib.r1_bvh_export_device(self.handle, device, nodes.ctypes.data, nodes.nbytes, leaves.ctypes.data if nl.value else None,
+                                        leaves.nbytes, C.byref(nn), C.byref(nl), C.byref(depth)), "r1_bvh_export_device")
         return nodes, leaves, int(depth.value)
 
     def filter_probe(self, org, dir_, n_spheres, layout=0):

@@ -4,6 +4,7 @@
 // file:line citations are relative to /root/reference/.
 #include "../../include/rays1_b200.h"
 #include "r1_bvh.h"
+#include "r1_bvh_device.h"
 #include "r1_internal.h"
 #include "r1_kernels.cuh"
 #include "r1_wavefront.cuh"
@@ -40,8 +41,9 @@ struct DeviceCtx {
     size_t block_bytes = 0;
     r1::DevScene dev;
     uint64_t generation = 0;            // r1_scene::generation at the commit
-    void *bvh_block = nullptr;          // R1_VARIANT_MEGAKERNEL_BVH: [nodes | leaf records], uploaded on first use
+    void *bvh_block = nullptr;          // R1_VARIANT_MEGAKERNEL_BVH: [nodes | leaf records], uploaded on first use or r1_scene_build_bvh
     const float4 *bvh_nodes = nullptr, *bvh_leaves = nullptr;
+    uint32_t bvh_n_nodes = 0, bvh_n_leaves = 0, bvh_depth = 0;
 };
 
 // Per-device scratch shared by every scene of the process (pixel accumulators, counters, staging, events).
@@ -397,9 +399,38 @@ int scene_bvh(r1_scene *scene, const r1::bvh::Bvh **out)
     return R1_OK;
 }
 
-// The scene's BVH on the context's device: built and uploaded on the first BVH render or trace there (a synchronous copy into an
-// allocation of its own, freed with the context).  Refused when the spheres changed after the commit: the device's shading and
-// exact records would no longer match the tree.
+// Makes blk = [n_nodes nodes | n_leaves leaf records] the tree BVH renders and traces on c's device use, freeing the one it replaces.
+void set_ctx_bvh(DeviceCtx &c, void *blk, uint32_t n_nodes, uint32_t n_leaves, uint32_t depth)
+{
+    if (c.bvh_block) cudaFree(c.bvh_block);
+    c.bvh_block = blk;
+    c.bvh_nodes = static_cast<const float4 *>(blk);
+    c.bvh_leaves = reinterpret_cast<const float4 *>(static_cast<unsigned char *>(blk) + (size_t)n_nodes * sizeof(r1::bvh::Node));
+    c.bvh_n_nodes = n_nodes; c.bvh_n_leaves = n_leaves; c.bvh_depth = depth;
+}
+
+// The host tree on c's device: a synchronous copy into an allocation of its own, freed with the context.  ms (optional): CUDA
+// events around the copies.
+int upload_bvh(DeviceCtx &c, const r1::bvh::Bvh &b, double *ms)
+{
+    const size_t nb = b.nodes.size() * sizeof(r1::bvh::Node), lb = b.leaves.size() * sizeof(r1::bvh::LeafRec);
+    R1_CUDA(cudaSetDevice(c.device));
+    void *blk = nullptr;
+    R1_CUDA(cudaMalloc(&blk, nb + lb + 16));
+    r1::PhaseTimer tm;
+    cudaError_t e = ms ? tm.start() : cudaSuccess;
+    if (e == cudaSuccess) e = cudaMemcpy(blk, b.nodes.data(), nb, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && lb) e = cudaMemcpy(static_cast<unsigned char *>(blk) + nb, b.leaves.data(), lb, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && ms) e = tm.stop();
+    if (e != cudaSuccess) { cudaFree(blk); return fail(R1_ERR_CUDA, "bvh upload: %s", cudaGetErrorString(e)); }
+    if (ms) *ms = tm.ms;
+    set_ctx_bvh(c, blk, (uint32_t)b.nodes.size(), (uint32_t)b.leaves.size(), b.depth);
+    return R1_OK;
+}
+
+// The scene's BVH on the context's device: unless r1_scene_build_bvh put one there, the host tree is built and uploaded on the
+// first BVH render or trace.  Refused when the spheres changed after the commit: the device's shading and exact records would no
+// longer match the tree.
 int ctx_bvh(r1_scene *scene, DeviceCtx &c)
 {
     if (c.bvh_block) return R1_OK;
@@ -407,17 +438,7 @@ int ctx_bvh(r1_scene *scene, DeviceCtx &c)
     const r1::bvh::Bvh *b = nullptr;
     int rc = scene_bvh(scene, &b);
     if (rc) return rc;
-    const size_t nb = b->nodes.size() * sizeof(r1::bvh::Node), lb = b->leaves.size() * sizeof(r1::bvh::LeafRec);
-    R1_CUDA(cudaSetDevice(c.device));
-    void *blk = nullptr;
-    R1_CUDA(cudaMalloc(&blk, nb + lb + 16));
-    cudaError_t e = cudaMemcpy(blk, b->nodes.data(), nb, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && lb) e = cudaMemcpy(static_cast<unsigned char *>(blk) + nb, b->leaves.data(), lb, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) { cudaFree(blk); return fail(R1_ERR_CUDA, "bvh upload: %s", cudaGetErrorString(e)); }
-    c.bvh_block = blk;
-    c.bvh_nodes = static_cast<const float4 *>(blk);
-    c.bvh_leaves = reinterpret_cast<const float4 *>(static_cast<unsigned char *>(blk) + nb);
-    return R1_OK;
+    return upload_bvh(c, *b, nullptr);
 }
 
 // R1_VARIANT_MEGAKERNEL = the fastest megakernel for the scene.  Measured on B200: the tensor-core filter wins on the large scene
@@ -965,9 +986,59 @@ int trace_rays_bvh(r1_scene *scene, DeviceCtx &c, int n, const float *org, const
     return R1_OK;
 }
 
+// The LBVH of the committed scene, built on c's device (r1_bvh_device.cu) and installed as its tree.
+int build_device_bvh(DeviceCtx &c, double *ms)
+{
+    R1_CUDA(cudaSetDevice(c.device));
+    r1::lbvh::Built out;
+    R1_TRY(r1::lbvh::build(c.dev.exact, c.dev.shade, (uint32_t)c.dev.n_real, &out, ms));
+    set_ctx_bvh(c, out.block, out.n_nodes, out.n_leaves, out.depth);
+    return R1_OK;
+}
+
 }  // namespace
 
 extern "C" {
+
+int r1_scene_build_bvh(r1_scene *scene, int device, int builder, double *device_ms)
+{
+    if (!scene) return fail(R1_ERR_ARG, "null scene");
+    if (builder != R1_BVH_BUILD_HOST && builder != R1_BVH_BUILD_DEVICE) return fail(R1_ERR_ARG, "unknown bvh builder %d", builder);
+    DeviceCtx *cp = nullptr;
+    R1_TRY(get_ctx(scene, &cp, device));
+    if (cp->generation != scene->generation) return fail(R1_ERR_STATE, "the scene's spheres changed after it was committed to device %d (commit it again)", cp->device);
+    double ms = 0;
+    if (builder == R1_BVH_BUILD_HOST) {
+        const r1::bvh::Bvh *b = nullptr;
+        R1_TRY(scene_bvh(scene, &b));
+        R1_TRY(upload_bvh(*cp, *b, &ms));
+    } else {
+        R1_TRY(build_device_bvh(*cp, &ms));
+    }
+    if (device_ms) *device_ms = ms;
+    return R1_OK;
+}
+
+int r1_bvh_export_device(r1_scene *scene, int device, void *nodes, uint64_t nodes_bytes, void *leaves, uint64_t leaves_bytes, uint32_t *n_nodes,
+                         uint32_t *n_leaf_records, uint32_t *depth)
+{
+    if (!scene) return fail(R1_ERR_ARG, "null scene");
+    if (device < 0) device = scene->current;
+    auto it = scene->ctx.find(device);
+    if (device < 0 || it == scene->ctx.end()) return fail(R1_ERR_STATE, "scene not committed to device %d (call r1_scene_commit)", device);
+    const DeviceCtx &c = it->second;
+    if (!c.bvh_block) return fail(R1_ERR_STATE, "device %d holds no bvh of this scene", device);
+    if (n_nodes) *n_nodes = c.bvh_n_nodes;
+    if (n_leaf_records) *n_leaf_records = c.bvh_n_leaves;
+    if (depth) *depth = c.bvh_depth;
+    const uint64_t nb = (uint64_t)c.bvh_n_nodes * sizeof(r1::bvh::Node), lb = (uint64_t)c.bvh_n_leaves * sizeof(r1::bvh::LeafRec);
+    if (nodes && nodes_bytes < nb) return fail(R1_ERR_ARG, "node buffer too small: %llu < %llu bytes", (unsigned long long)nodes_bytes, (unsigned long long)nb);
+    if (leaves && leaves_bytes < lb) return fail(R1_ERR_ARG, "leaf buffer too small: %llu < %llu bytes", (unsigned long long)leaves_bytes, (unsigned long long)lb);
+    R1_CUDA(cudaSetDevice(c.device));
+    if (nodes) R1_CUDA(cudaMemcpy(nodes, c.bvh_nodes, nb, cudaMemcpyDeviceToHost));
+    if (leaves && lb) R1_CUDA(cudaMemcpy(leaves, c.bvh_leaves, lb, cudaMemcpyDeviceToHost));
+    return R1_OK;
+}
 
 int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, float t_min, float t_max, int variant, int32_t *index, float *t,
                   float *p, float *normal)

@@ -12,7 +12,14 @@ also: the host build time of the BVH (r1_bvh_export on a fresh copy of the scene
 depth.  On `--config-scenes` every BVH thread count and two scheduling settings run too.  The card's name, power limit and SM
 clocks come from `nvidia-smi --query-gpu` (read-only) in the same call; the SM clock is sampled every 100 ms while renders run.
 
+With `--builders host device` the script compares the two trees of r1_scene_build_bvh instead of the variants.  Per scene: the
+host build time (as above); the device build time, median over `--builds` builds after one warm-up, as CUDA events around the
+device work and as host wall time of the call; node count, depth and SAH cost of each tree (from the exports; cost = 1 + sum over
+child slots of area(slot box) / area(root box) x (1 for an inner node, the sphere count for a leaf)); and BVH Mrays/s with each
+tree at `--builder-size`, alternated `--runs` times with L2 overwritten before every render, images and ray counts compared.
+
     python tools/bench_bvh.py [--runs 3] [--size 1280 720 250] [--out profiles/r03_bench_bvh.json]
+    python tools/bench_bvh.py --builders host device [--builds 7] [--builder-size 640 360 32] [--out profiles/r04_bench_bvh_build.json]
 
 There is no CPU path: without a CUDA device the script fails.
 """
@@ -63,6 +70,63 @@ def bvh_stats(r1, name, path):
     return {"host_build_s": dt, "nodes": len(nodes), "leaf_records": len(leaves), "bytes": int(nodes.nbytes + leaves.nbytes), "depth": depth}
 
 
+def sah_cost(nodes):
+    """1 + sum over used child slots of area / root area x (1 inner, count leaf); boxes as exported"""
+    lo = np.stack([nodes["lo0"], nodes["lo1"]], 1).astype(np.float64)
+    hi = np.stack([nodes["hi0"], nodes["hi1"]], 1).astype(np.float64)
+    ch = nodes["child"]
+    used = ch != -1
+    e = hi - lo
+    area = e[..., 0] * e[..., 1] + e[..., 1] * e[..., 2] + e[..., 2] * e[..., 0]
+    if not used[0].any():
+        return 0.0
+    rl, rh = lo[0][used[0]].min(0), hi[0][used[0]].max(0)
+    re = rh - rl
+    root_area = re[0] * re[1] + re[1] * re[2] + re[2] * re[0]
+    weight = np.where(ch >= 0, 1.0, (~ch) & 7)
+    return float(1.0 + (area * weight)[used].sum() / root_area)
+
+
+def tree_stats(nodes, leaves, depth):
+    return {"nodes": len(nodes), "leaf_records": len(leaves), "depth": depth, "sah_cost": sah_cost(nodes)}
+
+
+def compare_builders(r1, s, name, path, flush, torch, args):
+    """host and device trees of one scene: build times, tree statistics, BVH render rates with each (alternated)"""
+    entry = {"spheres": s.count(), "host": bvh_stats(r1, name, path)}
+    host_nodes, host_leaves, host_depth = s.bvh()
+    entry["host"].update(tree_stats(host_nodes, host_leaves, host_depth))
+    entry["host"]["upload_ms"] = s.build_bvh(r1.BVH_BUILD_HOST)
+    s.build_bvh(r1.BVH_BUILD_DEVICE)                                      # warm-up: module load, the sort's first launch
+    dev_ms, wall_s = [], []
+    for _ in range(args.builds):
+        t0 = time.perf_counter()
+        dev_ms.append(s.build_bvh(r1.BVH_BUILD_DEVICE))
+        wall_s.append(time.perf_counter() - t0)
+    dn, dl, dd = s.bvh_on_device()
+    entry["device"] = dict(tree_stats(dn, dl, dd), build_ms=dev_ms, build_ms_median=float(np.median(dev_ms)), wall_s=wall_s,
+                           wall_s_median=float(np.median(wall_s)))
+    size = tuple(args.builder_size)
+    entry["render_size"] = list(size)
+    runs = {"host": [], "device": []}
+    images = {}
+    for builder in ("host", "device"):                                    # warm-up of each tree
+        s.build_bvh(r1.BVH_BUILD_HOST if builder == "host" else r1.BVH_BUILD_DEVICE)
+        render(r1, s, flush, torch, (96, 54, 4), r1.VARIANT_MEGAKERNEL_BVH, 0, None)
+    for _ in range(args.runs):
+        for builder in ("host", "device"):
+            s.build_bvh(r1.BVH_BUILD_HOST if builder == "host" else r1.BVH_BUILD_DEVICE)
+            rgb, res = render(r1, s, flush, torch, size, r1.VARIANT_MEGAKERNEL_BVH, 0, None)
+            images.setdefault(builder, (rgb, int(res.num_rays)))
+            runs[builder].append({"mrays_per_s": res.num_rays / (res.kernel_ms * 1e-3) / 1e6, "kernel_ms": res.kernel_ms,
+                                  "num_rays": int(res.num_rays), "image_equal": bool(np.array_equal(rgb, images["host"][0])),
+                                  "rays_equal": int(res.num_rays) == images["host"][1]})
+    entry["runs"] = runs
+    entry["median_mrays_per_s"] = {b: float(np.median([r["mrays_per_s"] for r in rs])) for b, rs in runs.items()}
+    entry["all_images_equal"] = all(r["image_equal"] and r["rays_equal"] for rs in runs.values() for r in rs)
+    return entry
+
+
 def render(r1, s, flush, torch, size, v, threads, sched):
     if sched:
         os.environ["R1_SCHED"] = sched
@@ -84,8 +148,15 @@ def main():
     ap.add_argument("--small-size", type=int, nargs=3, default=(320, 180, 8), metavar=("W", "H", "SPP"))
     ap.add_argument("--scenes", nargs="+", default=["small", "medium", "large", "synth4096", "grid8016", "grid1e5", "cloud1e5", "grid1e6", "cloud1e6"])
     ap.add_argument("--config-scenes", nargs="*", default=["large", "cloud1e5"])
+    ap.add_argument("--builders", nargs="*", choices=("host", "device"), help="compare the host and device trees instead of the variants")
+    ap.add_argument("--builds", type=int, default=7, help="timed device builds per scene (after one warm-up)")
+    ap.add_argument("--builder-size", type=int, nargs=3, default=(640, 360, 32), metavar=("W", "H", "SPP"))
     ap.add_argument("--out", help="also write the JSON result here")
     args = ap.parse_args()
+    if args.builders is not None and sorted(args.builders) != ["device", "host"]:
+        ap.error("--builders compares both trees: pass `--builders host device`")
+    if args.builders and "--scenes" not in sys.argv:
+        args.scenes = ["large", "synth4096", "grid8016", "grid1e5", "cloud1e5", "grid1e6", "cloud1e6"]
 
     import torch
     if not torch.cuda.is_available():
@@ -100,6 +171,16 @@ def main():
     with tempfile.TemporaryDirectory() as tmp, ClockSampler() as clocks:
         for name in args.scenes:
             s, path = make(r1, name, tmp)
+            if args.builders:
+                entry = result["scenes"][name] = compare_builders(r1, s, name, path, flush, torch, args)
+                s.close()
+                print("%-10s %7d spheres: host build %.3f s, device build %.2f ms (wall %.2f ms); nodes %d / %d, depth %d / %d, SAH %.1f / %.1f; "
+                      "Mrays/s host tree %.0f, device tree %.0f; images equal: %s" % (
+                          name, entry["spheres"], entry["host"]["host_build_s"], entry["device"]["build_ms_median"], 1e3 * entry["device"]["wall_s_median"],
+                          entry["host"]["nodes"], entry["device"]["nodes"], entry["host"]["depth"], entry["device"]["depth"], entry["host"]["sah_cost"],
+                          entry["device"]["sah_cost"], entry["median_mrays_per_s"]["host"], entry["median_mrays_per_s"]["device"], entry["all_images_equal"]),
+                      file=sys.stderr, flush=True)
+                continue
             n = s.count()
             n32 = (n + 31) // 32 * 32
             entry = {"spheres": n, "real_spheres": int((s.soa()["inv_radius"] > 0).sum()), "bvh": bvh_stats(r1, name, path)}
