@@ -115,7 +115,8 @@ int r1_scene_add_sphere(r1_scene *scene, float cx, float cy, float cz, float rad
  * (rayweek1.cpp:575-576; SIMD_WIDTH = 8 there). */
 int r1_scene_pad(r1_scene *scene, uint32_t multiple);
 uint32_t r1_scene_count(const r1_scene *scene);
-/* Host copies of the SoA arrays, `count` entries each (albedo: 3 per sphere) -- for bit-parity checks. */
+/* Host copies of the SoA arrays, `count` entries each (albedo: 3 per sphere) -- for bit-parity checks.  They describe the scene as
+ * built on the host: r1_scene_move_spheres changes a device's records only. */
 int r1_scene_get_soa(const r1_scene *scene, float *cx, float *cy, float *cz, float *radius_sq, float *inv_radius, int32_t *kind,
                      float *albedo, float *param);
 /* out[22] = origin, lower-left corner, horizontal, vertical, u, v, w (3 each), lens radius (rayweek1.cpp:388-393). */
@@ -168,14 +169,16 @@ const char *r1_kernel_name(r1_scene *scene, int variant);
 /* Host only (no device needed): the sphere operand of the tensor-core filter for this scene -- n32 rows (sphere count padded to
  * 32) of 128 bytes: 32 TF32 words {hi x 11 | hi x 11 | lo x 10} of the 11 lifted features in the tcgen05 K-major no-swizzle
  * layout, byte offset of (row r, word k) = (r / 8) * 1024 + (k / 4) * 128 + (r % 8) * 16 + (k % 4) * 4.  out = NULL: only
- * *n32_out is set.  R1_ERR_LIMIT for empty scenes and above 768 spheres. */
+ * *n32_out is set.  R1_ERR_LIMIT for empty scenes and above 768 spheres.  Built from the host scene: spheres moved on a device by
+ * r1_scene_move_spheres are not seen here (r1_scene_export_device returns a device's operand). */
 int r1_tensor_operand(const r1_scene *scene, void *out, uint64_t out_bytes, uint32_t *n32_out);
 /* Host only (no device needed): the BVH of R1_VARIANT_MEGAKERNEL_BVH for this scene, built now if it is not cached yet (adding
  * spheres drops the cached tree).  nodes: n_nodes x 64 bytes {float lo0[3], hi0[3], lo1[3], hi1[3]; int32 child[2]; float diag[2]},
  * node 0 = root; child >= 0: inner node, child < 0: leaf with ~child = first record << 3 | count (1 .. 4), child = -1: none;
  * diag = bound on the box's diagonal.  leaves: n_leaf_records x 32 bytes {float cx, cy, cz, radius_sq (the scene's values); int32
  * sphere index; 3 x 0}, ascending index within a leaf.  Spheres with inv_radius == 0 are not in the tree.  depth = deepest inner
- * node (root = 1), at most 64.  A NULL buffer skips that copy (the counts are still returned). */
+ * node (root = 1), at most 64.  A NULL buffer skips that copy (the counts are still returned).  Built from the host scene: spheres
+ * moved on a device by r1_scene_move_spheres are not seen here (r1_bvh_export_device returns a device's tree). */
 int r1_bvh_export(const r1_scene *scene, void *nodes, uint64_t nodes_bytes, void *leaves, uint64_t leaves_bytes, uint32_t *n_nodes,
                   uint32_t *n_leaf_records, uint32_t *depth);
 /* Builders of r1_scene_build_bvh.  HOST: the tree r1_bvh_export returns (binned SAH, built on the host and cached in the scene).
@@ -194,6 +197,27 @@ int r1_scene_build_bvh(r1_scene *scene, int device, int builder, double *device_
  * for a null scene or a buffer smaller than the tree.  A NULL buffer skips that copy (the counts are still returned). */
 int r1_bvh_export_device(r1_scene *scene, int device, void *nodes, uint64_t nodes_bytes, void *leaves, uint64_t leaves_bytes,
                          uint32_t *n_nodes, uint32_t *n_leaf_records, uint32_t *depth);
+/* Moves spheres first .. first + n - 1 of the scene committed on `device` (< 0: device of the last commit), for animated scenes.
+ * d_centre: n x 3 floats (xyz interleaved).  d_radius: n floats, or NULL to keep the radii.  Both are DEVICE pointers on that device.
+ * The device's records of those spheres become exactly what r1_scene_commit writes for a scene with these values (radius_sq =
+ * radius * radius and inv_radius = radius > 0 ? 1 / radius : 0, as r1_scene_add_sphere derives them; materials are kept).
+ * If the device holds a BVH, it is refitted in place (same topology, new boxes and leaf records; DESIGN.md section 4.10).
+ * Runs on cuda_stream (NULL = legacy default stream) and returns when that work is done.
+ * device_ms (optional): CUDA events around the device work.
+ * Only that device changes.  The host scene keeps its values: r1_scene_get_soa, r1_tensor_operand and r1_bvh_export still describe
+ * the committed scene, and a re-commit restores its records there and drops the device's tree.  After a move, a BVH render or trace
+ * on a device without a tree is refused (R1_ERR_STATE) instead of uploading the host tree, and so is r1_scene_build_bvh with
+ * R1_BVH_BUILD_HOST; R1_BVH_BUILD_DEVICE builds from the moved records.
+ * R1_ERR_ARG: null scene; first + n > count (no wrap in uint32); n > 0 with a null d_centre; a sphere whose new radius changes
+ *   whether it can be hit (inv_radius != 0 before and after); a sphere that can be hit with a non-finite centre or radius_sq
+ *   (the rule of the device builder).  Nothing is written in any of these cases.
+ * R1_ERR_STATE: not committed there, or the spheres changed on the host since the commit. */
+int r1_scene_move_spheres(r1_scene *scene, int device, uint32_t first, uint32_t n, const float *d_centre, const float *d_radius,
+                          void *cuda_stream, double *device_ms);
+/* The device's scene records ([scan | exact | shade | tensor operand], the layout r1_scene_commit uploads), for parity checks:
+ * *bytes = the layout's size.  out = NULL: only *bytes is set.  R1_ERR_ARG for a null scene or out_bytes < *bytes, R1_ERR_STATE if
+ * the scene is not committed to `device` (< 0: device of the last commit). */
+int r1_scene_export_device(r1_scene *scene, int device, void *out, uint64_t out_bytes, uint64_t *bytes);
 /* Values of the tensor-core FILTER (R1_VARIANT_MEGAKERNEL_TENSOR) for n rays against every sphere: e[ray * n32 + sphere], n32 =
  * sphere count padded to 32; the filter flags a sphere iff the sign bit of e is clear, and must flag every sphere Hitable::hit's
  * discriminant test (rayweek1.cpp:192-204) accepts.  layout must be 0 (the renderer's operand layout); any other value returns

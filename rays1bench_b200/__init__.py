@@ -93,6 +93,8 @@ def _load():
         "r1_bvh_export": (ci, [vp, vp, C.c_uint64, vp, C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
         "r1_scene_build_bvh": (ci, [vp, ci, ci, C.POINTER(C.c_double)]),
         "r1_bvh_export_device": (ci, [vp, ci, vp, C.c_uint64, vp, C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+        "r1_scene_move_spheres": (ci, [vp, ci, C.c_uint32, C.c_uint32, vp, vp, vp, C.POINTER(C.c_double)]),
+        "r1_scene_export_device": (ci, [vp, ci, vp, C.c_uint64, C.POINTER(C.c_uint64)]),
         "r1_scatter": (ci, [vp, ci, f32p, f32p, f32p, i32p, f32p, f32p, i32p, f32p, f32p]),
         "r1_get_ray": (ci, [vp, ci, f32p, f32p, f32p, f32p, f32p]),
         "r1_replay_pixels": (ci, [vp, ci, i32p, ci, ci, ci, ci, u32p, u32p, f32p, u32p]),
@@ -275,6 +277,48 @@ class Scene:
         _check(lib.r1_bvh_export_device(self.handle, device, nodes.ctypes.data, nodes.nbytes, leaves.ctypes.data if nl.value else None,
                                         leaves.nbytes, C.byref(nn), C.byref(nl), C.byref(depth)), "r1_bvh_export_device")
         return nodes, leaves, int(depth.value)
+
+    def move_spheres(self, centres, radii=None, first=0, device=-1, stream=None):
+        """r1_scene_move_spheres: moves spheres first .. first + n - 1 on one device to `centres` (torch float32 CUDA tensor, contiguous,
+        shape (n, 3)) and, if given, `radii` (shape (n,)); the device's BVH, if it holds one, is refitted in place.  device: -1 = the
+        tensors' device (the scene must be committed there).  stream: a torch.cuda.Stream or raw cudaStream_t handle; default: torch's
+        current stream on that device, so the move is ordered after whatever produced the tensors.  Returns when the move is done,
+        with its device time in ms.  The host scene (soa(), bvh(), tensor_operand()) keeps its committed values."""
+        import torch
+        tensors = [("centres", centres, 2)] + ([("radii", radii, 1)] if radii is not None else [])
+        for what, t, dims in tensors:
+            if not isinstance(t, torch.Tensor) or not t.is_cuda:
+                raise ValueError("%s must be a torch CUDA tensor" % what)
+            if t.dtype != torch.float32:
+                raise ValueError("%s must be float32, not %s" % (what, t.dtype))
+            if not t.is_contiguous():
+                raise ValueError("%s must be contiguous" % what)
+        n = centres.shape[0] if centres.dim() == 2 else -1
+        if centres.dim() != 2 or centres.shape[1] != 3:
+            raise ValueError("centres must have shape (n, 3), not %s" % (tuple(centres.shape),))
+        if radii is not None and tuple(radii.shape) != (n,):
+            raise ValueError("radii must have shape (%d,), not %s" % (n, tuple(radii.shape)))
+        dev = centres.device.index if device is None or device < 0 else device
+        for what, t, _ in tensors:
+            if t.device.index != dev:
+                raise ValueError("%s is on cuda:%d, the move runs on device %d" % (what, t.device.index, dev))
+        if stream is None:
+            stream = torch.cuda.current_stream(dev)
+        handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
+        ms = C.c_double(0)
+        _check(lib.r1_scene_move_spheres(self.handle, dev, first, n, C.c_void_p(centres.data_ptr() if n else None),
+                                         C.c_void_p(radii.data_ptr() if radii is not None and n else None), C.c_void_p(handle or None),
+                                         C.byref(ms)), "r1_scene_move_spheres")
+        return ms.value
+
+    def device_records(self, device=-1):
+        """r1_scene_export_device: the records `device` (-1: the device of the last commit) holds for this scene, as uint8 bytes in
+        r1_scene_commit's layout [scan | exact | shade | tensor operand]."""
+        nb = C.c_uint64(0)
+        _check(lib.r1_scene_export_device(self.handle, device, None, 0, C.byref(nb)), "r1_scene_export_device")
+        out = np.zeros(nb.value, np.uint8)
+        _check(lib.r1_scene_export_device(self.handle, device, out.ctypes.data, out.nbytes, C.byref(nb)), "r1_scene_export_device")
+        return out
 
     def filter_probe(self, org, dir_, n_spheres, layout=0):
         """r1_filter_probe: values of the tensor-core filter, shape (rays, n32); sign bit clear = sphere flagged."""

@@ -44,7 +44,7 @@ def build(force=False, verbose=False):
     extra = ["-Xptxas", "-v"] if verbose else []
     if force or _stale(LIB, srcs):
         cmd = [nvcc, *ARCH, *COMMON, *extra, "-shared", "-o", LIB, os.path.join(CSRC, "r1_core.cu"), os.path.join(CSRC, "r1_bvh_device.cu"),
-               os.path.join(CSRC, "rays1_host.cpp"),
+               os.path.join(CSRC, "r1_move.cu"), os.path.join(CSRC, "rays1_host.cpp"),
                "-lcudart", "-ldl"]
         subprocess.run(cmd, check=True)
     if force or _stale(EXE, srcs + [LIB]):

@@ -55,6 +55,11 @@ __device__ __forceinline__ float unordered(unsigned int u) { return __uint_as_fl
 
 __device__ __forceinline__ bool finite4(float4 v) { return isfinite(v.x) && isfinite(v.y) && isfinite(v.z) && isfinite(v.w); }
 
+// step 1: the padded box of a sphere, [box_lo(c_k, rp), box_hi(c_k, rp)] per axis with rp = padded_radius(radius_sq)
+__device__ __forceinline__ double padded_radius(float r2) { return __dmul_rn(__dsqrt_rn((double)r2), bvh::kRadiusPad); }
+__device__ __forceinline__ float box_lo(float c, double rp) { return __double2float_rd(__dsub_rn((double)c, rp)); }
+__device__ __forceinline__ float box_hi(float c, double rp) { return __double2float_ru(__dadd_rn((double)c, rp)); }
+
 // step 1 for every sphere; centroid bounds and the real-sphere count
 __global__ void __launch_bounds__(kThreads) lbvh_boxes(const float4 *__restrict__ exact, const float4 *__restrict__ shade, uint32_t n,
                                                        float4 *__restrict__ box, Header *hdr)
@@ -64,12 +69,12 @@ __global__ void __launch_bounds__(kThreads) lbvh_boxes(const float4 *__restrict_
     if (shade[2 * (size_t)i + 1].x == 0.0f) return;               // inv_radius == 0: never hit, not in the tree
     const float4 e = exact[i];
     if (!finite4(e)) { atomicOr(&hdr->error, 1u); return; }
-    const double rp = __dmul_rn(__dsqrt_rn((double)e.w), bvh::kRadiusPad);
+    const double rp = padded_radius(e.w);
     const float c[3] = { e.x, e.y, e.z };
     float lo[3], hi[3];
     for (int k = 0; k < 3; ++k) {
-        lo[k] = __double2float_rd(__dsub_rn((double)c[k], rp));
-        hi[k] = __double2float_ru(__dadd_rn((double)c[k], rp));
+        lo[k] = box_lo(c[k], rp);
+        hi[k] = box_hi(c[k], rp);
         atomicMin(&hdr->bounds[k], ordered(c[k]));
         atomicMax(&hdr->bounds[3 + k], ordered(c[k]));
     }
@@ -271,6 +276,91 @@ __global__ void lbvh_small_root(const unsigned long long *__restrict__ keys, int
     put_node(nodes, lo, hi, put_leaf(keys, exact, 0, m, leaves), zero, zero, bvh::kEmpty);
 }
 
+// ---- refit (DESIGN.md section 4.10): new boxes and leaf records for moved spheres, same topology ---------------------------------
+//
+// Works on any tree in r1_bvh.h's layout, whichever builder made it and however its nodes are numbered (node 0 is the root).  Every
+// slot whose child is not kEmpty gets the float union of the padded boxes (step 1) of the spheres under it and its diagonal bound;
+// every leaf record gets the scene's new exact record.  Empty slots and child references keep their bytes.
+
+// parent[v] = p << 1 | slot for every node v referenced by slot `slot` of node p; the root keeps the -1 it was filled with
+__global__ void __launch_bounds__(kThreads) refit_parents(const float4 *__restrict__ nodes, uint32_t n_nodes, int *__restrict__ parent)
+{
+    const uint32_t v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= n_nodes) return;
+    const float4 c = nodes[4 * (size_t)v + 3];
+    const int32_t ref[2] = { __float_as_int(c.x), __float_as_int(c.y) };
+    for (int slot = 0; slot < 2; ++slot)
+        if (ref[slot] >= 0) parent[ref[slot]] = (int)(v << 1) | slot;
+}
+
+// writes a slot's box and diagonal bound; 4-byte stores, because the two slots of a node share float4s and may be written by two threads
+__device__ __forceinline__ void put_slot(float4 *node, int slot, float4 lo, float4 hi)
+{
+    float *f = reinterpret_cast<float *>(node);
+    __stcg(f + 6 * slot + 0, lo.x); __stcg(f + 6 * slot + 1, lo.y); __stcg(f + 6 * slot + 2, lo.z);
+    __stcg(f + 6 * slot + 3, hi.x); __stcg(f + 6 * slot + 4, hi.y); __stcg(f + 6 * slot + 5, hi.z);
+    __stcg(f + 14 + slot, diag_bound(lo, hi));
+}
+
+__device__ __forceinline__ void get_slot(const float4 *node, int slot, float4 &lo, float4 &hi)
+{
+    const float *f = reinterpret_cast<const float *>(node);
+    lo = make_float4(__ldcg(f + 6 * slot + 0), __ldcg(f + 6 * slot + 1), __ldcg(f + 6 * slot + 2), 0.0f);
+    hi = make_float4(__ldcg(f + 6 * slot + 3), __ldcg(f + 6 * slot + 4), __ldcg(f + 6 * slot + 5), 0.0f);
+}
+
+__device__ __forceinline__ int inner_children(int32_t r0, int32_t r1) { return (r0 >= 0 ? 1 : 0) + (r1 >= 0 ? 1 : 0); }
+
+// One thread per node: the boxes of its leaf slots (and their records), then an arrival at the node.  A node is complete after 1 +
+// (its inner children) arrivals; the last arriving thread writes the node's box into its parent's slot and arrives there.  No thread
+// waits for another, and float min / max are exact, so the arrival order cannot show.
+__global__ void __launch_bounds__(kThreads) refit_nodes(float4 *__restrict__ nodes, float4 *__restrict__ leaves, uint32_t n_nodes,
+                                                       const float4 *__restrict__ exact, const int *__restrict__ parent, unsigned int *arrivals)
+{
+    const uint32_t v0 = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v0 >= n_nodes) return;
+    const float inf = __int_as_float(0x7f800000);
+    {
+        float4 *node = nodes + 4 * (size_t)v0;
+        const float4 c = node[3];
+        const int32_t ref[2] = { __float_as_int(c.x), __float_as_int(c.y) };
+        for (int slot = 0; slot < 2; ++slot) {
+            if (ref[slot] >= 0 || ref[slot] == bvh::kEmpty) continue;
+            const uint32_t v = ~(uint32_t)ref[slot], first = v >> 3, count = v & 7u;
+            float4 lo = make_float4(inf, inf, inf, 0.0f), hi = make_float4(-inf, -inf, -inf, 0.0f);
+            for (uint32_t a = 0; a < count; ++a) {
+                const size_t rec = first + a;
+                const float4 e = exact[__float_as_int(leaves[2 * rec + 1].x)];
+                leaves[2 * rec] = e;
+                const double rp = padded_radius(e.w);
+                lo = make_float4(fminf(lo.x, box_lo(e.x, rp)), fminf(lo.y, box_lo(e.y, rp)), fminf(lo.z, box_lo(e.z, rp)), 0.0f);
+                hi = make_float4(fmaxf(hi.x, box_hi(e.x, rp)), fmaxf(hi.y, box_hi(e.y, rp)), fmaxf(hi.z, box_hi(e.z, rp)), 0.0f);
+            }
+            put_slot(node, slot, lo, hi);
+        }
+    }
+    for (uint32_t v = v0;;) {
+        const float4 *node = nodes + 4 * (size_t)v;
+        const int32_t r0 = __float_as_int(__ldcg(reinterpret_cast<const float *>(node) + 12)), r1 = __float_as_int(__ldcg(reinterpret_cast<const float *>(node) + 13));
+        __threadfence();
+        if (atomicAdd(&arrivals[v], 1u) != (unsigned int)inner_children(r0, r1)) return;   // not the last arrival
+        __threadfence();
+        const int p = __ldcg(&parent[v]);
+        if (p < 0) return;                                         // the root: its own box is not stored
+        // the union of the node's used slots; an empty slot (kEmpty) holds zeros, not a box, and is left out whichever slot it is
+        float4 lo = make_float4(inf, inf, inf, 0.0f), hi = make_float4(-inf, -inf, -inf, 0.0f);
+        for (int slot = 0; slot < 2; ++slot) {
+            if ((slot ? r1 : r0) == bvh::kEmpty) continue;
+            float4 l, h;
+            get_slot(node, slot, l, h);
+            lo = make_float4(fminf(lo.x, l.x), fminf(lo.y, l.y), fminf(lo.z, l.z), 0.0f);
+            hi = make_float4(fmaxf(hi.x, h.x), fmaxf(hi.y, h.y), fmaxf(hi.z, h.z), 0.0f);
+        }
+        put_slot(nodes + 4 * (size_t)(p >> 1), p & 1, lo, hi);
+        v = (uint32_t)(p >> 1);
+    }
+}
+
 #define R1_LBVH_CUDA(expr)                                                                                   \
     do {                                                                                                     \
         cudaError_t e_ = (expr);                                                                             \
@@ -367,6 +457,20 @@ int build(const float4 *exact, const float4 *shade, uint32_t n, Built *out, doub
     *out = Built{ blk.p, n_nodes, (uint32_t)m, h.depth };
     blk.p = nullptr;
     if (ms) *ms = tm.ms;
+    return R1_OK;
+}
+
+int refit(float4 *nodes, float4 *leaves, uint32_t n_nodes, const float4 *exact, int *parent, unsigned int *arrivals, bool parents_ready, cudaStream_t stream)
+{
+    const unsigned blocks = (n_nodes + kThreads - 1) / kThreads;
+    if (!parents_ready) {
+        R1_LBVH_CUDA(cudaMemsetAsync(parent, 0xff, (size_t)n_nodes * sizeof(int), stream));
+        refit_parents<<<blocks, kThreads, 0, stream>>>(nodes, n_nodes, parent);
+        R1_LBVH_CUDA(cudaGetLastError());
+    }
+    R1_LBVH_CUDA(cudaMemsetAsync(arrivals, 0, (size_t)n_nodes * sizeof(unsigned int), stream));
+    refit_nodes<<<blocks, kThreads, 0, stream>>>(nodes, leaves, n_nodes, exact, parent, arrivals);
+    R1_LBVH_CUDA(cudaGetLastError());
     return R1_OK;
 }
 

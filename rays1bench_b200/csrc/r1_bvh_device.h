@@ -42,5 +42,12 @@ struct Built {
 // kernels and the sort.
 int build(const float4 *exact, const float4 *shade, uint32_t n, Built *out, double *ms);
 
+// Refits a tree in r1_bvh.h's layout in place to the scene's exact records (DESIGN.md section 4.10): same topology, child references
+// and record order; every used slot gets the union of the padded boxes of its spheres and their diagonal bound, every leaf record the
+// sphere's exact record.  parent / arrivals: n_nodes words of scratch each; parent is derived from the child references unless
+// parents_ready says it already holds that (it depends on the topology alone).  Asynchronous on `stream`.
+int refit(float4 *nodes, float4 *leaves, uint32_t n_nodes, const float4 *exact, int *parent, unsigned int *arrivals, bool parents_ready,
+          cudaStream_t stream);
+
 }  // namespace lbvh
 }  // namespace r1

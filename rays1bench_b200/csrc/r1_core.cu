@@ -7,6 +7,7 @@
 #include "r1_bvh_device.h"
 #include "r1_internal.h"
 #include "r1_kernels.cuh"
+#include "r1_move.h"
 #include "r1_wavefront.cuh"
 
 #include <chrono>
@@ -44,6 +45,11 @@ struct DeviceCtx {
     void *bvh_block = nullptr;          // R1_VARIANT_MEGAKERNEL_BVH: [nodes | leaf records], uploaded on first use or r1_scene_build_bvh
     const float4 *bvh_nodes = nullptr, *bvh_leaves = nullptr;
     uint32_t bvh_n_nodes = 0, bvh_n_leaves = 0, bvh_depth = 0;
+    // r1_scene_move_spheres: set once spheres were moved here (the records no longer match the host SoA, the host tree no longer fits)
+    bool moved = false;
+    void *refit_block = nullptr;        // the tree's [parent | arrivals] for refits, n_nodes words each; freed with the tree
+    bool refit_parents = false;         // parent holds the tree's parent references
+    unsigned int *move_flag = nullptr;  // result word of the move's value check
 };
 
 // Per-device scratch shared by every scene of the process (pixel accumulators, counters, staging, events).
@@ -105,9 +111,11 @@ constexpr size_t kSceneBlockCache = 4;   // blocks kept per device (<= 4 x 260 K
 void free_ctx(DeviceCtx &c)
 {
     if (c.device < 0) return;
-    if (c.bvh_block) {
+    if (c.bvh_block || c.refit_block || c.move_flag) {
         cudaSetDevice(c.device);
-        cudaFree(c.bvh_block);
+        if (c.bvh_block) cudaFree(c.bvh_block);
+        if (c.refit_block) cudaFree(c.refit_block);
+        if (c.move_flag) cudaFree(c.move_flag);
     }
     bool kept = false;
     {
@@ -403,6 +411,9 @@ int scene_bvh(r1_scene *scene, const r1::bvh::Bvh **out)
 void set_ctx_bvh(DeviceCtx &c, void *blk, uint32_t n_nodes, uint32_t n_leaves, uint32_t depth)
 {
     if (c.bvh_block) cudaFree(c.bvh_block);
+    if (c.refit_block) cudaFree(c.refit_block);
+    c.refit_block = nullptr;
+    c.refit_parents = false;
     c.bvh_block = blk;
     c.bvh_nodes = static_cast<const float4 *>(blk);
     c.bvh_leaves = reinterpret_cast<const float4 *>(static_cast<unsigned char *>(blk) + (size_t)n_nodes * sizeof(r1::bvh::Node));
@@ -434,6 +445,8 @@ int upload_bvh(DeviceCtx &c, const r1::bvh::Bvh &b, double *ms)
 int ctx_bvh(r1_scene *scene, DeviceCtx &c)
 {
     if (c.bvh_block) return R1_OK;
+    if (c.moved)
+        return fail(R1_ERR_STATE, "spheres were moved on device %d and it holds no bvh of them: build one with r1_scene_build_bvh(..., R1_BVH_BUILD_DEVICE, ...)", c.device);
     if (c.generation != scene->generation) return fail(R1_ERR_STATE, "the scene's spheres changed after it was committed to device %d (commit it again)", c.device);
     const r1::bvh::Bvh *b = nullptr;
     int rc = scene_bvh(scene, &b);
@@ -553,8 +566,10 @@ int r1_scene_add_sphere(r1_scene *scene, float cx, float cy, float cz, float rad
     scene->bvh.reset();
     ++scene->generation;
     scene->cx.push_back(cx); scene->cy.push_back(cy); scene->cz.push_back(cz);
-    scene->radius_sq.push_back(radius * radius);
-    scene->inv_radius.push_back(radius > 0 ? (1.0f / radius) : 0);
+    float radius_sq, inv_radius;
+    r1::enc::radius_terms(radius, radius_sq, inv_radius);   // r1_encode.h: r1_scene_move_spheres derives new radii's terms the same way
+    scene->radius_sq.push_back(radius_sq);
+    scene->inv_radius.push_back(inv_radius);
     scene->kind.push_back(mat_kind);
     scene->albedo.push_back(r); scene->albedo.push_back(g); scene->albedo.push_back(b);
     scene->param.push_back(param);
@@ -665,7 +680,6 @@ int r1_scene_commit(r1_scene *scene, int device)
 
     const int n = (int)scene->cx.size();
     const int n_pad = (n + 15) / 16 * 16;  // one scan supergroup = 16 spheres (the reference pads to SIMD_WIDTH = 8, rayweek1.cpp:575)
-    const float inf = std::numeric_limits<float>::infinity();
     // host image of the device block: [scan n_pad f4 | exact n_pad f4 | shade n_pad x 2 f4 | tensor-filter operand n32 x 128 B].
     // The operand is built for every scene: the streamed filter (r1::tcs_operand) finds it after `shade` at any size, while `tcb`,
     // the resident filter's pointer, stays null above tc::kMaxSpheres.
@@ -679,21 +693,9 @@ int r1_scene_commit(r1_scene *scene, int device)
     float4 *shade = exact + n_pad;
     for (int i = 0; i < n_pad; ++i) {
         const bool real = i < n && scene->inv_radius[i] != 0;  // rayweek1.cpp:288-292: inv_radius == 0 spheres never hit
-        // supergroup layout (r1_device.cuh): group g = i / 4 at float4 index (g >> 2) * 16 + (g & 3); cy / cz / r2f at +4 / +8 / +12
-        const int g = i / 4, k = i % 4, f4 = (g >> 2) * 16 + (g & 3);
-        scan[4 * (f4 + 0) + k] = real ? -scene->cx[i] : 0.0f;
-        scan[4 * (f4 + 4) + k] = real ? -scene->cy[i] : 0.0f;
-        scan[4 * (f4 + 8) + k] = real ? -scene->cz[i] : 0.0f;
-        // kk = |c|^2 - r^2 - 2^-17 |c|^2, evaluated in double and rounded DOWN (r1_device.cuh "Filter arithmetic")
-        if (real) {
-            const double c2 = (double)scene->cx[i] * scene->cx[i] + (double)scene->cy[i] * scene->cy[i] + (double)scene->cz[i] * scene->cz[i];
-            const double kk = c2 - (double)scene->radius_sq[i] - c2 / 131072.0;
-            float kf = (float)kk;
-            if ((double)kf > kk) kf = std::nextafter(kf, -inf);
-            scan[4 * (f4 + 12) + k] = std::nextafter(kf, -inf);
-        } else {
-            scan[4 * (f4 + 12) + k] = inf;
-        }
+        // supergroup lanes and kk (r1_encode.h; r1_scene_move_spheres encodes moved spheres with the same function on the device)
+        if (real) r1::enc::scan_lanes(scan, i, true, scene->cx[i], scene->cy[i], scene->cz[i], scene->radius_sq[i]);
+        else r1::enc::scan_lanes(scan, i, false, 0.0f, 0.0f, 0.0f, 0.0f);
         int32_t kind = R1_MAT_NONE;
         float inv_r = 0.0f;
         if (i < n) {
@@ -1009,6 +1011,8 @@ int r1_scene_build_bvh(r1_scene *scene, int device, int builder, double *device_
     if (cp->generation != scene->generation) return fail(R1_ERR_STATE, "the scene's spheres changed after it was committed to device %d (commit it again)", cp->device);
     double ms = 0;
     if (builder == R1_BVH_BUILD_HOST) {
+        if (cp->moved)
+            return fail(R1_ERR_STATE, "spheres were moved on device %d: the host tree describes the committed positions (build with R1_BVH_BUILD_DEVICE, or commit again)", cp->device);
         const r1::bvh::Bvh *b = nullptr;
         R1_TRY(scene_bvh(scene, &b));
         R1_TRY(upload_bvh(*cp, *b, &ms));
@@ -1037,6 +1041,68 @@ int r1_bvh_export_device(r1_scene *scene, int device, void *nodes, uint64_t node
     R1_CUDA(cudaSetDevice(c.device));
     if (nodes) R1_CUDA(cudaMemcpy(nodes, c.bvh_nodes, nb, cudaMemcpyDeviceToHost));
     if (leaves && lb) R1_CUDA(cudaMemcpy(leaves, c.bvh_leaves, lb, cudaMemcpyDeviceToHost));
+    return R1_OK;
+}
+
+int r1_scene_move_spheres(r1_scene *scene, int device, uint32_t first, uint32_t n, const float *d_centre, const float *d_radius, void *cuda_stream,
+                          double *device_ms)
+{
+    if (!scene) return fail(R1_ERR_ARG, "null scene");
+    const uint64_t count = scene->cx.size();
+    if ((uint64_t)first + n > count)
+        return fail(R1_ERR_ARG, "spheres %u .. %u + %u - 1 are out of range (the scene has %llu)", first, first, n, (unsigned long long)count);
+    if (n > 0 && !d_centre) return fail(R1_ERR_ARG, "null centres");
+    DeviceCtx *cp = nullptr;
+    R1_TRY(get_ctx(scene, &cp, device));
+    DeviceCtx &c = *cp;
+    if (c.generation != scene->generation) return fail(R1_ERR_STATE, "the scene's spheres changed after it was committed to device %d (commit it again)", c.device);
+    if (device_ms) *device_ms = 0;
+    if (n == 0) return R1_OK;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    if (!c.move_flag) R1_CUDA(cudaMalloc(&c.move_flag, 16));
+    if (c.bvh_block && !c.refit_block) R1_CUDA(cudaMalloc(&c.refit_block, (size_t)c.bvh_n_nodes * 8 + 16));
+    struct Events {
+        cudaEvent_t a = nullptr, b = nullptr;
+        ~Events() { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); }
+    } ev;
+    if (device_ms) { R1_CUDA(cudaEventCreate(&ev.a)); R1_CUDA(cudaEventCreate(&ev.b)); R1_CUDA(cudaEventRecord(ev.a, stream)); }
+    float4 *block = static_cast<float4 *>(c.block);
+    const r1::move::Records rec = { block, block + c.dev.n_pad, block + 2 * (size_t)c.dev.n_pad,
+                                    static_cast<unsigned char *>(c.block) + (size_t)c.dev.n_pad * (16 + 16 + 32) };
+    R1_TRY(r1::move::check(rec, first, n, d_centre, d_radius, c.move_flag, stream));   // nothing is written unless every value passes
+    R1_TRY(r1::move::encode(rec, first, n, d_centre, d_radius, stream));
+    c.moved = true;                                                // the records no longer match the host scene
+    if (c.bvh_block) {
+        int *parent = static_cast<int *>(c.refit_block);
+        unsigned int *arrivals = reinterpret_cast<unsigned int *>(parent + c.bvh_n_nodes);
+        float4 *nodes = static_cast<float4 *>(c.bvh_block);
+        R1_TRY(r1::lbvh::refit(nodes, const_cast<float4 *>(c.bvh_leaves), c.bvh_n_nodes, rec.exact, parent, arrivals, c.refit_parents, stream));
+        c.refit_parents = true;
+    }
+    if (device_ms) {
+        R1_CUDA(cudaEventRecord(ev.b, stream));
+        R1_CUDA(cudaEventSynchronize(ev.b));
+        float ms = 0;
+        R1_CUDA(cudaEventElapsedTime(&ms, ev.a, ev.b));
+        *device_ms = ms;
+    }
+    R1_CUDA(cudaStreamSynchronize(stream));
+    return R1_OK;
+}
+
+int r1_scene_export_device(r1_scene *scene, int device, void *out, uint64_t out_bytes, uint64_t *bytes)
+{
+    if (!scene) return fail(R1_ERR_ARG, "null scene");
+    if (device < 0) device = scene->current;
+    auto it = scene->ctx.find(device);
+    if (device < 0 || it == scene->ctx.end()) return fail(R1_ERR_STATE, "scene not committed to device %d (call r1_scene_commit)", device);
+    const DeviceCtx &c = it->second;
+    const uint64_t nb = (uint64_t)c.dev.n_pad * (16 + 16 + 32) + (uint64_t)c.dev.n32 * r1::tc::kRowBytes;   // r1_scene_commit's layout
+    if (bytes) *bytes = nb;
+    if (!out) return R1_OK;
+    if (out_bytes < nb) return fail(R1_ERR_ARG, "record buffer too small: %llu < %llu bytes", (unsigned long long)out_bytes, (unsigned long long)nb);
+    R1_CUDA(cudaSetDevice(c.device));
+    R1_CUDA(cudaMemcpy(out, c.block, nb, cudaMemcpyDeviceToHost));
     return R1_OK;
 }
 

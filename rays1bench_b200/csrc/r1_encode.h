@@ -1,0 +1,187 @@
+// r1_encode.h -- the device records of one sphere, in one definition for the host and the device: r1_scene_commit encodes a scene
+// with these functions on the host, and r1_scene_move_spheres (r1_move.cu) re-encodes moved spheres with them on the device.  The
+// two must write the same bytes (DESIGN.md section 4.10), so every double operation goes through dmul / dadd / dsub / ddiv, which
+// are the _rn intrinsics on the device (nvcc would otherwise contract a product and a sum into an FMA) and the plain operators on
+// the host.  Conversions between float and double are exact (float -> double) or round to nearest (double -> float) on both.
+//
+// Records of sphere i in the committed block [scan | exact | shade | tensor operand]:
+//   scan    supergroup lanes -cx, -cy, -cz, kk (r1_device.cuh "Filter arithmetic"): scan_lanes
+//   exact   {cx, cy, cz, radius_sq}
+//   shade   [2i] material, [2i + 1] {inv_radius, kind, 1 / ior, r0}: only inv_radius depends on the geometry
+//   operand the sphere's row of the tensor-core filter's B operand (r1_tensor.cuh): sphere_row_words
+#pragma once
+#include <cuda_runtime.h>
+#include <stdint.h>
+
+#include <cmath>
+#include <cstring>
+
+#define R1_HD __host__ __device__ __forceinline__
+
+namespace r1 {
+namespace enc {
+
+R1_HD double dmul(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+R1_HD double dadd(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __dadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+R1_HD double dsub(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __dsub_rn(a, b);
+#else
+    return a - b;
+#endif
+}
+R1_HD double ddiv(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __ddiv_rn(a, b);
+#else
+    return a / b;
+#endif
+}
+R1_HD uint32_t bits(float x)
+{
+    uint32_t b;
+    memcpy(&b, &x, 4);
+    return b;
+}
+R1_HD float from_bits(uint32_t b)
+{
+    float x;
+    memcpy(&x, &b, 4);
+    return x;
+}
+R1_HD float neg(float x) { return from_bits(bits(x) ^ 0x80000000u); }   // the sign flip of the host's unary minus, NaN included
+
+// r1_scene_add_sphere's derived values (SphereSOA::add, soa_sphere.cpp:70-85): radius * radius and radius > 0 ? 1 / radius : 0, IEEE
+R1_HD void radius_terms(float radius, float &radius_sq, float &inv_radius)
+{
+#ifdef __CUDA_ARCH__
+    radius_sq = __fmul_rn(radius, radius);
+    inv_radius = radius > 0 ? __fdiv_rn(1.0f, radius) : 0.0f;
+#else
+    radius_sq = radius * radius;
+    inv_radius = radius > 0 ? (1.0f / radius) : 0;
+#endif
+}
+
+// The four scan lanes of sphere i in the supergroup layout (r1_device.cuh): group g = i / 4 at float4 index (g >> 2) * 16 + (g & 3);
+// cy / cz / kk at +4 / +8 / +12.  kk = |c|^2 - r^2 - 2^-17 |c|^2, evaluated in double, rounded down, then one more ulp down.  A sphere
+// that can never be hit (`real` false) gets 0, 0, 0, +inf: no ray flags it.
+R1_HD void scan_lanes(float *scan, int i, bool real, float cx, float cy, float cz, float radius_sq)
+{
+    const int g = i / 4, k = i % 4, f4 = (g >> 2) * 16 + (g & 3);
+    const float inf = from_bits(0x7f800000u);
+    scan[4 * (f4 + 0) + k] = real ? neg(cx) : 0.0f;
+    scan[4 * (f4 + 4) + k] = real ? neg(cy) : 0.0f;
+    scan[4 * (f4 + 8) + k] = real ? neg(cz) : 0.0f;
+    if (real) {
+        const double c2 = dadd(dadd(dmul((double)cx, (double)cx), dmul((double)cy, (double)cy)), dmul((double)cz, (double)cz));
+        const double kk = dsub(dsub(c2, (double)radius_sq), ddiv(c2, 131072.0));
+        float kf = (float)kk;
+        if ((double)kf > kk) kf = nextafterf(kf, -inf);
+        scan[4 * (f4 + 12) + k] = nextafterf(kf, -inf);
+    } else {
+        scan[4 * (f4 + 12) + k] = inf;
+    }
+}
+
+}  // namespace enc
+
+namespace tc {
+
+constexpr int kFeatures = 11;
+constexpr int kK = 32;                                  // 4 x (K = 8 tf32)
+constexpr int kRowBytes = kK * 4;                       // one ray / sphere row
+// canonical K-major, no-swizzle operand layout (core matrix = 8 rows x 16 bytes, stored contiguously):
+//   byte offset of (row r, k) = (r / 8) * kSBO + (k / 4) * kLBO + (r % 8) * 16 + (k % 4) * 4
+constexpr uint32_t kLBO = 128;                          // between the core matrices of adjacent K
+constexpr uint32_t kSBO = (kK / 4) * 128;               // between 8-row groups: 1024 bytes
+constexpr int kMaxSpheres = 768;                        // B tile of the whole scene resident in shared memory: 96 KB
+constexpr double kMargin = 1.0 / 65536.0;               // 2^-16 of |c|^2 (sphere side) and of |o|^2 (ray side)
+constexpr float kPadKK = 1.0e30f;                       // padded sphere rows: e = -1e30
+
+__host__ __device__ __forceinline__ uint32_t row_offset(int r, int k) { return (uint32_t)(r >> 3) * kSBO + (uint32_t)(k >> 2) * kLBO + (uint32_t)(r & 7) * 16u + (uint32_t)(k & 3) * 4u; }
+
+// ---- the sphere operand ------------------------------------------------------------------------------------------------------
+R1_HD uint32_t tf32_rna_bits(float x)                   // cvt.rna.tf32.f32: round to nearest, ties away, low 13 bits zero
+{
+    const uint32_t b = enc::bits(x);
+    if ((b & 0x7f800000u) == 0x7f800000u) return b & 0xffffe000u;
+    return (b + 0x1000u) & 0xffffe000u;
+}
+R1_HD void split_tf32(double v, uint32_t &hi, uint32_t &lo)
+{
+    hi = tf32_rna_bits((float)v);
+    lo = tf32_rna_bits((float)enc::dsub(v, (double)enc::from_bits(hi)));
+}
+// The 11 lifted features of one sphere (the B operand's row before the TF32 split); `real` = false for padding and for spheres
+// that can never be hit
+struct Features {
+    double f[kFeatures];
+};
+R1_HD Features sphere_features(bool real, double cx, double cy, double cz, double radius_sq)
+{
+    Features r = { { 0, 0, 0, 0, 0, 0, 0, 0, 0, (double)kPadKK, 0 } };
+    double *f = r.f;
+    if (real) {
+#ifdef __CUDA_ARCH__
+        using namespace enc;
+        const double nx = -cx, ny = -cy, nz = -cz, c2 = dadd(dadd(dmul(cx, cx), dmul(cy, cy)), dmul(cz, cz));
+        f[0] = dmul(nx, nx); f[1] = dmul(ny, ny); f[2] = dmul(nz, nz); f[3] = dmul(nx, ny); f[4] = dmul(nx, nz); f[5] = dmul(ny, nz);
+        f[6] = nx; f[7] = ny; f[8] = nz;
+        f[9] = dsub(dsub(c2, radius_sq), dmul(c2, kMargin));
+#else
+        // The same operations in the same order, spelled with operators: with NaN inputs the host compiler is free to pick which
+        // operand's NaN a product returns, and this spelling keeps the bytes r1_scene_commit has always written for them.  The device
+        // never encodes a NaN (r1_scene_move_spheres refuses them), and for every other input the two spellings round alike.
+        const double nx = -cx, ny = -cy, nz = -cz, c2 = cx * cx + cy * cy + cz * cz;
+        f[0] = nx * nx; f[1] = ny * ny; f[2] = nz * nz; f[3] = nx * ny; f[4] = nx * nz; f[5] = ny * nz;
+        f[6] = nx; f[7] = ny; f[8] = nz;
+        f[9] = c2 - radius_sq - c2 * kMargin;
+#endif
+        f[10] = 1.0;
+    }
+    return r;
+}
+// The 32 words of one sphere row in K order: {hi x 11 | hi x 11 | lo x 10} of the features (the ray side pairs them hi, lo, hi)
+R1_HD void sphere_row_words(bool real, double cx, double cy, double cz, double radius_sq, uint32_t (&w)[kK])
+{
+    const Features ft = sphere_features(real, cx, cy, cz, radius_sq);
+    for (int j = 0; j < kFeatures; ++j) {
+        uint32_t hi, lo;
+        split_tf32(ft.f[j], hi, lo);
+        w[j] = hi;
+        w[kFeatures + j] = hi;
+        if (j < kFeatures - 1) w[2 * kFeatures + j] = lo;
+    }
+}
+// one sphere row of the B tile in shared-memory layout: sphere_row_words, written at row i
+inline void sphere_row_host(unsigned char *tile, int i, bool real, double cx, double cy, double cz, double radius_sq)
+{
+    const Features ft = sphere_features(real, cx, cy, cz, radius_sq);
+    for (int j = 0; j < kFeatures; ++j) {
+        uint32_t hi, lo;
+        split_tf32(ft.f[j], hi, lo);
+        memcpy(tile + row_offset(i, j), &hi, 4);                                // x ray hi
+        memcpy(tile + row_offset(i, kFeatures + j), &hi, 4);                    // x ray lo
+        if (j < kFeatures - 1) memcpy(tile + row_offset(i, 2 * kFeatures + j), &lo, 4);   // x ray hi
+    }
+}
+
+}  // namespace tc
+}  // namespace r1

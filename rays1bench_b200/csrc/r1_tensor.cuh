@@ -11,62 +11,16 @@
 // the K dimension:  K = 11 + 11 + 10 = 32 (the constant sphere feature has no low part) = four K = 8 instructions.
 // Per test the CUDA cores are left with ONE instruction (the sign bit of e into the candidate mask) instead of eight packed FMA.
 // The split products carry 2^-21 relative error and the accumulation order inside the tensor core is not documented, so the
-// margins are wider than the FP32 filter's (kMargin below, against 2^-17); the measured error is in DESIGN.md section 4.0 and
+// margins are wider than the FP32 filter's (kMargin in r1_encode.h, against 2^-17); the measured error is in DESIGN.md section 4.0 and
 // tests/test_gpu_parity.py::test_tensor_filter_is_conservative checks the filter against the exact test on the GPU.
 #pragma once
 #include <cstdint>
 #include <cstring>
 
+#include "r1_encode.h"   // the operand layout and the sphere rows (kFeatures .. sphere_row_host)
+
 namespace r1 {
 namespace tc {
-
-constexpr int kFeatures = 11;
-constexpr int kK = 32;                                  // 4 x (K = 8 tf32)
-constexpr int kRowBytes = kK * 4;                       // one ray / sphere row
-// canonical K-major, no-swizzle operand layout (core matrix = 8 rows x 16 bytes, stored contiguously):
-//   byte offset of (row r, k) = (r / 8) * kSBO + (k / 4) * kLBO + (r % 8) * 16 + (k % 4) * 4
-constexpr uint32_t kLBO = 128;                          // between the core matrices of adjacent K
-constexpr uint32_t kSBO = (kK / 4) * 128;               // between 8-row groups: 1024 bytes
-constexpr int kMaxSpheres = 768;                        // B tile of the whole scene resident in shared memory: 96 KB
-constexpr double kMargin = 1.0 / 65536.0;               // 2^-16 of |c|^2 (sphere side) and of |o|^2 (ray side)
-constexpr float kPadKK = 1.0e30f;                       // padded sphere rows: e = -1e30
-
-__host__ __device__ __forceinline__ uint32_t row_offset(int r, int k) { return (uint32_t)(r >> 3) * kSBO + (uint32_t)(k >> 2) * kLBO + (uint32_t)(r & 7) * 16u + (uint32_t)(k & 3) * 4u; }
-
-// ---- host: the sphere operand ------------------------------------------------------------------------------------------------
-inline uint32_t tf32_rna_host(float x)                  // cvt.rna.tf32.f32: round to nearest, ties away, low 13 bits zero
-{
-    uint32_t b;
-    memcpy(&b, &x, 4);
-    if ((b & 0x7f800000u) == 0x7f800000u) return b & 0xffffe000u;
-    return (b + 0x1000u) & 0xffffe000u;
-}
-inline void split_host(double v, uint32_t &hi, uint32_t &lo)
-{
-    hi = tf32_rna_host((float)v);
-    float hf;
-    memcpy(&hf, &hi, 4);
-    lo = tf32_rna_host((float)(v - (double)hf));
-}
-// one sphere row of the B tile; `real` = false for padding and for spheres that can never be hit
-inline void sphere_row_host(unsigned char *tile, int i, bool real, double cx, double cy, double cz, double radius_sq)
-{
-    double f[kFeatures] = { 0, 0, 0, 0, 0, 0, 0, 0, 0, (double)kPadKK, 0 };
-    if (real) {
-        const double nx = -cx, ny = -cy, nz = -cz, c2 = cx * cx + cy * cy + cz * cz;
-        f[0] = nx * nx; f[1] = ny * ny; f[2] = nz * nz; f[3] = nx * ny; f[4] = nx * nz; f[5] = ny * nz;
-        f[6] = nx; f[7] = ny; f[8] = nz;
-        f[9] = c2 - radius_sq - c2 * kMargin;
-        f[10] = 1.0;
-    }
-    for (int j = 0; j < kFeatures; ++j) {
-        uint32_t hi, lo;
-        split_host(f[j], hi, lo);
-        memcpy(tile + row_offset(i, j), &hi, 4);                                // x ray hi
-        memcpy(tile + row_offset(i, kFeatures + j), &hi, 4);                    // x ray lo
-        if (j < kFeatures - 1) memcpy(tile + row_offset(i, 2 * kFeatures + j), &lo, 4);   // x ray hi
-    }
-}
 
 #ifdef __CUDACC__
 // ---- PTX wrappers ------------------------------------------------------------------------------------------------------------
