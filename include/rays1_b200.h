@@ -159,7 +159,9 @@ int r1_deinterleave_rows(int device, const void *d_gathered, uint64_t stride, vo
  * megakernel_bvh at any sphere count, while every other variant returns R1_ERR_LIMIT above 4096 (they stage the scene in shared memory); WAVEFRONT and DUAL have no per-ray
  * kernel and return R1_ERR_ARG.  t_min must be >= 2^-24
  * (renders use 0.001): below it the exact test's floored square root and the unsigned root keys of COOP and DEFERRED can differ
- * from Hitable::hit, so a smaller t_min or a NaN returns R1_ERR_ARG before any device is touched. */
+ * from Hitable::hit, so a smaller t_min or a NaN returns R1_ERR_ARG before any device is touched.  For every finite origin and
+ * scene every variant returns Hitable::hit's records bit for bit: the expanded filters hold their error bounds for |c|^2 and |o|^2
+ * below 2^120 and flag every sphere that can be hit beyond that (DESIGN.md section 4.1), so far scenes are slow, not wrong. */
 int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, float t_min, float t_max, int variant,
                   int32_t *index, float *t, float *p, float *normal);
 /* Name of the trace kernel `variant` resolves to for this scene with default tuning ("megakernel_tc3", "megakernel_tcs", "megakernel_bvh",
@@ -211,7 +213,9 @@ int r1_bvh_export_device(r1_scene *scene, int device, void *nodes, uint64_t node
  * R1_ERR_ARG: null scene; first + n > count (no wrap in uint32); n > 0 with a null d_centre; a sphere whose new radius changes
  *   whether it can be hit (inv_radius != 0 before and after); a sphere that can be hit with a non-finite centre or radius_sq
  *   (the rule of the device builder).  Nothing is written in any of these cases.
- * R1_ERR_STATE: not committed there, or the spheres changed on the host since the commit. */
+ * R1_ERR_STATE: not committed there, or the spheres changed on the host since the commit.
+ * Any finite position traces and renders like the oracle: spheres with |c|^2 >= 2^120 are encoded as candidates of every ray
+ * (DESIGN.md section 4.1). */
 int r1_scene_move_spheres(r1_scene *scene, int device, uint32_t first, uint32_t n, const float *d_centre, const float *d_radius,
                           void *cuda_stream, double *device_ms);
 /* The device's scene records ([scan | exact | shade | tensor operand], the layout r1_scene_commit uploads), for parity checks:

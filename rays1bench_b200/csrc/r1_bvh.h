@@ -10,8 +10,8 @@
 //   leaf record (32 B):  {cx, cy, cz, radius_sq} bit-equal to the scene's exact record, original sphere index, 3 x 0
 //
 // Node 0 is the root.  Its own box is not stored (every ray tests its two children).  A leaf's records are in ascending index
-// order.  Each sphere's box is [c - rp, c + rp] with rp = sqrt(radius_sq) (1 + 2^-16), evaluated in double and rounded outward
-// to float; an inner box is the union of its spheres' boxes.  The traversal widens every box per ray (r1_device.cuh,
+// order.  Each sphere's box is [c - rp, c + rp] with rp = sqrt(radius_sq) (1 + 2^-16), the exact bounds rounded outward to float
+// (box_lo / box_hi); an inner box is the union of its spheres' boxes.  The traversal widens every box per ray (r1_device.cuh,
 // bvh_child): the two together contain every point the exact test can accept, DESIGN.md section 4.8 derives the bound.
 //
 // Depth: the root is at depth 1; no inner node is deeper than kMaxDepth, which is also the traversal stack size.  Where the SAH
@@ -80,6 +80,22 @@ inline float round_up(double v)
 {
     float f = (float)v;
     if ((double)f < v) f = std::nextafter(f, std::numeric_limits<float>::infinity());
+    return f;
+}
+// The float below / above the exact c - rp / c + rp (rp >= 0).  The double sum rounds; its exact error (Knuth's TwoSum) says on
+// which side of it the exact value lies.  Without it, rp below half a double ulp of c (|c| above 2^53 rp) gave the box [c, c].
+inline float box_lo(float c, double rp)
+{
+    const double v = (double)c - rp, bv = v - (double)c, err = ((double)c - (v - bv)) + (-rp - bv);
+    float f = round_down(v);
+    if ((double)f == v && err < 0) f = std::nextafter(f, -std::numeric_limits<float>::infinity());
+    return f;
+}
+inline float box_hi(float c, double rp)
+{
+    const double v = (double)c + rp, bv = v - (double)c, err = ((double)c - (v - bv)) + (rp - bv);
+    float f = round_up(v);
+    if ((double)f == v && err > 0) f = std::nextafter(f, std::numeric_limits<float>::infinity());
     return f;
 }
 
@@ -234,7 +250,7 @@ inline bool build(const float *cx, const float *cy, const float *cz, const float
         bld.ids.push_back(i);
         const double rp = std::sqrt((double)radius_sq[i]) * kRadiusPad;
         const double c[3] = { cx[i], cy[i], cz[i] };
-        for (int k = 0; k < 3; ++k) { bld.box[i].lo[k] = detail::round_down(c[k] - rp); bld.box[i].hi[k] = detail::round_up(c[k] + rp); }
+        for (int k = 0; k < 3; ++k) { bld.box[i].lo[k] = detail::box_lo((float)c[k], rp); bld.box[i].hi[k] = detail::box_hi((float)c[k], rp); }
     }
     if (bld.ids.size() >= (1u << 28)) return false;
     out.nodes.reserve(bld.ids.size() / 2 + 1);

@@ -5,7 +5,7 @@
 // box and diagonal arithmetic, so the traversal (bvh_trace) and its correctness argument are unchanged.  The tree is a function
 // of the scene alone, specified step by step below, and tests/lbvh_restatement.py restates it on the CPU bit for bit:
 //
-//   1. box of a real sphere (inv_radius != 0): rp = sqrt((double)r2) (1 + 2^-16), [round_down(c - rp), round_up(c + rp)]
+//   1. box of a real sphere (inv_radius != 0): rp = sqrt((double)r2) (1 + 2^-16), [c - rp, c + rp] exactly, rounded outward to float
 //   2. q_k = ext_k > 0 ? min(1023, floor((c_k - lo_k) / ext_k * 1024)) : 0 over the centroid bounds [lo, hi] of the real spheres,
 //      ext_k = hi_k - lo_k, in double; morton = interleave(x -> bit 3b + 2, y -> 3b + 1, z -> 3b)
 //   3. key = morton << 32 | sphere index: unique, sorted ascending over bits [0, 62)
@@ -57,8 +57,9 @@ __device__ __forceinline__ bool finite4(float4 v) { return isfinite(v.x) && isfi
 
 // step 1: the padded box of a sphere, [box_lo(c_k, rp), box_hi(c_k, rp)] per axis with rp = padded_radius(radius_sq)
 __device__ __forceinline__ double padded_radius(float r2) { return __dmul_rn(__dsqrt_rn((double)r2), bvh::kRadiusPad); }
-__device__ __forceinline__ float box_lo(float c, double rp) { return __double2float_rd(__dsub_rn((double)c, rp)); }
-__device__ __forceinline__ float box_hi(float c, double rp) { return __double2float_ru(__dadd_rn((double)c, rp)); }
+// (directed in both steps: the float below / above the exact c -+ rp, even where rp is below half a double ulp of c)
+__device__ __forceinline__ float box_lo(float c, double rp) { return __double2float_rd(__dsub_rd((double)c, rp)); }
+__device__ __forceinline__ float box_hi(float c, double rp) { return __double2float_ru(__dadd_ru((double)c, rp)); }
 
 // step 1 for every sphere; centroid bounds and the real-sphere count
 __global__ void __launch_bounds__(kThreads) lbvh_boxes(const float4 *__restrict__ exact, const float4 *__restrict__ shade, uint32_t n,

@@ -79,18 +79,31 @@ R1_HD void radius_terms(float radius, float &radius_sq, float &inv_radius)
 #endif
 }
 
+// The range of the expanded filters (r1_device.cuh "Filter arithmetic", r1_tensor.cuh; DESIGN.md section 4.1).  Their error bounds
+// are relative and hold while no term overflows, which |c|^2 < 2^120 and |o|^2 < 2^120 guarantee with a wide margin.  A sphere that
+// can be hit with |c|^2 >= 2^120 (double; so from |c| = 2^60 on, and for infinite centres) is a FAR sphere: its filter records make
+// it a candidate of every ray.  A ray with |o|^2 >= 2^120 (float, or NaN) gets filter constants that flag every sphere that can be
+// hit.  The exact test decides both, and placeholders stay out.  From |c| = 2^60 on the margins exceed r^2 of any sphere the
+// ray's line passes within |c| of, so far spheres were candidates of nearly every ray already; the encoding only keeps that true
+// where |c|^2 overflows float (|c| > 2^64).
+constexpr double kFarC2 = 0x1p120;
+constexpr float kFarKK = -0x1p122f;                     // the kk of a far sphere, whose every other lane or feature is 0
+
 // The four scan lanes of sphere i in the supergroup layout (r1_device.cuh): group g = i / 4 at float4 index (g >> 2) * 16 + (g & 3);
 // cy / cz / kk at +4 / +8 / +12.  kk = |c|^2 - r^2 - 2^-17 |c|^2, evaluated in double, rounded down, then one more ulp down.  A sphere
-// that can never be hit (`real` false) gets 0, 0, 0, +inf: no ray flags it.
+// that can never be hit (`real` false) gets 0, 0, 0, +inf: no ray flags it.  A far sphere gets 0, 0, 0, kFarKK: every ray flags it.
 R1_HD void scan_lanes(float *scan, int i, bool real, float cx, float cy, float cz, float radius_sq)
 {
     const int g = i / 4, k = i % 4, f4 = (g >> 2) * 16 + (g & 3);
     const float inf = from_bits(0x7f800000u);
-    scan[4 * (f4 + 0) + k] = real ? neg(cx) : 0.0f;
-    scan[4 * (f4 + 4) + k] = real ? neg(cy) : 0.0f;
-    scan[4 * (f4 + 8) + k] = real ? neg(cz) : 0.0f;
-    if (real) {
-        const double c2 = dadd(dadd(dmul((double)cx, (double)cx), dmul((double)cy, (double)cy)), dmul((double)cz, (double)cz));
+    const double c2 = real ? dadd(dadd(dmul((double)cx, (double)cx), dmul((double)cy, (double)cy)), dmul((double)cz, (double)cz)) : 0.0;
+    const bool far = c2 >= kFarC2;                      // false for NaN: those keep the records r1_scene_commit has always written
+    scan[4 * (f4 + 0) + k] = real && !far ? neg(cx) : 0.0f;
+    scan[4 * (f4 + 4) + k] = real && !far ? neg(cy) : 0.0f;
+    scan[4 * (f4 + 8) + k] = real && !far ? neg(cz) : 0.0f;
+    if (far) {
+        scan[4 * (f4 + 12) + k] = kFarKK;
+    } else if (real) {
         const double kk = dsub(dsub(c2, (double)radius_sq), ddiv(c2, 131072.0));
         float kf = (float)kk;
         if ((double)kf > kk) kf = nextafterf(kf, -inf);
@@ -130,7 +143,8 @@ R1_HD void split_tf32(double v, uint32_t &hi, uint32_t &lo)
     lo = tf32_rna_bits((float)enc::dsub(v, (double)enc::from_bits(hi)));
 }
 // The 11 lifted features of one sphere (the B operand's row before the TF32 split); `real` = false for padding and for spheres
-// that can never be hit
+// that can never be hit.  A far sphere (enc::kFarC2) gets 0 x 9, kFarKK, 1: every live ray row flags it (its feature 10 lies in
+// [-2^120, 2^121], r1_tensor.cuh ray_row), and the idle row (-2^126) does not.
 struct Features {
     double f[kFeatures];
 };
@@ -138,7 +152,11 @@ R1_HD Features sphere_features(bool real, double cx, double cy, double cz, doubl
 {
     Features r = { { 0, 0, 0, 0, 0, 0, 0, 0, 0, (double)kPadKK, 0 } };
     double *f = r.f;
-    if (real) {
+    const bool far = real && enc::dadd(enc::dadd(enc::dmul(cx, cx), enc::dmul(cy, cy)), enc::dmul(cz, cz)) >= enc::kFarC2;
+    if (far) {
+        f[9] = (double)enc::kFarKK;
+        f[10] = 1.0;
+    } else if (real) {
 #ifdef __CUDA_ARCH__
         using namespace enc;
         const double nx = -cx, ny = -cy, nz = -cz, c2 = dadd(dadd(dmul(cx, cx), dmul(cy, cy)), dmul(cz, cz));

@@ -138,20 +138,25 @@ __device__ __forceinline__ uint32_t tf32_rna(float x)
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
     return r;
 }
-// The lifted TF32 row of one ray.  Rays without a path (`live` false) get a row that flags nothing: e = -1e30.
+// The lifted TF32 row of one ray.  Rays without a path (`live` false) get a row that flags nothing: 0 x 9, -1, -2^126, so
+// e = -(kk + 2^126) < 0 for every sphere with r^2 < 2^126, far spheres (r1_encode.h kFarC2) included, and -1e30 for padding.
+// A live ray with |o|^2 >= 2^120 (or NaN) is out of the filter's range (r1_device.cuh "Filter arithmetic"): its row 0 x 9, -1, 2^121
+// flags every sphere that can be hit (e = 2^121 - kk > 0 with kk < 2^120, or kk = -2^122) and no padding row (e = -1e30).  Every
+// row is finite, so no product the tensor core forms is infinite or NaN.
 __device__ __forceinline__ void ray_row(f3 o, f3 d, bool live, uint32_t (&row)[kK])
 {
     float f[kFeatures];
-    const float od = dot3(o, d);
+    const float od = dot3(o, d), oo = dot3(o, o);
     f[0] = fmul(d.x, d.x); f[1] = fmul(d.y, d.y); f[2] = fmul(d.z, d.z);
     f[3] = fmul(fadd(d.x, d.x), d.y); f[4] = fmul(fadd(d.x, d.x), d.z); f[5] = fmul(fadd(d.y, d.y), d.z);
     f[6] = fmul(2.0f, fsub(fmul(od, d.x), o.x)); f[7] = fmul(2.0f, fsub(fmul(od, d.y), o.y)); f[8] = fmul(2.0f, fsub(fmul(od, d.z), o.z));
     f[9] = -1.0f;
-    f[10] = fsub(fmul(od, od), fmul(dot3(o, o), (float)(1.0 - kMargin)));
-    if (!live) {
+    f[10] = fsub(fmul(od, od), fmul(oo, (float)(1.0 - kMargin)));
+    const bool in_range = oo < 0x1p120f;
+    if (!live || !in_range) {
 #pragma unroll
         for (int j = 0; j < 9; ++j) f[j] = 0.0f;
-        f[10] = -kPadKK;
+        f[10] = live ? 0x1p121f : -0x1p126f;
     }
 #pragma unroll
     for (int j = 0; j < kFeatures; ++j) {

@@ -24,6 +24,22 @@ def round_up(v):
     return np.where(f.astype(np.float64) < v, np.nextafter(f, np.float32(np.inf)), f)
 
 
+def box_bounds(c, rp):
+    """float64 centres [k, 3] (float32 values) and radii [k] -> the floats below c - rp and above c + rp, exactly (r1_bvh.h box_lo /
+    box_hi, __dsub_rd / __dadd_ru then directed to float): TwoSum gives the error of the double sum and so the side it rounded to"""
+    out = []
+    for sgn, rnd, step in ((-1.0, round_down, -np.inf), (1.0, round_up, np.inf)):
+        b = sgn * rp[:, None]
+        with np.errstate(invalid="ignore"):                 # infinite centres: err is NaN and the box stays infinite
+            v = c + b
+            bv = v - c
+            err = (c - (v - bv)) + (b - bv)
+        f = rnd(v)
+        off = (f.astype(np.float64) == v) & (err * sgn > 0)
+        out.append(np.where(off, np.nextafter(f, np.float32(step)), f))
+    return out[0], out[1]
+
+
 def spread3(v):
     """bit b of a 10-bit value -> bit 3b"""
     out = np.zeros_like(v, dtype=np.uint64)
@@ -36,7 +52,7 @@ def sphere_boxes(soa, real):
     """step 1: [n_real, 3] lo and hi of the padded sphere boxes, rounded outward to float32"""
     c = np.stack([soa["cx"][real], soa["cy"][real], soa["cz"][real]], 1).astype(np.float64)
     rp = np.sqrt(soa["radius_sq"][real].astype(np.float64)) * RADIUS_PAD
-    return round_down(c - rp[:, None]), round_up(c + rp[:, None])
+    return box_bounds(c, rp)
 
 
 def sorted_keys(soa, real):

@@ -5,7 +5,7 @@ The device refits bottom-up with one thread per node and atomic arrival counters
 result is specified as a function of the tree's topology and the spheres' exact records alone:
   - child references, record order and depth are unchanged; slots with child -1 keep their bytes;
   - every leaf record's {cx, cy, cz, radius_sq} becomes the sphere's exact record;
-  - every other slot gets the float union of the padded sphere boxes [round_down(c - rp), round_up(c + rp)],
+  - every other slot gets the float union of the padded sphere boxes [c - rp, c + rp] rounded outward,
     rp = sqrt((double) r2) (1 + 2^-16), of the spheres under it, and diag = round_up(sqrt(d2) (1 + 1e-12)) of that box.
 `refit(tree, exact)` takes (nodes, leaves, depth) as Scene.bvh() returns them and exact [n, 4] float32 (cx, cy, cz, radius_sq per
 sphere index), and returns the refitted (nodes, leaves, depth)."""
@@ -23,7 +23,7 @@ def record_boxes(ex):
     """padded boxes (lo, hi) [k, 3] float32 of exact records [k, 4] (step 1 of the builders)"""
     rp = np.sqrt(ex[:, 3].astype(np.float64)) * lbvh.RADIUS_PAD
     c = ex[:, :3].astype(np.float64)
-    return lbvh.round_down(c - rp[:, None]), lbvh.round_up(c + rp[:, None])
+    return lbvh.box_bounds(c, rp)
 
 
 def diag_bound(lo, hi):
