@@ -106,6 +106,11 @@ int r1_scene_set_camera(r1_scene *scene, const float lookfrom[3], const float lo
  * camera constants of their own (r1_scene_set_camera itself reproduces the reference's constants bit for bit: it evaluates
  * Camera::init the way gcc -ffast-math folds it for the reference's builders). */
 int r1_scene_set_camera_raw(r1_scene *scene, const float cam[22]);
+/* Host only (no device needed): the 22 constants r1_scene_set_camera installs for these arguments, in r1_scene_get_camera's order --
+ * r1_scene_set_camera is this function followed by r1_scene_set_camera_raw.  For r1_scene_move_camera.  R1_ERR_ARG for a null
+ * pointer. */
+int r1_camera_constants(const float lookfrom[3], const float lookat[3], const float vup[3], float vfov_deg, float aspect, float aperture,
+                        float focus_dist, float out[22]);
 /* SphereSOA::add (soa_sphere.cpp:70-85): stores radius*radius and radius > 0 ? 1/radius : 0.  Metal's `param` is the
  * fuzz (clamped to <= 1 as the Metal ctor does, rayweek1.cpp:424), Dielectric's the refraction index.  Returns the
  * sphere's index (>= 0) or a negative error. */
@@ -116,10 +121,11 @@ int r1_scene_add_sphere(r1_scene *scene, float cx, float cy, float cz, float rad
 int r1_scene_pad(r1_scene *scene, uint32_t multiple);
 uint32_t r1_scene_count(const r1_scene *scene);
 /* Host copies of the SoA arrays, `count` entries each (albedo: 3 per sphere) -- for bit-parity checks.  They describe the scene as
- * built on the host: r1_scene_move_spheres changes a device's records only. */
+ * built on the host: r1_scene_move_spheres and r1_scene_set_materials change a device's records only. */
 int r1_scene_get_soa(const r1_scene *scene, float *cx, float *cy, float *cz, float *radius_sq, float *inv_radius, int32_t *kind,
                      float *albedo, float *param);
-/* out[22] = origin, lower-left corner, horizontal, vertical, u, v, w (3 each), lens radius (rayweek1.cpp:388-393). */
+/* out[22] = origin, lower-left corner, horizontal, vertical, u, v, w (3 each), lens radius (rayweek1.cpp:388-393).  The host's
+ * camera: r1_scene_move_camera changes a device's camera only. */
 int r1_scene_get_camera(const r1_scene *scene, float *out);
 /* Uploads the scan / shading buffers to CUDA device `device` (replicated per device; may be called once per device). */
 int r1_scene_commit(r1_scene *scene, int device);
@@ -218,6 +224,36 @@ int r1_bvh_export_device(r1_scene *scene, int device, void *nodes, uint64_t node
  * (DESIGN.md section 4.1). */
 int r1_scene_move_spheres(r1_scene *scene, int device, uint32_t first, uint32_t n, const float *d_centre, const float *d_radius,
                           void *cuda_stream, double *device_ms);
+/* Installs 22 camera constants (r1_scene_get_camera's order; r1_camera_constants computes them) for renders and parity calls on
+ * `device` (< 0: device of the last commit), for animated scenes.  No upload: the constants reach a kernel by value when it is
+ * launched, so a render already enqueued with r1_render_device keeps the camera it was launched with, and the next one uses the new
+ * camera.  The wavefront variant's cached graph is rebuilt once for a new camera (r1_wavefront_graph_builds).  Values are not
+ * checked, as r1_scene_set_camera_raw does not check them.
+ * State rules (shared with r1_scene_set_materials; DESIGN.md section 4.11): only that device changes; the host scene keeps its
+ * camera (r1_scene_get_camera) and a re-commit restores it there; renders of every variant, r1_get_ray, r1_scatter and
+ * r1_replay_pixels on that device see the new constants; r1_trace_rays reads neither the camera nor the materials.
+ * R1_ERR_ARG: null scene or cam.  R1_ERR_STATE: not committed there, or the spheres changed on the host since the commit. */
+int r1_scene_move_camera(r1_scene *scene, int device, const float cam[22]);
+/* Sets the materials of spheres first .. first + n - 1 of the scene committed on `device` (< 0: device of the last commit), for
+ * animated scenes.  d_kind: n int32 (R1_MAT_*), d_albedo: n x 3 floats (rgb interleaved), d_param: n floats (Metal fuzz, Dielectric
+ * ior), all DEVICE pointers on that device; any one may be NULL to keep that field.  The device's shade records of those spheres
+ * become exactly what r1_scene_commit writes for a scene whose spheres were added with the resulting (kind, albedo, param): Metal's
+ * param clamped to <= 1 as r1_scene_add_sphere does (a NaN fuzz becomes 1; a kept param is clamped when it meets a new Metal kind),
+ * 1 / ior and the Schlick r0 of dielectrics in IEEE float (where an ior makes them NaN -- NaN or infinite ior -- the NaN's bits may
+ * differ from the host's); inv_radius is kept.  Geometry and BVH are untouched: the scan, exact and
+ * tensor-operand records stay, a tree the device holds stays valid, and a BVH render on a device without a tree still uploads the
+ * host tree (unless spheres were moved there).
+ * Runs on cuda_stream (NULL = legacy default stream) and returns when that work is done.  device_ms (optional): CUDA events around
+ * the device work.
+ * State rules: those of r1_scene_move_camera; r1_scene_get_soa still returns the host's materials and r1_scene_export_device the new
+ * shade records.
+ * R1_ERR_ARG: null scene; first + n > count (no wrap in uint32); n > 0 with all three pointers NULL; a kind outside -1 .. 2;
+ *   R1_MAT_NONE for a sphere that can be hit (inv_radius != 0) -- the device form of r1_scene_add_sphere's "radius > 0 needs a
+ *   material" rule, which differs from it only for radius +inf (inv_radius 0: never hit, so NONE is accepted here).  Nothing is
+ *   written in any of these cases.
+ * R1_ERR_STATE: not committed there, or the spheres changed on the host since the commit. */
+int r1_scene_set_materials(r1_scene *scene, int device, uint32_t first, uint32_t n, const int32_t *d_kind, const float *d_albedo,
+                           const float *d_param, void *cuda_stream, double *device_ms);
 /* The device's scene records ([scan | exact | shade | tensor operand], the layout r1_scene_commit uploads), for parity checks:
  * *bytes = the layout's size.  out = NULL: only *bytes is set.  R1_ERR_ARG for a null scene or out_bytes < *bytes, R1_ERR_STATE if
  * the scene is not committed to `device` (< 0: device of the last commit). */

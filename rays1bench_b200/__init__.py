@@ -95,6 +95,9 @@ def _load():
         "r1_bvh_export_device": (ci, [vp, ci, vp, C.c_uint64, vp, C.c_uint64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
         "r1_scene_move_spheres": (ci, [vp, ci, C.c_uint32, C.c_uint32, vp, vp, vp, C.POINTER(C.c_double)]),
         "r1_scene_export_device": (ci, [vp, ci, vp, C.c_uint64, C.POINTER(C.c_uint64)]),
+        "r1_camera_constants": (ci, [f32p, f32p, f32p, cf, cf, cf, cf, f32p]),
+        "r1_scene_move_camera": (ci, [vp, ci, vp]),
+        "r1_scene_set_materials": (ci, [vp, ci, C.c_uint32, C.c_uint32, vp, vp, vp, vp, C.POINTER(C.c_double)]),
         "r1_scatter": (ci, [vp, ci, f32p, f32p, f32p, i32p, f32p, f32p, i32p, f32p, f32p]),
         "r1_get_ray": (ci, [vp, ci, f32p, f32p, f32p, f32p, f32p]),
         "r1_replay_pixels": (ci, [vp, ci, i32p, ci, ci, ci, ci, u32p, u32p, f32p, u32p]),
@@ -311,6 +314,52 @@ class Scene:
                                          C.byref(ms)), "r1_scene_move_spheres")
         return ms.value
 
+    def move_camera(self, cam22, device=-1):
+        """r1_scene_move_camera: installs 22 camera constants (camera_constants() computes them) for renders and parity calls on
+        `device` (-1: the device of the last commit).  Renders already enqueued keep the camera they were launched with.  The host
+        scene (camera()) keeps its camera; a re-commit restores it on the device."""
+        cam = np.ascontiguousarray(cam22, np.float32)
+        if cam.shape != (22,):
+            raise ValueError("cam22 must hold 22 constants, not shape %s" % (cam.shape,))
+        _check(lib.r1_scene_move_camera(self.handle, device, cam.ctypes.data), "r1_scene_move_camera")
+
+    def set_materials(self, kind=None, albedo=None, param=None, first=0, device=-1, stream=None):
+        """r1_scene_set_materials: sets the materials of spheres first .. first + n - 1 on one device from torch CUDA tensors, each
+        contiguous: `kind` int32 (n,) of MAT_*, `albedo` float32 (n, 3), `param` float32 (n,) (Metal fuzz, Dielectric ior); a tensor
+        left out keeps that field, and at least one must be given.  device: -1 = the tensors' device (the scene must be committed
+        there).  stream: a torch.cuda.Stream or raw cudaStream_t handle; default: torch's current stream on that device.  Returns when
+        the change is done, with its device time in ms.  The host scene (soa()) keeps its committed materials."""
+        tensors = [(what, t, dtype, shape) for what, t, dtype, shape in (("kind", kind, "int32", 1), ("albedo", albedo, "float32", 3),
+                                                                           ("param", param, "float32", 1)) if t is not None]
+        if not tensors:
+            raise ValueError("set_materials needs at least one of kind, albedo and param")
+        import torch
+        for what, t, dtype, _ in tensors:
+            if not isinstance(t, torch.Tensor) or not t.is_cuda:
+                raise ValueError("%s must be a torch CUDA tensor" % what)
+            if t.dtype != getattr(torch, dtype):
+                raise ValueError("%s must be %s, not %s" % (what, dtype, t.dtype))
+            if not t.is_contiguous():
+                raise ValueError("%s must be contiguous" % what)
+        t0 = tensors[0][1]
+        n = t0.shape[0] if t0.dim() >= 1 else -1
+        for what, t, _, cols in tensors:
+            want = (n,) if cols == 1 else (n, cols)
+            if n < 0 or tuple(t.shape) != want:
+                raise ValueError("%s must have shape %s, not %s" % (what, "(n,)" if cols == 1 else "(n, %d)" % cols, tuple(t.shape)))
+        dev = t0.device.index if device is None or device < 0 else device
+        for what, t, _, _ in tensors:
+            if t.device.index != dev:
+                raise ValueError("%s is on cuda:%d, the change runs on device %d" % (what, t.device.index, dev))
+        if stream is None:
+            stream = torch.cuda.current_stream(dev)
+        handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
+        ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None and n else None)  # noqa: E731
+        ms = C.c_double(0)
+        _check(lib.r1_scene_set_materials(self.handle, dev, first, n, ptr(kind), ptr(albedo), ptr(param), C.c_void_p(handle or None),
+                                          C.byref(ms)), "r1_scene_set_materials")
+        return ms.value
+
     def device_records(self, device=-1):
         """r1_scene_export_device: the records `device` (-1: the device of the last commit) holds for this scene, as uint8 bytes in
         r1_scene_commit's layout [scan | exact | shade | tensor operand]."""
@@ -453,6 +502,18 @@ def log_results(version, scene, results):
     el = (C.c_double * n)(*[r.elapsed_seconds for r in results])
     rays = (C.c_uint64 * n)(*[r.num_rays for r in results])
     _check(lib.r1_host_log_results(version.encode(), scene.encode(), el, rays, n), "log_results")
+
+
+def camera_constants(lookfrom, lookat, vup, vfov, aspect, aperture, focus_dist):
+    """r1_camera_constants (host only): the 22 constants r1_scene_set_camera installs for these arguments, as float32[22] in camera()'s
+    order -- the argument of Scene.move_camera()."""
+    vecs = [np.ascontiguousarray(x, np.float32).reshape(-1) for x in (lookfrom, lookat, vup)]
+    for a, what in zip(vecs, ("lookfrom", "lookat", "vup")):
+        if a.shape != (3,):
+            raise ValueError("%s must hold 3 values, not %d" % (what, a.size))
+    out = np.zeros(22, np.float32)
+    _check(lib.r1_camera_constants(*vecs, vfov, aspect, aperture, focus_dist, out), "r1_camera_constants")
+    return out
 
 
 def rng_draws(pixel, sample, seed, n):

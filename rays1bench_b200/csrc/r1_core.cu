@@ -513,12 +513,33 @@ void r1_scene_destroy(r1_scene *scene)
     delete scene;
 }
 
-// Camera::init (rayweek1.cpp:366-379)
-int r1_scene_set_camera(r1_scene *scene, const float lookfrom[3], const float lookat[3], const float vup[3], float vfov_deg, float aspect,
-                        float aperture, float focus_dist)
+}  // extern "C"
+
+namespace {
+// The 22 camera constants in r1_scene_get_camera's order, to and from r1::Camera.
+void camera_to_constants(const r1::Camera &c, float *out)
 {
-    if (!scene || !lookfrom || !lookat || !vup) return fail(R1_ERR_ARG, "null argument");
-    r1::Camera &c = scene->cam;
+    const float *src[7] = { c.origin, c.llc, c.horizontal, c.vertical, c.u, c.v, c.w };
+    for (int k = 0; k < 7; ++k) memcpy(out + 3 * k, src[k], 12);
+    out[21] = c.lens_radius;
+}
+
+void camera_from_constants(const float *cam, r1::Camera &c)
+{
+    float *dst[7] = { c.origin, c.llc, c.horizontal, c.vertical, c.u, c.v, c.w };
+    for (int k = 0; k < 7; ++k) memcpy(dst[k], cam + 3 * k, 12);
+    c.lens_radius = cam[21];
+}
+}  // namespace
+
+extern "C" {
+
+// Camera::init (rayweek1.cpp:366-379)
+int r1_camera_constants(const float lookfrom[3], const float lookat[3], const float vup[3], float vfov_deg, float aspect, float aperture,
+                        float focus_dist, float out[22])
+{
+    if (!lookfrom || !lookat || !vup || !out) return fail(R1_ERR_ARG, "null argument");
+    r1::Camera c;
     // The reference's builders call Camera::init with constants, so gcc folds it at compile time -- after the fast-math
     // reassociation of `vfov * (float)M_PI / 180 / 2` into vfov * C, C = (float)M_PI * (1.0f / 360.0f) -- with tanf and the 1 / sqrtf
     // of unit_vector correctly rounded and everything else in source order.  Evaluated the same way here, the 22 constants have the
@@ -541,17 +562,24 @@ int r1_scene_set_camera(r1_scene *scene, const float lookfrom[3], const float lo
         c.horizontal[k] = (2 * half_width * focus_dist) * c.u[k];
         c.vertical[k] = (2 * half_height * focus_dist) * c.v[k];
     }
-    scene->have_camera = true;
+    camera_to_constants(c, out);
     return R1_OK;
+}
+
+int r1_scene_set_camera(r1_scene *scene, const float lookfrom[3], const float lookat[3], const float vup[3], float vfov_deg, float aspect,
+                        float aperture, float focus_dist)
+{
+    if (!scene || !lookfrom || !lookat || !vup) return fail(R1_ERR_ARG, "null argument");
+    float cam[22];
+    const int rc = r1_camera_constants(lookfrom, lookat, vup, vfov_deg, aspect, aperture, focus_dist, cam);
+    if (rc) return rc;
+    return r1_scene_set_camera_raw(scene, cam);
 }
 
 int r1_scene_set_camera_raw(r1_scene *scene, const float cam[22])
 {
     if (!scene || !cam) return fail(R1_ERR_ARG, "null argument");
-    r1::Camera &c = scene->cam;
-    float *dst[7] = { c.origin, c.llc, c.horizontal, c.vertical, c.u, c.v, c.w };
-    for (int k = 0; k < 7; ++k) memcpy(dst[k], cam + 3 * k, 12);
-    c.lens_radius = cam[21];
+    camera_from_constants(cam, scene->cam);
     scene->have_camera = true;
     return R1_OK;
 }
@@ -602,10 +630,7 @@ int r1_scene_get_soa(const r1_scene *scene, float *cx, float *cy, float *cz, flo
 int r1_scene_get_camera(const r1_scene *scene, float *out)
 {
     if (!scene || !out) return fail(R1_ERR_ARG, "null argument");
-    const r1::Camera &c = scene->cam;
-    const float *src[7] = { c.origin, c.llc, c.horizontal, c.vertical, c.u, c.v, c.w };
-    for (int k = 0; k < 7; ++k) memcpy(out + 3 * k, src[k], 12);
-    out[21] = c.lens_radius;
+    camera_to_constants(scene->cam, out);
     return R1_OK;
 }
 
@@ -696,22 +721,14 @@ int r1_scene_commit(r1_scene *scene, int device)
         // supergroup lanes and kk (r1_encode.h; r1_scene_move_spheres encodes moved spheres with the same function on the device)
         if (real) r1::enc::scan_lanes(scan, i, true, scene->cx[i], scene->cy[i], scene->cz[i], scene->radius_sq[i]);
         else r1::enc::scan_lanes(scan, i, false, 0.0f, 0.0f, 0.0f, 0.0f);
-        int32_t kind = R1_MAT_NONE;
-        float inv_r = 0.0f;
         if (i < n) {
             exact[i] = make_float4(scene->cx[i], scene->cy[i], scene->cz[i], scene->radius_sq[i]);
-            shade[2 * i] = make_float4(scene->albedo[3 * i], scene->albedo[3 * i + 1], scene->albedo[3 * i + 2], scene->param[i]);
-            inv_r = scene->inv_radius[i];
-            kind = scene->kind[i];
+            // material and inv_radius (r1_encode.h; r1_scene_set_materials encodes new materials with the same function on the device)
+            r1::enc::shade_records(scene->kind[i], scene->albedo[3 * i], scene->albedo[3 * i + 1], scene->albedo[3 * i + 2], scene->param[i],
+                                   scene->inv_radius[i], shade[2 * i], shade[2 * i + 1]);
+        } else {
+            r1::enc::shade_records(R1_MAT_NONE, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, shade[2 * i], shade[2 * i + 1]);
         }
-        float kind_bits, inv_ior = 0.0f, r0s = 0.0f;
-        memcpy(&kind_bits, &kind, 4);
-        if (kind == R1_MAT_DIELECTRIC) {   // Dielectric::scatter's two divisions (rayweek1.cpp:482, :456), once per sphere, IEEE float
-            const volatile float ior = scene->param[i];
-            inv_ior = 1.0f / ior;
-            r0s = (1.0f - ior) / (ior + 1.0f);
-        }
-        shade[2 * i + 1] = make_float4(inv_r, kind_bits, inv_ior, r0s);
     }
     build_tensor_operand(scene, host.data() + tcb_off, n32);
     rc = take_scene_block(*scr, bytes, &c.block, &c.block_bytes);
@@ -971,6 +988,35 @@ struct DevBuf {
 };
 #define R1_TRY(expr) do { int rc_ = (expr); if (rc_) return rc_; } while (0)
 
+// CUDA events around work enqueued on one stream (device_ms of r1_scene_move_spheres and r1_scene_set_materials)
+struct StreamTimer {
+    cudaEvent_t a = nullptr, b = nullptr;
+    ~StreamTimer() { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); }
+    int start(cudaStream_t stream)
+    {
+        R1_CUDA(cudaEventCreate(&a));
+        R1_CUDA(cudaEventCreate(&b));
+        R1_CUDA(cudaEventRecord(a, stream));
+        return R1_OK;
+    }
+    int stop(cudaStream_t stream, double *ms_out)
+    {
+        R1_CUDA(cudaEventRecord(b, stream));
+        R1_CUDA(cudaEventSynchronize(b));
+        float ms = 0;
+        R1_CUDA(cudaEventElapsedTime(&ms, a, b));
+        *ms_out = ms;
+        return R1_OK;
+    }
+};
+
+// the records of c's block, in r1_scene_commit's layout
+r1::move::Records ctx_records(DeviceCtx &c)
+{
+    float4 *block = static_cast<float4 *>(c.block);
+    return { block, block + c.dev.n_pad, block + 2 * (size_t)c.dev.n_pad, static_cast<unsigned char *>(c.block) + (size_t)c.dev.n_pad * (16 + 16 + 32) };
+}
+
 // r1_trace_rays through the BVH: any sphere count
 int trace_rays_bvh(r1_scene *scene, DeviceCtx &c, int n, const float *org, const float *dir, float t_min, float t_max, int32_t *index, float *t,
                    float *p, float *normal)
@@ -1061,14 +1107,9 @@ int r1_scene_move_spheres(r1_scene *scene, int device, uint32_t first, uint32_t 
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     if (!c.move_flag) R1_CUDA(cudaMalloc(&c.move_flag, 16));
     if (c.bvh_block && !c.refit_block) R1_CUDA(cudaMalloc(&c.refit_block, (size_t)c.bvh_n_nodes * 8 + 16));
-    struct Events {
-        cudaEvent_t a = nullptr, b = nullptr;
-        ~Events() { if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); }
-    } ev;
-    if (device_ms) { R1_CUDA(cudaEventCreate(&ev.a)); R1_CUDA(cudaEventCreate(&ev.b)); R1_CUDA(cudaEventRecord(ev.a, stream)); }
-    float4 *block = static_cast<float4 *>(c.block);
-    const r1::move::Records rec = { block, block + c.dev.n_pad, block + 2 * (size_t)c.dev.n_pad,
-                                    static_cast<unsigned char *>(c.block) + (size_t)c.dev.n_pad * (16 + 16 + 32) };
+    StreamTimer ev;
+    if (device_ms) R1_TRY(ev.start(stream));
+    const r1::move::Records rec = ctx_records(c);
     R1_TRY(r1::move::check(rec, first, n, d_centre, d_radius, c.move_flag, stream));   // nothing is written unless every value passes
     R1_TRY(r1::move::encode(rec, first, n, d_centre, d_radius, stream));
     c.moved = true;                                                // the records no longer match the host scene
@@ -1079,13 +1120,45 @@ int r1_scene_move_spheres(r1_scene *scene, int device, uint32_t first, uint32_t 
         R1_TRY(r1::lbvh::refit(nodes, const_cast<float4 *>(c.bvh_leaves), c.bvh_n_nodes, rec.exact, parent, arrivals, c.refit_parents, stream));
         c.refit_parents = true;
     }
-    if (device_ms) {
-        R1_CUDA(cudaEventRecord(ev.b, stream));
-        R1_CUDA(cudaEventSynchronize(ev.b));
-        float ms = 0;
-        R1_CUDA(cudaEventElapsedTime(&ms, ev.a, ev.b));
-        *device_ms = ms;
-    }
+    if (device_ms) R1_TRY(ev.stop(stream, device_ms));
+    R1_CUDA(cudaStreamSynchronize(stream));
+    return R1_OK;
+}
+
+int r1_scene_move_camera(r1_scene *scene, int device, const float cam[22])
+{
+    if (!scene) return fail(R1_ERR_ARG, "null scene");
+    if (!cam) return fail(R1_ERR_ARG, "null camera constants");
+    DeviceCtx *cp = nullptr;
+    R1_TRY(get_ctx(scene, &cp, device));
+    if (cp->generation != scene->generation) return fail(R1_ERR_STATE, "the scene's spheres changed after it was committed to device %d (commit it again)", cp->device);
+    camera_from_constants(cam, cp->dev.cam);   // read by value when a render or parity kernel is launched
+    return R1_OK;
+}
+
+int r1_scene_set_materials(r1_scene *scene, int device, uint32_t first, uint32_t n, const int32_t *d_kind, const float *d_albedo, const float *d_param,
+                           void *cuda_stream, double *device_ms)
+{
+    if (!scene) return fail(R1_ERR_ARG, "null scene");
+    const uint64_t count = scene->cx.size();
+    if ((uint64_t)first + n > count)
+        return fail(R1_ERR_ARG, "spheres %u .. %u + %u - 1 are out of range (the scene has %llu)", first, first, n, (unsigned long long)count);
+    if (n > 0 && !d_kind && !d_albedo && !d_param) return fail(R1_ERR_ARG, "no material field given (kind, albedo and param are all null)");
+    DeviceCtx *cp = nullptr;
+    R1_TRY(get_ctx(scene, &cp, device));
+    DeviceCtx &c = *cp;
+    if (c.generation != scene->generation) return fail(R1_ERR_STATE, "the scene's spheres changed after it was committed to device %d (commit it again)", c.device);
+    if (device_ms) *device_ms = 0;
+    if (n == 0) return R1_OK;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    if (d_kind && !c.move_flag) R1_CUDA(cudaMalloc(&c.move_flag, 16));
+    StreamTimer ev;
+    if (device_ms) R1_TRY(ev.start(stream));
+    const r1::move::Records rec = ctx_records(c);
+    if (d_kind) R1_TRY(r1::move::check_materials(rec, first, n, d_kind, c.move_flag, stream));   // only new kinds can be refused
+    R1_TRY(r1::move::encode_materials(rec, first, n, d_kind, d_albedo, d_param, stream));
+    // neither the geometry nor the tree changes: c.moved stays as it is, and a device without a tree may still upload the host's
+    if (device_ms) R1_TRY(ev.stop(stream, device_ms));
     R1_CUDA(cudaStreamSynchronize(stream));
     return R1_OK;
 }

@@ -1,17 +1,20 @@
 // r1_encode.h -- the device records of one sphere, in one definition for the host and the device: r1_scene_commit encodes a scene
-// with these functions on the host, and r1_scene_move_spheres (r1_move.cu) re-encodes moved spheres with them on the device.  The
-// two must write the same bytes (DESIGN.md section 4.10), so every double operation goes through dmul / dadd / dsub / ddiv, which
-// are the _rn intrinsics on the device (nvcc would otherwise contract a product and a sum into an FMA) and the plain operators on
-// the host.  Conversions between float and double are exact (float -> double) or round to nearest (double -> float) on both.
+// with these functions on the host, and r1_scene_move_spheres / r1_scene_set_materials (r1_move.cu) re-encode spheres with them on
+// the device.  The two must write the same bytes (DESIGN.md sections 4.10, 4.11), so every double operation goes through dmul /
+// dadd / dsub / ddiv, which are the _rn intrinsics on the device (nvcc would otherwise contract a product and a sum into an FMA) and
+// the plain operators on the host.  Conversions between float and double are exact (float -> double) or round to nearest (double ->
+// float) on both.
 //
 // Records of sphere i in the committed block [scan | exact | shade | tensor operand]:
 //   scan    supergroup lanes -cx, -cy, -cz, kk (r1_device.cuh "Filter arithmetic"): scan_lanes
 //   exact   {cx, cy, cz, radius_sq}
-//   shade   [2i] material, [2i + 1] {inv_radius, kind, 1 / ior, r0}: only inv_radius depends on the geometry
+//   shade   [2i] material, [2i + 1] {inv_radius, kind, 1 / ior, r0}: shade_records; only inv_radius depends on the geometry
 //   operand the sphere's row of the tensor-core filter's B operand (r1_tensor.cuh): sphere_row_words
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include "../../include/rays1_b200.h"
 
 #include <cmath>
 #include <cstring>
@@ -111,6 +114,28 @@ R1_HD void scan_lanes(float *scan, int i, bool real, float cx, float cy, float c
     } else {
         scan[4 * (f4 + 12) + k] = inf;
     }
+}
+
+// The two shade records of a sphere with material (kind, r, g, b, param): mat = {r, g, b, param}, Metal's param clamped as its ctor
+// does (rayweek1.cpp:424: param < 1 ? param : 1, so a NaN fuzz becomes 1); geo = {inv_radius, kind's bits, 1 / ior, (1 - ior) /
+// (ior + 1)}, Dielectric::scatter's two divisions (rayweek1.cpp:482, :456) done once per sphere in IEEE float, 0 and 0 for other
+// kinds.  r1_scene_commit's host scene holds Metal params clamped already; clamping again changes no bit.
+R1_HD void shade_records(int32_t kind, float r, float g, float b, float param, float inv_radius, float4 &mat, float4 &geo)
+{
+    if (kind == R1_MAT_METAL) param = param < 1 ? param : 1;
+    float inv_ior = 0.0f, r0 = 0.0f;
+    if (kind == R1_MAT_DIELECTRIC) {
+#ifdef __CUDA_ARCH__
+        inv_ior = __fdiv_rn(1.0f, param);
+        r0 = __fdiv_rn(__fsub_rn(1.0f, param), __fadd_rn(param, 1.0f));
+#else
+        const volatile float ior = param;
+        inv_ior = 1.0f / ior;
+        r0 = (1.0f - ior) / (ior + 1.0f);
+#endif
+    }
+    mat = make_float4(r, g, b, param);
+    geo = make_float4(inv_radius, from_bits((uint32_t)kind), inv_ior, r0);
 }
 
 }  // namespace enc
