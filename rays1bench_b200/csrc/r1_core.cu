@@ -222,156 +222,11 @@ Partition partition(int width, int height, int row_tile, int rank, int world)
 constexpr int kDefaultThreads = 1024;     // per-lane scans: 64 registers
 constexpr int kDefaultThreadsCoop = 512;  // cooperative scan: 4 rays per lane in flight, 127 registers
 
-template <int kScan, bool kStaged, int kThreads>
-int launch_megakernel_lanefetch(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
-{
-    constexpr int kBlocks = 1;
-    auto kern = r1::megakernel<kScan, kStaged, kThreads, kBlocks>;
-    const size_t smem = r1::kSmemSpheres + (kStaged ? (size_t)args.scene.n_pad * 32 : 0) + (kScan == r1::kScanCoop || kScan == r1::kScanLaneDeferred ? sizeof(r1::WarpScratch) * (kThreads / 32) : 0);
-    R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = sm_count * kBlocks;
-    if (prm.blocks_per_sm > 0) grid = sm_count * prm.blocks_per_sm;
-    // never launch more lanes than there are units
-    const long long max_ctas = ((long long)args.n_units + kThreads - 1) / kThreads;
-    if (grid > max_ctas) grid = (int)std::max<long long>(1, max_ctas);
-    kern<<<grid, kThreads, smem, stream>>>(args);
-    R1_CUDA(cudaGetLastError());
-    return R1_OK;
-}
-
-// warp sample-pool scheduling (r1::megakernel_pool): the default; R1_POOL=0 selects the per-lane unit fetch of r1::megakernel
-size_t megakernel_pool_smem(int scan, bool staged, int n_pad, int threads)
-{
-    return r1::kSmemSpheres + (staged ? (size_t)n_pad * 32 : 0) +
-           (scan == r1::kScanCoop || scan == r1::kScanLaneDeferred ? sizeof(r1::WarpScratch) * (threads / 32) : 0) + sizeof(r1::WarpPool) * (threads / 32);
-}
-
-template <int kScan, bool kStaged, int kThreads>
-int launch_megakernel_pool(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
-{
-    constexpr int kBlocks = 1;
-    auto kern = r1::megakernel_pool<kScan, kStaged, kThreads, kBlocks>;
-    const size_t smem = megakernel_pool_smem(kScan, kStaged, args.scene.n_pad, kThreads);
-    if (smem > 227 * 1024) return fail(R1_ERR_LIMIT, "%d threads need %zu bytes of shared memory for this scene (227 KB available)", kThreads, smem);
-    R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = sm_count * kBlocks;
-    if (prm.blocks_per_sm > 0) grid = sm_count * prm.blocks_per_sm;
-    const unsigned long long max_ctas = (args.n_samples + kThreads - 1) / kThreads;   // never launch more lanes than there are samples
-    if ((unsigned long long)grid > max_ctas) grid = (int)std::max<unsigned long long>(1, max_ctas);
-    kern<<<grid, kThreads, smem, stream>>>(args);
-    R1_CUDA(cudaGetLastError());
-    return R1_OK;
-}
-
-// two paths per lane (r1::megakernel_pool2, R1_VARIANT_MEGAKERNEL_DUAL)
-template <bool kStaged, int kThreads>
-int launch_megakernel_dual_t(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
-{
-    auto kern = r1::megakernel_pool2<kStaged, kThreads, 1>;
-    const size_t smem = r1::kSmemSpheres + (kStaged ? (size_t)args.scene.n_pad * 32 : 0) + sizeof(r1::WarpPool) * (kThreads / 32);
-    R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = sm_count * (prm.blocks_per_sm > 0 ? prm.blocks_per_sm : 1);
-    const unsigned long long max_ctas = (args.n_samples + 2 * kThreads - 1) / (2 * kThreads);
-    if ((unsigned long long)grid > max_ctas) grid = (int)std::max<unsigned long long>(1, max_ctas);
-    kern<<<grid, kThreads, smem, stream>>>(args);
-    R1_CUDA(cudaGetLastError());
-    return R1_OK;
-}
-
-template <bool kStaged>
-int launch_megakernel_dual(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
-{
-    const int threads = prm.threads > 0 ? prm.threads : 768;
-    if (threads == 512) return launch_megakernel_dual_t<kStaged, 512>(sm_count, args, prm, stream);
-    if (threads == 768) return launch_megakernel_dual_t<kStaged, 768>(sm_count, args, prm, stream);
-    return fail(R1_ERR_ARG, "the dual variant runs 512 or 768 threads (got %d)", threads);
-}
-
-// tensor-core filter (r1::megakernel_tc3, R1_VARIANT_MEGAKERNEL_TENSOR): `threads` / 128 = ray groups per CTA
-template <int kGroups>
-int launch_megakernel_tc3_t(int sm_count, const r1::RenderArgs &args, cudaStream_t stream)
-{
-    auto kern = r1::megakernel_tc3<kGroups>;
-    const size_t smem = r1::tc3_smem_bytes(kGroups, args.scene.n32);
-    if (smem > 227 * 1024) return fail(R1_ERR_LIMIT, "tensor variant: %d ray groups need %zu bytes of shared memory for this scene", kGroups, smem);
-    R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = sm_count;
-    const unsigned long long max_ctas = (args.n_samples + kGroups * 128 - 1) / (kGroups * 128);
-    if ((unsigned long long)grid > max_ctas) grid = (int)std::max<unsigned long long>(1, max_ctas);
-    kern<<<grid, kGroups * 128, smem, stream>>>(args);
-    R1_CUDA(cudaGetLastError());
-    return R1_OK;
-}
-
 // streamed tensor-core filter (r1::megakernel_tcs, R1_VARIANT_MEGAKERNEL_TENSOR_STREAM): `threads` / 128 = ray groups per CTA (one
 // 128-column TMEM accumulator each), R1_TCS_STAGES = depth of the operand ring.  Shared memory does not depend on the scene.
 // Measured on synth4096 at 1280x720x250 (B200, 1000 W; DESIGN.md section 4.7, profiles/r03_bench_tensor_stream.json): 4 groups with
 // 2 / 3 / 4 / 6 stages 1279 / 1324 / 1350 / 1358 Mrays/s; 3 / 2 / 1 groups with 6 stages 1120 / 806 / 415 (PACKED: 827).
 constexpr int kDefaultTcsGroups = 4, kDefaultTcsStages = 6;
-
-template <int kGroups, int kStages>
-int launch_megakernel_tcs_t(int sm_count, const r1::RenderArgs &args, cudaStream_t stream)
-{
-    auto kern = r1::megakernel_tcs<kGroups, kStages>;
-    const size_t smem = r1::tcs_smem_bytes(kGroups, kStages);
-    if (smem > 227 * 1024) return fail(R1_ERR_LIMIT, "tensor-stream variant: %d ray groups and %d stages need %zu bytes of shared memory", kGroups, kStages, smem);
-    R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = sm_count;                                         // one CTA per SM
-    const unsigned long long max_ctas = (args.n_samples + kGroups * 128 - 1) / (kGroups * 128);
-    if ((unsigned long long)grid > max_ctas) grid = (int)std::max<unsigned long long>(1, max_ctas);
-    kern<<<grid, kGroups * 128, smem, stream>>>(args);
-    R1_CUDA(cudaGetLastError());
-    return R1_OK;
-}
-
-int launch_megakernel_tcs(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
-{
-    const int groups = prm.threads > 0 ? prm.threads / 128 : kDefaultTcsGroups;
-    const int stages = getenv("R1_TCS_STAGES") ? atoi(getenv("R1_TCS_STAGES")) : kDefaultTcsStages;
-    if (groups == 4 && stages == 2) return launch_megakernel_tcs_t<4, 2>(sm_count, args, stream);
-    if (groups == 4 && stages == 3) return launch_megakernel_tcs_t<4, 3>(sm_count, args, stream);
-    if (groups == 4 && stages == 4) return launch_megakernel_tcs_t<4, 4>(sm_count, args, stream);
-    if (groups == 4 && stages == 6) return launch_megakernel_tcs_t<4, 6>(sm_count, args, stream);
-    if (groups == 3 && stages == 6) return launch_megakernel_tcs_t<3, 6>(sm_count, args, stream);
-    if (groups == 2 && stages == 6) return launch_megakernel_tcs_t<2, 6>(sm_count, args, stream);
-    if (groups == 1 && stages == 6) return launch_megakernel_tcs_t<1, 6>(sm_count, args, stream);
-    return fail(R1_ERR_ARG, "the tensor-stream variant runs 1 .. 4 groups of 128 ray threads per CTA (threads = 128 .. 512) with a 6-stage ring, "
-                            "or 4 groups with 2, 3, 4 or 6 stages (got %d groups, %d stages)", groups, stages);
-}
-
-int launch_megakernel_tc(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
-{
-    if (!args.scene.tcb) return fail(R1_ERR_LIMIT, "the tensor-core filter takes scenes of 1 .. %d spheres (its operand lives in shared memory)", r1::tc::kMaxSpheres);
-    // ray groups per CTA; measured on the large scene: 4 groups 9.70, 5: 10.34, 6: 9.92, 7: 9.69 G rays/s
-    const int groups = prm.threads > 0 ? prm.threads / 128 : 5;
-    if (groups == 4) return launch_megakernel_tc3_t<4>(sm_count, args, stream);
-    if (groups == 5) return launch_megakernel_tc3_t<5>(sm_count, args, stream);
-    if (groups == 6) return launch_megakernel_tc3_t<6>(sm_count, args, stream);
-    if (groups == 7) return launch_megakernel_tc3_t<7>(sm_count, args, stream);
-    return fail(R1_ERR_ARG, "the tensor variant runs 4 .. 7 groups of 128 ray threads per CTA (threads = 512 .. 896)");
-}
-
-template <int kScan, bool kStaged, int kThreads>
-int launch_megakernel_t(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
-{
-    const bool pool = !(getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0);   // read per render, like the other tuning knobs
-    if (pool) return launch_megakernel_pool<kScan, kStaged, kThreads>(sm_count, args, prm, stream);
-    return launch_megakernel_lanefetch<kScan, kStaged, kThreads>(sm_count, args, prm, stream);
-}
-
-template <int kScan, bool kStaged>
-int launch_megakernel(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
-{
-    int threads = prm.threads > 0 ? prm.threads : (kScan == r1::kScanCoop ? kDefaultThreadsCoop : kDefaultThreads);
-    // The deferred scan's 2 KB of queue per warp: with the sample pool, 1024 threads and more than 3 936 staged spheres exceed
-    // 227 KB of shared memory.  The default then runs 768 threads (the image does not depend on the thread count).
-    const bool pool = !(getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0);
-    if (prm.threads <= 0 && pool && megakernel_pool_smem(kScan, kStaged, args.scene.n_pad, threads) > 227 * 1024) threads = 768;
-    if (threads == 512) return launch_megakernel_t<kScan, kStaged, 512>(sm_count, args, prm, stream);
-    if (threads == 768) return launch_megakernel_t<kScan, kStaged, 768>(sm_count, args, prm, stream);
-    if (threads == 1024) return launch_megakernel_t<kScan, kStaged, 1024>(sm_count, args, prm, stream);
-    return fail(R1_ERR_ARG, "threads must be 512, 768 or 1024 (got %d)", threads);
-}
 
 // BVH traversal (megakernel_pool<kScanBvh>, R1_VARIANT_MEGAKERNEL_BVH): nothing is staged, every CTA shape runs the sample pool
 // (R1_POOL=0 does not apply).  Measured at 640x360x32 (B200, DESIGN.md section 4.8), Mrays/s for 512 / 768 / 1024 threads: large
@@ -380,16 +235,146 @@ int launch_megakernel(int sm_count, const r1::RenderArgs &args, const r1_render_
 constexpr int kDefaultThreadsBvh = 1024;
 constexpr uint32_t kBvhSchedKmax = 64, kBvhSchedDiv = 16;
 
+// The tuning knobs of the environment.  Read on every render, so that a caller can change them between renders.
+struct Knobs {
+    bool pool = true;                   // R1_POOL=0: r1::megakernel's per-lane unit fetch instead of the warp sample pool
+    bool force_unstaged = false;        // R1_FORCE_UNSTAGED: scan from global memory even where the scene could be staged
+    bool auto_tensor = true;            // R1_AUTO_TENSOR=0: R1_VARIANT_MEGAKERNEL never resolves to the tensor-core filter
+    int tcs_stages = kDefaultTcsStages; // R1_TCS_STAGES: depth of the tensor-stream variant's operand ring
+    uint32_t sched_kmax = 0, sched_div = 0;   // R1_SCHED "kmax,div" (1 .. 4096, 1 .. 1024) overrides the scheduling; 0: not set
+};
+
+Knobs read_knobs()
+{
+    const auto zero = [](const char *name) { const char *e = getenv(name); return e && atoi(e) == 0; };
+    Knobs k;
+    k.pool = !zero("R1_POOL");
+    k.force_unstaged = getenv("R1_FORCE_UNSTAGED") != nullptr;
+    k.auto_tensor = !zero("R1_AUTO_TENSOR");
+    if (const char *e = getenv("R1_TCS_STAGES")) k.tcs_stages = atoi(e);
+    if (const char *e = getenv("R1_SCHED")) {
+        unsigned kmax = 0, div = 0;
+        if (sscanf(e, "%u,%u", &kmax, &div) == 2 && kmax >= 1 && kmax <= 4096 && div >= 1 && div <= 1024) { k.sched_kmax = kmax; k.sched_div = div; }
+    }
+    return k;
+}
+
+// Samples per atomic (guided self-scheduling).  The sample pool: a WARP takes kmax x 32 consecutive samples per atomicAdd, shrinking
+// as left / (div x lanes) towards the end.  Measured on B200 (large scene, Mrays/s, full image | rank 0 of 8 = the per-GPU share of
+// the 8-GPU partition):  1,1: 6066 | 6057   2,16: 6102 | 6088   4,16: 6121 | 6088   8,16: 6132 | 6103.  Small scenes need long
+// ranges: with 32 samples per atomic the one counter line in L2 saturates (small scene 39 G rays/s instead of 58).  r1::megakernel
+// (R1_POOL=0) hands units to LANES; its round-1 tuning is kept: 1 unit per fetch on scan-heavy scenes (ranges held by lanes at the
+// end of a render are a serial tail), up to 64 on small ones.  BVH traversals are short at every scene size (DESIGN.md section 4.8).
+void pick_schedule(const r1::DevScene &dev, int variant, const Knobs &k, r1::RenderArgs &a)
+{
+    if (variant == R1_VARIANT_MEGAKERNEL_BVH) { a.sched_kmax = kBvhSchedKmax; a.sched_div = kBvhSchedDiv; }
+    else if (dev.n8 >= 256) { a.sched_kmax = k.pool ? 8 : 1; a.sched_div = k.pool ? 16 : 1; }
+    else { a.sched_kmax = 64; a.sched_div = 16; }
+    if (k.sched_kmax) { a.sched_kmax = k.sched_kmax; a.sched_div = k.sched_div; }
+}
+
+using RenderKernel = void (*)(r1::RenderArgs);
+
+// Launches a persistent render kernel: blocks_per_sm CTAs per SM (at least one), but never more CTAs than ceil(work / work_per_cta),
+// the CTAs that have work to take.  `what` names the kernel in the shared-memory refusal.
+int launch_persistent(RenderKernel kern, int threads, size_t smem, unsigned long long work, unsigned long long work_per_cta, int blocks_per_sm,
+                      int sm_count, const char *what, const r1::RenderArgs &args, cudaStream_t stream)
+{
+    if (smem > 227 * 1024) return fail(R1_ERR_LIMIT, "%s: %d threads need %zu bytes of shared memory for this scene (227 KB available)", what, threads, smem);
+    R1_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const unsigned long long max_ctas = std::max<unsigned long long>(1, (work + work_per_cta - 1) / work_per_cta);
+    const int grid = (int)std::min<unsigned long long>((unsigned long long)sm_count * (unsigned long long)std::max(blocks_per_sm, 1), max_ctas);
+    kern<<<grid, threads, smem, stream>>>(args);
+    R1_CUDA(cudaGetLastError());
+    return R1_OK;
+}
+
+// [mbarrier 16 B | rsqrtss table 4 KB | staged spheres n_pad * 32 B | per-warp scan scratch (coop / deferred) | per-warp sample pools]
+size_t megakernel_smem(int scan, bool staged, int n_pad, int threads, bool pool)
+{
+    return r1::kSmemSpheres + (staged ? (size_t)n_pad * 32 : 0) +
+           (scan == r1::kScanCoop || scan == r1::kScanLaneDeferred ? sizeof(r1::WarpScratch) * (threads / 32) : 0) + (pool ? sizeof(r1::WarpPool) * (threads / 32) : 0);
+}
+
+// warp sample-pool scheduling (r1::megakernel_pool): the default; R1_POOL=0 selects the per-lane unit fetch of r1::megakernel
+template <int kScan, bool kStaged>
+int launch_megakernel(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, bool pool, cudaStream_t stream)
+{
+    int threads = prm.threads > 0 ? prm.threads : (kScan == r1::kScanCoop ? kDefaultThreadsCoop : kDefaultThreads);
+    // The deferred scan's 2 KB of queue per warp: with the sample pool, 1024 threads and more than 3 936 staged spheres exceed
+    // 227 KB of shared memory.  The default then runs 768 threads (the image does not depend on the thread count).
+    if (prm.threads <= 0 && pool && megakernel_smem(kScan, kStaged, args.scene.n_pad, threads, true) > 227 * 1024) threads = 768;
+    RenderKernel kern = nullptr;
+    if (threads == 512) kern = pool ? r1::megakernel_pool<kScan, kStaged, 512, 1> : r1::megakernel<kScan, kStaged, 512, 1>;
+    if (threads == 768) kern = pool ? r1::megakernel_pool<kScan, kStaged, 768, 1> : r1::megakernel<kScan, kStaged, 768, 1>;
+    if (threads == 1024) kern = pool ? r1::megakernel_pool<kScan, kStaged, 1024, 1> : r1::megakernel<kScan, kStaged, 1024, 1>;
+    if (!kern) return fail(R1_ERR_ARG, "threads must be 512, 768 or 1024 (got %d)", threads);
+    const size_t smem = megakernel_smem(kScan, kStaged, args.scene.n_pad, threads, pool);
+    if (pool) return launch_persistent(kern, threads, smem, args.n_samples, threads, prm.blocks_per_sm, sm_count, "megakernel_pool", args, stream);
+    return launch_persistent(kern, threads, smem, args.n_units, threads, prm.blocks_per_sm, sm_count, "megakernel", args, stream);
+}
+
 int launch_megakernel_bvh(int sm_count, const r1::RenderArgs &args, const float4 *nodes, const float4 *leaves, const r1_render_params &prm,
                           cudaStream_t stream)
 {
     const int threads = prm.threads > 0 ? prm.threads : kDefaultThreadsBvh;
     const r1::BvhArgs b = { nodes, leaves };
     R1_CUDA(cudaMemcpyToSymbolAsync(r1::c_bvh, &b, sizeof(b), 0, cudaMemcpyHostToDevice, stream));
-    if (threads == 512) return launch_megakernel_pool<r1::kScanBvh, false, 512>(sm_count, args, prm, stream);
-    if (threads == 768) return launch_megakernel_pool<r1::kScanBvh, false, 768>(sm_count, args, prm, stream);
-    if (threads == 1024) return launch_megakernel_pool<r1::kScanBvh, false, 1024>(sm_count, args, prm, stream);
-    return fail(R1_ERR_ARG, "the bvh variant runs 512, 768 or 1024 threads (got %d)", threads);
+    RenderKernel kern = nullptr;
+    if (threads == 512) kern = r1::megakernel_pool<r1::kScanBvh, false, 512, 1>;
+    if (threads == 768) kern = r1::megakernel_pool<r1::kScanBvh, false, 768, 1>;
+    if (threads == 1024) kern = r1::megakernel_pool<r1::kScanBvh, false, 1024, 1>;
+    if (!kern) return fail(R1_ERR_ARG, "the bvh variant runs 512, 768 or 1024 threads (got %d)", threads);
+    return launch_persistent(kern, threads, megakernel_smem(r1::kScanBvh, false, args.scene.n_pad, threads, true), args.n_samples, threads, prm.blocks_per_sm,
+                             sm_count, "bvh variant", args, stream);
+}
+
+// two paths per lane (r1::megakernel_pool2, R1_VARIANT_MEGAKERNEL_DUAL)
+template <bool kStaged>
+int launch_megakernel_dual(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
+{
+    const int threads = prm.threads > 0 ? prm.threads : 768;
+    RenderKernel kern = nullptr;
+    if (threads == 512) kern = r1::megakernel_pool2<kStaged, 512, 1>;
+    if (threads == 768) kern = r1::megakernel_pool2<kStaged, 768, 1>;
+    if (!kern) return fail(R1_ERR_ARG, "the dual variant runs 512 or 768 threads (got %d)", threads);
+    return launch_persistent(kern, threads, megakernel_smem(r1::kScanLanePacked, kStaged, args.scene.n_pad, threads, true), args.n_samples, 2ull * threads,
+                             prm.blocks_per_sm, sm_count, "dual variant", args, stream);
+}
+
+// tensor-core filter (r1::megakernel_tc3, R1_VARIANT_MEGAKERNEL_TENSOR): `threads` / 128 = ray groups per CTA, one CTA per SM
+int launch_megakernel_tc(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
+{
+    if (!args.scene.tcb) return fail(R1_ERR_LIMIT, "the tensor-core filter takes scenes of 1 .. %d spheres (its operand lives in shared memory)", r1::tc::kMaxSpheres);
+    // ray groups per CTA; measured on the large scene: 4 groups 9.70, 5: 10.34, 6: 9.92, 7: 9.69 G rays/s
+    const int groups = prm.threads > 0 ? prm.threads / 128 : 5;
+    RenderKernel kern = nullptr;
+    if (groups == 4) kern = r1::megakernel_tc3<4>;
+    if (groups == 5) kern = r1::megakernel_tc3<5>;
+    if (groups == 6) kern = r1::megakernel_tc3<6>;
+    if (groups == 7) kern = r1::megakernel_tc3<7>;
+    if (!kern) return fail(R1_ERR_ARG, "the tensor variant runs 4 .. 7 groups of 128 ray threads per CTA (threads = 512 .. 896)");
+    return launch_persistent(kern, groups * 128, r1::tc3_smem_bytes(groups, args.scene.n32), args.n_samples, groups * 128, 1, sm_count, "tensor variant", args,
+                             stream);
+}
+
+// streamed tensor-core filter (r1::megakernel_tcs): one CTA per SM
+int launch_megakernel_tcs(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, int stages, cudaStream_t stream)
+{
+    const int groups = prm.threads > 0 ? prm.threads / 128 : kDefaultTcsGroups;
+    RenderKernel kern = nullptr;
+    if (groups == 4 && stages == 2) kern = r1::megakernel_tcs<4, 2>;
+    if (groups == 4 && stages == 3) kern = r1::megakernel_tcs<4, 3>;
+    if (groups == 4 && stages == 4) kern = r1::megakernel_tcs<4, 4>;
+    if (groups == 4 && stages == 6) kern = r1::megakernel_tcs<4, 6>;
+    if (groups == 3 && stages == 6) kern = r1::megakernel_tcs<3, 6>;
+    if (groups == 2 && stages == 6) kern = r1::megakernel_tcs<2, 6>;
+    if (groups == 1 && stages == 6) kern = r1::megakernel_tcs<1, 6>;
+    if (!kern)
+        return fail(R1_ERR_ARG, "the tensor-stream variant runs 1 .. 4 groups of 128 ray threads per CTA (threads = 128 .. 512) with a 6-stage ring, "
+                                "or 4 groups with 2, 3, 4 or 6 stages (got %d groups, %d stages)", groups, stages);
+    return launch_persistent(kern, groups * 128, r1::tcs_smem_bytes(groups, stages), args.n_samples, groups * 128, 1, sm_count, "tensor-stream variant", args,
+                             stream);
 }
 
 // The host BVH of the scene, built on first need (r1_bvh.h).
@@ -457,12 +442,11 @@ int ctx_bvh(r1_scene *scene, DeviceCtx &c)
 // R1_VARIANT_MEGAKERNEL = the fastest megakernel for the scene.  Measured on B200: the tensor-core filter wins on the large scene
 // (485 spheres: 10.3 against 6.2 G rays/s) and loses where a scan is short (medium, 58 spheres: 25 against 34 G).  Explicit
 // tuning knobs (blocks_per_sm, threads, R1_POOL=0) address the packed kernel; R1_AUTO_TENSOR=0 keeps it everywhere.
-int resolve_variant(const r1::DevScene &dev, const r1_render_params &prm)
+int resolve_variant(const r1::DevScene &dev, const r1_render_params &prm, const Knobs &k)
 {
     if (prm.variant != R1_VARIANT_MEGAKERNEL) return prm.variant;
-    const bool tuned = prm.blocks_per_sm > 0 || prm.threads > 0 || (getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0) || getenv("R1_FORCE_UNSTAGED");
-    const bool off = getenv("R1_AUTO_TENSOR") && atoi(getenv("R1_AUTO_TENSOR")) == 0;
-    if (dev.tcb && dev.n8 >= 256 && !tuned && !off) return R1_VARIANT_MEGAKERNEL_TENSOR;
+    const bool tuned = prm.blocks_per_sm > 0 || prm.threads > 0 || !k.pool || k.force_unstaged;
+    if (dev.tcb && dev.n8 >= 256 && !tuned && k.auto_tensor) return R1_VARIANT_MEGAKERNEL_TENSOR;
     return R1_VARIANT_MEGAKERNEL_PACKED;
 }
 
@@ -822,22 +806,9 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
     a.magic_chunks = r1::div_magic((uint32_t)a.n_chunks);
     a.magic_width = r1::div_magic((uint32_t)prm.width);
     a.magic_row_tile = r1::div_magic((uint32_t)prm.row_tile);
-    // Samples per atomic (guided self-scheduling).  r1::megakernel_pool: a WARP takes kmax x 32 consecutive samples per atomicAdd,
-    // shrinking as left / (div x lanes) towards the end.  Measured on B200 (large scene, Mrays/s, full image | rank 0 of 8 = the
-    // per-GPU share of the 8-GPU partition):  1,1: 6066 | 6057   2,16: 6102 | 6088   4,16: 6121 | 6088   8,16: 6132 | 6103.
-    // Small scenes need long ranges: with 32 samples per atomic the one counter line in L2 saturates (small scene 39 G rays/s
-    // instead of 58).  r1::megakernel (R1_POOL=0) hands units to LANES; its round-1 tuning is kept: 1 unit per fetch on
-    // scan-heavy scenes (ranges held by lanes at the end of a render are a serial tail), up to 64 on small ones.
-    const bool pool_sched = !(getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0);
-    if (c.dev.n8 >= 256) { a.sched_kmax = pool_sched ? 8 : 1; a.sched_div = pool_sched ? 16 : 1; }
-    else { a.sched_kmax = 64; a.sched_div = 16; }
-    if (prm.variant == R1_VARIANT_MEGAKERNEL_BVH) {   // traversals are short at every scene size (DESIGN.md section 4.8)
-        a.sched_kmax = kBvhSchedKmax; a.sched_div = kBvhSchedDiv;
-    }
-    if (const char *e = getenv("R1_SCHED")) {  // tuning knob: "kmax,div"
-        unsigned k = 0, d = 0;
-        if (sscanf(e, "%u,%u", &k, &d) == 2 && k >= 1 && k <= 4096 && d >= 1 && d <= 1024) { a.sched_kmax = k; a.sched_div = d; }
-    }
+    const Knobs knobs = read_knobs();
+    const int variant = resolve_variant(c.dev, prm, knobs);
+    pick_schedule(c.dev, variant, knobs, a);
     a.rgb = (uint8_t *)d_rgb;
     a.num_rays = (unsigned long long *)d_num_rays;
     a.unit_counter = x.unit_counter;
@@ -861,9 +832,8 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
         R1_CUDA(cudaMemsetAsync(x.unit_counter, 0, sizeof(unsigned int), stream));
         R1_CUDA(cudaMemsetAsync(x.sample_counter, 0, sizeof(unsigned long long), stream));
         // scenes of up to 4096 spheres are staged in shared memory; R1_FORCE_UNSTAGED=1 exercises the global-memory path on small scenes
-        const bool staged = c.dev.n_pad <= r1::kMaxStagedSpheres && !getenv("R1_FORCE_UNSTAGED");
+        const bool staged = c.dev.n_pad <= r1::kMaxStagedSpheres && !knobs.force_unstaged;
         R1_CUDA(cudaEventRecord(x.ev[1], stream));
-        const int variant = resolve_variant(c.dev, prm);
         if (variant == R1_VARIANT_WAVEFRONT) {
             if (c.dev.n_pad > r1::kMaxStagedSpheres) return fail(R1_ERR_LIMIT, "the wavefront variant stages at most %d spheres", r1::kMaxStagedSpheres);
             uint32_t launches = 0;
@@ -871,19 +841,19 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
             if (rc) return fail(R1_ERR_CUDA, "wavefront: %s", cudaGetErrorString((cudaError_t)rc));
             x.last_launches += launches;
         } else {
-            if (variant == R1_VARIANT_MEGAKERNEL_PACKED) rc = staged ? launch_megakernel<r1::kScanLanePacked, true>(x.sm_count, a, prm, stream)
-                                                                  : launch_megakernel<r1::kScanLanePacked, false>(x.sm_count, a, prm, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_COOP) rc = staged ? launch_megakernel<r1::kScanCoop, true>(x.sm_count, a, prm, stream)
-                                                                            : launch_megakernel<r1::kScanCoop, false>(x.sm_count, a, prm, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_DEFERRED) rc = staged ? launch_megakernel<r1::kScanLaneDeferred, true>(x.sm_count, a, prm, stream)
-                                                                                : launch_megakernel<r1::kScanLaneDeferred, false>(x.sm_count, a, prm, stream);
+            if (variant == R1_VARIANT_MEGAKERNEL_PACKED) rc = staged ? launch_megakernel<r1::kScanLanePacked, true>(x.sm_count, a, prm, knobs.pool, stream)
+                                                                  : launch_megakernel<r1::kScanLanePacked, false>(x.sm_count, a, prm, knobs.pool, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_COOP) rc = staged ? launch_megakernel<r1::kScanCoop, true>(x.sm_count, a, prm, knobs.pool, stream)
+                                                                            : launch_megakernel<r1::kScanCoop, false>(x.sm_count, a, prm, knobs.pool, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_DEFERRED) rc = staged ? launch_megakernel<r1::kScanLaneDeferred, true>(x.sm_count, a, prm, knobs.pool, stream)
+                                                                                : launch_megakernel<r1::kScanLaneDeferred, false>(x.sm_count, a, prm, knobs.pool, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR) rc = launch_megakernel_tc(x.sm_count, a, prm, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) rc = launch_megakernel_tcs(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) rc = launch_megakernel_tcs(x.sm_count, a, prm, knobs.tcs_stages, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_BVH) rc = launch_megakernel_bvh(x.sm_count, a, c.bvh_nodes, c.bvh_leaves, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_DUAL) rc = staged ? launch_megakernel_dual<true>(x.sm_count, a, prm, stream)
                                                                             : launch_megakernel_dual<false>(x.sm_count, a, prm, stream);
-            else rc = staged ? launch_megakernel<r1::kScanLaneScalar, true>(x.sm_count, a, prm, stream)
-                             : launch_megakernel<r1::kScanLaneScalar, false>(x.sm_count, a, prm, stream);
+            else rc = staged ? launch_megakernel<r1::kScanLaneScalar, true>(x.sm_count, a, prm, knobs.pool, stream)
+                             : launch_megakernel<r1::kScanLaneScalar, false>(x.sm_count, a, prm, knobs.pool, stream);
             if (rc) return rc;
             x.last_launches += 1;
         }
@@ -1193,7 +1163,7 @@ int r1_trace_rays(r1_scene *scene, int n, const float *org, const float *dir, fl
     memset(&prm, 0, sizeof(prm));
     prm.variant = variant;
     if (!known_variant(variant)) return fail(R1_ERR_ARG, "unknown variant %d", variant);
-    const int v = resolve_variant(cp->dev, prm);
+    const int v = resolve_variant(cp->dev, prm, read_knobs());
     if (v == R1_VARIANT_WAVEFRONT || v == R1_VARIANT_MEGAKERNEL_DUAL) return fail(R1_ERR_ARG, "r1_trace_rays has no kernel for variant %d (wavefront, dual)", v);
     if (v == R1_VARIANT_MEGAKERNEL_TENSOR && !cp->dev.tcb)
         return fail(R1_ERR_LIMIT, "the tensor-core filter takes scenes of 1 .. %d spheres (this scene pads to %d)", r1::tc::kMaxSpheres, cp->dev.n32);
@@ -1234,13 +1204,14 @@ const char *r1_kernel_name(r1_scene *scene, int variant)
     r1_render_params prm;
     memset(&prm, 0, sizeof(prm));
     prm.variant = variant;
-    switch (resolve_variant(cp->dev, prm)) {
+    const Knobs k = read_knobs();
+    switch (resolve_variant(cp->dev, prm, k)) {
     case R1_VARIANT_WAVEFRONT: return "wf_intersect + wf_shade (graph loop)";
     case R1_VARIANT_MEGAKERNEL_TENSOR: return "megakernel_tc3";
     case R1_VARIANT_MEGAKERNEL_DUAL: return "megakernel_pool2";
     case R1_VARIANT_MEGAKERNEL_TENSOR_STREAM: return "megakernel_tcs";
     case R1_VARIANT_MEGAKERNEL_BVH: return "megakernel_bvh";
-    default: return (getenv("R1_POOL") && atoi(getenv("R1_POOL")) == 0) ? "megakernel" : "megakernel_pool";
+    default: return k.pool ? "megakernel_pool" : "megakernel";
     }
 }
 

@@ -122,6 +122,15 @@ __device__ __forceinline__ void accumulate_sample(const RenderArgs &a, uint32_t 
     accumulate_quantised(a, lp, quantise_radiance(c.x), quantise_radiance(c.y), quantise_radiance(c.z));
 }
 
+// total-rays counter (rayweek1.cpp:809-813): warp reduce, one 64-bit atomic per warp
+__device__ __forceinline__ void count_rays(const RenderArgs &a, uint32_t nrays, unsigned lane)
+{
+    unsigned long long total = nrays;
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
+    if (lane == 0 && total) atomicAdd(a.num_rays, total);
+}
+
 // start sample s of a pixel: jitter (rayweek1.cpp:759), lens disk + camera ray (:760, :381-386)
 __device__ __forceinline__ void primary_ray(const RenderArgs &a, uint32_t pixel, float fx, float fy, int s, const uint16_t *__restrict__ tab, Rng &rng, f3 &o,
                                             f3 &d)
@@ -273,7 +282,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel(const __gri
             }
         }
     }
-    // -- total-rays counter (rayweek1.cpp:809-813): warp reduce, one 64-bit atomic per warp
+    // count_rays written out: through the helper, ptxas allocates this kernel's registers differently
     unsigned long long total = nrays;
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
@@ -291,12 +300,108 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel(const __gri
 // the path state loses unit / sample bookkeeping, eight registers the scan loop can use), numbered g = lp * spp + s in 64 bits.
 // Which lane traces which sample is irrelevant to the result: RNG streams are keyed by (pixel, sample) and the accumulators are
 // integer sums -- the image is bit-identical to the other variants'.
+// Every persistent kernel except `megakernel` takes its work this way, and all of them produce through pool_produce.
+// megakernel_tc3 and megakernel_tcs pop through pool_take; megakernel_pool writes the same pop out (faster there), and
+// megakernel_pool2, which ranks two slots per lane, pops on its own.
 struct __align__(16) WarpPool {
     float4 a[32];                     // origin.xyz, local pixel index (uint bits; kPoolInvalid = past the end of the work)
     float4 b[32];                     // direction.xyz, rng key word 0 (uint bits)
     uint32_t k1[32];                  // rng key word 1
 };
 constexpr uint32_t kPoolInvalid = 0xffffffffu;
+
+// The producer side of a warp's pool; warp-uniform.
+struct PoolState {
+    bool dry;                         // the sample counter has run past the end
+    uint32_t ready;                   // rays in the pool, entries [0, ready)
+    // The warp's private range of samples [w_next, w_end).  Scan-heavy scenes take 32 samples per atomic; small scenes, where a
+    // scan is a few hundred instructions and one atomic per 32 samples would saturate the counter's L2 line, take up to
+    // sched_kmax x 32, shrinking as left / (sched_div x lanes) so that the last warps finish together.
+    unsigned long long w_next, w_end;
+};
+
+// The whole warp produces the next 32 consecutive samples into its pool (every lane has popped what it takes from it): takes a
+// new range when its own is used up, decodes sample g = lp * spp + s under the interleaved row-tile partition and generates the
+// primary ray.  lanes_x = lanes of the grid x sched_div.
+__device__ __forceinline__ void pool_produce(const RenderArgs &a, WarpPool &pool, PoolState &ps, const uint16_t *tab, unsigned lane, uint32_t lanes_x)
+{
+    __syncwarp();
+    if (ps.w_next >= ps.w_end) {
+        unsigned long long base = 0;
+        uint32_t k = 1;
+        if (lane == 0) {
+            const unsigned long long left = a.n_samples > ps.w_end ? a.n_samples - ps.w_end : 0ull;
+            const unsigned long long want_k = left / lanes_x;
+            k = want_k >= a.sched_kmax ? a.sched_kmax : (want_k < 1 ? 1u : (uint32_t)want_k);
+            base = atomicAdd(a.sample_counter, 32ull * k);
+        }
+        base = __shfl_sync(kFull, base, 0);
+        k = __shfl_sync(kFull, k, 0);
+        ps.w_next = base;
+        ps.w_end = base + 32ull * k < a.n_samples ? base + 32ull * k : a.n_samples;
+    }
+    if (ps.w_next >= a.n_samples) {
+        ps.dry = true;
+        ps.ready = 0;
+    } else {
+        const unsigned long long g = ps.w_next + lane;
+        ps.w_next += 32;
+        float4 pa = make_float4(0, 0, 0, __uint_as_float(kPoolInvalid)), pb = make_float4(0, 0, 0, 0);
+        uint32_t pk1 = 0;
+        if (g < a.n_samples) {
+            const uint32_t plp = a.magic_spp ? (uint32_t)__umul64hi(g, a.magic_spp) : (uint32_t)g;
+            const uint32_t smp = (uint32_t)(g - (unsigned long long)plp * (uint32_t)a.spp);
+            const uint32_t lr = fast_div(plp, a.magic_width);
+            const int x = (int)(plp - lr * (uint32_t)a.width);
+            const uint32_t tile = fast_div(lr, a.magic_row_tile);
+            const int y = (int)((tile * (uint32_t)a.world + (uint32_t)a.rank) * (uint32_t)a.row_tile + (lr - tile * (uint32_t)a.row_tile));
+            Rng r;
+            f3 po, pd;
+            primary_ray(a, (uint32_t)y * (uint32_t)a.width + (uint32_t)x, (float)x, (float)y, (int)smp, tab, r, po, pd);
+            pa = make_float4(po.x, po.y, po.z, __uint_as_float(plp));
+            pb = make_float4(pd.x, pd.y, pd.z, __uint_as_float(r.k0));
+            pk1 = r.k1;
+        }
+        pool.a[lane] = pa; pool.b[lane] = pb; pool.k1[lane] = pk1;
+        ps.ready = 32;
+    }
+    __syncwarp();
+}
+
+// Lanes without a path (`want`, ballot `need`) take a ray from the warp's pool; the warp produces more when the pool runs short.
+// A lane that finds the work exhausted keeps its o / d.
+__device__ __forceinline__ void pool_take(const RenderArgs &a, WarpPool &pool, PoolState &ps, const uint16_t *tab, unsigned lane, unsigned lt_mask,
+                                          uint32_t lanes_x, unsigned need, bool want, bool &active, bool &exhausted, f3 &o, f3 &d, uint32_t &lp, Rng &rng,
+                                          f3 &thr, int &depth)
+{
+    const uint32_t n_need = (uint32_t)__popc(need), rank = (uint32_t)__popc(need & lt_mask);
+    int entry = -1;
+    if (want && rank < ps.ready) entry = (int)(ps.ready - 1u - rank);
+    const uint32_t n_first = min(n_need, ps.ready);
+    float4 ea = make_float4(0, 0, 0, __uint_as_float(kPoolInvalid)), eb = make_float4(0, 0, 0, 0);
+    uint32_t ek1 = 0;
+    if (entry >= 0) { ea = pool.a[entry]; eb = pool.b[entry]; ek1 = pool.k1[entry]; }   // pop before the pool is overwritten
+    if (n_need > ps.ready && !ps.dry) {                          // warp-uniform: not enough rays
+        pool_produce(a, pool, ps, tab, lane, lanes_x);
+        const uint32_t rank2 = rank - n_first;                   // rank among the lanes the old pool could not serve
+        if (want && entry < 0 && rank2 < ps.ready) {
+            entry = (int)(ps.ready - 1u - rank2);
+            ea = pool.a[entry]; eb = pool.b[entry]; ek1 = pool.k1[entry];
+        }
+        ps.ready -= min(n_need - n_first, ps.ready);
+    } else {                                                     // the pool serves everybody (or there is nothing left to produce)
+        ps.ready -= n_first;
+    }
+    if (want) {
+        if (entry >= 0 && __float_as_uint(ea.w) != kPoolInvalid) {
+            o = mk3(ea.x, ea.y, ea.z); d = mk3(eb.x, eb.y, eb.z); lp = __float_as_uint(ea.w);
+            rng.k0 = __float_as_uint(eb.w); rng.k1 = ek1;
+            thr = mk3(1, 1, 1); depth = 0; active = true;
+        } else {
+            exhausted = true;                                    // past the end of the work
+        }
+    }
+}
 
 template <int kScan, bool kStaged, int kThreads, int kBlocksPerSM>
 __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool(const __grid_constant__ RenderArgs a)
@@ -326,12 +431,8 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool(const 
     WarpPool &pool = reinterpret_cast<WarpPool *>(after_spheres + (kScratch ? sizeof(WarpScratch) * (kThreads / 32) : 0))[threadIdx.x >> 5];
 
     bool active = false, exhausted = false;
-    bool dry = false;                                            // warp-uniform: the sample counter has run past the end
-    uint32_t ready = 0;                                          // warp-uniform: rays in the pool, entries [0, ready)
-    // warp-uniform: the warp's private range of samples [w_next, w_end).  Scan-heavy scenes take 32 samples per atomic; small
-    // scenes, where a scan is a few hundred instructions and one atomic per 32 samples would saturate the counter's L2 line,
-    // take up to sched_kmax x 32, shrinking as left / (sched_div x lanes) so that the last warps finish together.
-    unsigned long long w_next = 0, w_end = 0;
+    PoolState ps;
+    ps.dry = false; ps.ready = 0; ps.w_next = 0; ps.w_end = 0;
     const uint32_t lanes_x = gridDim.x * blockDim.x * a.sched_div;
     uint32_t lp = 0, nrays = 0;
     int depth = 0;
@@ -341,66 +442,26 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool(const 
     rng.k0 = 0; rng.k1 = 0;
 
     for (;;) {
-        // -- lanes without a path take a ray from the warp's pool; the warp refills the pool when it runs short
+        // -- lanes without a path take a ray from the warp's pool; the warp produces more when the pool runs short.  pool_take's
+        //    logic, written out: through pool_take this kernel measured 0.8-3.4 % slower on B200 (DESIGN.md section 4.12)
         const bool want = !active && !exhausted;
         const unsigned need = __ballot_sync(kFull, want);
         if (need) {
             const uint32_t n_need = (uint32_t)__popc(need), rank = (uint32_t)__popc(need & lt_mask);
             int entry = -1;                                      // pool entry this lane pops
-            if (want && rank < ready) entry = (int)(ready - 1u - rank);
-            const uint32_t n_first = min(n_need, ready);
-            if (n_need > ready && !dry) {                        // warp-uniform: not enough rays, produce the next 32 samples
+            if (want && rank < ps.ready) entry = (int)(ps.ready - 1u - rank);
+            const uint32_t n_first = min(n_need, ps.ready);
+            if (n_need > ps.ready && !ps.dry) {                  // warp-uniform: not enough rays
                 float4 ea = make_float4(0, 0, 0, 0), eb = make_float4(0, 0, 0, 0);
                 uint32_t ek1 = 0;
                 if (entry >= 0) { ea = pool.a[entry]; eb = pool.b[entry]; ek1 = pool.k1[entry]; }   // pop before the pool is overwritten
-                __syncwarp();
-                if (w_next >= w_end) {                           // the private range is used up: take the next one
-                    unsigned long long base = 0;
-                    uint32_t k = 1;
-                    if (lane == 0) {
-                        const unsigned long long left = a.n_samples > w_end ? a.n_samples - w_end : 0ull;
-                        const unsigned long long want_k = left / lanes_x;
-                        k = want_k >= a.sched_kmax ? a.sched_kmax : (want_k < 1 ? 1u : (uint32_t)want_k);
-                        base = atomicAdd(a.sample_counter, 32ull * k);
-                    }
-                    base = __shfl_sync(kFull, base, 0);
-                    k = __shfl_sync(kFull, k, 0);
-                    w_next = base;
-                    w_end = base + 32ull * k < a.n_samples ? base + 32ull * k : a.n_samples;
-                }
-                if (w_next >= a.n_samples) {
-                    dry = true;
-                    ready = 0;
-                } else {
-                    const unsigned long long g = w_next + lane;
-                    w_next += 32;
-                    float4 pa = make_float4(0, 0, 0, __uint_as_float(kPoolInvalid)), pb = make_float4(0, 0, 0, 0);
-                    uint32_t pk1 = 0;
-                    if (g < a.n_samples) {
-                        // sample g -> (local pixel, sample index) -> global pixel under the interleaved row-tile partition
-                        const uint32_t plp = a.magic_spp ? (uint32_t)__umul64hi(g, a.magic_spp) : (uint32_t)g;
-                        const uint32_t smp = (uint32_t)(g - (unsigned long long)plp * (uint32_t)a.spp);
-                        const uint32_t lr = fast_div(plp, a.magic_width);
-                        const int x = (int)(plp - lr * (uint32_t)a.width);
-                        const uint32_t tile = fast_div(lr, a.magic_row_tile);
-                        const int y = (int)((tile * (uint32_t)a.world + (uint32_t)a.rank) * (uint32_t)a.row_tile + (lr - tile * (uint32_t)a.row_tile));
-                        Rng r;
-                        f3 po, pd;
-                        primary_ray(a, (uint32_t)y * (uint32_t)a.width + (uint32_t)x, (float)x, (float)y, (int)smp, tab, r, po, pd);
-                        pa = make_float4(po.x, po.y, po.z, __uint_as_float(plp));
-                        pb = make_float4(pd.x, pd.y, pd.z, __uint_as_float(r.k0));
-                        pk1 = r.k1;
-                    }
-                    pool.a[lane] = pa; pool.b[lane] = pb; pool.k1[lane] = pk1;
-                    ready = 32;
-                }
-                __syncwarp();
+                pool_produce(a, pool, ps, tab, lane, lanes_x);
                 const uint32_t rank2 = rank - n_first;           // rank among the lanes the old pool could not serve
-                if (want && entry < 0 && rank2 < ready) {
-                    entry = (int)(ready - 1u - rank2);
+                if (want && entry < 0 && rank2 < ps.ready) {
+                    entry = (int)(ps.ready - 1u - rank2);
                     ea = pool.a[entry]; eb = pool.b[entry]; ek1 = pool.k1[entry];
                 }
-                ready -= min(n_need - n_first, ready);
+                ps.ready -= min(n_need - n_first, ps.ready);
                 if (want) {
                     if (entry >= 0 && __float_as_uint(ea.w) != kPoolInvalid) {
                         o = mk3(ea.x, ea.y, ea.z); d = mk3(eb.x, eb.y, eb.z); lp = __float_as_uint(ea.w);
@@ -412,7 +473,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool(const 
                     }
                 }
             } else {                                             // the pool serves everybody (or there is nothing left to produce)
-                ready -= n_first;
+                ps.ready -= n_first;
                 if (want) {
                     bool got = false;
                     if (entry >= 0) {
@@ -452,11 +513,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool(const 
             }
         }
     }
-    // -- total-rays counter (rayweek1.cpp:809-813): warp reduce, one 64-bit atomic per warp
-    unsigned long long total = nrays;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
-    if (lane == 0 && total) atomicAdd(a.num_rays, total);
+    count_rays(a, nrays, lane);
 }
 
 // ------------------------------------------------------------------------------------------------ megakernel, two paths per lane
@@ -491,9 +548,8 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool2(const
     WarpPool &pool = reinterpret_cast<WarpPool *>(smem_raw + kSmemSpheres + (kStaged ? (size_t)a.scene.n_pad * 32 : 0))[threadIdx.x >> 5];
 
     bool active[2] = { false, false };
-    bool dry = false;                                            // warp-uniform
-    uint32_t ready = 0;                                          // warp-uniform
-    unsigned long long w_next = 0, w_end = 0;                    // warp-uniform private sample range
+    PoolState ps;
+    ps.dry = false; ps.ready = 0; ps.w_next = 0; ps.w_end = 0;
     const uint32_t lanes_x = gridDim.x * blockDim.x * a.sched_div;
     uint32_t lp[2] = { 0, 0 }, nrays = 0;
     int depth[2] = { 0, 0 };
@@ -510,7 +566,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool2(const
             const uint32_t rank[2] = { (uint32_t)__popc(need0 & lt_mask), n0 + (uint32_t)__popc(need1 & lt_mask) };
             uint32_t served = 0;                                 // warp-uniform: slots with rank < served have been handled
             for (;;) {
-                const uint32_t avail = ready;
+                const uint32_t avail = ps.ready;
 #pragma unroll
                 for (int r = 0; r < 2; ++r) {
                     if (!active[r] && rank[r] >= served && rank[r] < served + avail) {
@@ -524,58 +580,18 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool2(const
                     }
                 }
                 const uint32_t take = min(avail, n_need - served);
-                ready -= take;
+                ps.ready -= take;
                 served += avail;
-                if (served >= n_need || dry) break;
-                // produce the next 32 samples (everything in the pool has been popped: ready == 0)
-                __syncwarp();
-                if (w_next >= w_end) {
-                    unsigned long long base = 0;
-                    uint32_t k = 1;
-                    if (lane == 0) {
-                        const unsigned long long left = a.n_samples > w_end ? a.n_samples - w_end : 0ull;
-                        const unsigned long long want_k = left / lanes_x;
-                        k = want_k >= a.sched_kmax ? a.sched_kmax : (want_k < 1 ? 1u : (uint32_t)want_k);
-                        base = atomicAdd(a.sample_counter, 32ull * k);
-                    }
-                    base = __shfl_sync(kFull, base, 0);
-                    k = __shfl_sync(kFull, k, 0);
-                    w_next = base;
-                    w_end = base + 32ull * k < a.n_samples ? base + 32ull * k : a.n_samples;
-                }
-                if (w_next >= a.n_samples) {
-                    dry = true;
-                } else {
-                    const unsigned long long g = w_next + lane;
-                    w_next += 32;
-                    float4 pa = make_float4(0, 0, 0, __uint_as_float(kPoolInvalid)), pb = make_float4(0, 0, 0, 0);
-                    uint32_t pk1 = 0;
-                    if (g < a.n_samples) {
-                        const uint32_t plp = a.magic_spp ? (uint32_t)__umul64hi(g, a.magic_spp) : (uint32_t)g;
-                        const uint32_t smp = (uint32_t)(g - (unsigned long long)plp * (uint32_t)a.spp);
-                        const uint32_t lr = fast_div(plp, a.magic_width);
-                        const int x = (int)(plp - lr * (uint32_t)a.width);
-                        const uint32_t tile = fast_div(lr, a.magic_row_tile);
-                        const int y = (int)((tile * (uint32_t)a.world + (uint32_t)a.rank) * (uint32_t)a.row_tile + (lr - tile * (uint32_t)a.row_tile));
-                        Rng r;
-                        f3 po, pd;
-                        primary_ray(a, (uint32_t)y * (uint32_t)a.width + (uint32_t)x, (float)x, (float)y, (int)smp, tab, r, po, pd);
-                        pa = make_float4(po.x, po.y, po.z, __uint_as_float(plp));
-                        pb = make_float4(pd.x, pd.y, pd.z, __uint_as_float(r.k0));
-                        pk1 = r.k1;
-                    }
-                    pool.a[lane] = pa; pool.b[lane] = pb; pool.k1[lane] = pk1;
-                    ready = 32;
-                }
-                __syncwarp();
-                if (dry) break;
+                if (served >= n_need || ps.dry) break;
+                pool_produce(a, pool, ps, tab, lane, lanes_x);   // everything in the pool has been popped: ready == 0
+                if (ps.dry) break;
             }
 #pragma unroll
             for (int r = 0; r < 2; ++r)
                 if (!active[r]) { o[r] = mk3(0.0f, 1.0e18f, 0.0f); d[r] = mk3(0.0f, 0.0f, 0.0f); }   // nothing left for this slot
         }
         // the warp is done when the work has run dry, the pool is empty and no slot holds a path
-        if (dry && ready == 0 && __all_sync(kFull, !active[0] && !active[1])) break;
+        if (ps.dry && ps.ready == 0 && __all_sync(kFull, !active[0] && !active[1])) break;
 
         // -- Hitable::hit for both rays against the same sphere loads
         float t[2] = { kTMax, kTMax };
@@ -596,10 +612,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool2(const
             }
         }
     }
-    unsigned long long total = nrays;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
-    if (lane == 0 && total) atomicAdd(a.num_rays, total);
+    count_rays(a, nrays, lane);
 }
 
 // ------------------------------------------------------------------------------------------------ megakernel, tensor-core filter
@@ -628,85 +641,6 @@ struct TcControl {
     uint32_t pad_[2];
 };
 static_assert(sizeof(TcControl) % 16 == 0, "TcControl is followed by 16-byte aligned tiles");
-
-// Lanes without a path take a ray from the warp's pool; the warp refills the pool when it runs short (megakernel_pool's refill).
-struct PoolState {
-    bool dry;
-    uint32_t ready;
-    unsigned long long w_next, w_end;
-};
-__device__ __forceinline__ void pool_take(const RenderArgs &a, WarpPool &pool, PoolState &ps, const uint16_t *tab, unsigned lane, unsigned lt_mask,
-                                          uint32_t lanes_x, unsigned need, bool want, bool &active, bool &exhausted, f3 &o, f3 &d, uint32_t &lp, Rng &rng,
-                                          f3 &thr, int &depth)
-{
-    const uint32_t n_need = (uint32_t)__popc(need), rank = (uint32_t)__popc(need & lt_mask);
-    int entry = -1;
-    if (want && rank < ps.ready) entry = (int)(ps.ready - 1u - rank);
-    const uint32_t n_first = min(n_need, ps.ready);
-    float4 ea = make_float4(0, 0, 0, __uint_as_float(kPoolInvalid)), eb = make_float4(0, 0, 0, 0);
-    uint32_t ek1 = 0;
-    if (entry >= 0) { ea = pool.a[entry]; eb = pool.b[entry]; ek1 = pool.k1[entry]; }
-    if (n_need > ps.ready && !ps.dry) {                          // warp-uniform: produce the next 32 samples
-        __syncwarp();
-        if (ps.w_next >= ps.w_end) {
-            unsigned long long base = 0;
-            uint32_t k = 1;
-            if (lane == 0) {
-                const unsigned long long left = a.n_samples > ps.w_end ? a.n_samples - ps.w_end : 0ull;
-                const unsigned long long want_k = left / lanes_x;
-                k = want_k >= a.sched_kmax ? a.sched_kmax : (want_k < 1 ? 1u : (uint32_t)want_k);
-                base = atomicAdd(a.sample_counter, 32ull * k);
-            }
-            base = __shfl_sync(kFull, base, 0);
-            k = __shfl_sync(kFull, k, 0);
-            ps.w_next = base;
-            ps.w_end = base + 32ull * k < a.n_samples ? base + 32ull * k : a.n_samples;
-        }
-        if (ps.w_next >= a.n_samples) {
-            ps.dry = true;
-            ps.ready = 0;
-        } else {
-            const unsigned long long g = ps.w_next + lane;
-            ps.w_next += 32;
-            float4 pa = make_float4(0, 0, 0, __uint_as_float(kPoolInvalid)), pb = make_float4(0, 0, 0, 0);
-            uint32_t pk1 = 0;
-            if (g < a.n_samples) {
-                const uint32_t plp = a.magic_spp ? (uint32_t)__umul64hi(g, a.magic_spp) : (uint32_t)g;
-                const uint32_t smp = (uint32_t)(g - (unsigned long long)plp * (uint32_t)a.spp);
-                const uint32_t lr = fast_div(plp, a.magic_width);
-                const int x = (int)(plp - lr * (uint32_t)a.width);
-                const uint32_t tile = fast_div(lr, a.magic_row_tile);
-                const int y = (int)((tile * (uint32_t)a.world + (uint32_t)a.rank) * (uint32_t)a.row_tile + (lr - tile * (uint32_t)a.row_tile));
-                Rng r;
-                f3 po, pd;
-                primary_ray(a, (uint32_t)y * (uint32_t)a.width + (uint32_t)x, (float)x, (float)y, (int)smp, tab, r, po, pd);
-                pa = make_float4(po.x, po.y, po.z, __uint_as_float(plp));
-                pb = make_float4(pd.x, pd.y, pd.z, __uint_as_float(r.k0));
-                pk1 = r.k1;
-            }
-            pool.a[lane] = pa; pool.b[lane] = pb; pool.k1[lane] = pk1;
-            ps.ready = 32;
-        }
-        __syncwarp();
-        const uint32_t rank2 = rank - n_first;                   // rank among the lanes the old pool could not serve
-        if (want && entry < 0 && rank2 < ps.ready) {
-            entry = (int)(ps.ready - 1u - rank2);
-            ea = pool.a[entry]; eb = pool.b[entry]; ek1 = pool.k1[entry];
-        }
-        ps.ready -= min(n_need - n_first, ps.ready);
-    } else {
-        ps.ready -= n_first;
-    }
-    if (want) {
-        if (entry >= 0 && __float_as_uint(ea.w) != kPoolInvalid) {
-            o = mk3(ea.x, ea.y, ea.z); d = mk3(eb.x, eb.y, eb.z); lp = __float_as_uint(ea.w);
-            rng.k0 = __float_as_uint(eb.w); rng.k1 = ek1;
-            thr = mk3(1, 1, 1); depth = 0; active = true;
-        } else {
-            exhausted = true;                                    // past the end of the work
-        }
-    }
-}
 
 constexpr size_t tc3_smem_bytes(int groups, int n32)
 {
@@ -888,10 +822,7 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tc3(const __grid_
             }
         }
     }
-    unsigned long long total = nrays;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
-    if (lane == 0 && total) atomicAdd(a.num_rays, total);
+    count_rays(a, nrays, lane);
     tc::tc_fence_before();
     __syncthreads();
     if (threadIdx.x < 32) tc::tmem_dealloc(tmem_base, 512);
@@ -1160,10 +1091,7 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tcs(const __grid_
             }
         }
     }
-    unsigned long long total = nrays;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
-    if (lane == 0 && total) atomicAdd(a.num_rays, total);
+    count_rays(a, nrays, lane);
     tc::tc_fence_before();
     __syncthreads();
     if (threadIdx.x == 0) {                                      // no bulk copy may still be writing when the CTA ends

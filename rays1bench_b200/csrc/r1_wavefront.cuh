@@ -159,10 +159,7 @@ __global__ void __launch_bounds__(kThreads, 1) wf_intersect(const __grid_constan
             }
         }
     }
-    unsigned long long total = nrays;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
-    if (lane == 0 && total) atomicAdd(a.num_rays, total);
+    count_rays(a, nrays, lane);
 }
 
 // color() + (on path end) accumulate, next sample / next unit, next primary ray -- class by class.
