@@ -223,13 +223,13 @@ constexpr int kDefaultThreads = 1024;     // per-lane scans: 64 registers
 constexpr int kDefaultThreadsCoop = 512;  // cooperative scan: 4 rays per lane in flight, 127 registers
 
 // streamed tensor-core filter (r1::megakernel_tcs, R1_VARIANT_MEGAKERNEL_TENSOR_STREAM): `threads` / 128 = ray groups per CTA (one
-// 128-column TMEM accumulator each), R1_TCS_STAGES = depth of the operand ring.  Shared memory does not depend on the scene.
+// 128-column TMEM accumulator each), kDefaultTcsStages = depth of the operand ring.  Shared memory does not depend on the scene.
 // Measured on synth4096 at 1280x720x250 (B200, 1000 W; DESIGN.md section 4.7, profiles/r03_bench_tensor_stream.json): 4 groups with
 // 2 / 3 / 4 / 6 stages 1279 / 1324 / 1350 / 1358 Mrays/s; 3 / 2 / 1 groups with 6 stages 1120 / 806 / 415 (PACKED: 827).
 constexpr int kDefaultTcsGroups = 4, kDefaultTcsStages = 6;
 
-// BVH traversal (megakernel_pool<kScanBvh>, R1_VARIANT_MEGAKERNEL_BVH): nothing is staged, every CTA shape runs the sample pool
-// (R1_POOL=0 does not apply).  Measured at 640x360x32 (B200, DESIGN.md section 4.8), Mrays/s for 512 / 768 / 1024 threads: large
+// BVH traversal (megakernel_pool<kScanBvh>, R1_VARIANT_MEGAKERNEL_BVH): nothing is staged.
+// Measured at 640x360x32 (B200, DESIGN.md section 4.8), Mrays/s for 512 / 768 / 1024 threads: large
 // 7143 / 8264 / 8531, 10^5-sphere cloud 527 / 705 / 789, 10^5-sphere grid 2603 / 3331 / 3565.  Samples per atomic (sched_kmax x 32,
 // shrinking by sched_div) at 512 threads, kmax,div = 64,16 / 8,16 / 1,1: large 7143 / 7114 / 6716, cloud 527 / 529 / 525.
 constexpr int kDefaultThreadsBvh = 1024;
@@ -237,21 +237,14 @@ constexpr uint32_t kBvhSchedKmax = 64, kBvhSchedDiv = 16;
 
 // The tuning knobs of the environment.  Read on every render, so that a caller can change them between renders.
 struct Knobs {
-    bool pool = true;                   // R1_POOL=0: r1::megakernel's per-lane unit fetch instead of the warp sample pool
     bool force_unstaged = false;        // R1_FORCE_UNSTAGED: scan from global memory even where the scene could be staged
-    bool auto_tensor = true;            // R1_AUTO_TENSOR=0: R1_VARIANT_MEGAKERNEL never resolves to the tensor-core filter
-    int tcs_stages = kDefaultTcsStages; // R1_TCS_STAGES: depth of the tensor-stream variant's operand ring
     uint32_t sched_kmax = 0, sched_div = 0;   // R1_SCHED "kmax,div" (1 .. 4096, 1 .. 1024) overrides the scheduling; 0: not set
 };
 
 Knobs read_knobs()
 {
-    const auto zero = [](const char *name) { const char *e = getenv(name); return e && atoi(e) == 0; };
     Knobs k;
-    k.pool = !zero("R1_POOL");
     k.force_unstaged = getenv("R1_FORCE_UNSTAGED") != nullptr;
-    k.auto_tensor = !zero("R1_AUTO_TENSOR");
-    if (const char *e = getenv("R1_TCS_STAGES")) k.tcs_stages = atoi(e);
     if (const char *e = getenv("R1_SCHED")) {
         unsigned kmax = 0, div = 0;
         if (sscanf(e, "%u,%u", &kmax, &div) == 2 && kmax >= 1 && kmax <= 4096 && div >= 1 && div <= 1024) { k.sched_kmax = kmax; k.sched_div = div; }
@@ -262,13 +255,12 @@ Knobs read_knobs()
 // Samples per atomic (guided self-scheduling).  The sample pool: a WARP takes kmax x 32 consecutive samples per atomicAdd, shrinking
 // as left / (div x lanes) towards the end.  Measured on B200 (large scene, Mrays/s, full image | rank 0 of 8 = the per-GPU share of
 // the 8-GPU partition):  1,1: 6066 | 6057   2,16: 6102 | 6088   4,16: 6121 | 6088   8,16: 6132 | 6103.  Small scenes need long
-// ranges: with 32 samples per atomic the one counter line in L2 saturates (small scene 39 G rays/s instead of 58).  r1::megakernel
-// (R1_POOL=0) hands units to LANES; its round-1 tuning is kept: 1 unit per fetch on scan-heavy scenes (ranges held by lanes at the
-// end of a render are a serial tail), up to 64 on small ones.  BVH traversals are short at every scene size (DESIGN.md section 4.8).
+// ranges: with 32 samples per atomic the one counter line in L2 saturates (small scene 39 G rays/s instead of 58).  BVH traversals
+// are short at every scene size (DESIGN.md section 4.8).
 void pick_schedule(const r1::DevScene &dev, int variant, const Knobs &k, r1::RenderArgs &a)
 {
     if (variant == R1_VARIANT_MEGAKERNEL_BVH) { a.sched_kmax = kBvhSchedKmax; a.sched_div = kBvhSchedDiv; }
-    else if (dev.n8 >= 256) { a.sched_kmax = k.pool ? 8 : 1; a.sched_div = k.pool ? 16 : 1; }
+    else if (dev.n8 >= 256) { a.sched_kmax = 8; a.sched_div = 16; }
     else { a.sched_kmax = 64; a.sched_div = 16; }
     if (k.sched_kmax) { a.sched_kmax = k.sched_kmax; a.sched_div = k.sched_div; }
 }
@@ -290,28 +282,27 @@ int launch_persistent(RenderKernel kern, int threads, size_t smem, unsigned long
 }
 
 // [mbarrier 16 B | rsqrtss table 4 KB | staged spheres n_pad * 32 B | per-warp scan scratch (coop / deferred) | per-warp sample pools]
-size_t megakernel_smem(int scan, bool staged, int n_pad, int threads, bool pool)
+size_t megakernel_smem(int scan, bool staged, int n_pad, int threads)
 {
     return r1::kSmemSpheres + (staged ? (size_t)n_pad * 32 : 0) +
-           (scan == r1::kScanCoop || scan == r1::kScanLaneDeferred ? sizeof(r1::WarpScratch) * (threads / 32) : 0) + (pool ? sizeof(r1::WarpPool) * (threads / 32) : 0);
+           (scan == r1::kScanCoop || scan == r1::kScanLaneDeferred ? sizeof(r1::WarpScratch) * (threads / 32) : 0) + sizeof(r1::WarpPool) * (threads / 32);
 }
 
-// warp sample-pool scheduling (r1::megakernel_pool): the default; R1_POOL=0 selects the per-lane unit fetch of r1::megakernel
+// r1::megakernel_pool with the packed, scalar, cooperative or deferred scan
 template <int kScan, bool kStaged>
-int launch_megakernel(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, bool pool, cudaStream_t stream)
+int launch_megakernel(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
 {
     int threads = prm.threads > 0 ? prm.threads : (kScan == r1::kScanCoop ? kDefaultThreadsCoop : kDefaultThreads);
     // The deferred scan's 2 KB of queue per warp: with the sample pool, 1024 threads and more than 3 936 staged spheres exceed
     // 227 KB of shared memory.  The default then runs 768 threads (the image does not depend on the thread count).
-    if (prm.threads <= 0 && pool && megakernel_smem(kScan, kStaged, args.scene.n_pad, threads, true) > 227 * 1024) threads = 768;
+    if (prm.threads <= 0 && megakernel_smem(kScan, kStaged, args.scene.n_pad, threads) > 227 * 1024) threads = 768;
     RenderKernel kern = nullptr;
-    if (threads == 512) kern = pool ? r1::megakernel_pool<kScan, kStaged, 512, 1> : r1::megakernel<kScan, kStaged, 512, 1>;
-    if (threads == 768) kern = pool ? r1::megakernel_pool<kScan, kStaged, 768, 1> : r1::megakernel<kScan, kStaged, 768, 1>;
-    if (threads == 1024) kern = pool ? r1::megakernel_pool<kScan, kStaged, 1024, 1> : r1::megakernel<kScan, kStaged, 1024, 1>;
+    if (threads == 512) kern = r1::megakernel_pool<kScan, kStaged, 512, 1>;
+    if (threads == 768) kern = r1::megakernel_pool<kScan, kStaged, 768, 1>;
+    if (threads == 1024) kern = r1::megakernel_pool<kScan, kStaged, 1024, 1>;
     if (!kern) return fail(R1_ERR_ARG, "threads must be 512, 768 or 1024 (got %d)", threads);
-    const size_t smem = megakernel_smem(kScan, kStaged, args.scene.n_pad, threads, pool);
-    if (pool) return launch_persistent(kern, threads, smem, args.n_samples, threads, prm.blocks_per_sm, sm_count, "megakernel_pool", args, stream);
-    return launch_persistent(kern, threads, smem, args.n_units, threads, prm.blocks_per_sm, sm_count, "megakernel", args, stream);
+    return launch_persistent(kern, threads, megakernel_smem(kScan, kStaged, args.scene.n_pad, threads), args.n_samples, threads, prm.blocks_per_sm, sm_count,
+                             "megakernel_pool", args, stream);
 }
 
 int launch_megakernel_bvh(int sm_count, const r1::RenderArgs &args, const float4 *nodes, const float4 *leaves, const r1_render_params &prm,
@@ -325,7 +316,7 @@ int launch_megakernel_bvh(int sm_count, const r1::RenderArgs &args, const float4
     if (threads == 768) kern = r1::megakernel_pool<r1::kScanBvh, false, 768, 1>;
     if (threads == 1024) kern = r1::megakernel_pool<r1::kScanBvh, false, 1024, 1>;
     if (!kern) return fail(R1_ERR_ARG, "the bvh variant runs 512, 768 or 1024 threads (got %d)", threads);
-    return launch_persistent(kern, threads, megakernel_smem(r1::kScanBvh, false, args.scene.n_pad, threads, true), args.n_samples, threads, prm.blocks_per_sm,
+    return launch_persistent(kern, threads, megakernel_smem(r1::kScanBvh, false, args.scene.n_pad, threads), args.n_samples, threads, prm.blocks_per_sm,
                              sm_count, "bvh variant", args, stream);
 }
 
@@ -338,7 +329,7 @@ int launch_megakernel_dual(int sm_count, const r1::RenderArgs &args, const r1_re
     if (threads == 512) kern = r1::megakernel_pool2<kStaged, 512, 1>;
     if (threads == 768) kern = r1::megakernel_pool2<kStaged, 768, 1>;
     if (!kern) return fail(R1_ERR_ARG, "the dual variant runs 512 or 768 threads (got %d)", threads);
-    return launch_persistent(kern, threads, megakernel_smem(r1::kScanLanePacked, kStaged, args.scene.n_pad, threads, true), args.n_samples, 2ull * threads,
+    return launch_persistent(kern, threads, megakernel_smem(r1::kScanLanePacked, kStaged, args.scene.n_pad, threads), args.n_samples, 2ull * threads,
                              prm.blocks_per_sm, sm_count, "dual variant", args, stream);
 }
 
@@ -359,22 +350,17 @@ int launch_megakernel_tc(int sm_count, const r1::RenderArgs &args, const r1_rend
 }
 
 // streamed tensor-core filter (r1::megakernel_tcs): one CTA per SM
-int launch_megakernel_tcs(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, int stages, cudaStream_t stream)
+int launch_megakernel_tcs(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
 {
     const int groups = prm.threads > 0 ? prm.threads / 128 : kDefaultTcsGroups;
     RenderKernel kern = nullptr;
-    if (groups == 4 && stages == 2) kern = r1::megakernel_tcs<4, 2>;
-    if (groups == 4 && stages == 3) kern = r1::megakernel_tcs<4, 3>;
-    if (groups == 4 && stages == 4) kern = r1::megakernel_tcs<4, 4>;
-    if (groups == 4 && stages == 6) kern = r1::megakernel_tcs<4, 6>;
-    if (groups == 3 && stages == 6) kern = r1::megakernel_tcs<3, 6>;
-    if (groups == 2 && stages == 6) kern = r1::megakernel_tcs<2, 6>;
-    if (groups == 1 && stages == 6) kern = r1::megakernel_tcs<1, 6>;
-    if (!kern)
-        return fail(R1_ERR_ARG, "the tensor-stream variant runs 1 .. 4 groups of 128 ray threads per CTA (threads = 128 .. 512) with a 6-stage ring, "
-                                "or 4 groups with 2, 3, 4 or 6 stages (got %d groups, %d stages)", groups, stages);
-    return launch_persistent(kern, groups * 128, r1::tcs_smem_bytes(groups, stages), args.n_samples, groups * 128, 1, sm_count, "tensor-stream variant", args,
-                             stream);
+    if (groups == 4) kern = r1::megakernel_tcs<4, kDefaultTcsStages>;
+    if (groups == 3) kern = r1::megakernel_tcs<3, kDefaultTcsStages>;
+    if (groups == 2) kern = r1::megakernel_tcs<2, kDefaultTcsStages>;
+    if (groups == 1) kern = r1::megakernel_tcs<1, kDefaultTcsStages>;
+    if (!kern) return fail(R1_ERR_ARG, "the tensor-stream variant runs 1 .. 4 groups of 128 ray threads per CTA (threads = 128 .. 512, got %d groups)", groups);
+    return launch_persistent(kern, groups * 128, r1::tcs_smem_bytes(groups, kDefaultTcsStages), args.n_samples, groups * 128, 1, sm_count, "tensor-stream variant",
+                             args, stream);
 }
 
 // The host BVH of the scene, built on first need (r1_bvh.h).
@@ -441,12 +427,12 @@ int ctx_bvh(r1_scene *scene, DeviceCtx &c)
 
 // R1_VARIANT_MEGAKERNEL = the fastest megakernel for the scene.  Measured on B200: the tensor-core filter wins on the large scene
 // (485 spheres: 10.3 against 6.2 G rays/s) and loses where a scan is short (medium, 58 spheres: 25 against 34 G).  Explicit
-// tuning knobs (blocks_per_sm, threads, R1_POOL=0) address the packed kernel; R1_AUTO_TENSOR=0 keeps it everywhere.
+// tuning knobs (blocks_per_sm, threads, R1_FORCE_UNSTAGED) address the packed kernel.
 int resolve_variant(const r1::DevScene &dev, const r1_render_params &prm, const Knobs &k)
 {
     if (prm.variant != R1_VARIANT_MEGAKERNEL) return prm.variant;
-    const bool tuned = prm.blocks_per_sm > 0 || prm.threads > 0 || !k.pool || k.force_unstaged;
-    if (dev.tcb && dev.n8 >= 256 && !tuned && k.auto_tensor) return R1_VARIANT_MEGAKERNEL_TENSOR;
+    const bool tuned = prm.blocks_per_sm > 0 || prm.threads > 0 || k.force_unstaged;
+    if (dev.tcb && dev.n8 >= 256 && !tuned) return R1_VARIANT_MEGAKERNEL_TENSOR;
     return R1_VARIANT_MEGAKERNEL_PACKED;
 }
 
@@ -841,19 +827,19 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
             if (rc) return fail(R1_ERR_CUDA, "wavefront: %s", cudaGetErrorString((cudaError_t)rc));
             x.last_launches += launches;
         } else {
-            if (variant == R1_VARIANT_MEGAKERNEL_PACKED) rc = staged ? launch_megakernel<r1::kScanLanePacked, true>(x.sm_count, a, prm, knobs.pool, stream)
-                                                                  : launch_megakernel<r1::kScanLanePacked, false>(x.sm_count, a, prm, knobs.pool, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_COOP) rc = staged ? launch_megakernel<r1::kScanCoop, true>(x.sm_count, a, prm, knobs.pool, stream)
-                                                                            : launch_megakernel<r1::kScanCoop, false>(x.sm_count, a, prm, knobs.pool, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_DEFERRED) rc = staged ? launch_megakernel<r1::kScanLaneDeferred, true>(x.sm_count, a, prm, knobs.pool, stream)
-                                                                                : launch_megakernel<r1::kScanLaneDeferred, false>(x.sm_count, a, prm, knobs.pool, stream);
+            if (variant == R1_VARIANT_MEGAKERNEL_PACKED) rc = staged ? launch_megakernel<r1::kScanLanePacked, true>(x.sm_count, a, prm, stream)
+                                                                  : launch_megakernel<r1::kScanLanePacked, false>(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_COOP) rc = staged ? launch_megakernel<r1::kScanCoop, true>(x.sm_count, a, prm, stream)
+                                                                            : launch_megakernel<r1::kScanCoop, false>(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_DEFERRED) rc = staged ? launch_megakernel<r1::kScanLaneDeferred, true>(x.sm_count, a, prm, stream)
+                                                                                : launch_megakernel<r1::kScanLaneDeferred, false>(x.sm_count, a, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR) rc = launch_megakernel_tc(x.sm_count, a, prm, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) rc = launch_megakernel_tcs(x.sm_count, a, prm, knobs.tcs_stages, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) rc = launch_megakernel_tcs(x.sm_count, a, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_BVH) rc = launch_megakernel_bvh(x.sm_count, a, c.bvh_nodes, c.bvh_leaves, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_DUAL) rc = staged ? launch_megakernel_dual<true>(x.sm_count, a, prm, stream)
                                                                             : launch_megakernel_dual<false>(x.sm_count, a, prm, stream);
-            else rc = staged ? launch_megakernel<r1::kScanLaneScalar, true>(x.sm_count, a, prm, knobs.pool, stream)
-                             : launch_megakernel<r1::kScanLaneScalar, false>(x.sm_count, a, prm, knobs.pool, stream);
+            else rc = staged ? launch_megakernel<r1::kScanLaneScalar, true>(x.sm_count, a, prm, stream)
+                             : launch_megakernel<r1::kScanLaneScalar, false>(x.sm_count, a, prm, stream);
             if (rc) return rc;
             x.last_launches += 1;
         }
@@ -1204,14 +1190,13 @@ const char *r1_kernel_name(r1_scene *scene, int variant)
     r1_render_params prm;
     memset(&prm, 0, sizeof(prm));
     prm.variant = variant;
-    const Knobs k = read_knobs();
-    switch (resolve_variant(cp->dev, prm, k)) {
+    switch (resolve_variant(cp->dev, prm, read_knobs())) {
     case R1_VARIANT_WAVEFRONT: return "wf_intersect + wf_shade (graph loop)";
     case R1_VARIANT_MEGAKERNEL_TENSOR: return "megakernel_tc3";
     case R1_VARIANT_MEGAKERNEL_DUAL: return "megakernel_pool2";
     case R1_VARIANT_MEGAKERNEL_TENSOR_STREAM: return "megakernel_tcs";
     case R1_VARIANT_MEGAKERNEL_BVH: return "megakernel_bvh";
-    default: return k.pool ? "megakernel_pool" : "megakernel";
+    default: return "megakernel_pool";
     }
 }
 

@@ -9,8 +9,8 @@ namespace r1 {
 
 constexpr unsigned kFull = 0xffffffffu;
 
-// Work decomposition.  r1::megakernel_pool (default): work items are single samples g = lp * spp + s, handed to WARPS 32..2048
-// at a time from one 64-bit counter.  r1::megakernel (round-1 scheduling, R1_POOL=0) and the wavefront variant: unit
+// Work decomposition.  The persistent megakernels: work items are single samples g = lp * spp + s, handed to WARPS 32..2048
+// at a time from one 64-bit counter (the warp sample pool, WarpPool below).  The wavefront variant: unit
 // u = lp * n_chunks + c = `samples_per_unit` consecutive samples of one pixel (1 sample for spp <= 256), handed to LANES from a
 // 32-bit counter.  Either way every finished sample is added to its pixel's accumulator in 64-bit FIXED POINT (2^-24) with a
 // fire-and-forget atomic (RED.ADD.64).  Integer addition is associative: the sums, and therefore the RGB8 image, are
@@ -30,8 +30,8 @@ struct RenderArgs {
     float inv_w, inv_h, inv_spp;
     uint64_t seed;                   // Rng::seed_hash(global seed)
     uint64_t magic_chunks, magic_width, magic_row_tile;  // floor(2^64 / d) + 1: exact n / d for 32-bit n via one 64-bit mul-high (0 when d == 1)
-    uint32_t sched_kmax, sched_div;      // guided self-scheduling: min(kmax, max(1, left / (lanes * div))) units per lane (megakernel) or
-                                         // x 32 samples per warp (megakernel_pool) per atomic
+    uint32_t sched_kmax, sched_div;      // guided self-scheduling: min(kmax, max(1, left / (lanes * div))) x 32 samples per warp
+                                         // per atomic (the sample pool)
     // sample-pool scheduling (megakernel_pool): work items are single samples g = lp * spp + s, handed out 32 at a time
     unsigned long long *sample_counter;  // next sample to hand out (64-bit: 3840 x 2160 x 1024 = 8.5e9 samples)
     uint64_t n_samples, magic_spp;       // npix_local * spp; floor(2^64 / spp) + 1 (exact g / spp for g < 2^64 / spp; 0 when spp == 1)
@@ -172,135 +172,25 @@ __device__ __forceinline__ bool shade_step(const RenderArgs &a, int hit, float t
     return false;
 }
 
-// ------------------------------------------------------------------------------------------------ megakernel
-// Persistent CTAs; every lane runs  loop { take a unit | start a sample | SCAN | shade }  so that all 32 lanes enter
-// every scan with a live ray and divergence is confined to the short fetch / generate / shade steps.
+// ------------------------------------------------------------------------------------------------ megakernel, warp sample pool
+// Persistent CTAs; every lane runs  loop { take a sample | SCAN | shade }  so that all 32 lanes enter every scan with a live
+// ray and divergence is confined to the short take / shade steps.
 // Replaces render_tile + color + TileRenderScheduler (rayweek1.cpp:722-842, 515-536).
 // kScan: which Hitable::hit implementation the lanes run
 enum ScanKind { kScanCoop = 0, kScanLanePacked = 1, kScanLaneScalar = 2, kScanLaneDeferred = 3, kScanBvh = 4 };   // kScanBvh: megakernel_pool only
 __host__ __device__ constexpr int scan_filter(int kScan) { return kScan == kScanLaneScalar ? 0 : 1; }
 
-// (Round-1 scheduling, kept as the A/B alternative of megakernel_pool below: R1_POOL=0.)
-template <int kScan, bool kStaged, int kThreads, int kBlocksPerSM>
-__global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel(const __grid_constant__ RenderArgs a)
-{
-    // shared memory: [mbarrier 16 B | rsqrtss table 4 KB | staged spheres n_pad * 32 B | per-warp scratch (cooperative scan)]
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    uint16_t *s_tab = reinterpret_cast<uint16_t *>(smem_raw + 16);
-    for (int i = threadIdx.x; i < R1_RSQRT12_ENTRIES / 2; i += kThreads)
-        reinterpret_cast<uint32_t *>(s_tab)[i] = reinterpret_cast<const uint32_t *>(g_rsqrt12)[i];
-    const float4 *s_scan, *s_exact;
-    if (kStaged) {
-        float4 *s_spheres = reinterpret_cast<float4 *>(smem_raw + kSmemSpheres);
-        stage_spheres(a.scene, s_spheres, reinterpret_cast<uint64_t *>(smem_raw));   // its __syncthreads also publishes the table
-        s_scan = s_spheres;
-        s_exact = s_spheres + a.scene.n_pad;
-    } else {  // scenes beyond the staging limit scan straight from global memory (L1/L2 resident)
-        s_scan = a.scene.scan;
-        s_exact = a.scene.exact;
-        __syncthreads();
-    }
-    const uint16_t *tab = s_tab;
-    const int n_pad = a.scene.n_pad;
-    const unsigned lane = threadIdx.x & 31u;
-    // per-warp scratch of the cooperative scan, behind the staged spheres
-    WarpScratch *ws = reinterpret_cast<WarpScratch *>(smem_raw + kSmemSpheres + (kStaged ? (size_t)n_pad * 32 : 0)) + (threadIdx.x >> 5);
-
-    bool active = false, exhausted = false, need_primary = false;
-    uint32_t unit = 0, unit_end = 0, lp = 0, pixel = 0, nrays = 0, last_base = 0;
-    int s = 0, s_end = 0, depth = 0;
-    float fx = 0.0f, fy = 0.0f;
-    f3 thr = mk3(1, 1, 1);
-    f3 o = mk3(0.0f, 1.0e18f, 0.0f), d = mk3(0.0f, 0.0f, 0.0f);  // idle lanes scan a ray that passes no filter
-    Rng rng;
-    rng.k0 = 0; rng.k1 = 0;
-    const uint32_t lanes_x4 = gridDim.x * blockDim.x * a.sched_div;
-
-    for (;;) {
-        // -- take a range of units (warp-aggregated: one atomic per warp per refill round).  Guided self-scheduling:
-        //    16 units per lane while more than 64 per lane remain, shrinking to 1 at the end.
-        const bool want = !active && !exhausted;
-        const unsigned need = __ballot_sync(kFull, want);
-        if (need) {
-            const int leader = __ffs(need) - 1;
-            unsigned base = 0, k = 0;
-            if ((int)lane == leader) {
-                const uint32_t left = a.n_units > last_base ? a.n_units - last_base : 0u;
-                k = min(a.sched_kmax, max(1u, left / lanes_x4));
-                base = atomicAdd(a.unit_counter, k * (unsigned)__popc(need));
-            }
-            base = __shfl_sync(kFull, base, leader);
-            k = __shfl_sync(kFull, k, leader);
-            last_base = base;
-            if (want) {
-                unit = base + k * __popc(need & ((1u << lane) - 1u));
-                unit_end = min(unit + k, a.n_units);
-                if (unit < a.n_units) {
-                    unit_begin(a, unit, lp, pixel, fx, fy, s, s_end);
-                    active = true; need_primary = true;
-                } else {
-                    exhausted = true;
-                    o = mk3(0.0f, 1.0e18f, 0.0f); d = mk3(0.0f, 0.0f, 0.0f);
-                }
-            }
-        }
-        if (__all_sync(kFull, exhausted)) break;
-
-        // -- start a sample
-        if (active && need_primary) {
-            primary_ray(a, pixel, fx, fy, s, tab, rng, o, d);
-            thr = mk3(1, 1, 1);
-            depth = 0;
-            need_primary = false;
-        }
-
-        // -- Hitable::hit (rayweek1.cpp:152-339): uniform trip count, all lanes
-        float t = kTMax;
-        int hit = -1;
-        if (kScan == kScanCoop) scan_coop<(kThreads <= 512 ? 2 : 1)>(*ws, s_scan, s_exact, n_pad, o, d, kTMin, kTMax, t, hit);
-        else if (kScan == kScanLaneDeferred) scan_deferred(*reinterpret_cast<DeferScratch *>(ws), s_scan, s_exact, a.scene.n8, o, d, kTMin, kTMax, t, hit);
-        else scan<scan_filter(kScan)>(s_scan, s_exact, a.scene.n8, o, d, kTMin, t, hit);
-
-        // -- color() body (rayweek1.cpp:515-536)
-        if (active) {
-            ++nrays;
-            f3 contrib;
-            const float4 e = hit >= 0 ? s_exact[hit] : make_float4(0, 0, 0, 0);
-            if (shade_step(a, hit, t, e, tab, o, d, thr, depth, rng, contrib)) {
-                accumulate_sample(a, lp, contrib);
-                need_primary = true;
-                if (++s == s_end) {                          // unit done: the next one of my range, or a new range
-                    if (++unit == unit_end) {
-                        active = false;
-                        o = mk3(0.0f, 1.0e18f, 0.0f); d = mk3(0.0f, 0.0f, 0.0f);
-                    } else if (s == a.spp) {
-                        unit_begin(a, unit, lp, pixel, fx, fy, s, s_end);   // first chunk of the next pixel
-                    } else {
-                        s_end = min(s + a.samples_per_unit, a.spp);        // next chunk of the same pixel
-                    }
-                }
-            }
-        }
-    }
-    // count_rays written out: through the helper, ptxas allocates this kernel's registers differently
-    unsigned long long total = nrays;
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(kFull, total, off);
-    if (lane == 0 && total) atomicAdd(a.num_rays, total);
-}
-
-// ------------------------------------------------------------------------------------------------ megakernel, warp sample pool
-// The same per-lane path state machine, with the START of a path taken out of the divergent part.  In `megakernel` above a
-// lane that finishes a sample fetches its next unit and generates its primary ray at once, together with whichever other
-// lanes happen to finish in the same iteration: 12 of 32 lanes on the large scene, so the ~300 instructions of fetch + unit
-// decode + RNG seeding + jitter + lens sample + Camera::getRay are paid at 37 % occupancy in every iteration.
+// The START of a path is taken out of the divergent part.  A lane that fetched its own next sample and generated its primary
+// ray at once would do so together with whichever other lanes happen to finish in the same iteration: 12 of 32 lanes on the
+// large scene, so the ~300 instructions of fetch + decode + RNG seeding + jitter + lens sample + Camera::getRay would be paid
+// at 37 % occupancy in every iteration (round 1's lane-fetch scheduling, DESIGN.md section 4.1).
 // Here each WARP keeps a pool of up to 32 ready-made primary rays in shared memory.  When the lanes in need outnumber the pool,
 // the whole warp produces the next 32 consecutive samples at once -- one atomicAdd per 32 samples, every lane busy -- and a
 // finishing lane just pops a ray (ballot + popc ranks, three 16-byte loads).  Work items are single samples (no unit ranges:
-// the path state loses unit / sample bookkeeping, eight registers the scan loop can use), numbered g = lp * spp + s in 64 bits.
+// the path state has no unit / sample bookkeeping, registers the scan loop can use), numbered g = lp * spp + s in 64 bits.
 // Which lane traces which sample is irrelevant to the result: RNG streams are keyed by (pixel, sample) and the accumulators are
 // integer sums -- the image is bit-identical to the other variants'.
-// Every persistent kernel except `megakernel` takes its work this way, and all of them produce through pool_produce.
+// Every persistent kernel takes its work this way, and all of them produce through pool_produce.
 // megakernel_tc3 and megakernel_tcs pop through pool_take; megakernel_pool writes the same pop out (faster there), and
 // megakernel_pool2, which ranks two slots per lane, pops on its own.
 struct __align__(16) WarpPool {

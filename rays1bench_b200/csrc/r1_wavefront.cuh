@@ -16,9 +16,6 @@
 #include <cstring>
 #include "r1_kernels.cuh"
 
-#include <cstdio>
-#include <cstdlib>
-
 namespace r1 {
 
 constexpr int kWfRays = 2;          // rays per lane in wf_intersect (measured: 4 x 512 threads 3815, 2 x 768 3988, 2 x 1024 4070,
@@ -43,8 +40,7 @@ struct WfState {
 struct WfGraphKey {
     RenderArgs a;
     WfState w;
-    void (*ikern)(RenderArgs, WfState);
-    int igrid, ithreads, sgrid;
+    int igrid, sgrid;
     size_t smem;
 };
 struct WavefrontBuffers {
@@ -236,7 +232,8 @@ __global__ void __launch_bounds__(256) wf_shade(const __grid_constant__ RenderAr
     }
 }
 
-// loop control: one thread.  (handle == 0: host-driven loop, the flag is read back by the host instead)
+// loop control: one thread.  Sets the WHILE node's condition through `handle`; host_flag, when not null, receives the live-slot
+// count (the graph passes null).
 __global__ void wf_decide(const __grid_constant__ WfState w, cudaGraphConditionalHandle handle, uint32_t *host_flag)
 {
     const uint32_t alive = w.counters[4];
@@ -261,7 +258,7 @@ inline uint32_t wavefront_slots(uint32_t n_units, int sm_count)
     return (uint32_t)slots;
 }
 
-// returns a cudaError_t (0 = ok).  Asynchronous on `stream` (graph mode); the unit counter must already be zeroed.
+// returns a cudaError_t (0 = ok).  Asynchronous on `stream`; the unit counter must already be zeroed.
 inline int wavefront_render(WavefrontBuffers &b, const RenderArgs &a, int sm_count, cudaStream_t stream, uint32_t *launches)
 {
     *launches = 0;
@@ -291,58 +288,18 @@ inline int wavefront_render(WavefrontBuffers &b, const RenderArgs &a, int sm_cou
     *launches += 1;
 
     const size_t smem = 16 + (size_t)a.scene.n_pad * 32;
-    // rays per lane / threads per CTA of wf_intersect (R1_WF_CONFIG=R,threads overrides the tuned default for experiments)
-    int cfg_r = kWfRays, cfg_t = kWfThreads;
-    if (const char *env = getenv("R1_WF_CONFIG")) sscanf(env, "%d,%d", &cfg_r, &cfg_t);
-    void (*ikern)(RenderArgs, WfState) = nullptr;
-    if (cfg_r == 4 && cfg_t == 512) ikern = wf_intersect<4, 512>;
-    else if (cfg_r == 2 && cfg_t == 768) ikern = wf_intersect<2, 768>;
-    else if (cfg_r == 2 && cfg_t == 512) ikern = wf_intersect<2, 512>;
-    else if (cfg_r == 2 && cfg_t == 1024) ikern = wf_intersect<2, 1024>;
-    else if (cfg_r == 1 && cfg_t == 1024) ikern = wf_intersect<1, 1024>;
-    else return (int)cudaErrorInvalidValue;
+    const auto ikern = wf_intersect<kWfRays, kWfThreads>;
     R1_WF_CUDA(cudaFuncSetAttribute(ikern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const uint32_t n_tiles = (w.n_slots + 32 * cfg_r - 1) / (32 * cfg_r);
-    const int igrid = (int)std::min<uint32_t>((uint32_t)sm_count, (n_tiles * 32 + cfg_t - 1) / cfg_t);
+    const uint32_t n_tiles = (w.n_slots + 32 * kWfRays - 1) / (32 * kWfRays);
+    const int igrid = (int)std::min<uint32_t>((uint32_t)sm_count, (n_tiles * 32 + kWfThreads - 1) / kWfThreads);
     const int sgrid = sm_count * 8;
 
-    if (getenv("R1_WF_HOSTLOOP")) {
-        // debugging / per-kernel timing path: the same three kernels driven from the host (synchronous)
-        uint32_t *flag = nullptr;
-        R1_WF_CUDA(cudaMallocHost(&flag, sizeof(uint32_t)));
-        cudaEvent_t ev[4];
-        for (auto &e : ev) R1_WF_CUDA(cudaEventCreate(&e));
-        double ms_i = 0, ms_s = 0, ms_d = 0;
-        uint32_t iters = 0;
-        *flag = 1;
-        while (*flag) {
-            R1_WF_CUDA(cudaEventRecord(ev[0], stream));
-            ikern<<<igrid, cfg_t, smem, stream>>>(a, w);
-            R1_WF_CUDA(cudaEventRecord(ev[1], stream));
-            wf_shade<<<sgrid, 256, 0, stream>>>(a, w);
-            R1_WF_CUDA(cudaEventRecord(ev[2], stream));
-            wf_decide<<<1, 1, 0, stream>>>(w, 0, flag);
-            R1_WF_CUDA(cudaEventRecord(ev[3], stream));
-            R1_WF_CUDA(cudaStreamSynchronize(stream));
-            float t;
-            cudaEventElapsedTime(&t, ev[0], ev[1]); ms_i += t;
-            cudaEventElapsedTime(&t, ev[1], ev[2]); ms_s += t;
-            cudaEventElapsedTime(&t, ev[2], ev[3]); ms_d += t;
-            ++iters;
-        }
-        fprintf(stderr, "[r1 wavefront host loop] slots %u iterations %u: intersect %.2f ms, shade %.2f ms, decide %.2f ms\n", w.n_slots, iters, ms_i, ms_s, ms_d);
-        for (auto &e : ev) cudaEventDestroy(e);
-        cudaFreeHost(flag);
-        *launches += 3 * iters;
-        b.d_iterations = nullptr;
-        return 0;
-    }
     // the loop as a CUDA-graph WHILE node: intersect -> shade -> decide, repeated on the device until no slot is alive.
     // Kernel arguments are baked into the instantiated graph, so it is cached and re-launched while they stay the same
-    // (every render of a benchmark loop); any change -- another scene block, image size, buffers, kernel configuration -- rebuilds it.
+    // (every render of a benchmark loop); any change -- another scene block, image size, buffers, grid -- rebuilds it.
     WfGraphKey key;
     memset(&key, 0, sizeof(key));
-    key.a = a; key.w = w; key.ikern = ikern; key.igrid = igrid; key.ithreads = cfg_t; key.sgrid = sgrid; key.smem = smem;
+    key.a = a; key.w = w; key.igrid = igrid; key.sgrid = sgrid; key.smem = smem;
     if (b.exec && memcmp(&key, &b.key, sizeof(key)) != 0) {
         R1_WF_CUDA(cudaStreamSynchronize(stream));   // the previous render's graph may still be running on this stream
         cudaGraphExecDestroy(b.exec);
@@ -363,7 +320,7 @@ inline int wavefront_render(WavefrontBuffers &b, const RenderArgs &a, int sm_cou
         cudaStream_t cap;
         R1_WF_CUDA(cudaStreamCreateWithFlags(&cap, cudaStreamNonBlocking));
         R1_WF_CUDA(cudaStreamBeginCaptureToGraph(cap, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
-        ikern<<<igrid, cfg_t, smem, cap>>>(a, w);
+        ikern<<<igrid, kWfThreads, smem, cap>>>(a, w);
         wf_shade<<<sgrid, 256, 0, cap>>>(a, w);
         wf_decide<<<1, 1, 0, cap>>>(w, handle, nullptr);
         R1_WF_CUDA(cudaStreamEndCapture(cap, nullptr));

@@ -221,18 +221,12 @@ def test_tensor_renders_the_same_bytes_at_every_group_count(r1, scenes):
         scenes["synth4096"].render(64, 36, 2, variant=r1.VARIANT_MEGAKERNEL_TENSOR)   # above the shared-memory limit of the B tile
 
 
-def test_default_variant_picks_the_kernel_by_scene(r1, scenes, monkeypatch):
+def test_default_variant_picks_the_kernel_by_scene(r1, scenes):
     """R1_VARIANT_MEGAKERNEL: the tensor-core filter for scan-heavy scenes that fit its shared-memory operand, else the packed filter"""
     name = lambda scene, v=r1.VARIANT_MEGAKERNEL: r1.lib.r1_kernel_name(scenes[scene].handle, v).decode()  # noqa: E731
     assert name("large") == "megakernel_tc3" and name("medium") == "megakernel_pool" and name("small") == "megakernel_pool"
     assert name("synth4096") == "megakernel_pool"
     assert name("large", r1.VARIANT_MEGAKERNEL_PACKED) == "megakernel_pool" and name("large", r1.VARIANT_MEGAKERNEL_TENSOR) == "megakernel_tc3"
-    monkeypatch.setenv("R1_AUTO_TENSOR", "0")
-    assert name("large") == "megakernel_pool"
-    a, ra = scenes["large"].render(96, 54, 8)
-    monkeypatch.delenv("R1_AUTO_TENSOR")
-    b, rb = scenes["large"].render(96, 54, 8)
-    assert np.array_equal(a, b) and ra.num_rays == rb.num_rays
 
 
 def test_trace_rays_refuses_variants_without_a_ray_kernel(r1, scenes):
@@ -459,22 +453,6 @@ def test_wavefront_graph_is_cached_across_renders(r1, scenes):
     assert r1.lib.r1_wavefront_graph_builds(0) == n0 + 1, "another spp: rebuilt once"
     ref, rr = s.render(160, 90, 9)
     assert np.array_equal(c, ref) and rc.num_rays == rr.num_rays
-
-
-def test_sample_pool_and_lane_fetch_scheduling_render_the_same_bytes(r1, scenes, monkeypatch):
-    """r1::megakernel_pool (default: warps produce 32 primary rays at a time, finishing lanes pop them) against r1::megakernel
-    (round-1 scheduling: every lane fetches and generates its own next sample, R1_POOL=0), incl. ragged sizes and partitions"""
-    for name, (w, h, spp) in (("large", (200, 117, 40)), ("small", (33, 7, 3)), ("synth4096", (64, 36, 5))):
-        s = scenes[name]
-        monkeypatch.delenv("R1_POOL", raising=False)
-        a, ra = s.render(w, h, spp)
-        a2, ra2 = s.render(w, h, spp, rank=1, world=3)
-        monkeypatch.setenv("R1_POOL", "0")
-        b, rb = s.render(w, h, spp)
-        b2, rb2 = s.render(w, h, spp, rank=1, world=3)
-        assert np.array_equal(a, b) and ra.num_rays == rb.num_rays and ra.num_samples == rb.num_samples == w * h * spp
-        assert np.array_equal(a2, b2) and ra2.num_rays == rb2.num_rays
-    monkeypatch.delenv("R1_POOL", raising=False)
 
 
 # ---- determinism / partition invariance --------------------------------------------------------------------------------

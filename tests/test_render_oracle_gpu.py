@@ -210,15 +210,12 @@ def variant_runs(r1):
             "deferred": (V.VARIANT_MEGAKERNEL_DEFERRED, 0, 0, {}), "dual768": (V.VARIANT_MEGAKERNEL_DUAL, 768, 0, {}),
             "dual512": (V.VARIANT_MEGAKERNEL_DUAL, 512, 0, {}), "packed": (V.VARIANT_MEGAKERNEL_PACKED, 0, 0, {}),
             "tensor": (V.VARIANT_MEGAKERNEL_TENSOR, 0, 0, {}), "wavefront": (V.VARIANT_WAVEFRONT, 0, 0, {}),
-            "pool0": (V.VARIANT_MEGAKERNEL, 0, 0, {"R1_POOL": "0"}), "pool0_coop": (V.VARIANT_MEGAKERNEL_COOP, 0, 0, {"R1_POOL": "0"}),
             "unstaged": (V.VARIANT_MEGAKERNEL, 0, 0, {"R1_FORCE_UNSTAGED": "1"}),
             "unstaged_deferred": (V.VARIANT_MEGAKERNEL_DEFERRED, 0, 0, {"R1_FORCE_UNSTAGED": "1"}),
             "threads512": (V.VARIANT_MEGAKERNEL, 512, 0, {}), "threads768": (V.VARIANT_MEGAKERNEL, 768, 0, {}),
             "blocks2": (V.VARIANT_MEGAKERNEL, 0, 2, {})}
     for g in (1, 2, 3, 4):
         runs["stream%dg" % g] = (V.VARIANT_MEGAKERNEL_TENSOR_STREAM, 128 * g, 0, {})
-    for st in (2, 3, 4):
-        runs["stream_stages%d" % st] = (V.VARIANT_MEGAKERNEL_TENSOR_STREAM, 512, 0, {"R1_TCS_STAGES": str(st)})
     for g in (4, 5, 6, 7):
         runs["tc3_%dg" % g] = (V.VARIANT_MEGAKERNEL_TENSOR, 128 * g, 0, {})
     return runs
@@ -237,7 +234,7 @@ def test_every_variant_and_knob(r1, expected, scenes, monkeypatch, name, run):  
 
 # ---- more than 256 samples per pixel --------------------------------------------------------------------------------------------
 
-SPP_VARIANTS = {"default": (0, 0, {}), "packed": (7, 0, {}), "pool0": (0, 0, {"R1_POOL": "0"}), "wavefront": (1, 0, {}), "stream": (9, 0, {})}
+SPP_VARIANTS = {"default": (0, 0, {}), "packed": (7, 0, {}), "wavefront": (1, 0, {}), "stream": (9, 0, {})}
 
 
 @pytest.mark.parametrize("spp", (257, 514, 1000))
@@ -246,19 +243,6 @@ def test_more_than_256_samples_per_pixel(r1, expected, scenes, monkeypatch, name
     """units of ceil(spp / 256) samples (514: a one-sample last unit) on a 5x3 image"""
     for run, (v, threads, env) in SPP_VARIANTS.items():
         check(r1, expected, monkeypatch, scenes[name], 5, 3, spp, variant=v, threads=threads, env=env, what="%s %s" % (name, run))
-
-
-@pytest.mark.parametrize("spp", (257, 514, 1000))
-@pytest.mark.parametrize("name", ("small", "medium", "large"))
-def test_lane_fetch_continues_a_pixel_across_units(r1, expected, scenes, monkeypatch, name, spp):  # noqa: F811
-    """R1_POOL=0: a lane takes k = min(kmax, left / (lanes x div)) units per fetch and continues a pixel from one unit to the next
-    (r1::megakernel, `s_end = min(s + samples_per_unit, spp)`).  k >= 2 needs more than 2 x lanes x div units: 512 threads on every
-    SM, div = 1 (R1_SCHED; the large scene's default kmax is 1) and a 40x32 image (>= 154 000 units at 257 spp)"""
-    if name == "large" and spp == 1000:
-        pytest.skip("1000 = 4 x 250 has no short last unit; covered on small and medium")
-    env = {"R1_POOL": "0", "R1_SCHED": "8,1" if name == "large" else "64,1"}
-    check(r1, expected, monkeypatch, scenes[name], 40, 32, spp, variant=r1.VARIANT_MEGAKERNEL_PACKED, threads=512, env=env,
-          what="%s lane fetch" % name)
 
 
 # ---- partitions -----------------------------------------------------------------------------------------------------------------
@@ -287,7 +271,7 @@ def test_rank_shares(r1, expected, scenes, monkeypatch, run):  # noqa: F811
 
 def edge_runs(r1, n):
     runs = [(0, 0, {}), (r1.VARIANT_MEGAKERNEL_PACKED, 0, {}), (r1.VARIANT_MEGAKERNEL_TENSOR_STREAM, 0, {}), (r1.VARIANT_WAVEFRONT, 0, {}),
-            (r1.VARIANT_MEGAKERNEL_COOP, 0, {"R1_POOL": "0"})]
+            (r1.VARIANT_MEGAKERNEL_COOP, 0, {})]
     if (n + 31) // 32 * 32 <= 768:
         runs.append((r1.VARIANT_MEGAKERNEL_TENSOR, 0, {}))
     return runs
@@ -338,8 +322,7 @@ def test_8016_sphere_grid(r1, expected, big_scenes, monkeypatch):  # noqa: F811
     """beyond the staging limit: the default (the packed scan from global memory) and the streamed tensor-core filter"""
     s = big_scenes[8016]
     assert r1.lib.r1_kernel_name(s.handle, 0).decode() == "megakernel_pool"
-    for v, threads, env in ((0, 0, {}), (r1.VARIANT_MEGAKERNEL_TENSOR_STREAM, 0, {}), (r1.VARIANT_MEGAKERNEL_TENSOR_STREAM, 256, {}),
-                            (r1.VARIANT_MEGAKERNEL_PACKED, 0, {"R1_POOL": "0"})):
+    for v, threads, env in ((0, 0, {}), (r1.VARIANT_MEGAKERNEL_TENSOR_STREAM, 0, {}), (r1.VARIANT_MEGAKERNEL_TENSOR_STREAM, 256, {})):
         check(r1, expected, monkeypatch, s, 48, 27, 2, variant=v, threads=threads, env=env, what="grid8016")
 
 

@@ -439,8 +439,6 @@ def render_runs(r1, name):
     n = count_of(name)
     if n32_of(n) <= 768 and (not name.startswith("flood") or n in FLOOD_RENDER_TENSOR):
         runs.append((V.VARIANT_MEGAKERNEL_TENSOR, 0, {}))
-    for v in (V.VARIANT_MEGAKERNEL_PACKED, V.VARIANT_MEGAKERNEL_SCALAR, V.VARIANT_MEGAKERNEL_COOP, V.VARIANT_MEGAKERNEL_DEFERRED):
-        runs.append((v, 0, {"R1_POOL": "0"}))
     for v in (V.VARIANT_MEGAKERNEL_PACKED, V.VARIANT_MEGAKERNEL_COOP, V.VARIANT_MEGAKERNEL_DEFERRED, V.VARIANT_MEGAKERNEL_DUAL):
         runs.append((v, 0, {"R1_FORCE_UNSTAGED": "1"}))
     return runs
@@ -448,7 +446,7 @@ def render_runs(r1, name):
 
 @pytest.mark.parametrize("name", RENDER_SCENES)
 def test_every_variant_renders_like_packed(r1, edge_scenes, monkeypatch, name):
-    """E: scalar, coop, deferred, DUAL (768 and 512 threads), WAVEFRONT, TENSOR, R1_POOL=0 and R1_FORCE_UNSTAGED=1 renders
+    """E: scalar, coop, deferred, DUAL (768 and 512 threads), WAVEFRONT, TENSOR and R1_FORCE_UNSTAGED=1 renders
     byte-identical to PACKED with the same ray count, on a 48x27 frame, a 7x3 image and as rank 1 of 3"""
     s = edge_scenes[name]
     for w, h, spp, rank, world in RENDER_CASES:

@@ -28,9 +28,8 @@ import make_scene  # noqa: E402
 
 STREAM = ("tensor_stream",)
 ALL = ("small", "medium", "large", "synth4096")
-# (threads, environment) of every configuration the render kernel has: 1 .. 4 ray groups with the default 6-stage ring, and
-# 4 groups with 2, 3 and 4 stages
-CONFIGS = ((0, {}), (128, {}), (256, {}), (384, {}), (512, {"R1_TCS_STAGES": "2"}), (512, {"R1_TCS_STAGES": "3"}), (512, {"R1_TCS_STAGES": "4"}))
+# threads of every configuration the render kernel has: 1 .. 4 ray groups (0: the default, 4), each with the 6-stage ring
+CONFIGS = (0, 128, 256, 384)
 # (width, height, spp, rank, world): a frame, images with fewer samples than one CTA (or one group) has lanes, and a rank
 RENDER_CASES = ((96, 54, 8, 0, 1), (7, 3, 5, 0, 1), (1, 1, 3, 0, 1), (96, 54, 8, 1, 3))
 # sweep scenes above 768 spheres: n32 mod 128 = 32, 64, 96 and 0
@@ -51,16 +50,12 @@ def assert_same(got, want, what):
         assert np.array_equal(bits(a), bits(b)), "%s: %s differs" % (what, name)
 
 
-def render_like_packed(r1, s, cases, configs, monkeypatch, what):
+def render_like_packed(r1, s, cases, configs, what):
     for w, h, spp, rank, world in cases:
         base, r0 = s.render(w, h, spp, rank=rank, world=world, variant=r1.VARIANT_MEGAKERNEL_PACKED)
-        for threads, env in configs:
-            for k, v in env.items():
-                monkeypatch.setenv(k, v)
+        for threads in configs:
             rgb, res = s.render(w, h, spp, rank=rank, world=world, variant=r1.VARIANT_MEGAKERNEL_TENSOR_STREAM, threads=threads)
-            for k in env:
-                monkeypatch.delenv(k)
-            assert np.array_equal(rgb, base) and res.num_rays == r0.num_rays, (what, (w, h, spp, rank, world), threads, env)
+            assert np.array_equal(rgb, base) and res.num_rays == r0.num_rays, (what, (w, h, spp, rank, world), threads)
 
 
 def grid(r1, directory, gw, gh, lookfrom, focus):
@@ -260,17 +255,17 @@ def test_scenes_beyond_staging_match_oracle(r1, oracle, big_scenes, count):
 # ---- renders ----------------------------------------------------------------------------------------------------------------
 
 @pytest.mark.parametrize("name", ALL)
-def test_builtin_scenes_render_like_packed(r1, scenes, monkeypatch, name):  # noqa: F811
-    render_like_packed(r1, scenes[name], RENDER_CASES, CONFIGS, monkeypatch, name)
+def test_builtin_scenes_render_like_packed(r1, scenes, name):  # noqa: F811
+    render_like_packed(r1, scenes[name], RENDER_CASES, CONFIGS, name)
 
 
 @pytest.mark.parametrize("name", ABOVE_768 + ("flood4096",))
-def test_scenes_above_768_spheres_render_like_packed(r1, edge_scenes, monkeypatch, name):
+def test_scenes_above_768_spheres_render_like_packed(r1, edge_scenes, name):
     s = edge_scenes[name]
     n32 = (s.count() + 31) // 32 * 32
     assert n32 > 768
     cases = RENDER_CASES if not name.startswith("flood") else ((48, 27, 4, 0, 1), (7, 3, 5, 0, 1))
-    render_like_packed(r1, s, cases, CONFIGS, monkeypatch, name)
+    render_like_packed(r1, s, cases, CONFIGS, name)
 
 
 def test_above_768_sweep_covers_every_last_chunk(edge_scenes):
@@ -278,8 +273,8 @@ def test_above_768_sweep_covers_every_last_chunk(edge_scenes):
 
 
 @pytest.mark.parametrize("count", (5048, 8016))
-def test_scenes_beyond_staging_render_like_packed(r1, big_scenes, monkeypatch, count):
-    render_like_packed(r1, big_scenes[count], RENDER_CASES[:2] + RENDER_CASES[3:], ((0, {}), (128, {})), monkeypatch, count)
+def test_scenes_beyond_staging_render_like_packed(r1, big_scenes, count):
+    render_like_packed(r1, big_scenes[count], RENDER_CASES[:2] + RENDER_CASES[3:], (0, 128), count)
 
 
 def test_full_size_synth4096_renders_like_packed(r1, scenes):  # noqa: F811
@@ -290,15 +285,11 @@ def test_full_size_synth4096_renders_like_packed(r1, scenes):  # noqa: F811
     print("synth4096 1280x720x250: packed %.1f ms, tensor_stream %.1f ms (trace)" % (r0.trace_ms, res.trace_ms))
 
 
-def test_unsupported_configurations_are_refused(r1, scenes, monkeypatch):  # noqa: F811
+def test_unsupported_configurations_are_refused(r1, scenes):  # noqa: F811
     s = scenes["large"]
     for threads in (640, 1024):
         with pytest.raises(r1.Rays1Error, match=r"\(-1\).*tensor-stream"):
             s.render(16, 9, 2, variant=r1.VARIANT_MEGAKERNEL_TENSOR_STREAM, threads=threads)
-    monkeypatch.setenv("R1_TCS_STAGES", "5")
-    with pytest.raises(r1.Rays1Error, match=r"\(-1\).*tensor-stream"):
-        s.render(16, 9, 2, variant=r1.VARIANT_MEGAKERNEL_TENSOR_STREAM)
-    monkeypatch.delenv("R1_TCS_STAGES")
     base, r0 = s.render(16, 9, 2, variant=r1.VARIANT_MEGAKERNEL_PACKED)
     rgb, res = s.render(16, 9, 2, variant=r1.VARIANT_MEGAKERNEL_TENSOR_STREAM)   # no sticky error
     assert np.array_equal(rgb, base) and res.num_rays == r0.num_rays

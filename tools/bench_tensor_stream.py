@@ -32,8 +32,8 @@ sys.path.insert(0, os.path.join(ROOT, "tools"))
 
 # grid scenes of tools/make_scene.py: (grid w, grid h) -> spheres after the loader's padding to 8
 GRIDS = {"grid1000": (32, 31), "grid2000": (45, 44), "grid8000": (90, 89)}
-# (threads, R1_TCS_STAGES) of the streamed kernel: 0 / None = the defaults (4 groups, 6 stages)
-TCS_CONFIGS = ((0, None), (512, "2"), (512, "3"), (512, "4"), (384, "6"), (256, "6"), (128, "6"))
+# threads of the streamed kernel (128 per ray group): 0 = the default, 4 groups
+TCS_CONFIGS = (0, 384, 256, 128)
 
 
 def gpu_info():
@@ -100,27 +100,21 @@ def main():
             n = s.count()
             n_real = int((soa["inv_radius"] > 0).sum())
             n32, n_pad = (n + 31) // 32 * 32, (n + 15) // 16 * 16
-            runs = [("packed", r1.VARIANT_MEGAKERNEL_PACKED, 0, None)]
+            runs = [("packed", r1.VARIANT_MEGAKERNEL_PACKED, 0)]
             if n32 <= 768:
-                runs.append(("tensor", r1.VARIANT_MEGAKERNEL_TENSOR, 0, None))
-            for threads, stages in (TCS_CONFIGS if name == args.config_scene else TCS_CONFIGS[:1]):
-                label = "tensor_stream" + ("" if not threads else "_g%d_s%s" % (threads // 128, stages))
-                runs.append((label, r1.VARIANT_MEGAKERNEL_TENSOR_STREAM, threads, stages))
-            for label, v, threads, stages in runs:                    # warm-up: module load, first launch of every kernel
-                if stages:
-                    os.environ["R1_TCS_STAGES"] = stages
+                runs.append(("tensor", r1.VARIANT_MEGAKERNEL_TENSOR, 0))
+            for threads in (TCS_CONFIGS if name == args.config_scene else TCS_CONFIGS[:1]):
+                label = "tensor_stream" + ("" if not threads else "_g%d" % (threads // 128))
+                runs.append((label, r1.VARIANT_MEGAKERNEL_TENSOR_STREAM, threads))
+            for label, v, threads in runs:                            # warm-up: module load, first launch of every kernel
                 s.render(96, 54, 4, variant=v, threads=threads)
-                os.environ.pop("R1_TCS_STAGES", None)
-            entry = {"spheres": n, "real_spheres": n_real, "n32": n32, "kernels": {}, "runs": {label: [] for label, _, _, _ in runs}}
+            entry = {"spheres": n, "real_spheres": n_real, "n32": n32, "kernels": {}, "runs": {label: [] for label, _, _ in runs}}
             for rep in range(args.runs):
                 base = None
-                for label, v, threads, stages in runs:
-                    if stages:
-                        os.environ["R1_TCS_STAGES"] = stages
+                for label, v, threads in runs:
                     flush.zero_()
                     torch.cuda.synchronize()
                     rgb, res = s.render(W, H, SPP, variant=v, threads=threads)
-                    os.environ.pop("R1_TCS_STAGES", None)
                     if base is None:
                         base = (rgb, res.num_rays)
                     flops = float(res.num_rays) * (16.0 * n_real + 70.0)
