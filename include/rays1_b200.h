@@ -144,6 +144,25 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
 /* Blocks until the last r1_render_device of this scene on `device` (< 0: device of the last commit) has finished and
  * fills kernel_ms / trace_ms (CUDA events recorded on the launching stream), launches, n_units, num_samples. */
 int r1_render_wait(r1_scene *scene, int device, r1_result *result);
+/* A batch of views: K = n_views images of one scene state in one persistent launch and one resolve (two above 2^31 batch
+ * pixels: the resolve's index is 32-bit, so it runs in pieces of at most 2^31 pixels).  View v is byte for byte what
+ * r1_scene_move_camera(cams + 22 v) followed by r1_render_sums with params->seed = seeds[v] gives on that device: the same pixel
+ * sums, bytes and rank rows; num_rays is the sum of those K renders' counts.  The batch renders the device's current records
+ * (moved spheres, changed materials) and does NOT change the device's camera.
+ * cams: n_views x 22 floats (r1_scene_get_camera's order; r1_camera_constants computes them).  seeds: n_views, or NULL for
+ * params->seed in every view.  Both are HOST arrays, read before the call returns.
+ * Outputs are view-major, each view laid out as r1_render lays out one image: rgb_host n_views x r1_local_pixels() x 3 bytes,
+ * sums_host (NULL: not returned) n_views x r1_local_pixels() x 3 uint64 as r1_render_sums returns them.
+ * Variants: R1_VARIANT_MEGAKERNEL (resolved as for r1_render), PACKED, TENSOR, TENSOR_STREAM and BVH (with a single render's tree
+ * rules); the A/B variants, WAVEFRONT and tuning (threads or blocks_per_sm > 0) are refused with R1_ERR_ARG.  Before any device
+ * is looked up: bad params, n_views == 0, a null cams or output pointer: R1_ERR_ARG; n_views x r1_local_pixels() >= 2^32 - 1, or
+ * too many samples: R1_ERR_LIMIT.  result->n_units is 0 (the batch's kernels take samples, not units).
+ * r1_render_views_device: d_rgb as rgb_host, d_num_rays one uint64; asynchronous on cuda_stream like r1_render_device (num_rays
+ * not filled; r1_render_wait completes it).  The cameras are copied on the stream, so a batch already enqueued keeps its own. */
+int r1_render_views(r1_scene *scene, const r1_render_params *params, uint32_t n_views, const float *cams, const uint32_t *seeds,
+                    uint8_t *rgb_host, uint64_t *sums_host, r1_result *result);
+int r1_render_views_device(r1_scene *scene, const r1_render_params *params, uint32_t n_views, const float *cams, const uint32_t *seeds,
+                           void *d_rgb, void *d_num_rays, void *cuda_stream, r1_result *result);
 /* Diagnostics: how many times the wavefront variant had to (re)build its CUDA-graph WHILE loop on `device` -- the
  * instantiated graph is cached and re-launched while the render arguments stay the same.  Negative on error. */
 int r1_wavefront_graph_builds(int device);

@@ -82,6 +82,8 @@ def _load():
         "r1_render": (ci, [vp, C.POINTER(RenderParams), u8p, C.POINTER(Result)]),
         "r1_render_device": (ci, [vp, C.POINTER(RenderParams), vp, vp, vp, C.POINTER(Result)]),
         "r1_render_wait": (ci, [vp, ci, C.POINTER(Result)]),
+        "r1_render_views": (ci, [vp, C.POINTER(RenderParams), C.c_uint32, vp, vp, vp, vp, C.POINTER(Result)]),
+        "r1_render_views_device": (ci, [vp, C.POINTER(RenderParams), C.c_uint32, vp, vp, vp, vp, vp, C.POINTER(Result)]),
         "r1_wavefront_graph_builds": (ci, [ci]),
         "r1_local_rows": (C.c_int64, [ci, ci, ci, ci]),
         "r1_local_pixels": (C.c_int64, [ci, ci, ci, ci, ci]),
@@ -222,6 +224,56 @@ class Scene:
         res = Result()
         _check(lib.r1_render_device(self.handle, C.byref(p), C.c_void_p(d_rgb_ptr), C.c_void_p(d_num_rays_ptr),
                                     C.c_void_p(stream_ptr or 0), C.byref(res)), "r1_render_device")
+        return res
+
+    def _views_args(self, cams, seeds):
+        """cams (K, 22) float32 and seeds (K,) integers in 0 .. 2^32 - 1 (None: none) as the C arrays r1_render_views takes"""
+        cams = np.asarray(cams)
+        if cams.dtype != np.float32:
+            raise ValueError("cams must be float32 camera constants, not %s" % cams.dtype)
+        if cams.ndim != 2 or cams.shape[1] != 22:
+            raise ValueError("cams must hold 22 constants per view, shape (K, 22), not shape %s" % (cams.shape,))
+        cams = np.ascontiguousarray(cams)
+        if seeds is not None:
+            seeds = np.asarray(seeds)
+            if seeds.dtype.kind not in "iu":
+                raise ValueError("seeds must be integers, not %s" % seeds.dtype)
+            if seeds.shape != (cams.shape[0],):
+                raise ValueError("seeds must hold one seed per view, shape (%d,), not shape %s" % (cams.shape[0], seeds.shape))
+            if seeds.size and (seeds.min() < 0 or seeds.max() > 0xFFFFFFFF):
+                raise ValueError("seeds must lie in 0 .. 2^32 - 1")
+            seeds = np.ascontiguousarray(seeds, np.uint32)
+        return cams, seeds
+
+    def render_views(self, cams, seeds=None, width=SCREEN_W, height=SCREEN_H, spp=NUM_SAMPLES_PER_PIXEL, max_bounces=MAX_BOUNCES,
+                     variant=VARIANT_MEGAKERNEL, seed=0, rank=0, world=1, row_tile=DEFAULT_ROW_TILE, device=-1, sums=False):
+        """r1_render_views: K = len(cams) views of the scene in one launch.  cams: float32 (K, 22), e.g. a stack of camera_constants();
+        seeds: K seeds, or None for `seed` in every view.  View v equals move_camera(cams[v]) + render_sums(seed=seeds[v]) byte for
+        byte; the device's camera does not change.  Returns (rgb[K, local_rows, width, 3] uint8, [sums[K, local_rows, width, 3]
+        uint64 when sums=True,] Result), num_rays summed over the views."""
+        cams, seeds = self._views_args(cams, seeds)
+        k = cams.shape[0]
+        p = RenderParams(width, height, spp, max_bounces, variant, seed, rank, world, row_tile, 0, 0, device)
+        rows = int(lib.r1_local_rows(height, row_tile, rank, world))
+        rgb = np.zeros((k, rows, width, 3), np.uint8)
+        out_sums = np.zeros((k, rows, width, 3), np.uint64) if sums else None
+        res = Result()
+        buf = rgb if rgb.size else np.zeros(16, np.uint8)
+        _check(lib.r1_render_views(self.handle, C.byref(p), k, cams.ctypes.data, seeds.ctypes.data if seeds is not None else None, buf.ctypes.data,
+                                   out_sums.ctypes.data if sums and out_sums.size else None, C.byref(res)), "r1_render_views")
+        return (rgb, out_sums, res) if sums else (rgb, res)
+
+    def render_views_device(self, cams, d_rgb_ptr, d_num_rays_ptr, seeds=None, stream_ptr=None, **kw):
+        """r1_render_views_device: render_views() into device pointers, asynchronous on the stream like render_device();
+        render_wait() completes it."""
+        cams, seeds = self._views_args(cams, seeds)
+        p = RenderParams(kw.get("width", SCREEN_W), kw.get("height", SCREEN_H), kw.get("spp", NUM_SAMPLES_PER_PIXEL),
+                         kw.get("max_bounces", MAX_BOUNCES), kw.get("variant", VARIANT_MEGAKERNEL), kw.get("seed", 0), kw.get("rank", 0),
+                         kw.get("world", 1), kw.get("row_tile", DEFAULT_ROW_TILE), kw.get("blocks_per_sm", 0), kw.get("threads", 0), kw.get("device", -1))
+        res = Result()
+        _check(lib.r1_render_views_device(self.handle, C.byref(p), cams.shape[0], cams.ctypes.data, seeds.ctypes.data if seeds is not None else None,
+                                          C.c_void_p(d_rgb_ptr), C.c_void_p(d_num_rays_ptr), C.c_void_p(stream_ptr or 0), C.byref(res)),
+               "r1_render_views_device")
         return res
 
     def render_wait(self, device=-1):

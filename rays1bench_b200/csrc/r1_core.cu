@@ -64,6 +64,7 @@ struct Scratch {
     uint8_t *rgb = nullptr; size_t rgb_cap = 0;
     unsigned long long *num_rays = nullptr;
     unsigned long long *host_rays = nullptr;  // pinned
+    r1::ViewRec *views = nullptr; size_t views_cap = 0;          // the view table of the last batch (r1_render_views_device)
     r1::WavefrontBuffers wf;
     // scene blocks of destroyed scenes, kept for the next commit on this device: the reference-facing call builds a new scene
     // per benchmark() (rayweek1.cpp:969-984), and a cudaMalloc + cudaFree per scene and device is most of what the 8-GPU
@@ -207,6 +208,9 @@ constexpr int kDefaultRowTile = 1;
 // order-free, so the unit size affects scheduling granularity only, never the image.
 int samples_per_unit(int spp) { return std::max(1, (spp + 255) / 256); }
 
+// Pixels per r1::resolve launch: its 32-bit grid-stride index (at most sm_count x 8 x 256 apart) cannot wrap below 2^31 pixels.
+constexpr uint32_t kResolvePixels = 1u << 31;
+
 struct Partition { int local_rows; uint32_t npix_local; };
 
 Partition partition(int width, int height, int row_tile, int rank, int world)
@@ -288,8 +292,9 @@ size_t megakernel_smem(int scan, bool staged, int n_pad, int threads)
            (scan == r1::kScanCoop || scan == r1::kScanLaneDeferred ? sizeof(r1::WarpScratch) * (threads / 32) : 0) + sizeof(r1::WarpPool) * (threads / 32);
 }
 
-// r1::megakernel_pool with the packed, scalar, cooperative or deferred scan
-template <int kScan, bool kStaged>
+// r1::megakernel_pool with the packed, scalar, cooperative or deferred scan.  kViews (a batch of views, packed scan only): the
+// default thread count is the only instance.
+template <int kScan, bool kStaged, bool kViews>
 int launch_megakernel(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
 {
     int threads = prm.threads > 0 ? prm.threads : (kScan == r1::kScanCoop ? kDefaultThreadsCoop : kDefaultThreads);
@@ -297,14 +302,17 @@ int launch_megakernel(int sm_count, const r1::RenderArgs &args, const r1_render_
     // 227 KB of shared memory.  The default then runs 768 threads (the image does not depend on the thread count).
     if (prm.threads <= 0 && megakernel_smem(kScan, kStaged, args.scene.n_pad, threads) > 227 * 1024) threads = 768;
     RenderKernel kern = nullptr;
-    if (threads == 512) kern = r1::megakernel_pool<kScan, kStaged, 512, 1>;
-    if (threads == 768) kern = r1::megakernel_pool<kScan, kStaged, 768, 1>;
-    if (threads == 1024) kern = r1::megakernel_pool<kScan, kStaged, 1024, 1>;
+    if constexpr (!kViews) {
+        if (threads == 512) kern = r1::megakernel_pool<kScan, kStaged, 512, 1, false>;
+        if (threads == 768) kern = r1::megakernel_pool<kScan, kStaged, 768, 1, false>;
+    }
+    if (threads == 1024) kern = r1::megakernel_pool<kScan, kStaged, 1024, 1, kViews>;
     if (!kern) return fail(R1_ERR_ARG, "threads must be 512, 768 or 1024 (got %d)", threads);
     return launch_persistent(kern, threads, megakernel_smem(kScan, kStaged, args.scene.n_pad, threads), args.n_samples, threads, prm.blocks_per_sm, sm_count,
                              "megakernel_pool", args, stream);
 }
 
+template <bool kViews>
 int launch_megakernel_bvh(int sm_count, const r1::RenderArgs &args, const float4 *nodes, const float4 *leaves, const r1_render_params &prm,
                           cudaStream_t stream)
 {
@@ -312,9 +320,11 @@ int launch_megakernel_bvh(int sm_count, const r1::RenderArgs &args, const float4
     const r1::BvhArgs b = { nodes, leaves };
     R1_CUDA(cudaMemcpyToSymbolAsync(r1::c_bvh, &b, sizeof(b), 0, cudaMemcpyHostToDevice, stream));
     RenderKernel kern = nullptr;
-    if (threads == 512) kern = r1::megakernel_pool<r1::kScanBvh, false, 512, 1>;
-    if (threads == 768) kern = r1::megakernel_pool<r1::kScanBvh, false, 768, 1>;
-    if (threads == 1024) kern = r1::megakernel_pool<r1::kScanBvh, false, 1024, 1>;
+    if constexpr (!kViews) {
+        if (threads == 512) kern = r1::megakernel_pool<r1::kScanBvh, false, 512, 1, false>;
+        if (threads == 768) kern = r1::megakernel_pool<r1::kScanBvh, false, 768, 1, false>;
+    }
+    if (threads == 1024) kern = r1::megakernel_pool<r1::kScanBvh, false, 1024, 1, kViews>;
     if (!kern) return fail(R1_ERR_ARG, "the bvh variant runs 512, 768 or 1024 threads (got %d)", threads);
     return launch_persistent(kern, threads, megakernel_smem(r1::kScanBvh, false, args.scene.n_pad, threads), args.n_samples, threads, prm.blocks_per_sm,
                              sm_count, "bvh variant", args, stream);
@@ -334,30 +344,36 @@ int launch_megakernel_dual(int sm_count, const r1::RenderArgs &args, const r1_re
 }
 
 // tensor-core filter (r1::megakernel_tc3, R1_VARIANT_MEGAKERNEL_TENSOR): `threads` / 128 = ray groups per CTA, one CTA per SM
+template <bool kViews>
 int launch_megakernel_tc(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
 {
     if (!args.scene.tcb) return fail(R1_ERR_LIMIT, "the tensor-core filter takes scenes of 1 .. %d spheres (its operand lives in shared memory)", r1::tc::kMaxSpheres);
     // ray groups per CTA; measured on the large scene: 4 groups 9.70, 5: 10.34, 6: 9.92, 7: 9.69 G rays/s
     const int groups = prm.threads > 0 ? prm.threads / 128 : 5;
     RenderKernel kern = nullptr;
-    if (groups == 4) kern = r1::megakernel_tc3<4>;
-    if (groups == 5) kern = r1::megakernel_tc3<5>;
-    if (groups == 6) kern = r1::megakernel_tc3<6>;
-    if (groups == 7) kern = r1::megakernel_tc3<7>;
+    if (groups == 5) kern = r1::megakernel_tc3<5, kViews>;
+    if constexpr (!kViews) {
+        if (groups == 4) kern = r1::megakernel_tc3<4, false>;
+        if (groups == 6) kern = r1::megakernel_tc3<6, false>;
+        if (groups == 7) kern = r1::megakernel_tc3<7, false>;
+    }
     if (!kern) return fail(R1_ERR_ARG, "the tensor variant runs 4 .. 7 groups of 128 ray threads per CTA (threads = 512 .. 896)");
     return launch_persistent(kern, groups * 128, r1::tc3_smem_bytes(groups, args.scene.n32), args.n_samples, groups * 128, 1, sm_count, "tensor variant", args,
                              stream);
 }
 
 // streamed tensor-core filter (r1::megakernel_tcs): one CTA per SM
+template <bool kViews>
 int launch_megakernel_tcs(int sm_count, const r1::RenderArgs &args, const r1_render_params &prm, cudaStream_t stream)
 {
     const int groups = prm.threads > 0 ? prm.threads / 128 : kDefaultTcsGroups;
     RenderKernel kern = nullptr;
-    if (groups == 4) kern = r1::megakernel_tcs<4, kDefaultTcsStages>;
-    if (groups == 3) kern = r1::megakernel_tcs<3, kDefaultTcsStages>;
-    if (groups == 2) kern = r1::megakernel_tcs<2, kDefaultTcsStages>;
-    if (groups == 1) kern = r1::megakernel_tcs<1, kDefaultTcsStages>;
+    if (groups == 4) kern = r1::megakernel_tcs<4, kDefaultTcsStages, kViews>;
+    if constexpr (!kViews) {
+        if (groups == 3) kern = r1::megakernel_tcs<3, kDefaultTcsStages, false>;
+        if (groups == 2) kern = r1::megakernel_tcs<2, kDefaultTcsStages, false>;
+        if (groups == 1) kern = r1::megakernel_tcs<1, kDefaultTcsStages, false>;
+    }
     if (!kern) return fail(R1_ERR_ARG, "the tensor-stream variant runs 1 .. 4 groups of 128 ray threads per CTA (threads = 128 .. 512, got %d groups)", groups);
     return launch_persistent(kern, groups * 128, r1::tcs_smem_bytes(groups, kDefaultTcsStages), args.n_samples, groups * 128, 1, sm_count, "tensor-stream variant",
                              args, stream);
@@ -753,7 +769,36 @@ int r1_deinterleave_rows(int device, const void *d_gathered, uint64_t stride, vo
     return R1_OK;
 }
 
-int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rgb, void *d_num_rays, void *cuda_stream, r1_result *result)
+}  // extern "C"
+
+namespace {
+
+// A batch of views (r1_render_views_device): n host camera records of 22 floats and n seeds (null: the render's seed for every view).
+struct Views { uint32_t n; const float *cams; const uint32_t *seeds; };
+
+// The refusals of a batch that need no device, in the header's order.  `outputs`: the output pointers are not null.
+int check_views(const r1_render_params *params, uint32_t n_views, const float *cams, bool outputs)
+{
+    int rc = validate(params);
+    if (rc) return rc;
+    if (n_views == 0) return fail(R1_ERR_ARG, "a batch needs at least one view");
+    if (!cams || !outputs) return fail(R1_ERR_ARG, "null argument");
+    const int v = params->variant;
+    if (v != R1_VARIANT_MEGAKERNEL && v != R1_VARIANT_MEGAKERNEL_PACKED && v != R1_VARIANT_MEGAKERNEL_TENSOR && v != R1_VARIANT_MEGAKERNEL_TENSOR_STREAM &&
+        v != R1_VARIANT_MEGAKERNEL_BVH)
+        return fail(R1_ERR_ARG, "a batch of views renders with the megakernel, packed, tensor, tensor-stream or bvh variant, not %d", v);
+    if (params->threads > 0 || params->blocks_per_sm > 0) return fail(R1_ERR_ARG, "a batch of views runs with default tuning only (threads and blocks_per_sm <= 0)");
+    const Partition part = partition(params->width, params->height, params->row_tile, params->rank, params->world);
+    const uint64_t batch_pix = (uint64_t)n_views * part.npix_local;
+    // a batch pixel is a 32-bit pool entry, and 0xffffffff marks an empty one (kPoolInvalid)
+    if (batch_pix >= 0xffffffffull) return fail(R1_ERR_LIMIT, "too many pixels in the batch (%u views x %u local pixels)", n_views, part.npix_local);
+    if ((long double)batch_pix * params->spp * params->spp >= 18.0e18L)
+        return fail(R1_ERR_LIMIT, "too many samples (%llu x %d spp)", (unsigned long long)batch_pix, params->spp);
+    return R1_OK;
+}
+
+// r1_render_device, and with `views` r1_render_views_device: enqueues the memsets, the trace kernel and the resolve on the stream.
+int enqueue_render(r1_scene *scene, const r1_render_params *params, const Views *views, void *d_rgb, void *d_num_rays, void *cuda_stream, r1_result *result)
 {
     int rc = validate(params);
     if (rc) return rc;
@@ -780,12 +825,14 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
     a.scene = c.dev;
     a.width = prm.width; a.height = prm.height; a.spp = prm.spp; a.max_bounces = prm.max_bounces;
     a.rank = prm.rank; a.world = prm.world; a.row_tile = prm.row_tile;
-    a.npix_local = part.npix_local;
+    a.npix_local = views ? views->n * part.npix_local : part.npix_local;   // a batch: the views' pixels one after the other
     a.samples_per_unit = samples_per_unit(prm.spp);
     a.n_chunks = (prm.spp + a.samples_per_unit - 1) / a.samples_per_unit;
-    const uint64_t n_units = (uint64_t)a.npix_local * (uint64_t)a.n_chunks;
-    if (n_units >= (1ull << 32) - (1ull << 24)) return fail(R1_ERR_LIMIT, "too many work units (%llu)", (unsigned long long)n_units);
-    a.n_units = (uint32_t)n_units;
+    if (!views) {   // work units are the wavefront variant's; the kernels a batch runs take samples
+        const uint64_t n_units = (uint64_t)a.npix_local * (uint64_t)a.n_chunks;
+        if (n_units >= (1ull << 32) - (1ull << 24)) return fail(R1_ERR_LIMIT, "too many work units (%llu)", (unsigned long long)n_units);
+        a.n_units = (uint32_t)n_units;
+    }
     a.seed = r1::Rng::seed_hash(prm.seed);
     a.inv_w = 1.0f / prm.width; a.inv_h = 1.0f / prm.height;  // rayweek1.cpp:746
     a.inv_spp = (float)(1.0f / prm.spp);                       // rayweek1.cpp:765
@@ -817,6 +864,18 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
         R1_CUDA(cudaMemsetAsync(x.accum, 0, (size_t)a.npix_local * 4 * sizeof(unsigned long long), stream));
         R1_CUDA(cudaMemsetAsync(x.unit_counter, 0, sizeof(unsigned int), stream));
         R1_CUDA(cudaMemsetAsync(x.sample_counter, 0, sizeof(unsigned long long), stream));
+        if (views) {   // the view table, on the stream: a batch enqueued before keeps its own
+            std::vector<r1::ViewRec> recs(views->n);
+            for (uint32_t v = 0; v < views->n; ++v) {
+                camera_from_constants(views->cams + 22 * (size_t)v, recs[v].cam);
+                recs[v].seed = r1::Rng::seed_hash(views->seeds ? views->seeds[v] : prm.seed);
+            }
+            rc = grow(x.views, x.views_cap, views->n);
+            if (rc) return rc;
+            R1_CUDA(cudaMemcpyAsync(x.views, recs.data(), recs.size() * sizeof(r1::ViewRec), cudaMemcpyHostToDevice, stream));
+            const r1::ViewArgs va = { x.views, part.npix_local, r1::div_magic(part.npix_local) };
+            R1_CUDA(cudaMemcpyToSymbolAsync(r1::c_views, &va, sizeof(va), 0, cudaMemcpyHostToDevice, stream));
+        }
         // scenes of up to 4096 spheres are staged in shared memory; R1_FORCE_UNSTAGED=1 exercises the global-memory path on small scenes
         const bool staged = c.dev.n_pad <= r1::kMaxStagedSpheres && !knobs.force_unstaged;
         R1_CUDA(cudaEventRecord(x.ev[1], stream));
@@ -826,28 +885,44 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
             rc = r1::wavefront_render(x.wf, a, x.sm_count, stream, &launches);
             if (rc) return fail(R1_ERR_CUDA, "wavefront: %s", cudaGetErrorString((cudaError_t)rc));
             x.last_launches += launches;
+        } else if (views) {   // one instance per production kernel, default tuning (check_views)
+            if (variant == R1_VARIANT_MEGAKERNEL_PACKED) rc = staged ? launch_megakernel<r1::kScanLanePacked, true, true>(x.sm_count, a, prm, stream)
+                                                                  : launch_megakernel<r1::kScanLanePacked, false, true>(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR) rc = launch_megakernel_tc<true>(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) rc = launch_megakernel_tcs<true>(x.sm_count, a, prm, stream);
+            else rc = launch_megakernel_bvh<true>(x.sm_count, a, c.bvh_nodes, c.bvh_leaves, prm, stream);
+            if (rc) return rc;
+            x.last_launches += 1;
         } else {
-            if (variant == R1_VARIANT_MEGAKERNEL_PACKED) rc = staged ? launch_megakernel<r1::kScanLanePacked, true>(x.sm_count, a, prm, stream)
-                                                                  : launch_megakernel<r1::kScanLanePacked, false>(x.sm_count, a, prm, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_COOP) rc = staged ? launch_megakernel<r1::kScanCoop, true>(x.sm_count, a, prm, stream)
-                                                                            : launch_megakernel<r1::kScanCoop, false>(x.sm_count, a, prm, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_DEFERRED) rc = staged ? launch_megakernel<r1::kScanLaneDeferred, true>(x.sm_count, a, prm, stream)
-                                                                                : launch_megakernel<r1::kScanLaneDeferred, false>(x.sm_count, a, prm, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR) rc = launch_megakernel_tc(x.sm_count, a, prm, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) rc = launch_megakernel_tcs(x.sm_count, a, prm, stream);
-            else if (variant == R1_VARIANT_MEGAKERNEL_BVH) rc = launch_megakernel_bvh(x.sm_count, a, c.bvh_nodes, c.bvh_leaves, prm, stream);
+            if (variant == R1_VARIANT_MEGAKERNEL_PACKED) rc = staged ? launch_megakernel<r1::kScanLanePacked, true, false>(x.sm_count, a, prm, stream)
+                                                                  : launch_megakernel<r1::kScanLanePacked, false, false>(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_COOP) rc = staged ? launch_megakernel<r1::kScanCoop, true, false>(x.sm_count, a, prm, stream)
+                                                                            : launch_megakernel<r1::kScanCoop, false, false>(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_DEFERRED) rc = staged ? launch_megakernel<r1::kScanLaneDeferred, true, false>(x.sm_count, a, prm, stream)
+                                                                                : launch_megakernel<r1::kScanLaneDeferred, false, false>(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR) rc = launch_megakernel_tc<false>(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_TENSOR_STREAM) rc = launch_megakernel_tcs<false>(x.sm_count, a, prm, stream);
+            else if (variant == R1_VARIANT_MEGAKERNEL_BVH) rc = launch_megakernel_bvh<false>(x.sm_count, a, c.bvh_nodes, c.bvh_leaves, prm, stream);
             else if (variant == R1_VARIANT_MEGAKERNEL_DUAL) rc = staged ? launch_megakernel_dual<true>(x.sm_count, a, prm, stream)
                                                                             : launch_megakernel_dual<false>(x.sm_count, a, prm, stream);
-            else rc = staged ? launch_megakernel<r1::kScanLaneScalar, true>(x.sm_count, a, prm, stream)
-                             : launch_megakernel<r1::kScanLaneScalar, false>(x.sm_count, a, prm, stream);
+            else rc = staged ? launch_megakernel<r1::kScanLaneScalar, true, false>(x.sm_count, a, prm, stream)
+                             : launch_megakernel<r1::kScanLaneScalar, false, false>(x.sm_count, a, prm, stream);
             if (rc) return rc;
             x.last_launches += 1;
         }
         R1_CUDA(cudaEventRecord(x.ev[2], stream));
-        const int rgrid = (int)std::min<uint64_t>(((uint64_t)a.npix_local + 255) / 256, (uint64_t)x.sm_count * 8);
-        r1::resolve<<<rgrid, 256, 0, stream>>>(a);
-        R1_CUDA(cudaGetLastError());
-        x.last_launches += 1;
+        // resolve's grid-stride index is 32-bit: it ends only while npix_local + stride stays below 2^32.  A single render has at most
+        // 2^31 pixels (validate); a batch up to 2^32 - 2, so it is resolved in pieces of at most 2^31 pixels.
+        for (uint32_t first = 0; first < a.npix_local; first += std::min<uint32_t>(a.npix_local - first, kResolvePixels)) {
+            r1::RenderArgs ra = a;
+            ra.accum = a.accum + (size_t)first * 4;
+            ra.rgb = a.rgb + (size_t)first * 3;
+            ra.npix_local = std::min<uint32_t>(a.npix_local - first, kResolvePixels);
+            const int rgrid = (int)std::min<uint64_t>(((uint64_t)ra.npix_local + 255) / 256, (uint64_t)x.sm_count * 8);
+            r1::resolve<<<rgrid, 256, 0, stream>>>(ra);
+            R1_CUDA(cudaGetLastError());
+            x.last_launches += 1;
+        }
     } else {
         R1_CUDA(cudaEventRecord(x.ev[1], stream));
         R1_CUDA(cudaEventRecord(x.ev[2], stream));
@@ -860,6 +935,26 @@ int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rg
         result->n_units = x.last_units;
     }
     return R1_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int r1_render_device(r1_scene *scene, const r1_render_params *params, void *d_rgb, void *d_num_rays, void *cuda_stream, r1_result *result)
+{
+    return enqueue_render(scene, params, nullptr, d_rgb, d_num_rays, cuda_stream, result);
+}
+
+int r1_render_views_device(r1_scene *scene, const r1_render_params *params, uint32_t n_views, const float *cams, const uint32_t *seeds, void *d_rgb,
+                           void *d_num_rays, void *cuda_stream, r1_result *result)
+{
+    int rc = check_views(params, n_views, cams, d_rgb && d_num_rays);
+    if (rc) return rc;
+    int ndev = 0;
+    R1_CUDA(cudaGetDeviceCount(&ndev));   // no device: R1_ERR_CUDA, whether or not the scene was committed
+    const Views views = { n_views, cams, seeds };
+    return enqueue_render(scene, params, &views, d_rgb, d_num_rays, cuda_stream, result);
 }
 
 int r1_render_wait(r1_scene *scene, int device, r1_result *result)
@@ -924,6 +1019,44 @@ int r1_render(r1_scene *scene, const r1_render_params *params, uint8_t *rgb_host
     rc = r1_render_wait(scene, params->device, &res);
     if (rc) return rc;
     res.num_rays = *x.host_rays;
+    res.elapsed_seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+    if (result) *result = res;
+    return R1_OK;
+}
+
+int r1_render_views(r1_scene *scene, const r1_render_params *params, uint32_t n_views, const float *cams, const uint32_t *seeds, uint8_t *rgb_host,
+                    uint64_t *sums_host, r1_result *result)
+{
+    const auto t0 = std::chrono::steady_clock::now();
+    int rc = check_views(params, n_views, cams, rgb_host != nullptr);
+    if (rc) return rc;
+    int ndev = 0;
+    R1_CUDA(cudaGetDeviceCount(&ndev));
+    DeviceCtx *cp = nullptr;
+    rc = get_ctx(scene, &cp, params->device);
+    if (rc) return rc;
+    Scratch *xp = nullptr;
+    rc = get_scratch(cp->device, &xp);
+    if (rc) return rc;
+    Scratch &x = *xp;
+    const size_t npix = (size_t)n_views * partition(params->width, params->height, params->row_tile, params->rank, params->world).npix_local;
+    rc = grow(x.rgb, x.rgb_cap, std::max<size_t>(npix * 3, 16));
+    if (rc) return rc;
+    r1_result res;
+    rc = r1_render_views_device(scene, params, n_views, cams, seeds, x.rgb, x.num_rays, nullptr, &res);
+    if (rc) return rc;
+    if (npix) R1_CUDA(cudaMemcpyAsync(rgb_host, x.rgb, npix * 3, cudaMemcpyDeviceToHost, nullptr));
+    R1_CUDA(cudaMemcpyAsync(x.host_rays, x.num_rays, sizeof(unsigned long long), cudaMemcpyDeviceToHost, nullptr));
+    R1_CUDA(cudaStreamSynchronize(nullptr));
+    rc = r1_render_wait(scene, params->device, &res);
+    if (rc) return rc;
+    res.num_rays = *x.host_rays;
+    if (sums_host && npix) {
+        std::vector<unsigned long long> accum(npix * 4);   // (r, g, b, unused) per batch pixel
+        R1_CUDA(cudaMemcpy(accum.data(), x.accum, accum.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+        for (size_t p = 0; p < npix; ++p)
+            for (int c = 0; c < 3; ++c) sums_host[3 * p + c] = accum[4 * p + c];
+    }
     res.elapsed_seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     if (result) *result = res;
     return R1_OK;

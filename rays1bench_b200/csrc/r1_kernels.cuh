@@ -43,6 +43,19 @@ struct RenderArgs {
 struct BvhArgs { const float4 *nodes, *leaves; };
 __constant__ BvhArgs c_bvh;
 
+// A batch of views (r1_render_views): the kernels' kViews instances render K images of one scene as one work space of
+// K x npix local pixels, batch pixel plp = v * npix + lp.  View v's camera and hashed seed come from table[v]; everything past the
+// primary ray -- pool entries, accumulators, resolve -- carries plp and never needs v.  Written on the launching stream before
+// every batch launch, for the reason c_bvh is.
+struct ViewRec { Camera cam; uint64_t seed; };   // the 22 constants; Rng::seed_hash(seed of the view)
+static_assert(sizeof(ViewRec) == 96, "view records are loaded as six float4");
+struct ViewArgs {
+    const ViewRec *table;
+    uint32_t npix;                    // local pixels of one view
+    uint64_t magic_npix;              // div_magic(npix)
+};
+__constant__ ViewArgs c_views;
+
 constexpr int kSmemSpheres = 16 + R1_RSQRT12_ENTRIES * 2;   // megakernel: byte offset of the staged spheres (mbarrier, rsqrtss table first)
 constexpr float kFixedScale = 16777216.0f;                 // 2^24: one sample saturates at 2^32 - 1 (radiance 256; scenes stay <= 1)
 constexpr float kFixedInvScale = 5.9604644775390625e-8f;   // 2^-24
@@ -131,15 +144,21 @@ __device__ __forceinline__ void count_rays(const RenderArgs &a, uint32_t nrays, 
     if (lane == 0 && total) atomicAdd(a.num_rays, total);
 }
 
-// start sample s of a pixel: jitter (rayweek1.cpp:759), lens disk + camera ray (:760, :381-386)
-__device__ __forceinline__ void primary_ray(const RenderArgs &a, uint32_t pixel, float fx, float fy, int s, const uint16_t *__restrict__ tab, Rng &rng, f3 &o,
-                                            f3 &d)
+// start sample s of a pixel: jitter (rayweek1.cpp:759), lens disk + camera ray (:760, :381-386); seed = Rng::seed_hash(global seed)
+__device__ __forceinline__ void primary_ray(const RenderArgs &a, const Camera &cam, uint64_t seed, uint32_t pixel, float fx, float fy, int s,
+                                            const uint16_t *__restrict__ tab, Rng &rng, f3 &o, f3 &d)
 {
-    rng.seed(pixel, (uint32_t)s, a.seed);
+    rng.seed(pixel, (uint32_t)s, seed);
     const float u = fmul(fadd(rng.rand01(0), fx), a.inv_w), v = fmul(fadd(rng.rand01(1), fy), a.inv_h);
     float px, py;
     random_in_unit_disk(rng, 2, px, py);
-    camera_ray(a.scene.cam, u, v, px, py, tab, o, d);
+    camera_ray(cam, u, v, px, py, tab, o, d);
+}
+// the render's own camera and seed
+__device__ __forceinline__ void primary_ray(const RenderArgs &a, uint32_t pixel, float fx, float fy, int s, const uint16_t *__restrict__ tab, Rng &rng, f3 &o,
+                                            f3 &d)
+{
+    primary_ray(a, a.scene.cam, a.seed, pixel, fx, fy, s, tab, rng, o, d);
 }
 
 // color() body after hit() (rayweek1.cpp:515-536).  Returns true when the path ends (contrib = its radiance);
@@ -212,7 +231,9 @@ struct PoolState {
 
 // The whole warp produces the next 32 consecutive samples into its pool (every lane has popped what it takes from it): takes a
 // new range when its own is used up, decodes sample g = lp * spp + s under the interleaved row-tile partition and generates the
-// primary ray.  lanes_x = lanes of the grid x sched_div.
+// primary ray.  lanes_x = lanes of the grid x sched_div.  kViews: plp is a batch pixel (c_views), decoded per lane -- the 32
+// samples of a warp can straddle a view boundary.
+template <bool kViews>
 __device__ __forceinline__ void pool_produce(const RenderArgs &a, WarpPool &pool, PoolState &ps, const uint16_t *tab, unsigned lane, uint32_t lanes_x)
 {
     __syncwarp();
@@ -241,13 +262,26 @@ __device__ __forceinline__ void pool_produce(const RenderArgs &a, WarpPool &pool
         if (g < a.n_samples) {
             const uint32_t plp = a.magic_spp ? (uint32_t)__umul64hi(g, a.magic_spp) : (uint32_t)g;
             const uint32_t smp = (uint32_t)(g - (unsigned long long)plp * (uint32_t)a.spp);
-            const uint32_t lr = fast_div(plp, a.magic_width);
-            const int x = (int)(plp - lr * (uint32_t)a.width);
+            uint32_t lp = plp, v = 0;
+            if constexpr (kViews) {
+                v = fast_div(plp, c_views.magic_npix);
+                lp = plp - v * c_views.npix;
+            }
+            const uint32_t lr = fast_div(lp, a.magic_width);
+            const int x = (int)(lp - lr * (uint32_t)a.width);
             const uint32_t tile = fast_div(lr, a.magic_row_tile);
             const int y = (int)((tile * (uint32_t)a.world + (uint32_t)a.rank) * (uint32_t)a.row_tile + (lr - tile * (uint32_t)a.row_tile));
             Rng r;
             f3 po, pd;
-            primary_ray(a, (uint32_t)y * (uint32_t)a.width + (uint32_t)x, (float)x, (float)y, (int)smp, tab, r, po, pd);
+            if constexpr (kViews) {
+                union { float4 q[6]; ViewRec rec; } vr;
+                const float4 *src = reinterpret_cast<const float4 *>(c_views.table + v);
+#pragma unroll
+                for (int k = 0; k < 6; ++k) vr.q[k] = __ldg(src + k);
+                primary_ray(a, vr.rec.cam, vr.rec.seed, (uint32_t)y * (uint32_t)a.width + (uint32_t)x, (float)x, (float)y, (int)smp, tab, r, po, pd);
+            } else {
+                primary_ray(a, (uint32_t)y * (uint32_t)a.width + (uint32_t)x, (float)x, (float)y, (int)smp, tab, r, po, pd);
+            }
             pa = make_float4(po.x, po.y, po.z, __uint_as_float(plp));
             pb = make_float4(pd.x, pd.y, pd.z, __uint_as_float(r.k0));
             pk1 = r.k1;
@@ -260,6 +294,7 @@ __device__ __forceinline__ void pool_produce(const RenderArgs &a, WarpPool &pool
 
 // Lanes without a path (`want`, ballot `need`) take a ray from the warp's pool; the warp produces more when the pool runs short.
 // A lane that finds the work exhausted keeps its o / d.
+template <bool kViews>
 __device__ __forceinline__ void pool_take(const RenderArgs &a, WarpPool &pool, PoolState &ps, const uint16_t *tab, unsigned lane, unsigned lt_mask,
                                           uint32_t lanes_x, unsigned need, bool want, bool &active, bool &exhausted, f3 &o, f3 &d, uint32_t &lp, Rng &rng,
                                           f3 &thr, int &depth)
@@ -272,7 +307,7 @@ __device__ __forceinline__ void pool_take(const RenderArgs &a, WarpPool &pool, P
     uint32_t ek1 = 0;
     if (entry >= 0) { ea = pool.a[entry]; eb = pool.b[entry]; ek1 = pool.k1[entry]; }   // pop before the pool is overwritten
     if (n_need > ps.ready && !ps.dry) {                          // warp-uniform: not enough rays
-        pool_produce(a, pool, ps, tab, lane, lanes_x);
+        pool_produce<kViews>(a, pool, ps, tab, lane, lanes_x);
         const uint32_t rank2 = rank - n_first;                   // rank among the lanes the old pool could not serve
         if (want && entry < 0 && rank2 < ps.ready) {
             entry = (int)(ps.ready - 1u - rank2);
@@ -293,7 +328,7 @@ __device__ __forceinline__ void pool_take(const RenderArgs &a, WarpPool &pool, P
     }
 }
 
-template <int kScan, bool kStaged, int kThreads, int kBlocksPerSM>
+template <int kScan, bool kStaged, int kThreads, int kBlocksPerSM, bool kViews>
 __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool(const __grid_constant__ RenderArgs a)
 {
     // shared memory: [mbarrier 16 B | rsqrtss table 4 KB | staged spheres n_pad * 32 B | per-warp scan scratch (coop / deferred) | per-warp pools]
@@ -345,7 +380,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool(const 
                 float4 ea = make_float4(0, 0, 0, 0), eb = make_float4(0, 0, 0, 0);
                 uint32_t ek1 = 0;
                 if (entry >= 0) { ea = pool.a[entry]; eb = pool.b[entry]; ek1 = pool.k1[entry]; }   // pop before the pool is overwritten
-                pool_produce(a, pool, ps, tab, lane, lanes_x);
+                pool_produce<kViews>(a, pool, ps, tab, lane, lanes_x);
                 const uint32_t rank2 = rank - n_first;           // rank among the lanes the old pool could not serve
                 if (want && entry < 0 && rank2 < ps.ready) {
                     entry = (int)(ps.ready - 1u - rank2);
@@ -473,7 +508,7 @@ __global__ void __launch_bounds__(kThreads, kBlocksPerSM) megakernel_pool2(const
                 ps.ready -= take;
                 served += avail;
                 if (served >= n_need || ps.dry) break;
-                pool_produce(a, pool, ps, tab, lane, lanes_x);   // everything in the pool has been popped: ready == 0
+                pool_produce<false>(a, pool, ps, tab, lane, lanes_x);   // everything in the pool has been popped: ready == 0
                 if (ps.dry) break;
             }
 #pragma unroll
@@ -538,7 +573,7 @@ constexpr size_t tc3_smem_bytes(int groups, int n32)
            (size_t)groups * 4 * sizeof(WarpPool) + 256;          // + alignment slack
 }
 
-template <int kGroups>
+template <int kGroups, bool kViews>
 __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tc3(const __grid_constant__ RenderArgs a)
 {
     constexpr int kChunk = 128, kPool = 4;
@@ -601,7 +636,7 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tc3(const __grid_
     for (;;) {
         const bool want = !active && !exhausted;
         const unsigned need = __ballot_sync(kFull, want);
-        if (need) pool_take(a, pool, ps, tab, lane, lt_mask, lanes_x, need, want, active, exhausted, o, d, lp, rng, thr, depth);
+        if (need) pool_take<kViews>(a, pool, ps, tab, lane, lt_mask, lanes_x, need, want, active, exhausted, o, d, lp, rng, thr, depth);
         const bool warp_done = __all_sync(kFull, exhausted);
 
         tc::write_ray_row(a_tile, r, o, d, active);
@@ -820,7 +855,7 @@ constexpr size_t tcs_smem_bytes(int groups, int stages)
            (size_t)groups * 128 * tc::kRowBytes + (size_t)groups * 4 * sizeof(WarpPool);
 }
 
-template <int kGroups, int kStages>
+template <int kGroups, int kStages, bool kViews>
 __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tcs(const __grid_constant__ RenderArgs a)
 {
     constexpr int kChunk = kTcsChunk, kPieces = kChunk / 32;
@@ -884,7 +919,7 @@ __global__ void __launch_bounds__(kGroups * 128, 1) megakernel_tcs(const __grid_
     for (;;) {
         const bool want = !active && !exhausted;
         const unsigned need = __ballot_sync(kFull, want);
-        if (need) pool_take(a, pool, ps, tab, lane, lt_mask, lanes_x, need, want, active, exhausted, o, d, lp, rng, thr, depth);
+        if (need) pool_take<kViews>(a, pool, ps, tab, lane, lt_mask, lanes_x, need, want, active, exhausted, o, d, lp, rng, thr, depth);
         const bool warp_done = __all_sync(kFull, exhausted);
 
         tc::write_ray_row(a_tile, r, o, d, active);
